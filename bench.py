@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the batched simplex hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload config2|...]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (the batched simplex kernel) over one batch of synthetic LPs.
 N=1 workload = BASELINE.json configs[1]: 65,536 synthetic feasible dense LPs 32x64 (tableau 33x65 fp64),
@@ -22,6 +23,9 @@ collective: LPs are independent); the time is the max over ranks, the value the 
             available) on the box's host cores, bounded sample of the same workload
 
 --impl reference times that CPU restatement alone (all host threads) and prints the same JSON shape.
+
+--dump-outputs DIR writes what the last timed step returned for rank 0's LPs (status, value, pivots, RHS, basis) as
+DIR/<name>.npy, so that two builds can be compared output for output on the same generated inputs.
 """
 import argparse
 import json
@@ -285,6 +289,9 @@ def run_native(args):
     barrier()
     h2d_s = eng.measure_h2d_seconds(h_in, reps=3, nstreams=2)
     clocks = sampler.stop() if rank == 0 else None  # sampled over the device-timed and the end-to-end regions
+    if args.dump_outputs and rank == 0:  # the timed step's outputs: the end-to-end calls use their own buffers
+        dump_outputs(args.dump_outputs, {"status": d_status, "value": d_value, "pivots": d_piv, "rhs": d_rhs,
+                                         "pos": d_pos, "var": d_var})
     h2d = n * cells * 8
     d2h = n * (4 + 8 + 16 + H * 8 + 2 * (W + H) * 4)
 
@@ -400,6 +407,26 @@ def run_native(args):
     return 0
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Per-LP device outputs -> out_dir/<name>.npy: int32 fields as float32 (exact: they are far below 2**24), the
+    rest as float64.  When the batch's outputs exceed DUMP_BYTES, every file holds the same fixed seeded sample of LPs
+    (identical from run to run); lp_index.npy lists the LPs written, in order."""
+    import numpy as np
+    host = {k: v.cpu().numpy() for k, v in arrays.items()}
+    host = {k: a.astype(np.float32 if a.dtype == np.int32 else np.float64) for k, a in host.items()}
+    n = len(host["status"])
+    per_lp = 8 + sum(a[:1].nbytes for a in host.values())  # lp_index included
+    keep = min(n, (DUMP_BYTES - 4096) // per_lp)  # 4096: room for the .npy headers
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "lp_index.npy"), idx.astype(np.float64))
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a[idx]))
+
+
 def emit_line(line):
     """The JSON line goes to the REAL stdout; everything else a library prints there (NCCL's version banner) was
     sent to stderr by quiet_stdout()."""
@@ -426,7 +453,13 @@ def main():
     ap.add_argument("--threads", type=int, default=0, help="threads per LP (0 = auto)")
     ap.add_argument("--path", type=int, default=0, help="0 auto, 1 smem (K1), 2 gmem (K2), 6 tmem (K1t)")
     ap.add_argument("--no-secondary", action="store_true", help="skip the configs 3/4/5 block of the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32/float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
     quiet_stdout()
     if args.impl == "reference":
         return run_reference(args)
