@@ -283,6 +283,45 @@ int yalps_solve_sparse(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nn
                        double *result, int32_t *out_height, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                        int32_t *root_status, double *root_value, int64_t *root_pivots, int64_t *stats);
 
+/* ---- dual values: shadow prices and reduced costs ------------------------------------------------------------
+ * Each *_duals entry point takes the arguments of its sibling plus a trailing reduced_out (NULL: the sibling exactly).
+ * reduced_out holds one double per variable id and is packed like pos_out (width + height per LP):
+ *     reduced_out[v] = M[0, pos[v]]   if 1 <= pos[v] < width  (v non-basic: its column's row-0 cell, bits as they are)
+ *     reduced_out[v] = +0.0           otherwise                (basic variables, and ids 0 and width)
+ * where M, pos are the final tableau and positionOfVariable the call reports.  Ids 1..width-1 are the structural
+ * columns, id width + r is the slack of row r.  It is written for every status (it is row 0 re-indexed) and costs
+ * 8*(width+height) bytes of device-to-host copy per LP.  With the reference's conventions (entering column = positive
+ * row-0 cell, result = -sign * M[0,0]) these are the partial derivatives of result:
+ *     d result / d x_j   =  sign * reduced_out[j]           (structural variable j)
+ *     d result / d rhs_r = -sign * reduced_out[width + r]   (right-hand side of row r)
+ * e.g. max 3x s.t. x <= 4 ends with row 0 = [-12, -3]: sign = 1, the shadow price of the row is 3.
+ */
+/* yalps_solve_batch_basis + reduced_out (pos_in = var_in = NULL: yalps_solve_batch) */
+int yalps_solve_batch_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
+                            const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt, int32_t *status,
+                            double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                            double *matrices_out, double *reduced_out);
+/* yalps_solve_ragged_basis + reduced_out (packed by cumulative width + height, like pos_out) */
+int yalps_solve_ragged_duals(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
+                             const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                             const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                             int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                             double *matrices_out, double *reduced_out);
+int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
+                               const double *rhs, const yalps_options *opt, int32_t *status, double *value,
+                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                               double *reduced_out);
+/* d_reduced_out is device memory, like every other buffer of yalps_solve_batch_device */
+int yalps_solve_batch_device_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                                   double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
+                                   int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
+                                   double *d_matrices_out, void *stream, double *d_reduced_out);
+/* The root LP of yalps_solve_sparse (no branch and cut): status, value (as yalps_solve_batch), pivots[2], rhs_out[height],
+ * pos_out/var_out[width+height], reduced_out[width+height]. */
+int yalps_solve_sparse_duals(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nnz, const int32_t *cell,
+                             const double *val, const yalps_options *opt, int32_t *status, double *value, int64_t *pivots,
+                             double *rhs_out, int32_t *pos_out, int32_t *var_out, double *reduced_out);
+
 /* ---- one process, several GPUs (SURVEY 8b/8e) ------------------------------------------------------------
  * The reference is single-process and synchronous (src/YALPS.ts:73-92); a Node addon cannot use torchrun.  A
  * yalps_multi owns one ctx (plus worker ctxs for concurrent branch-and-cut searches) per entry of `devices` and one
@@ -308,6 +347,19 @@ int yalps_multi_solve_ragged(yalps_multi *m, int64_t n, const int32_t *heights, 
 int yalps_multi_solve_replicas(yalps_multi *m, int64_t n, int32_t height, int32_t width, const double *base,
                                const double *rhs, const yalps_options *opt, int32_t *status, double *value,
                                int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out);
+/* the three above + reduced_out (see "dual values"), sharded like pos_out */
+int yalps_multi_solve_batch_duals(yalps_multi *m, int64_t n, int32_t height, int32_t width, const double *matrices,
+                                  const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt,
+                                  int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
+                                  int32_t *var_out, double *matrices_out, double *reduced_out);
+int yalps_multi_solve_ragged_duals(yalps_multi *m, int64_t n, const int32_t *heights, const int32_t *widths,
+                                   const int64_t *mat_offsets, const double *matrices, const yalps_options *opt,
+                                   int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
+                                   int32_t *var_out, double *matrices_out, double *reduced_out);
+int yalps_multi_solve_replicas_duals(yalps_multi *m, int64_t n, int32_t height, int32_t width, const double *base,
+                                     const double *rhs, const yalps_options *opt, int32_t *status, double *value,
+                                     int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                                     double *reduced_out);
 /*
  * incumbent_allreduce (SURVEY 8b, north_star): min-allreduce of one fp64 per rank -- the incumbent objective of a
  * branch-and-bound search, lower is better internally (src/branchAndCut.ts:124,130).  local[ndev] in, agreed[ndev]

@@ -141,6 +141,10 @@ struct FollowArgs {
   int *fork_ids;          // [n] their indices, in arrival order
   int *fork_step;         // [n] (indexed by replica) the step at which it left
   long long *fork_resume; // [n][3] (indexed by replica) phase and pivot counters at that step
+  // optional reduced costs [n][W + H] (BatchArgs::red_out): a replica that finishes on the path has the leader's final
+  // row 0 in columns 1..W-1 (column 0 never feeds the others) and its basis, so it copies the leader's vector
+  double *red_out;
+  const double *leader_red;
 };
 
 constexpr int kFollowWarps = 8;
@@ -279,6 +283,7 @@ __global__ void __launch_bounds__(kFollowWarps * 32) k_replica_follow(const Foll
         const int v = a.leader_var[p];
         if (a.var_out) a.var_out[(size_t)i * (W + H) + p] = v;
         if (a.pos_out) a.pos_out[(size_t)i * (W + H) + v] = p;
+        if (a.red_out) a.red_out[(size_t)i * (W + H) + p] = a.leader_red[p];
       }
     }
     __syncwarp();
@@ -309,8 +314,8 @@ __global__ void k_replica_materialise(int first, int m, int H, int W, const int 
 // Results of the forked replicas [first, first + m) (compact, as solved) back to their replica slots.
 __global__ void k_replica_scatter(int first, int m, int H, int W, const int *fork_ids, const int *c_status,
                                   const double *c_value, const long long *c_pivots, const double *c_rhs, const int *c_pos,
-                                  const int *c_var, int *status, double *value, long long *pivots, double *rhs_out,
-                                  int *pos_out, int *var_out) {
+                                  const int *c_var, const double *c_red, int *status, double *value, long long *pivots,
+                                  double *rhs_out, int *pos_out, int *var_out, double *red_out) {
   for (int f = blockIdx.x; f < m; f += gridDim.x) {
     const size_t i = (size_t)fork_ids[first + f];
     if (threadIdx.x == 0) {
@@ -325,6 +330,7 @@ __global__ void k_replica_scatter(int first, int m, int H, int W, const int *for
     for (int p = threadIdx.x; p < W + H; p += blockDim.x) {
       if (pos_out) pos_out[i * (W + H) + p] = c_pos[(size_t)f * (W + H) + p];
       if (var_out) var_out[i * (W + H) + p] = c_var[(size_t)f * (W + H) + p];
+      if (red_out) red_out[i * (W + H) + p] = c_red[(size_t)f * (W + H) + p];
     }
   }
 }

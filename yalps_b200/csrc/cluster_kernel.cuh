@@ -770,6 +770,8 @@ __global__ void __launch_bounds__(NWC *NWR * 32, 1) k_simplex_cluster(const Batc
         for (int k = tid; k < W + H; k += NT) a.pos_out[poff + var[k]] = k;
       if (a.var_out)
         for (int k = tid; k < W + H; k += NT) a.var_out[poff + k] = var[k];
+      if (a.red_out)  // the private objective row: column k >= 1 is obj[k - 1]
+        for (int k = tid; k < W + H; k += NT) a.red_out[poff + var[k]] = (k >= 1 && k < W) ? obj[k - 1] : 0.0;
       if (a.mat_out)
         for (int c = tid; c < W; c += NT) a.mat_out[moff + c] = (c == 0) ? obj[bslot] : obj[c - 1];
     }

@@ -58,6 +58,7 @@ struct GridArgs {
   int *flags;                  // [2] cycle / history-overflow verdict of CTA 0, by iteration parity
   unsigned long long *barrier; // grid barrier arrival counter, zeroed before the launch
   unsigned long long *rows_out; // optional: rows rewritten by the updates are ADDED here (roofline diagnostics)
+  double *red_out;  // optional reduced costs [W+H] (BatchArgs::red_out), from the CTAs' identical objective-row copies
 };
 
 constexpr int kGridThreads = 1024;
@@ -389,6 +390,8 @@ __global__ void __launch_bounds__(kGridThreads, 1) k_simplex_grid(const GridArgs
     for (int r = blockIdx.x * NT + tid; r < H; r += gridDim.x * NT) a.rhs_out[r] = M[(size_t)r * W];
   if (a.pos_out)
     for (int k = blockIdx.x * NT + tid; k < W + H; k += gridDim.x * NT) a.pos_out[a.var[k]] = k;
+  if (a.red_out)
+    for (int k = blockIdx.x * NT + tid; k < W + H; k += gridDim.x * NT) a.red_out[a.var[k]] = (k >= 1 && k < W) ? row0[k] : 0.0;
 }
 
 }  // namespace yalps

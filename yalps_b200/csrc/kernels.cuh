@@ -59,6 +59,9 @@ struct BatchArgs {
   double *cl_scratch;  // cluster kernel: per cluster 2 * C * ldA doubles (published candidate pivot rows)
   int tma_mode;        // cluster kernel: how the winner's row is staged (0 ld.global.cg, 1 cp.async.bulk, 2 multicast)
   uint4 *gx_slots;     // grid-resident kernel (KG): [2][gridDim.x][gridDim.x] selection records (inbox per CTA); `counter` is its grid barrier
+  // optional reduced costs, packed like pos_out: red_out[v] = M[0, pos[v]] for a non-basic structural or slack
+  // variable (1 <= pos[v] < W), +0.0 for the basic ones and for ids 0 and W (row 0 re-indexed, written for every status)
+  double *red_out;
 };
 
 // Shared-memory carve-up, identical on host and device.
@@ -333,6 +336,8 @@ __global__ void __launch_bounds__(NWC *NWR * 32, min_ctas_per_sm(NWC, NWR)) k_si
       for (int k = tid; k < W + H; k += NT) a.pos_out[poff + t.var[k]] = k;
     if ((kResident || kSplit) && a.var_out)
       for (int k = tid; k < W + H; k += NT) a.var_out[poff + k] = t.var[k];
+    if (a.red_out)  // row 0, column k >= 1, is t.A[k - 1]
+      for (int k = tid; k < W + H; k += NT) a.red_out[poff + t.var[k]] = (k >= 1 && k < W) ? t.A[k - 1] : 0.0;
     if (a.mat_out) {
       double *dst = a.mat_out + moff;
       if (kResident || dst != a.work + moff) {

@@ -639,6 +639,11 @@ __global__ void __launch_bounds__(kTmemWarps * 32, TmemShape<HR>::kCtasPerSm) k_
       for (int k = lane; k < W + H; k += 32) a.pos_out[poff + var[k]] = k;
     if (a.var_out)
       for (int k = lane; k < W + H; k += 32) a.var_out[poff + k] = var[k];
+    if (a.red_out) {  // row 0 is in registers: lane l holds columns 2l+1 (o0) and 2l+2 (o1)
+      if (v0) a.red_out[poff + var[1 + j0]] = o0;
+      if (v1) a.red_out[poff + var[2 + j0]] = o1;
+      for (int k = lane; k < H + 1; k += 32) a.red_out[poff + var[k == 0 ? 0 : W - 1 + k]] = 0.0;
+    }
     tm_wait_st();
     if (a.mat_out) {
       double *dst = a.mat_out + moff;

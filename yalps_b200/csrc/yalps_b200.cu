@@ -790,7 +790,7 @@ int yalps_host_free(yalps_ctx *ctx, void *ptr) {
 static int launch_grid(yalps_ctx *ctx, int H, int W, double *d_M, const yalps_options *opt, int *d_status,
                        double *d_value, long long *d_pivots, double *d_rhs, int *d_pos, int *d_var,
                        cudaStream_t stream, const int *d_init_var = nullptr, int init_n = 0, int max_ctas = 0,
-                       const std::string &slot = "", unsigned long long *d_rows = nullptr) {
+                       const std::string &slot = "", unsigned long long *d_rows = nullptr, double *d_red = nullptr) {
   const GridSmem L(H, W);
   if (L.total > (size_t)ctx->smem_optin)
     return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d: pivot row/column staging exceeds shared memory", H, W);
@@ -818,6 +818,7 @@ static int launch_grid(yalps_ctx *ctx, int H, int W, double *d_M, const yalps_op
   a.pivots = d_pivots;
   a.rhs_out = d_rhs;
   a.pos_out = d_pos;
+  a.red_out = d_red;
   a.precision = opt->precision;
   a.max_pivots = opt->max_pivots;
   a.check_cycles = opt->check_cycles ? 1 : 0;
@@ -851,7 +852,8 @@ static int launch_grid(yalps_ctx *ctx, int H, int W, double *d_M, const yalps_op
 static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
                                    double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
                                    int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
-                                   double *d_matrices_out, void *stream, const std::string &slot, int64_t rows_base = 0) {
+                                   double *d_matrices_out, void *stream, const std::string &slot, int64_t rows_base = 0,
+                                   double *d_red_out = nullptr) {
   if (!ctx) return YALPS_ERR_ARGUMENT;
   if (n < 0 || height < 1 || width < 1 || !opt || (n > 0 && !d_matrices))
     return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", (long long)n, height, width);
@@ -895,6 +897,7 @@ static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, in
   a.rhs_out = d_rhs_out;
   a.pos_out = d_pos_out;
   a.var_out = d_var_out;
+  a.red_out = d_red_out;
   fill_options(a, opt);
   a.rows_out = ctx->d_rows ? ctx->d_rows + (ctx->rows_per_lp ? rows_base : 0) : nullptr;
   a.rows_per_lp = ctx->rows_per_lp;
@@ -914,7 +917,8 @@ static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, in
                                d_rhs_out ? d_rhs_out + i * height : nullptr,
                                d_pos_out ? d_pos_out + i * (width + height) : nullptr,
                                d_var_out ? d_var_out + i * (width + height) : nullptr, st, nullptr, 0, 0, slot,
-                               ctx->d_rows ? ctx->d_rows + (ctx->rows_per_lp ? rows_base + i : 0) : nullptr))
+                               ctx->d_rows ? ctx->d_rows + (ctx->rows_per_lp ? rows_base + i : 0) : nullptr,
+                               d_red_out ? d_red_out + i * (width + height) : nullptr))
         return rc;
     }
     if (d_matrices_out && d_matrices_out != d_work)
@@ -941,12 +945,20 @@ int yalps_solve_batch_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t 
                                  d_pos_out, d_var_out, d_matrices_out, stream, "dev");
 }
 
+int yalps_solve_batch_device_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                                   double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
+                                   int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
+                                   double *d_matrices_out, void *stream, double *d_reduced_out) {
+  return solve_batch_device_impl(ctx, n, height, width, d_matrices, d_work, opt, d_status, d_value, d_pivots, d_rhs_out,
+                                 d_pos_out, d_var_out, d_matrices_out, stream, "dev", 0, d_reduced_out);
+}
+
 // Shared host-side pipeline for uniform and ragged batches.
 static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const int32_t *heights,
                       const int32_t *widths, const int64_t *mat_offsets, const double *matrices,
                       const yalps_options *opt, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
                       int32_t *pos_out, int32_t *var_out, double *matrices_out, const int32_t *pos_in = nullptr,
-                      const int32_t *var_in = nullptr) {
+                      const int32_t *var_in = nullptr, double *reduced_out = nullptr) {
   if (!ctx) return YALPS_ERR_ARGUMENT;
   if (n < 0 || !opt || (n > 0 && !matrices)) return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments");
   if ((pos_in == nullptr) != (var_in == nullptr))
@@ -1008,7 +1020,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
   // let the kernel read the tableaus and write the results zero-copy: launch + synchronise, no memcpy calls.
   {
     const size_t in_b = (size_t)cells_upto(n) * 8, rows_b = (size_t)rows_upto(n) * 8, pv_b = (size_t)pv_upto(n) * 4;
-    const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (matrices_out ? in_b : 0);
+    const size_t red_b = reduced_out ? 2 * pv_b : 0;  // doubles, packed like pos_out
+    const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (matrices_out ? in_b : 0) + (red_b ? red_b + 16 : 0);
     const size_t desc_b = (ragged ? (size_t)n * 32 + 64 : 0) + (var_in ? pv_b + 16 : 0);
     LaunchPlan plan;
     // density of (a sample of) the first tableau: the latency-mode policy distinguishes dense from very sparse LPs
@@ -1039,6 +1052,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       const size_t o_pos = o; o += up16(pv_b);
       const size_t o_var = o; o += up16(pv_b);
       const size_t o_mat = o; o += matrices_out ? up16(in_b) : 0;
+      const size_t o_red = o; o += up16(red_b);
       void *hb, *db;
       int rc;
       if ((rc = pin_ensure(ctx, "small_io", o + 16, &hb))) return rc;
@@ -1073,6 +1087,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       a.pos_out = (int *)(d + o_pos);
       a.var_out = (int *)(d + o_var);
       a.var_in = var_in ? (const int *)(d + o_vin) : nullptr;
+      a.red_out = reduced_out ? (double *)(d + o_red) : nullptr;
       if (ragged) {
         a.heights = (const int *)(d + o_h);
         a.widths = (const int *)(d + o_w);
@@ -1090,6 +1105,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       if (rhs_out) std::memcpy(rhs_out, h + o_rhs, rows_b);
       if (pos_out) std::memcpy(pos_out, h + o_pos, pv_b);
       if (var_out) std::memcpy(var_out, h + o_var, pv_b);
+      if (reduced_out) std::memcpy(reduced_out, h + o_red, red_b);
       if (matrices_out) {
         if (ragged)
           for (int64_t i = 0; i < n; i++)
@@ -1151,6 +1167,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     if ((rc = dev_ensure(ctx, "rhs" + s, crows * 8, &d_rhs))) return rc;
     if ((rc = dev_ensure(ctx, "pos" + s, cpv * 4, &d_pos))) return rc;
     if ((rc = dev_ensure(ctx, "var" + s, cpv * 4, &d_var))) return rc;
+    void *d_red = nullptr;
+    if (reduced_out && (rc = dev_ensure(ctx, "red" + s, cpv * 8, &d_red))) return rc;
     void *d_vin = nullptr;
     if (var_in) {
       if ((rc = dev_ensure(ctx, "varin" + s, cpv * 4, &d_vin))) return rc;
@@ -1219,6 +1237,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     a.pos_out = (int *)d_pos;
     a.var_out = (int *)d_var;
     a.var_in = (const int *)d_vin;
+    a.red_out = (double *)d_red;
     if (ragged) {
       void *d_h, *d_w, *d_mo, *d_ro, *d_po;
       std::vector<long long> lm(cn), lr(cn), lpv(cn);
@@ -1260,7 +1279,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
                                 (long long *)d_piv + 2 * i, (double *)d_rhs + (size_t)i * height,
                                 (int *)d_pos + (size_t)i * (width + height), (int *)d_var + (size_t)i * (width + height),
                                 st, d_vin ? (const int *)d_vin + (size_t)i * (width + height) : nullptr,
-                                d_vin ? width + height : 0)))
+                                d_vin ? width + height : 0, 0, "", nullptr,
+                                d_red ? (double *)d_red + (size_t)i * (width + height) : nullptr)))
             return rc;
         }
         a.mat_out = want_mat ? (double *)d_in : nullptr;
@@ -1319,7 +1339,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
                             po = poff[begin + id] - poff[begin];
             if ((rc = launch_grid(ctx, hi, wi, (double *)d_in + mo, opt, (int *)d_status + id, (double *)d_value + id,
                                   (long long *)d_piv + 2 * id, (double *)d_rhs + ro, (int *)d_pos + po, (int *)d_var + po,
-                                  st, d_vin ? (const int *)d_vin + po : nullptr, d_vin ? wi + hi : 0)))
+                                  st, d_vin ? (const int *)d_vin + po : nullptr, d_vin ? wi + hi : 0, 0, "", nullptr,
+                                  d_red ? (double *)d_red + po : nullptr)))
               return rc;
             if (matrices_out)
               CU(ctx, cudaMemcpyAsync((double *)d_out + mo, (double *)d_in + mo, (size_t)hi * wi * 8,
@@ -1343,6 +1364,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     if (rhs_out) CU(ctx, cudaMemcpyAsync(rhs_out + rows_upto(begin), d_rhs, crows * 8, cudaMemcpyDeviceToHost, st));
     if (pos_out) CU(ctx, cudaMemcpyAsync(pos_out + pv_upto(begin), d_pos, cpv * 4, cudaMemcpyDeviceToHost, st));
     if (var_out) CU(ctx, cudaMemcpyAsync(var_out + pv_upto(begin), d_var, cpv * 4, cudaMemcpyDeviceToHost, st));
+    if (reduced_out)
+      CU(ctx, cudaMemcpyAsync(reduced_out + pv_upto(begin), d_red, cpv * 8, cudaMemcpyDeviceToHost, st));
     if (ctx->keep_final && n == 1 && !ragged) ctx->kept_final = a.mat_out;
     if (matrices_out) {
       if (ragged) {
@@ -1397,6 +1420,24 @@ int yalps_solve_ragged_basis(yalps_ctx *ctx, int64_t n, const int32_t *heights, 
                     pos_out, var_out, matrices_out, pos_in, var_in);
 }
 
+int yalps_solve_batch_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
+                            const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt, int32_t *status,
+                            double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                            double *matrices_out, double *reduced_out) {
+  return solve_host(ctx, n, height, width, nullptr, nullptr, nullptr, matrices, opt, status, value, pivots, rhs_out,
+                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out);
+}
+
+int yalps_solve_ragged_duals(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
+                             const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                             const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                             int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                             double *matrices_out, double *reduced_out) {
+  if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
+  return solve_host(ctx, n, 0, 0, heights, widths, mat_offsets, matrices, opt, status, value, pivots, rhs_out,
+                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out);
+}
+
 // ---- replica path sharing (aux_kernels.cuh: k_replica_follow) ------------------------------------------------------
 // The leader (the base tableau itself) is solved once by a row-split kernel that records its trace; see the comment
 // above FollowArgs for why following it gives every replica its own result, bit for bit.
@@ -1405,11 +1446,12 @@ struct ReplicaTrace {
   int K = 0, Hp = 0, cap = 0, leader_done = 0, leader_status = 0;
   int *steps = nullptr, *var = nullptr;
   double *q = nullptr, *col = nullptr, *snap = nullptr;
+  double *red = nullptr;  // the leader's final reduced costs (when the caller asked for them)
   double density = -1.0;
 };
 
 static int replica_leader_trace(yalps_ctx *ctx, int H, int W, const double *base_host, const double *d_base,
-                                const yalps_options *opt, cudaStream_t st, ReplicaTrace *tr) {
+                                const yalps_options *opt, cudaStream_t st, ReplicaTrace *tr, bool want_red) {
   tr->ok = false;
   if (!ctx->replica_sharing || opt->check_cycles || getenv("YALPS_NO_REPLICA_SHARING")) return 0;
   if (ctx->tune_path != YALPS_PATH_AUTO) return 0;  // a forced kernel path means "measure that kernel"
@@ -1445,6 +1487,11 @@ static int replica_leader_trace(yalps_ctx *ctx, int H, int W, const double *base
   if ((rc = dev_ensure(ctx, "rs_lwork", cells * 8, &d_lwork))) return rc;
   if ((rc = dev_ensure(ctx, "rs_lres", 64, &d_lres))) return rc;
   if ((rc = dev_ensure(ctx, "rs_lpv", 2 * pv * sizeof(int), &d_lpv))) return rc;
+  tr->red = nullptr;
+  if (want_red) {
+    if ((rc = dev_ensure(ctx, "rs_lred", pv * 8, &p))) return rc;
+    tr->red = (double *)p;
+  }
   BatchArgs a{};
   a.n = 1;
   a.mode = kModeBatch;
@@ -1457,6 +1504,7 @@ static int replica_leader_trace(yalps_ctx *ctx, int H, int W, const double *base
   a.pivots = (long long *)((char *)d_lres + 16);
   a.pos_out = (int *)d_lpv;
   a.var_out = (int *)d_lpv + pv;
+  a.red_out = tr->red;
   fill_options(a, opt);
   a.tr_steps = tr->steps;
   a.tr_q = tr->q;
@@ -1487,8 +1535,8 @@ static int replica_leader_trace(yalps_ctx *ctx, int H, int W, const double *base
 // (tableau = the leader's snapshot of the fork step + their own column 0) through the ordinary batch kernels.
 static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t cn, int H, int W, const double *d_rin,
                                 double *d_work, const yalps_options *opt, int *d_status, double *d_value, long long *d_piv,
-                                double *d_rhs, int *d_pos, int *d_var, cudaStream_t st, const std::string &s,
-                                int64_t *forks_out) {
+                                double *d_rhs, int *d_pos, int *d_var, double *d_red, cudaStream_t st,
+                                const std::string &s, int64_t *forks_out) {
   const size_t cells = (size_t)H * W, pv = (size_t)H + W;
   void *p, *hp;
   int rc;
@@ -1527,6 +1575,8 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   fa.fork_ids = d_fids;
   fa.fork_step = d_fstep;
   fa.fork_resume = d_fres;
+  fa.red_out = d_red;
+  fa.leader_red = tr.red;
   const int grid = (int)std::min<int64_t>((cn + kFollowWarps - 1) / kFollowWarps, (int64_t)ctx->prop.multiProcessorCount * 8);
   k_replica_follow<<<grid, kFollowWarps * 32, (size_t)kFollowWarps * tr.Hp * 8, st>>>(fa);
   CU(ctx, cudaGetLastError());
@@ -1553,6 +1603,11 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   int *c_pos = (int *)p;
   if ((rc = dev_ensure(ctx, "rs_cvar" + s, (size_t)nf * pv * 4, &p))) return rc;
   int *c_var = (int *)p;
+  double *c_red = nullptr;
+  if (d_red) {
+    if ((rc = dev_ensure(ctx, "rs_cred" + s, (size_t)nf * pv * 8, &p))) return rc;
+    c_red = (double *)p;
+  }
   {
     const dim3 g((unsigned)std::min<size_t>((cells + 255) / 256, 64), (unsigned)std::min(nf, 32768));
     k_replica_materialise<<<g, 256, 0, st>>>(0, nf, H, W, d_fids, d_fstep, d_fres, d_rhs, tr.snap, tr.var, d_work, c_vin, c_resume);
@@ -1582,19 +1637,22 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   a.pos_out = c_pos;
   a.var_out = c_var;
   a.var_in = c_vin;
+  a.red_out = c_red;
   a.resume = c_resume;
   fill_options(a, opt);
   if ((rc = launch_simplex(ctx, plan, a, "rs_fork" + s, st))) return rc;
   k_replica_scatter<<<(unsigned)std::min(nf, ctx->prop.multiProcessorCount * 8), 128, 0, st>>>(
-      0, nf, H, W, d_fids, c_status, c_value, c_piv, c_rhs, c_pos, c_var, d_status, d_value, d_piv, d_rhs, d_pos, d_var);
+      0, nf, H, W, d_fids, c_status, c_value, c_piv, c_rhs, c_pos, c_var, c_red, d_status, d_value, d_piv, d_rhs, d_pos,
+      d_var, d_red);
   CU(ctx, cudaGetLastError());
   ctx->launches++;
   return 0;
 }
 
-int yalps_solve_replicas(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
-                         const double *rhs, const yalps_options *opt, int32_t *status, double *value, int64_t *pivots,
-                         double *rhs_out, int32_t *pos_out, int32_t *var_out) {
+int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
+                               const double *rhs, const yalps_options *opt, int32_t *status, double *value,
+                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                               double *reduced_out) {
   if (!ctx) return YALPS_ERR_ARGUMENT;
   if (n < 0 || height < 1 || width < 1 || !opt || (n > 0 && (!base || !rhs)))
     return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", (long long)n, height, width);
@@ -1607,7 +1665,9 @@ int yalps_solve_replicas(yalps_ctx *ctx, int64_t n, int32_t height, int32_t widt
   if ((rc = dev_ensure(ctx, "rep_base", cells * 8, &d_base))) return rc;
   CU(ctx, cudaMemcpy(d_base, base, cells * 8, cudaMemcpyHostToDevice));
   ReplicaTrace trace;
-  if ((rc = replica_leader_trace(ctx, height, width, base, (const double *)d_base, opt, ctx->streams[0], &trace))) return rc;
+  if ((rc = replica_leader_trace(ctx, height, width, base, (const double *)d_base, opt, ctx->streams[0], &trace,
+                                 reduced_out != nullptr)))
+    return rc;
   ctx->replica_forks = trace.ok ? 0 : -1;
   // two pipeline slots of at most ~1.5 GiB of working copies each: the H2D of chunk k+1's right-hand sides and the
   // D2H of chunk k-1's results overlap the solve of chunk k
@@ -1629,11 +1689,13 @@ int yalps_solve_replicas(yalps_ctx *ctx, int64_t n, int32_t height, int32_t widt
     if ((rc = dev_ensure(ctx, "rhs" + s, (size_t)cn * height * 8, &d_rhs))) return rc;
     if ((rc = dev_ensure(ctx, "pos" + s, (size_t)cn * pv * 4, &d_pos))) return rc;
     if ((rc = dev_ensure(ctx, "var" + s, (size_t)cn * pv * 4, &d_var))) return rc;
+    void *d_red = nullptr;
+    if (reduced_out && (rc = dev_ensure(ctx, "red" + s, (size_t)cn * pv * 8, &d_red))) return rc;
     CU(ctx, cudaMemcpyAsync(d_rin, rhs + (size_t)begin * height, (size_t)cn * height * 8, cudaMemcpyHostToDevice, st));
     if (trace.ok) {
       if ((rc = replica_chunk_shared(ctx, trace, cn, height, width, (const double *)d_rin, (double *)d_work, opt, (int *)d_status,
-                                     (double *)d_value, (long long *)d_piv, (double *)d_rhs, (int *)d_pos, (int *)d_var, st, s,
-                                     &ctx->replica_forks)))
+                                     (double *)d_value, (long long *)d_piv, (double *)d_rhs, (int *)d_pos, (int *)d_var,
+                                     (double *)d_red, st, s, &ctx->replica_forks)))
         return rc;
     } else {
       const size_t total = (size_t)cn * cells;
@@ -1643,7 +1705,7 @@ int yalps_solve_replicas(yalps_ctx *ctx, int64_t n, int32_t height, int32_t widt
       ctx->launches++;
       if ((rc = solve_batch_device_impl(ctx, cn, height, width, (const double *)d_work, (double *)d_work, opt,
                                         (int32_t *)d_status, (double *)d_value, (int64_t *)d_piv, (double *)d_rhs,
-                                        (int32_t *)d_pos, (int32_t *)d_var, nullptr, st, s, begin)))
+                                        (int32_t *)d_pos, (int32_t *)d_var, nullptr, st, s, begin, (double *)d_red)))
         return rc;
     }
     if (status) CU(ctx, cudaMemcpyAsync(status + begin, d_status, (size_t)cn * 4, cudaMemcpyDeviceToHost, st));
@@ -1652,12 +1714,21 @@ int yalps_solve_replicas(yalps_ctx *ctx, int64_t n, int32_t height, int32_t widt
     if (rhs_out) CU(ctx, cudaMemcpyAsync(rhs_out + (size_t)begin * height, d_rhs, (size_t)cn * height * 8, cudaMemcpyDeviceToHost, st));
     if (pos_out) CU(ctx, cudaMemcpyAsync(pos_out + (size_t)begin * pv, d_pos, (size_t)cn * pv * 4, cudaMemcpyDeviceToHost, st));
     if (var_out) CU(ctx, cudaMemcpyAsync(var_out + (size_t)begin * pv, d_var, (size_t)cn * pv * 4, cudaMemcpyDeviceToHost, st));
+    if (reduced_out)
+      CU(ctx, cudaMemcpyAsync(reduced_out + (size_t)begin * pv, d_red, (size_t)cn * pv * 8, cudaMemcpyDeviceToHost, st));
     CU(ctx, cudaEventRecord(ctx->events[slot], st));
     used[slot] = true;
   }
   for (int i = 0; i < 2; i++)
     if (used[i]) CU(ctx, cudaStreamSynchronize(ctx->streams[i]));
   return check_device_status(ctx, status, n);
+}
+
+int yalps_solve_replicas(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
+                         const double *rhs, const yalps_options *opt, int32_t *status, double *value, int64_t *pivots,
+                         double *rhs_out, int32_t *pos_out, int32_t *var_out) {
+  return yalps_solve_replicas_duals(ctx, n, height, width, base, rhs, opt, status, value, pivots, rhs_out, pos_out,
+                                    var_out, nullptr);
 }
 
 int yalps_set_replica_sharing(yalps_ctx *ctx, int32_t on) {

@@ -24,6 +24,15 @@ def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
+def _basis_in(pos_in, var_in, size: int) -> tuple:
+    p = None if pos_in is None else np.ascontiguousarray(pos_in, np.int32).reshape(-1)
+    v = None if var_in is None else np.ascontiguousarray(var_in, np.int32).reshape(-1)
+    for arr in (p, v):
+        if arr is not None and arr.size != size:
+            raise ValueError("pos_in / var_in need n*(width+height) entries")
+    return p, v
+
+
 def make_options(precision=1e-8, max_pivots=8192, check_cycles=False, tolerance=0.0, timeout_ms=math.inf,
                  max_iterations=32768) -> Options:
     o = Options()
@@ -105,7 +114,7 @@ class Engine:
 
     # ------------------------------------------------------------------ simplex batches
     def batch_outputs(self, n: int, height: int, width: int, want_matrices: bool = False, want_basis: bool = True,
-                      pinned: bool = False) -> dict:
+                      pinned: bool = False, want_duals: bool = False) -> dict:
         """Output buffers for solve_batch; pinned=True allocates them page-locked (reusable across calls)."""
         mk = self.pinned_empty if pinned else (lambda shape, dtype: np.empty(shape, dtype))
         return {
@@ -116,15 +125,19 @@ class Engine:
             "pos": mk((n, width + height), np.int32) if want_basis else None,
             "var": mk((n, width + height), np.int32) if want_basis else None,
             "matrices": mk((n, height * width), np.float64) if want_matrices else None,
+            "reduced": mk((n, width + height), np.float64) if want_duals else None,
         }
 
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, want_basis: bool = True, out: Optional[dict] = None,
-                    pos_in: Optional[np.ndarray] = None, var_in: Optional[np.ndarray] = None) -> dict:
+                    pos_in: Optional[np.ndarray] = None, var_in: Optional[np.ndarray] = None,
+                    want_duals: bool = False) -> dict:
         """n same-shape tableaus, `matrices` float64 of n*height*width values (not modified).
         `out` may be a dict from batch_outputs() to reuse (pinned) result buffers.
         pos_in / var_in (int32, n*(width+height)): the basis bookkeeping the tableaus arrive with (the node LPs of
-        src/branchAndCut.ts:127); None = the identity of a fresh tableau (src/tableau.ts:95-98)."""
+        src/branchAndCut.ts:127); None = the identity of a fresh tableau (src/tableau.ts:95-98).
+        want_duals: also out["reduced"] (n, width+height), row 0 of the final tableau per variable id
+        (yalps_solve_batch_duals; yalps_b200.sensitivity turns it into shadow prices and reduced costs)."""
         opt = options or make_options()
         m = np.ascontiguousarray(matrices, dtype=np.float64).reshape(-1)
         cells = height * width
@@ -132,20 +145,25 @@ class Engine:
             raise ValueError(f"matrices has {m.size} values, not a multiple of {height}x{width}")
         n = m.size // cells
         if out is None:
-            out = self.batch_outputs(n, height, width, want_matrices, want_basis)
+            out = self.batch_outputs(n, height, width, want_matrices, want_basis, want_duals=want_duals)
         elif out["status"].shape[0] != n:
             raise ValueError("out was allocated for a different batch size")
+        if want_duals and out.get("reduced") is None:
+            out["reduced"] = np.empty((n, width + height), np.float64)
+        if want_duals:
+            p, v = _basis_in(pos_in, var_in, n * (width + height))
+            self._check(self._lib.yalps_solve_batch_duals(self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v),
+                                                          C.byref(opt), _ptr(out["status"]), _ptr(out["value"]),
+                                                          _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]),
+                                                          _ptr(out["var"]), _ptr(out["matrices"]), _ptr(out["reduced"])))
+            return out
         if pos_in is None and var_in is None:
             self._check(self._lib.yalps_solve_batch(self._ctx, n, height, width, _ptr(m), C.byref(opt),
                                                     _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
                                                     _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
                                                     _ptr(out["matrices"])))
             return out
-        p = None if pos_in is None else np.ascontiguousarray(pos_in, np.int32).reshape(-1)
-        v = None if var_in is None else np.ascontiguousarray(var_in, np.int32).reshape(-1)
-        for arr in (p, v):
-            if arr is not None and arr.size != n * (width + height):
-                raise ValueError("pos_in / var_in need n*(width+height) entries")
+        p, v = _basis_in(pos_in, var_in, n * (width + height))
         self._check(self._lib.yalps_solve_batch_basis(self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt),
                                                       _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
                                                       _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
@@ -172,8 +190,10 @@ class Engine:
         return STATUS_NAMES[int(status[0])], float(value[0])
 
     def solve_replicas(self, base: np.ndarray, rhs: np.ndarray, height: int, width: int,
-                       options: Optional[Options] = None, want_basis: bool = True, out: Optional[dict] = None) -> dict:
-        """n replicas of `base` (height*width) that differ only in column 0: rhs is float64 (n, height)."""
+                       options: Optional[Options] = None, want_basis: bool = True, out: Optional[dict] = None,
+                       want_duals: bool = False) -> dict:
+        """n replicas of `base` (height*width) that differ only in column 0: rhs is float64 (n, height).
+        want_duals: also out["reduced"] (n, width+height), as solve_batch."""
         opt = options or make_options()
         b = np.ascontiguousarray(base, np.float64).reshape(-1)
         r = np.ascontiguousarray(rhs, np.float64).reshape(-1)
@@ -181,10 +201,18 @@ class Engine:
             raise ValueError("base must hold height*width values and rhs n*height")
         n = r.size // height
         if out is None:
-            out = self.batch_outputs(n, height, width, False, want_basis)
-        self._check(self._lib.yalps_solve_replicas(self._ctx, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
-                                                   _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
-                                                   _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"])))
+            out = self.batch_outputs(n, height, width, False, want_basis, want_duals=want_duals)
+        if not want_duals:
+            self._check(self._lib.yalps_solve_replicas(self._ctx, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
+                                                       _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
+                                                       _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"])))
+            return out
+        if out.get("reduced") is None:
+            out["reduced"] = np.empty((n, width + height), np.float64)
+        self._check(self._lib.yalps_solve_replicas_duals(self._ctx, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
+                                                         _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
+                                                         _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
+                                                         _ptr(out["reduced"])))
         return out
 
     def set_replica_sharing(self, on: bool = True):
@@ -197,8 +225,9 @@ class Engine:
         return int(self._lib.yalps_replica_forks(self._ctx))
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
-                     want_matrices: bool = False) -> list:
-        """LPs of different shapes in one call.  tableaus[i] is float64 of height_i*width_i values."""
+                     want_matrices: bool = False, want_duals: bool = False) -> list:
+        """LPs of different shapes in one call.  tableaus[i] is float64 of height_i*width_i values.
+        want_duals: every result also has "reduced" (width_i+height_i values, as solve_batch)."""
         opt = options or make_options()
         n = len(tableaus)
         if n == 0:
@@ -222,9 +251,16 @@ class Engine:
         pos = np.empty(int(poffs[-1]), np.int32)
         var = np.empty(int(poffs[-1]), np.int32)
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
-        self._check(self._lib.yalps_solve_ragged(self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()),
-                                                 _ptr(packed), C.byref(opt), _ptr(status), _ptr(value), _ptr(pivots),
-                                                 _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats)))
+        if want_duals:
+            red = np.empty(int(poffs[-1]), np.float64)
+            self._check(self._lib.yalps_solve_ragged_duals(self._ctx, n, _ptr(heights), _ptr(widths),
+                                                           _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
+                                                           _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos),
+                                                           _ptr(var), _ptr(mats), _ptr(red)))
+        else:
+            self._check(self._lib.yalps_solve_ragged(self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()),
+                                                     _ptr(packed), C.byref(opt), _ptr(status), _ptr(value), _ptr(pivots),
+                                                     _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats)))
         res = []
         for i in range(n):
             res.append({
@@ -232,14 +268,24 @@ class Engine:
                 "rhs": rhs[roffs[i]:roffs[i + 1]], "pos": pos[poffs[i]:poffs[i + 1]], "var": var[poffs[i]:poffs[i + 1]],
                 "matrix": mats[offs[i]:offs[i + 1]] if want_matrices else None,
             })
+            if want_duals:
+                res[i]["reduced"] = red[poffs[i]:poffs[i + 1]]
         return res
 
     def solve_batch_device(self, n: int, height: int, width: int, d_matrices: int, options: Optional[Options] = None,
                            d_work: int = 0, d_status: int = 0, d_value: int = 0, d_pivots: int = 0, d_rhs: int = 0,
-                           d_pos: int = 0, d_var: int = 0, d_matrices_out: int = 0, stream: int = 0):
-        """Everything already in device memory (raw pointers); enqueues on `stream` and returns."""
+                           d_pos: int = 0, d_var: int = 0, d_matrices_out: int = 0, stream: int = 0,
+                           d_reduced: int = 0):
+        """Everything already in device memory (raw pointers); enqueues on `stream` and returns.
+        d_reduced (float64, n*(width+height)): reduced costs per variable id, as solve_batch's out["reduced"]."""
         opt = options or make_options()
         z = lambda p: C.c_void_p(p) if p else None
+        if d_reduced:
+            self._check(self._lib.yalps_solve_batch_device_duals(self._ctx, n, height, width, z(d_matrices), z(d_work),
+                                                                 C.byref(opt), z(d_status), z(d_value), z(d_pivots),
+                                                                 z(d_rhs), z(d_pos), z(d_var), z(d_matrices_out),
+                                                                 z(stream), z(d_reduced)))
+            return
         self._check(self._lib.yalps_solve_batch_device(self._ctx, n, height, width, z(d_matrices), z(d_work),
                                                        C.byref(opt), z(d_status), z(d_value), z(d_pivots), z(d_rhs),
                                                        z(d_pos), z(d_var), z(d_matrices_out), z(stream)))
@@ -302,6 +348,27 @@ class Engine:
         if cells.size != values.size:
             raise ValueError("cells and values must have the same length")
         return self.solve_tableau(values, height, width, integers, sign, options, cells=cells)
+
+    def solve_lp_sparse(self, cells: np.ndarray, values: np.ndarray, height: int, width: int,
+                        options: Optional[Options] = None) -> dict:
+        """One LP given as ordered (cell, value) stores into a zero matrix (yalps_solve_sparse_duals): status, value,
+        pivots, rhs, pos, var and reduced, as solve_batch with n = 1 and want_duals."""
+        opt = options or make_options()
+        cells = np.ascontiguousarray(cells, np.int32).reshape(-1)
+        values = np.ascontiguousarray(values, np.float64).reshape(-1)
+        if cells.size != values.size:
+            raise ValueError("cells and values must have the same length")
+        status, value = C.c_int32(), C.c_double()
+        piv = np.zeros(2, np.int64)
+        rhs, pos, var = np.empty(height), np.empty(width + height, np.int32), np.empty(width + height, np.int32)
+        red = np.empty(width + height, np.float64)
+        self._check(self._lib.yalps_solve_sparse_duals(self._ctx, height, width, int(cells.size),
+                                                       _ptr(cells) if cells.size else None,
+                                                       _ptr(values) if values.size else None, C.byref(opt),
+                                                       C.byref(status), C.byref(value), _ptr(piv), _ptr(rhs), _ptr(pos),
+                                                       _ptr(var), _ptr(red)))
+        return {"status": status.value, "value": value.value, "pivots": (int(piv[0]), int(piv[1])), "rhs": rhs,
+                "pos": pos, "var": var, "reduced": red}
 
     def solve_tableau(self, matrix: np.ndarray, height: int, width: int, integers: Sequence[int], sign: float,
                       options: Optional[Options] = None, cells: Optional[np.ndarray] = None) -> dict:
@@ -452,20 +519,30 @@ class MultiEngine:
                 raise YalpsError(-2, (self._lib.yalps_last_error(ctx) or b"").decode())
 
     @staticmethod
-    def _outputs(n, height, width, want_matrices):
+    def _outputs(n, height, width, want_matrices, want_duals=False):
         return {"status": np.empty(n, np.int32), "value": np.empty(n, np.float64), "pivots": np.empty((n, 2), np.int64),
                 "rhs": np.empty((n, height), np.float64), "pos": np.empty((n, width + height), np.int32),
                 "var": np.empty((n, width + height), np.int32),
-                "matrices": np.empty((n, height * width), np.float64) if want_matrices else None}
+                "matrices": np.empty((n, height * width), np.float64) if want_matrices else None,
+                "reduced": np.empty((n, width + height), np.float64) if want_duals else None}
 
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
-                    want_matrices: bool = False, pos_in=None, var_in=None, out: Optional[dict] = None) -> dict:
+                    want_matrices: bool = False, pos_in=None, var_in=None, out: Optional[dict] = None,
+                    want_duals: bool = False) -> dict:
         opt = options or make_options()
         m = np.ascontiguousarray(matrices, np.float64).reshape(-1)
         n = m.size // (height * width)
-        out = out or self._outputs(n, height, width, want_matrices)
+        out = out or self._outputs(n, height, width, want_matrices, want_duals)
         p = None if pos_in is None else np.ascontiguousarray(pos_in, np.int32).reshape(-1)
         v = None if var_in is None else np.ascontiguousarray(var_in, np.int32).reshape(-1)
+        if want_duals:
+            if out.get("reduced") is None:
+                out["reduced"] = np.empty((n, width + height), np.float64)
+            self._check(self._lib.yalps_multi_solve_batch_duals(
+                self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
+                _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
+                _ptr(out["matrices"]), _ptr(out["reduced"])))
+            return out
         self._check(self._lib.yalps_multi_solve_batch(self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt),
                                                       _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
                                                       _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
@@ -473,19 +550,26 @@ class MultiEngine:
         return out
 
     def solve_replicas(self, base: np.ndarray, rhs: np.ndarray, height: int, width: int,
-                       options: Optional[Options] = None, out: Optional[dict] = None) -> dict:
+                       options: Optional[Options] = None, out: Optional[dict] = None, want_duals: bool = False) -> dict:
         opt = options or make_options()
         b = np.ascontiguousarray(base, np.float64).reshape(-1)
         r = np.ascontiguousarray(rhs, np.float64).reshape(-1)
         n = r.size // height
-        out = out or self._outputs(n, height, width, False)
+        out = out or self._outputs(n, height, width, False, want_duals)
+        if want_duals:
+            if out.get("reduced") is None:
+                out["reduced"] = np.empty((n, width + height), np.float64)
+            self._check(self._lib.yalps_multi_solve_replicas_duals(
+                self._m, n, height, width, _ptr(b), _ptr(r), C.byref(opt), _ptr(out["status"]), _ptr(out["value"]),
+                _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]), _ptr(out["reduced"])))
+            return out
         self._check(self._lib.yalps_multi_solve_replicas(self._m, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
                                                          _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
                                                          _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"])))
         return out
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
-                     want_matrices: bool = False) -> list:
+                     want_matrices: bool = False, want_duals: bool = False) -> list:
         opt = options or make_options()
         n = len(tableaus)
         if n == 0:
@@ -502,12 +586,22 @@ class MultiEngine:
         status, value, pivots = np.empty(n, np.int32), np.empty(n, np.float64), np.empty((n, 2), np.int64)
         rhs, pos, var = np.empty(int(roffs[-1])), np.empty(int(poffs[-1]), np.int32), np.empty(int(poffs[-1]), np.int32)
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
-        self._check(self._lib.yalps_multi_solve_ragged(self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()),
-                                                       _ptr(packed), C.byref(opt), _ptr(status), _ptr(value),
-                                                       _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats)))
-        return [{"status": int(status[i]), "value": float(value[i]), "pivots": (int(pivots[i, 0]), int(pivots[i, 1])),
-                 "rhs": rhs[roffs[i]:roffs[i + 1]], "pos": pos[poffs[i]:poffs[i + 1]], "var": var[poffs[i]:poffs[i + 1]],
-                 "matrix": mats[offs[i]:offs[i + 1]] if want_matrices else None} for i in range(n)]
+        if want_duals:
+            red = np.empty(int(poffs[-1]), np.float64)
+            self._check(self._lib.yalps_multi_solve_ragged_duals(
+                self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
+                _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red)))
+        else:
+            self._check(self._lib.yalps_multi_solve_ragged(self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()),
+                                                           _ptr(packed), C.byref(opt), _ptr(status), _ptr(value),
+                                                           _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats)))
+        res = [{"status": int(status[i]), "value": float(value[i]), "pivots": (int(pivots[i, 0]), int(pivots[i, 1])),
+                "rhs": rhs[roffs[i]:roffs[i + 1]], "pos": pos[poffs[i]:poffs[i + 1]], "var": var[poffs[i]:poffs[i + 1]],
+                "matrix": mats[offs[i]:offs[i + 1]] if want_matrices else None} for i in range(n)]
+        if want_duals:
+            for i in range(n):
+                res[i]["reduced"] = red[poffs[i]:poffs[i + 1]]
+        return res
 
     def solve_large(self, matrix: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrix: bool = False) -> dict:

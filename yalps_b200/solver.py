@@ -6,6 +6,10 @@ Model, Options and Solution keep the reference's shapes and spellings (src/types
   options = {"precision", "checkCycles", "maxPivots", "tolerance", "timeout", "maxIterations",
              "includeZeroVariables"}
   solution = {"status": "optimal"|"infeasible"|"unbounded"|"timedout"|"cycled", "result", "variables"}
+One option goes beyond the reference: `sensitivity` (default False).  When it is true (LP models only), every
+Solution also has "reducedCosts" ([[variable, d result / d variable], ...], model order) and "shadowPrices"
+([[constraint key, d result / d bound], ...], first-seen order): raw doubles for an optimal LP, empty lists
+otherwise (yalps_b200.sensitivity has the conventions).
 The tableau is built on the host (tableau.py), the simplex and branch-and-cut numerics run on the GPU
 through the C ABI; there is no CPU solve path.
 """
@@ -17,7 +21,8 @@ from typing import Optional, Sequence
 import numpy as np
 
 from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
-from .tableau import SPARSE_OVER_BYTES, TableauModel, tableau_model
+from .sensitivity import model_sensitivity
+from .tableau import SPARSE_OVER_BYTES, TableauModel, constraint_rows, entries, tableau_model
 
 # src/YALPS.ts:52-60
 _DEFAULTS = {
@@ -87,16 +92,49 @@ def _solution(tabmod: TableauModel, status: str, result: float, rhs, pos, var, o
     return {"status": status, "result": math.nan, "variables": []}
 
 
+def _check_lp(tabmod: TableauModel):
+    if tabmod.integers:
+        raise ValueError("sensitivity: duals are defined for LP models only (this model has integer or binary variables)")
+
+
+def _with_sensitivity(sol: dict, tabmod: TableauModel, model: dict, reduced) -> dict:
+    """Solution + reducedCosts / shadowPrices (empty unless optimal)."""
+    if sol["status"] != "optimal":
+        return {**sol, "reducedCosts": [], "shadowPrices": []}
+    rows = constraint_rows(list(entries(model["constraints"])))
+    rc, sp = model_sensitivity(tabmod.variables, rows, reduced, tabmod.tableau.width, tabmod.sign)
+    return {**sol, "reducedCosts": rc, "shadowPrices": sp}
+
+
 def solve(model: dict, options: Optional[dict] = None, *, engine: Optional[Engine] = None,
           info: Optional[dict] = None) -> dict:
     """Runs the solver on `model` (src/YALPS.ts:73-92).  `info`, if given, receives engine statistics."""
     opt = {**_DEFAULTS, **(options or {})}
-    eng = engine or get_engine()
     # big model tableaus are almost all zeros: they go to the device as (cell, value) pairs (yalps_solve_sparse) and
     # never exist densely on the host; small ones take the library's zero-copy path as a dense image
-    sparse_ok = hasattr(eng, "solve_tableau_sparse")
+    sparse_ok = hasattr(engine, "solve_tableau_sparse") if engine is not None else True
     tabmod = tableau_model(model, SPARSE_OVER_BYTES if sparse_ok else None)
     t = tabmod.tableau
+    if opt.get("sensitivity"):
+        _check_lp(tabmod)
+    eng = engine or get_engine()
+    if opt.get("sensitivity"):
+        # the root LP is the whole solve: one LP with its reduced-cost row (dense batch of one, or the cell pairs)
+        if t.matrix is None:
+            r = eng.solve_lp_sparse(t.cells, t.values, t.height, t.width, _c_options(opt))
+            status, value, rhs, pos, var, red = (r["status"], r["value"], r["rhs"], r["pos"], r["var"], r["reduced"])
+            piv = r["pivots"]
+        else:
+            r = eng.solve_batch(t.matrix, t.height, t.width, _c_options(opt), want_duals=True)
+            status, value = int(r["status"][0]), float(r["value"][0])
+            rhs, pos, var, red = r["rhs"][0], r["pos"][0], r["var"][0], r["reduced"][0]
+            piv = (int(r["pivots"][0, 0]), int(r["pivots"][0, 1]))
+        if info is not None:
+            info.update(nodes=0, node_pivots=0, max_cuts=0, max_heap=0, waves=0, device_nodes=0, wave_us=0, bnb_us=0,
+                        root_status=STATUS_NAMES[status], root_value=value, root_pivots=piv, height=t.height,
+                        width=t.width, final_rhs=rhs, final_pos=pos, final_var=var)
+        sol = _solution(tabmod, STATUS_NAMES[status], value, rhs, pos, var, opt)
+        return _with_sensitivity(sol, tabmod, model, red)
     if t.matrix is None:
         r = eng.solve_tableau_sparse(t.cells, t.values, t.height, t.width, tabmod.integers, tabmod.sign, _c_options(opt))
     else:
@@ -130,10 +168,18 @@ def solve_many(models: Sequence[dict], options: Optional[dict] = None, *, engine
     Results are identical to calling solve() per model."""
     opt = {**_DEFAULTS, **(options or {})}
     copt = _c_options(opt)
-    eng = engine or get_engine()
     tabmods = [tableau_model(m) for m in models]
+    if opt.get("sensitivity"):
+        for tm in tabmods:
+            _check_lp(tm)
+    eng = engine or get_engine()
     if not tabmods:
         return []
+    if opt.get("sensitivity"):  # LP models only: the ragged root batch is the whole solve (one GPU or sharded)
+        roots = eng.solve_ragged([tm.tableau.matrix for tm in tabmods],
+                                 [(tm.tableau.height, tm.tableau.width) for tm in tabmods], copt, want_duals=True)
+        return [_with_sensitivity(_solution(tm, STATUS_NAMES[r["status"]], r["value"], r["rhs"], r["pos"], r["var"], opt),
+                                  tm, m, r["reduced"]) for tm, m, r in zip(tabmods, models, roots)]
     if isinstance(eng, MultiEngine):  # one C-ABI call: roots sharded over the GPUs, searches dealt to worker contexts
         res = eng.solve_many_tableaus(tabmods, copt, searches_per_device=milp_workers)
         return [_solution(tm, STATUS_NAMES[r["status"]], r["result"], r["rhs"], r["pos"], r["var"], opt)

@@ -93,9 +93,15 @@ class TableauModel:
     integers: list  # variable ids (1-based columns) that must be integral
 
 
-def _stores_python(variables: list, constraints: list, objective, sign: float, width: int, binary_cols: list):
-    """The ordered stores of src/tableau.ts:73-134 as (cells, values, rows); specification of csrc/tabfast.c."""
-    # merge constraints per key, first-seen order (src/tableau.ts:73-80)
+def constraint_rows(constraints: list) -> list:
+    """Merged constraint keys in first-seen order with their tableau rows (src/tableau.ts:73-86):
+    [(key, upper row or -1, lower row or -1)].  A key's bounds are intersected over its entries; the upper row
+    (`a.x <= max`) comes before the lower row (`-a.x <= -min`), rows count from 1, and an infinite bound has no row."""
+    return [(key, up, lo) for key, up, lo, _, _ in _merged_rows(constraints)]
+
+
+def _merged_rows(constraints: list) -> list:
+    """constraint_rows plus each key's merged (upper, lower) bounds."""
     lower: dict[Any, float] = {}
     upper: dict[Any, float] = {}
     for key, con in constraints:
@@ -110,32 +116,41 @@ def _stores_python(variables: list, constraints: list, objective, sign: float, w
         else:
             lower[key] = max(-math.inf, lo)
             upper[key] = min(math.inf, hi)
-
-    # row numbering: upper row first, then lower row (src/tableau.ts:82-86)
-    up_row: dict[Any, int] = {}
-    lo_row: dict[Any, int] = {}
+    out = []
     rows = 1
-    rhs_rows: list[int] = []
-    rhs_vals: list[float] = []
     for key in lower:
+        up = lo = -1
         if math.isfinite(upper[key]):
-            up_row[key] = rows
-            rhs_rows.append(rows)
-            rhs_vals.append(upper[key])
+            up = rows
             rows += 1
         if math.isfinite(lower[key]):
-            lo_row[key] = rows
-            rhs_rows.append(rows)
-            rhs_vals.append(-lower[key])
+            lo = rows
             rows += 1
+        out.append((key, up, lo, upper[key], lower[key]))
+    return out
+
+
+def _stores_python(variables: list, constraints: list, objective, sign: float, width: int, binary_cols: list):
+    """The ordered stores of src/tableau.ts:73-134 as (cells, values, rows); specification of csrc/tabfast.c."""
+    # merge constraints per key, first-seen order, and number their rows (src/tableau.ts:73-86)
+    merged = _merged_rows(constraints)
+    rows = 1 + sum((u >= 0) + (l >= 0) for _, u, l, _, _ in merged)
+    rhs_rows: list[int] = []
+    rhs_vals: list[float] = []
+    for _, u, l, hi, lo in merged:
+        if u >= 0:
+            rhs_rows.append(u)
+            rhs_vals.append(hi)
+        if l >= 0:
+            rhs_rows.append(l)
+            rhs_vals.append(-lo)
 
     # coefficients: later duplicates of a key overwrite earlier ones (src/tableau.ts:100-117)
     # one lookup per coefficient: key -> (row offset of the upper row or -1, row offset of the lower row or -1, is objective)
     where: dict[Any, tuple] = {}
-    for key in lower:
-        u, l = up_row.get(key), lo_row.get(key)
-        if u is not None or l is not None:
-            where[key] = (-1 if u is None else u * width, -1 if l is None else l * width, False)
+    for key, u, l, _, _ in merged:
+        if u >= 0 or l >= 0:
+            where[key] = (-1 if u < 0 else u * width, -1 if l < 0 else l * width, False)
     if objective is not None:
         u, l, _ = where.get(objective, (-1, -1, False))
         where[objective] = (u, l, True)
