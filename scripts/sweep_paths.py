@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """K1 (shared-memory resident) vs K2 (HBM/L2 resident) across tableau sizes and CTA widths, dense synthetic LPs
-and sparse Netlib replicas: the data behind the automatic path / width policy (plan_launch in yalps_b200.cu)."""
+and sparse Netlib replicas: the data behind the automatic path / width policy (choose_route in yalps_b200.cu)."""
 import json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))

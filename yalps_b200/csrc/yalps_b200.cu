@@ -233,27 +233,74 @@ int default_warps(long long cells, bool resident) {
   return 32;
 }
 
-struct LaunchPlan {
-  bool tmem = false;  // K1t: tableau in tensor memory, one LP per warp (tmem_kernel.cuh)
-  bool small_for_grid = false;  // few LPs outside shared memory, yet small enough that one row-split CTA beats K4
-  bool resident;
-  const KernelEntry *k;
-  size_t smem;
-  int grid;
+// ---- kernel path: which kernels a launch takes (choose_route) and how they are enqueued (launch_route) --------------
+enum RouteKind {
+  ROUTE_K1T,       // K1t: tableau in tensor memory, one LP per warp (tmem_kernel.cuh)
+  ROUTE_SIMPLEX,   // k_simplex table: K1/K1s (tableau in shared memory) or K2/K2s (HBM/L2), one LP per CTA
+  ROUTE_CLUSTER,   // KC: one LP per thread-block cluster (cluster_kernel.cuh)
+  ROUTE_GRID_RES,  // KG: one LP over the cooperative grid, tableau in the SMs' shared memory
+  ROUTE_GRID,      // K4: one LP over the cooperative grid, tableau in HBM/L2, the LPs one after another
 };
 
-// density: fraction of non-zero cells of a sample of the input (< 0 = unknown).  Sparse tableaus skip most of
-// the rank-1 update, their pivots are latency-bound, and the HBM/L2-resident kernel wins because it needs no
-// shared memory for the tableau and therefore runs many more LPs per SM (profiles/r01_sweep_paths.jsonl).
-int plan_launch(yalps_ctx *ctx, long long n, int Hcap, int Wcap, bool check_cycles, LaunchPlan *plan,
-                double density = -1.0, bool allow_tmem = false) {
-  // a forced cluster path is resolved by maybe_cluster(); what it cannot take is planned as in automatic mode
-  const int tune_path = (ctx->tune_path == YALPS_PATH_CLUSTER || ctx->tune_path == YALPS_PATH_GRID_RESIDENT) ? (int)YALPS_PATH_AUTO : ctx->tune_path;
+struct Route {
+  RouteKind kind = ROUTE_GRID;
+  const KernelEntry *k = nullptr;  // SIMPLEX, CLUSTER, GRID_RES
+  bool resident = false;   // K1t, K1/K1s; under GRID what the k_simplex plan said (node waves stage their I/O by it)
+  bool assembled = false;  // node waves: K3 assembles the nodes before the row-split kernel runs (big, very sparse nodes)
+  size_t smem = 0;
+  int grid = 0;            // K1T, SIMPLEX: CTAs
+  int C = 0;               // CLUSTER: CTAs per cluster; GRID_RES: CTAs
+  int clusters = 0;        // CLUSTER: co-resident clusters
+};
+
+struct RouteRequest {
+  long long n;
+  int Hcap, Wcap;
+  // fraction of non-zero cells of a sample of the input (< 0 = unknown).  Sparse tableaus skip most of the rank-1
+  // update, their pivots are latency-bound, and the HBM/L2-resident kernel wins because it needs no shared memory for
+  // the tableau and therefore runs many more LPs per SM (profiles/r01_sweep_paths.jsonl).
+  double density = -1.0;
+  bool check_cycles = false;
+  bool allow_k1t = false;
+  // replica leader and forks: the k_simplex kernel as planned, never KC, KG or K4 in its place (GRID only when no
+  // kernel of the table is wide enough).  The forks resume mid-solve, which only k_simplex can.
+  bool table_only = false;
+  // node waves: KC and KG have no node mode (a forced KC path plans as AUTO, a forced KG path as a forced k_simplex
+  // one); root_density is that of the root optimum (big-sparse-node rule)
+  bool nodes = false;
+  double root_density = 1.0;
+};
+
+int plan_cluster(yalps_ctx *ctx, int Hcap, int Wcap, Route *r);
+int plan_gridres(yalps_ctx *ctx, int Hcap, int Wcap, Route *r);
+
+// The kernel path of one launch of q.n LPs of at most q.Hcap x q.Wcap: the tuning of yalps_set_tuning /
+// yalps_set_row_groups, the YALPS_* switches, and otherwise the rules measured on B200 (comments below).  A forced path
+// that cannot take the tableau fails with YALPS_ERR_TOO_LARGE.
+int choose_route(yalps_ctx *ctx, const RouteRequest &q, Route *r) {
+  *r = Route{};
+  const long long n = q.n;
+  const int Hcap = q.Hcap, Wcap = q.Wcap;
+  const int path = ctx->tune_path;
+  if (!q.nodes && !q.table_only && path == YALPS_PATH_CLUSTER) {
+    if (int rc = plan_cluster(ctx, Hcap, Wcap, r)) return rc;
+    if (!r->k)
+      return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d does not fit the shared memory of a %d-CTA cluster", Hcap, Wcap, kMaxCluster);
+    return 0;
+  }
+  if (!q.nodes && !q.table_only && path == YALPS_PATH_GRID_RESIDENT) {
+    if (int rc = plan_gridres(ctx, Hcap, Wcap, r)) return rc;
+    if (!r->k)
+      return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d does not fit the shared memory of the grid (or is wider than 2049)", Hcap, Wcap);
+    return 0;
+  }
+  // ---- the k_simplex table (and K1t)
+  const int tune_path = (path == YALPS_PATH_CLUSTER || path == YALPS_PATH_GRID_RESIDENT) ? (int)YALPS_PATH_AUTO : path;
   SmemLayout Lr(Hcap, Wcap, true, 32), Lg(Hcap, Wcap, false, 32);
   bool resident = Lr.total <= (size_t)ctx->smem_optin;
   // (throughput mode only: with at most two LPs per SM the shared-memory row-split kernels are 3x faster than K2 on
   // sparse Netlib models -- AFIRO, 148 LPs: 46 vs 155 us)
-  if (resident && tune_path == YALPS_PATH_AUTO && density >= 0.0 && density < 0.35 &&
+  if (resident && tune_path == YALPS_PATH_AUTO && q.density >= 0.0 && q.density < 0.35 &&
       n > std::max(64LL, 2LL * ctx->prop.multiProcessorCount))
     resident = false;
   if (tune_path == YALPS_PATH_SMEM) {
@@ -262,7 +309,6 @@ int plan_launch(yalps_ctx *ctx, long long n, int Hcap, int Wcap, bool check_cycl
     resident = false;
   }
   const bool grid_ok = tune_path == YALPS_PATH_GRID || (tune_path == YALPS_PATH_AUTO && n <= 16);
-  plan->tmem = false;
   // K1t (tensor-memory resident, one LP per warp, no CTA barrier in the pivot loop): every batch whose tableaus fit
   // it, whatever its size and density.  Measured against the previous choices on B200: 1.47-1.68x K1 on big dense
   // batches of every shape from 9x17 to 33x65 (scripts/tmem_vs_smem.py); 1.5-2.3x K2 on big batches with 70-90 % zeros
@@ -277,34 +323,30 @@ int plan_launch(yalps_ctx *ctx, long long n, int Hcap, int Wcap, bool check_cycl
   // active rows: 90 % zeros, 33x65, one LP: 18.8 vs 18.9 us for K1s; scripts/tmem_small_batches.py).
   const bool tmem_auto = tune_path == YALPS_PATH_AUTO && ctx->tune_threads <= 0 && ctx->tune_rows <= 0 &&
                          (!tmem_kernel_is_tall(Hcap) ||
-                          (latency_mode ? density >= 0.5
+                          (latency_mode ? q.density >= 0.5
                                         // throughput mode (scripts/policy_mid_batches.py): KLEIN1 55x55 (density 0.24) 2.2-2.6x
                                         // the HBM-resident K2; very sparse AFIRO 36x33 (0.1) only while one wave of
                                         // 8 LPs per SM covers the batch, beyond that K2 is 20-30 % faster
-                                        : (density < 0.0 || density >= 0.15 || n <= 8LL * ctx->prop.multiProcessorCount)));
-  if (allow_tmem && tmem_kernel_fits(Hcap, Wcap) && (tune_path == YALPS_PATH_TMEM || tmem_auto)) {
-    plan->tmem = true;
-    plan->resident = true;
-    plan->k = nullptr;
-    plan->smem = tmem_kernel_dynamic_smem(Hcap);
-    CU(ctx, raise_smem_limit(ctx->device, tmem_kernel_fn(Hcap, false, check_cycles), (int)plan->smem));
-    if (ctx->d_rows) CU(ctx, raise_smem_limit(ctx->device, tmem_kernel_fn(Hcap, true, check_cycles), (int)plan->smem));
+                                        : (q.density < 0.0 || q.density >= 0.15 || n <= 8LL * ctx->prop.multiProcessorCount)));
+  if (q.allow_k1t && tmem_kernel_fits(Hcap, Wcap) && (tune_path == YALPS_PATH_TMEM || tmem_auto)) {
+    r->kind = ROUTE_K1T;
+    r->resident = true;
+    r->smem = tmem_kernel_dynamic_smem(Hcap);
+    CU(ctx, raise_smem_limit(ctx->device, tmem_kernel_fn(Hcap, false, q.check_cycles), (int)r->smem));
+    if (ctx->d_rows) CU(ctx, raise_smem_limit(ctx->device, tmem_kernel_fn(Hcap, true, q.check_cycles), (int)r->smem));
     // checkCycles: one history buffer per warp, so one CTA per SM bounds the memory (4 warps x 2 x hist_cap ints each)
-    const long long ctas = (long long)(check_cycles ? 1 : tmem_kernel_ctas_per_sm(Hcap)) * ctx->prop.multiProcessorCount;
-    plan->grid = (int)std::max(1LL, std::min(ctas, n));  // few LPs: one per CTA (the kernel deals LP i to CTA i % grid)
+    const long long ctas = (long long)(q.check_cycles ? 1 : tmem_kernel_ctas_per_sm(Hcap)) * ctx->prop.multiProcessorCount;
+    r->grid = (int)std::max(1LL, std::min(ctas, n));  // few LPs: one per CTA (the kernel deals LP i to CTA i % grid)
     return 0;
   }
   if (tune_path == YALPS_PATH_TMEM)
     return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d does not fit the tensor-memory kernel (max %dx%d, no node mode)",
                 Hcap, Wcap, 65, 65);
-  plan->resident = resident;
-  plan->k = nullptr;
-  plan->smem = 0;
-  plan->grid = 0;
-  if (!resident && Lg.total > (size_t)ctx->smem_optin) {
-    if (grid_ok) return 0;  // only the grid kernel (K4) can take it
+  r->resident = resident;
+  // pivot row/column staging beyond shared memory: only the grid kernel (K4) can take the tableau
+  const bool staged = resident || Lg.total <= (size_t)ctx->smem_optin;
+  if (!staged && !grid_ok)
     return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d: pivot row/column staging exceeds shared memory", Hcap, Wcap);
-  }
   // CTA shape.  Explicit tuning wins; otherwise (scripts/single_lp_latency.py, scripts/sweep_config3.py on B200):
   //  * latency mode (every LP can have an SM to itself): row-split CTAs, sized by the tableau;
   //  * throughput mode: one row group and many CTAs per SM for tableaus in shared memory, a small row split for
@@ -312,7 +354,7 @@ int plan_launch(yalps_ctx *ctx, long long n, int Hcap, int Wcap, bool check_cycl
   const long long cells = (long long)Hcap * Wcap;
   int want_threads = ctx->tune_threads, want_rows = ctx->tune_rows;
   if (want_threads <= 0 && want_rows <= 0) {
-    if (n <= 2LL * ctx->prop.multiProcessorCount) {
+    if (latency_mode) {
       // latency mode wants the row-split layout (compacted row list next to the tableau): a tableau that only fits
       // shared memory without it is better off on the cluster / HBM-resident split kernels than on one-row-group K1
       if (resident && tune_path == YALPS_PATH_AUTO && SmemLayout(Hcap, Wcap, true, 16, true).total > (size_t)ctx->smem_optin)
@@ -335,68 +377,92 @@ int plan_launch(yalps_ctx *ctx, long long n, int Hcap, int Wcap, bool check_cycl
       if (cells >= 5000) want_threads = Wcap <= 129 ? 64 : 128, want_rows = 2;
     }
   }
-  plan->small_for_grid = !resident && cells < 40000;
+  const bool small_for_grid = !resident && cells < 40000;  // few LPs outside shared memory, yet one row-split CTA beats K4
   const int nw = want_threads > 0 ? std::max(1, want_threads / 32) : default_warps(cells, resident);
   int nwr = want_rows > 0 ? want_rows : 1;
   const KernelEntry *k = nullptr;
-  if (nwr > 1) {
+  if (staged && nwr > 1) {
     k = pick_kernel(std::max(1, nw / nwr), nwr, Wcap, resident);
     if (k && SmemLayout(Hcap, Wcap, resident, k->nw * k->nwr, true).total > (size_t)ctx->smem_optin) k = nullptr;
   }
-  if (!k) {
+  if (staged && !k) {
     nwr = 1;
     k = pick_kernel(nw, 1, Wcap, resident);
   }
+  if (!k && !grid_ok) return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau width %d exceeds the widest kernel", Wcap);
   if (k) {
-    Lr = SmemLayout(Hcap, Wcap, true, k->nw * k->nwr, k->nwr > 1);
-    Lg = SmemLayout(Hcap, Wcap, false, k->nw * k->nwr, k->nwr > 1);
-  }
-  if (k) {  // the attribute / occupancy queries cost microseconds: remember them per (kernel, shared memory size)
-    const size_t smem_c = resident ? Lr.total : Lg.total;
-    const std::string key = std::to_string((size_t)(resident ? (void *)k->resident : (void *)k->global)) + ":" + std::to_string(smem_c);
+    SimplexKernel fn = resident ? k->resident : k->global;
+    const size_t smem = SmemLayout(Hcap, Wcap, resident, k->nw * k->nwr, k->nwr > 1).total;
+    CU(ctx, raise_smem_limit(ctx->device, (const void *)fn, (int)smem));
+    // the occupancy query costs microseconds: remember it per (kernel, shared memory size)
+    const std::string key = std::to_string((size_t)(void *)fn) + ":" + std::to_string(smem);
     auto it = ctx->occ_cache.find(key);
+    int occ = 0;
     if (it != ctx->occ_cache.end()) {
-      CU(ctx, raise_smem_limit(ctx->device, (const void *)(resident ? k->resident : k->global), (int)smem_c));
-      int occ_c = it->second;
-      if (check_cycles) occ_c = std::min(occ_c, 4);
-      if (const char *env = getenv("YALPS_CTAS_PER_SM")) occ_c = std::max(1, std::min(occ_c, atoi(env)));  // experiments
-      long long grid_c = std::max(1LL, std::min((long long)occ_c * ctx->prop.multiProcessorCount, n));
-      plan->resident = resident;
-      plan->k = k;
-      plan->smem = smem_c;
-      plan->grid = (int)grid_c;
+      occ = it->second;
+    } else {
+      CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, k->nw * k->nwr * 32, smem));
+      if (occ < 1) return fail(ctx, YALPS_ERR_TOO_LARGE, "kernel does not fit on an SM (smem %zu)", smem);
+      ctx->occ_cache[key] = occ;
+    }
+    if (q.check_cycles) occ = std::min(occ, 4);  // bounds the history buffer
+    if (const char *env = getenv("YALPS_CTAS_PER_SM")) occ = std::max(1, std::min(occ, atoi(env)));  // experiments
+    r->k = k;
+    r->resident = resident;
+    r->smem = smem;
+    r->grid = (int)std::max(1LL, std::min((long long)occ * ctx->prop.multiProcessorCount, n));
+  }
+  // K4 (whole grid per LP, LPs one after another) beats K2 (one CTA per LP) when the tableaus do not fit in
+  // shared memory and there are too few of them to give every SM its own LP.
+  const bool k4 = !r->k || (!q.table_only && (path == YALPS_PATH_GRID ||
+                                               ((path == YALPS_PATH_AUTO || path == YALPS_PATH_CLUSTER) && !r->resident &&
+                                                n <= 16 && !small_for_grid)));
+  if (path == YALPS_PATH_AUTO && !r->resident && !q.nodes && !q.table_only) {
+    // few LPs that do not fit one SM's shared memory: KC when they fit a cluster's
+    Route c;
+    if (int rc = plan_cluster(ctx, Hcap, Wcap, &c)) return rc;
+    if (c.k && n <= 2LL * std::max(1, c.clusters)) {
+      *r = c;
       return 0;
     }
+    // the batches K4 would take (beyond one cluster's shared memory too) go to KG when the tableau fits the grid's
+    if (k4 && !getenv("YALPS_NO_KG")) {
+      if (int rc = plan_gridres(ctx, Hcap, Wcap, &c)) return rc;
+      if (c.k) {
+        *r = c;
+        return 0;
+      }
+    }
   }
-  if (!k) {
-    if (grid_ok) return 0;
-    return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau width %d exceeds the widest kernel", Wcap);
+  // Big, very sparse nodes (Monster-class models: ~1 % non-zeros, ~10 rows rewritten per pivot): the row-split HBM/L2
+  // kernel with one CTA per node compacts the few active rows and needs no grid barrier -- 5.8 us per pivot for every
+  // node of the wave at once, against 9.5 us per pivot and node on K4 (scripts/big_sparse_paths.py).  Denser nodes
+  // (Vendor Selection: 28 % non-zeros at the root optimum) stay on K4.
+  if (q.nodes && k4 && !r->resident && path == YALPS_PATH_AUTO && ctx->tune_threads <= 0 && ctx->tune_rows <= 0 &&
+      q.root_density < 0.03) {
+    int split_nwc = 8, split_nwr = 2;
+    if (const char *env = getenv("YALPS_NODE_SPLIT")) sscanf(env, "%d,%d", &split_nwc, &split_nwr);  // experiments: "column warps,row groups"
+    if (const KernelEntry *k = pick_kernel(split_nwc, split_nwr, Wcap, false)) {
+      if (k->nwr == split_nwr) {
+        const size_t smem_k = SmemLayout(Hcap, Wcap, false, k->nw * k->nwr, true).total;
+        if (smem_k <= (size_t)ctx->smem_optin) {
+          CU(ctx, raise_smem_limit(ctx->device, (const void *)k->global, (int)smem_k));
+          int occ = 0;
+          CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k->global, k->nw * k->nwr * 32, smem_k));
+          if (occ >= 1) {
+            r->kind = ROUTE_SIMPLEX;
+            r->k = k;
+            r->smem = smem_k;
+            r->grid = (int)std::max<long long>(1, std::min<long long>((long long)occ * ctx->prop.multiProcessorCount, n));
+            r->assembled = true;
+            return 0;
+          }
+        }
+      }
+    }
   }
-  SimplexKernel fn = resident ? k->resident : k->global;
-  const size_t smem = resident ? Lr.total : Lg.total;
-  CU(ctx, raise_smem_limit(ctx->device, (const void *)fn, (int)smem));
-  int occ = 0;
-  CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, k->nw * k->nwr * 32, smem));
-  if (occ < 1) return fail(ctx, YALPS_ERR_TOO_LARGE, "kernel does not fit on an SM (smem %zu)", smem);
-  ctx->occ_cache[std::to_string((size_t)(void *)fn) + ":" + std::to_string(smem)] = occ;
-  if (check_cycles) occ = std::min(occ, 4);  // bounds the history buffer
-  if (const char *env = getenv("YALPS_CTAS_PER_SM")) occ = std::max(1, std::min(occ, atoi(env)));  // experiments
-  long long grid = (long long)occ * ctx->prop.multiProcessorCount;
-  grid = std::max(1LL, std::min(grid, n));
-  plan->resident = resident;
-  plan->k = k;
-  plan->smem = smem;
-  plan->grid = (int)grid;
+  r->kind = k4 ? ROUTE_GRID : ROUTE_SIMPLEX;
   return 0;
-}
-
-// K4 (whole grid per LP, LPs one after another) beats K2 (one CTA per LP) when the tableaus do not fit in
-// shared memory and there are too few of them to give every SM its own LP.
-bool use_grid_path(const yalps_ctx *ctx, long long n, const LaunchPlan &plan) {
-  if (plan.tmem) return false;
-  if (ctx->tune_path == YALPS_PATH_GRID || plan.k == nullptr) return true;
-  if (ctx->tune_path != YALPS_PATH_AUTO && ctx->tune_path != YALPS_PATH_CLUSTER) return false;
-  return !plan.resident && n <= 16 && !plan.small_for_grid;
 }
 
 int hist_capacity(const yalps_options *opt) {
@@ -407,12 +473,12 @@ int hist_capacity(const yalps_options *opt) {
   return (int)cap;
 }
 
-// Enqueue one kernel launch for `args` (device pointers filled in by the caller).
-int launch_simplex(yalps_ctx *ctx, const LaunchPlan &plan, BatchArgs &args, const std::string &slot,
-                   cudaStream_t stream) {
+// K1t, K1/K1s, K2/K2s: one launch.
+int launch_simplex(yalps_ctx *ctx, const Route &r, BatchArgs &args, const std::string &slot, cudaStream_t stream) {
+  const bool tmem = r.kind == ROUTE_K1T;
   if (!args.rows_out && ctx->d_rows && !ctx->rows_per_lp) args.rows_out = ctx->d_rows;  // total mode: every launch of the ctx
   args.counter = nullptr;
-  const long long solvers = plan.tmem ? (long long)plan.grid * tmem_kernel_warps() : plan.grid;  // K1t: one LP per warp
+  const long long solvers = tmem ? (long long)r.grid * tmem_kernel_warps() : r.grid;  // K1t: one LP per warp
   if (args.n > solvers) {  // more LPs than CTAs: dynamic queue (pivot counts vary per LP)
     void *counter = nullptr;
     if (int rc = dev_ensure(ctx, "counter" + slot, 8, &counter)) return rc;
@@ -421,36 +487,29 @@ int launch_simplex(yalps_ctx *ctx, const LaunchPlan &plan, BatchArgs &args, cons
   }
   if (args.check_cycles) {
     void *hist = nullptr;
-    const size_t per_cta = (size_t)(plan.tmem ? tmem_kernel_warps() : 1) * 2 * args.hist_cap * sizeof(int);  // K1t: per warp
-    if (int rc = dev_ensure(ctx, "hist" + slot, (size_t)plan.grid * per_cta, &hist)) return rc;
+    const size_t per_cta = (size_t)(tmem ? tmem_kernel_warps() : 1) * 2 * args.hist_cap * sizeof(int);  // K1t: per warp
+    if (int rc = dev_ensure(ctx, "hist" + slot, (size_t)r.grid * per_cta, &hist)) return rc;
     args.hist = (int *)hist;
   } else {
     args.hist = nullptr;
   }
-  if (plan.tmem) {
-    CU(ctx, launch_simplex_tmem(args, plan.grid, stream));
+  if (tmem) {
+    CU(ctx, launch_simplex_tmem(args, r.grid, stream));
     ctx->launches++;
     return 0;
   }
-  SimplexKernel fn = plan.resident ? plan.k->resident : plan.k->global;
-  fn<<<plan.grid, plan.k->nw * plan.k->nwr * 32, plan.smem, stream>>>(args);
+  SimplexKernel fn = r.resident ? r.k->resident : r.k->global;
+  fn<<<r.grid, r.k->nw * r.k->nwr * 32, r.smem, stream>>>(args);
   CU(ctx, cudaGetLastError());
   ctx->launches++;
   return 0;
 }
 
 // ---- KC: one LP per thread-block cluster (cluster_kernel.cuh) -------------------------------------------
-struct ClusterPlan {
-  const KernelEntry *k = nullptr;
-  int C = 0;          // CTAs per cluster
-  size_t smem = 0;
-  int clusters = 0;   // co-resident clusters
-};
-
 // Smallest cluster (2, 4, 8, 16 CTAs) whose shared memory holds the tableau, and the kernel covering its width.
-// plan->k stays null when the tableau does not fit or the device cannot co-schedule such a cluster.
-int plan_cluster(yalps_ctx *ctx, int Hcap, int Wcap, ClusterPlan *plan) {
-  plan->k = nullptr;
+// r->k stays null when the tableau does not fit or the device cannot co-schedule such a cluster.
+int plan_cluster(yalps_ctx *ctx, int Hcap, int Wcap, Route *r) {
+  r->k = nullptr;
   int count = 0;
   const KernelEntry *tab = kernel_table_cluster(&count);
   const KernelEntry *k = nullptr;
@@ -488,57 +547,55 @@ int plan_cluster(yalps_ctx *ctx, int Hcap, int Wcap, ClusterPlan *plan) {
     }
     if (ncl < 1) continue;
     CU(ctx, raise_smem_limit(ctx->device, (const void *)k->resident, (int)L.total));
-    plan->k = k;
-    plan->C = C;
-    plan->smem = L.total;
-    plan->clusters = ncl;
+    r->kind = ROUTE_CLUSTER;
+    r->k = k;
+    r->C = C;
+    r->smem = L.total;
+    r->clusters = ncl;
     return 0;
   }
   return 0;
 }
 
-int launch_cluster(yalps_ctx *ctx, const ClusterPlan &plan, BatchArgs &args, const std::string &slot, cudaStream_t stream) {
-  const int ncl = (int)std::max<long long>(1, std::min<long long>(plan.clusters, args.n));
+// KC: one LP per thread-block cluster.
+int launch_cluster(yalps_ctx *ctx, const Route &r, BatchArgs &args, const std::string &slot, cudaStream_t stream) {
+  const int ncl = (int)std::max<long long>(1, std::min<long long>(r.clusters, args.n));
   if (!args.rows_out && ctx->d_rows && !ctx->rows_per_lp) args.rows_out = ctx->d_rows;
   args.counter = nullptr;
   args.hist = nullptr;
   if (args.check_cycles) {
     void *hist = nullptr;
-    if (int rc = dev_ensure(ctx, "hist_cl" + slot, (size_t)ncl * plan.C * 2 * args.hist_cap * sizeof(int), &hist)) return rc;
+    if (int rc = dev_ensure(ctx, "hist_cl" + slot, (size_t)ncl * r.C * 2 * args.hist_cap * sizeof(int), &hist)) return rc;
     args.hist = (int *)hist;
   }
   {
     void *scr = nullptr;
-    const size_t per_cluster = (size_t)2 * plan.C * SmemLayout::ld_for(args.Wcap) * sizeof(double);
+    const size_t per_cluster = (size_t)2 * r.C * SmemLayout::ld_for(args.Wcap) * sizeof(double);
     if (int rc = dev_ensure(ctx, "cl_scratch" + slot, per_cluster * ncl, &scr)) return rc;
     args.cl_scratch = (double *)scr;
   }
   args.tma_mode = ctx->kc_tma;
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(ncl * plan.C));
-  cfg.blockDim = dim3((unsigned)(plan.k->nw * plan.k->nwr * 32));
-  cfg.dynamicSmemBytes = plan.smem;
+  cfg.gridDim = dim3((unsigned)(ncl * r.C));
+  cfg.blockDim = dim3((unsigned)(r.k->nw * r.k->nwr * 32));
+  cfg.dynamicSmemBytes = r.smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)plan.C;
+  attr[0].val.clusterDim.x = (unsigned)r.C;
   attr[0].val.clusterDim.y = attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  CU(ctx, cudaLaunchKernelEx(&cfg, plan.k->resident, (const BatchArgs)args));
+  CU(ctx, cudaLaunchKernelEx(&cfg, r.k->resident, (const BatchArgs)args));
   ctx->launches++;
   return 0;
 }
 
 // ---- KG: the cluster kernel with the whole cooperative grid as its "cluster" (tableau resident in the SMs' shared memory)
-struct GridResPlan {
-  const KernelEntry *k = nullptr;
-  int C = 0;  // CTAs (one per SM at most)
-  size_t smem = 0;
-};
-
-int plan_gridres(yalps_ctx *ctx, int Hcap, int Wcap, GridResPlan *plan) {
-  plan->k = nullptr;
+// KG: the cluster kernel with the whole cooperative grid as its "cluster".  r->k stays null when the tableau does not
+// fit the shared memory of the grid.
+int plan_gridres(yalps_ctx *ctx, int Hcap, int Wcap, Route *r) {
+  r->k = nullptr;
   int count = 0, coop = 0;
   const KernelEntry *tab = kernel_table_cluster(&count);
   const KernelEntry *k = nullptr;
@@ -570,28 +627,30 @@ int plan_gridres(yalps_ctx *ctx, int Hcap, int Wcap, GridResPlan *plan) {
     ctx->occ_cache[key] = occ;
   }
   if ((long long)occ * ctx->prop.multiProcessorCount < C) return 0;
-  plan->k = k;
-  plan->C = C;
-  plan->smem = L.total;
+  r->kind = ROUTE_GRID_RES;
+  r->k = k;
+  r->C = C;
+  r->smem = L.total;
   return 0;
 }
 
-int launch_gridres(yalps_ctx *ctx, const GridResPlan &plan, BatchArgs &args, const std::string &slot, cudaStream_t stream) {
+// KG: one LP over the cooperative grid, tableau resident in the SMs' shared memory.
+int launch_gridres(yalps_ctx *ctx, const Route &r, BatchArgs &args, const std::string &slot, cudaStream_t stream) {
   if (!args.rows_out && ctx->d_rows && !ctx->rows_per_lp) args.rows_out = ctx->d_rows;
   args.hist = nullptr;
   if (args.check_cycles) {
     void *hist = nullptr;
-    if (int rc = dev_ensure(ctx, "hist_kg" + slot, (size_t)plan.C * 2 * args.hist_cap * sizeof(int), &hist)) return rc;
+    if (int rc = dev_ensure(ctx, "hist_kg" + slot, (size_t)r.C * 2 * args.hist_cap * sizeof(int), &hist)) return rc;
     args.hist = (int *)hist;
   }
   void *p = nullptr;
   const size_t ldA = (size_t)SmemLayout::ld_for(args.Wcap);
   // candidate rows as 16-byte flag-in-data slots {low word, sequence, high word, sequence}: [2][C][ldA]
-  const size_t pub_bytes = (size_t)2 * plan.C * ldA * sizeof(uint4);
+  const size_t pub_bytes = (size_t)2 * r.C * ldA * sizeof(uint4);
   if (int rc = dev_ensure(ctx, "kg_scratch" + slot, pub_bytes, &p)) return rc;
   args.cl_scratch = (double *)p;
   CU(ctx, cudaMemsetAsync(p, 0, pub_bytes, stream));  // sequence numbers of an earlier launch must not look current
-  const size_t inbox_bytes = (size_t)2 * plan.C * plan.C * sizeof(uint4);  // [2][receiver][sender] selection records
+  const size_t inbox_bytes = (size_t)2 * r.C * r.C * sizeof(uint4);  // [2][receiver][sender] selection records
   if (int rc = dev_ensure(ctx, "kg_slots" + slot, inbox_bytes + 64, &p)) return rc;
   args.gx_slots = (uint4 *)p;
   args.counter = (unsigned long long *)((char *)p + inbox_bytes);
@@ -599,58 +658,105 @@ int launch_gridres(yalps_ctx *ctx, const GridResPlan &plan, BatchArgs &args, con
   CU(ctx, cudaMemsetAsync(p, 0, inbox_bytes + 64, stream));
   args.tma_mode = 0;
   void *params[] = {&args};
-  CU(ctx, cudaLaunchCooperativeKernel((const void *)plan.k->global, dim3((unsigned)plan.C),
-                                      dim3((unsigned)(plan.k->nw * plan.k->nwr * 32)), params, plan.smem, stream));
+  CU(ctx, cudaLaunchCooperativeKernel((const void *)r.k->global, dim3((unsigned)r.C),
+                                      dim3((unsigned)(r.k->nw * r.k->nwr * 32)), params, r.smem, stream));
   ctx->launches++;
   return 0;
 }
 
-// The batches K4 would take (few LPs beyond one SM's -- and one cluster's -- shared memory) go to KG when the tableau
-// fits the shared memory of the whole grid.  1: launched, 0: not applicable, < 0: error.
-int maybe_gridres(yalps_ctx *ctx, long long n, int Hcap, int Wcap, const LaunchPlan *plan, BatchArgs &a, const std::string &slot,
-                  cudaStream_t stream) {
-  const bool forced = ctx->tune_path == YALPS_PATH_GRID_RESIDENT;
-  if (!forced) {
-    if (!plan || ctx->tune_path != YALPS_PATH_AUTO || !use_grid_path(ctx, n, *plan)) return 0;
-    if (getenv("YALPS_NO_KG")) return 0;
+// K4: one LP over the whole grid.  d_M (H*W doubles, reference layout) is solved in place; the options come from `o`
+// (fill_options).
+int launch_grid(yalps_ctx *ctx, int H, int W, double *d_M, const BatchArgs &o, int *d_status, double *d_value,
+                long long *d_pivots, double *d_rhs, int *d_pos, int *d_var, cudaStream_t stream, const int *d_init_var,
+                int init_n, int max_ctas, const std::string &slot, unsigned long long *d_rows, double *d_red = nullptr) {
+  const GridSmem L(H, W);
+  if (L.total > (size_t)ctx->smem_optin)
+    return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d: pivot row/column staging exceeds shared memory", H, W);
+  int coop = 0;
+  CU(ctx, cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device));
+  if (!coop) return fail(ctx, YALPS_ERR_CUDA, "device does not support cooperative launches");
+  CU(ctx, raise_smem_limit(ctx->device, (const void *)k_simplex_grid, (int)L.total));
+  int occ = 0;
+  CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_simplex_grid, kGridThreads, L.total));
+  if (occ < 1) return fail(ctx, YALPS_ERR_TOO_LARGE, "grid kernel does not fit on an SM");
+  // at most ~2 update items (row x 256-column segment) per warp, never more CTAs than can be co-resident
+  int grid = ctx->prop.multiProcessorCount;
+  {
+    const long long items = (long long)H * ((W + kSegCols - 1) / kSegCols);
+    grid = (int)std::min<long long>(grid, std::max(1LL, (items + 2 * kGridWarps - 1) / (2 * kGridWarps)));
   }
-  GridResPlan gp;
-  if (int rc = plan_gridres(ctx, Hcap, Wcap, &gp)) return rc;
-  if (!gp.k) {
-    if (forced)
-      return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d does not fit the shared memory of the grid (or is wider than 2049)", Hcap, Wcap);
-    return 0;
+  if (const char *env = getenv("YALPS_GRID_CTAS")) grid = std::max(1, std::min(atoi(env), ctx->prop.multiProcessorCount * occ));
+  if (max_ctas > 0) grid = std::max(1, std::min(grid, max_ctas));  // several K4 launches sharing the GPU (node waves)
+  GridArgs a{};
+  a.M = d_M;
+  a.H = H;
+  a.W = W;
+  a.status = d_status;
+  a.value = d_value;
+  a.pivots = d_pivots;
+  a.rhs_out = d_rhs;
+  a.pos_out = d_pos;
+  a.red_out = d_red;
+  a.precision = o.precision;
+  a.max_pivots = o.max_pivots;
+  a.check_cycles = o.check_cycles;
+  a.hist_cap = o.hist_cap;
+  void *p = nullptr;
+  if (!d_var) {
+    if (int rc = dev_ensure(ctx, "grid_var" + slot, (size_t)(W + H) * 4, &p)) return rc;
+    d_var = (int *)p;
   }
-  if (int rc = launch_gridres(ctx, gp, a, slot, stream)) return rc;
-  return 1;
+  a.var = d_var;
+  a.init_var = d_init_var;
+  a.init_n = init_n;
+  a.rows_out = d_rows ? d_rows : ((ctx->d_rows && !ctx->rows_per_lp) ? ctx->d_rows : nullptr);
+  if (int rc = dev_ensure(ctx, "grid_flags" + slot, 64, &p)) return rc;
+  a.flags = (int *)p;
+  a.barrier = (unsigned long long *)((char *)p + 32);
+  CU(ctx, cudaMemsetAsync(p, 0, 64, stream));
+  if (a.check_cycles) {
+    if (int rc = dev_ensure(ctx, "grid_hist" + slot, (size_t)2 * a.hist_cap * sizeof(int), &p)) return rc;
+    a.hist = (int *)p;
+  }
+  void *params[] = {&a};
+  CU(ctx, cudaLaunchCooperativeKernel((void *)k_simplex_grid, dim3(grid), dim3(kGridThreads), params, L.total, stream));
+  ctx->launches++;
+  return 0;
 }
 
-// Few LPs that do not fit one SM's shared memory: KC when they fit a cluster's (tune_path AUTO or CLUSTER).
-bool want_cluster(const yalps_ctx *ctx, long long n, const LaunchPlan &plan, const ClusterPlan &cp) {
-  if (!cp.k) return false;
-  if (ctx->tune_path == YALPS_PATH_CLUSTER) return true;
-  if (ctx->tune_path != YALPS_PATH_AUTO || plan.tmem) return false;
-  return !plan.resident && n <= 2LL * std::max(1, cp.clusters);
-}
-
-// 1 = launched on the cluster path, 0 = not applicable (caller goes on with its plan), < 0 = error.
-// plan == nullptr: before plan_launch, only the forced YALPS_PATH_CLUSTER is considered.
-int maybe_cluster(yalps_ctx *ctx, long long n, int Hcap, int Wcap, const LaunchPlan *plan, BatchArgs &a,
-                  const std::string &slot, cudaStream_t stream) {
-  const bool forced = ctx->tune_path == YALPS_PATH_CLUSTER;
-  if (ctx->tune_path == YALPS_PATH_GRID_RESIDENT) return plan ? 0 : maybe_gridres(ctx, n, Hcap, Wcap, nullptr, a, slot, stream);
-  if (!plan && !forced) return 0;
-  if (plan && (forced || ctx->tune_path != YALPS_PATH_AUTO || plan->resident || plan->tmem)) return 0;
-  ClusterPlan cp;
-  if (int rc = plan_cluster(ctx, Hcap, Wcap, &cp)) return rc;
-  if (forced) {
-    if (!cp.k)
-      return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d does not fit the shared memory of a %d-CTA cluster", Hcap, Wcap, kMaxCluster);
-  } else if (!want_cluster(ctx, n, *plan, cp)) {
-    return maybe_gridres(ctx, n, Hcap, Wcap, plan, a, slot, stream);  // beyond a cluster: the whole grid's shared memory (KG)
+// Enqueue route `r` for the LPs of `args` (device pointers filled in by the caller).  K4 solves them one after another
+// in args.work, LP i being LP args.index[i] of the launch; a ragged batch's shapes, offsets and index are read from
+// `host`, host-side copies of those fields of `args`.  Final tableaus under K4: one bulk copy in and one out for a
+// uniform batch whose work buffer is not its input / output, one copy per LP into mat_out for a ragged batch.
+int launch_route(yalps_ctx *ctx, const Route &r, BatchArgs &args, const std::string &slot, cudaStream_t stream,
+                 const BatchArgs *host = nullptr) {
+  if (r.kind == ROUTE_CLUSTER) return launch_cluster(ctx, r, args, slot, stream);
+  if (r.kind == ROUTE_GRID_RES) return launch_gridres(ctx, r, args, slot, stream);
+  if (r.kind != ROUTE_GRID) return launch_simplex(ctx, r, args, slot, stream);
+  const bool ragged = args.heights != nullptr;
+  const BatchArgs &h = ragged ? *host : args;
+  const long long cells = (long long)args.H * args.W;
+  if (!ragged && args.work != args.in)
+    CU(ctx, cudaMemcpyAsync(args.work, args.in, (size_t)(args.n * cells) * 8, cudaMemcpyDeviceToDevice, stream));
+  for (long long i = 0; i < args.n; i++) {
+    const long long id = h.index ? h.index[i] : i;
+    const int H = ragged ? h.heights[id] : args.H, W = ragged ? h.widths[id] : args.W;
+    const long long mo = ragged ? h.mat_off[id] : id * cells, ro = ragged ? h.rhs_off[id] : id * args.H,
+                    po = ragged ? h.pos_off[id] : id * (args.H + args.W);
+    if (int rc = launch_grid(ctx, H, W, args.work + mo, args, args.status ? args.status + id : nullptr,
+                             args.value ? args.value + id : nullptr, args.pivots ? args.pivots + 2 * id : nullptr,
+                             args.rhs_out ? args.rhs_out + ro : nullptr, args.pos_out ? args.pos_out + po : nullptr,
+                             args.var_out ? args.var_out + po : nullptr, stream,
+                             args.var_in ? args.var_in + po : nullptr, args.var_in ? W + H : 0, 0, slot,
+                             args.rows_out ? args.rows_out + (args.rows_per_lp ? id : 0) : nullptr,
+                             args.red_out ? args.red_out + po : nullptr))
+      return rc;
+    if (ragged && args.mat_out)
+      CU(ctx, cudaMemcpyAsync(args.mat_out + mo, args.work + mo, (size_t)H * W * 8, cudaMemcpyDeviceToDevice, stream));
   }
-  if (int rc = launch_cluster(ctx, cp, a, slot, stream)) return rc;
-  return 1;
+  if (!ragged && args.mat_out && args.mat_out != args.work)
+    CU(ctx, cudaMemcpyAsync(args.mat_out, args.work, (size_t)(args.n * cells) * 8, cudaMemcpyDeviceToDevice, stream));
+  return 0;
 }
 
 void fill_options(BatchArgs &a, const yalps_options *opt) {
@@ -786,66 +892,6 @@ int yalps_host_free(yalps_ctx *ctx, void *ptr) {
   return 0;
 }
 
-// K4: one LP over the whole grid.  d_M (H*W doubles, reference layout) is solved in place.
-static int launch_grid(yalps_ctx *ctx, int H, int W, double *d_M, const yalps_options *opt, int *d_status,
-                       double *d_value, long long *d_pivots, double *d_rhs, int *d_pos, int *d_var,
-                       cudaStream_t stream, const int *d_init_var = nullptr, int init_n = 0, int max_ctas = 0,
-                       const std::string &slot = "", unsigned long long *d_rows = nullptr, double *d_red = nullptr) {
-  const GridSmem L(H, W);
-  if (L.total > (size_t)ctx->smem_optin)
-    return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d: pivot row/column staging exceeds shared memory", H, W);
-  int coop = 0;
-  CU(ctx, cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device));
-  if (!coop) return fail(ctx, YALPS_ERR_CUDA, "device does not support cooperative launches");
-  CU(ctx, raise_smem_limit(ctx->device, (const void *)k_simplex_grid, (int)L.total));
-  int occ = 0;
-  CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_simplex_grid, kGridThreads, L.total));
-  if (occ < 1) return fail(ctx, YALPS_ERR_TOO_LARGE, "grid kernel does not fit on an SM");
-  // at most ~2 update items (row x 256-column segment) per warp, never more CTAs than can be co-resident
-  int grid = ctx->prop.multiProcessorCount;
-  {
-    const long long items = (long long)H * ((W + kSegCols - 1) / kSegCols);
-    grid = (int)std::min<long long>(grid, std::max(1LL, (items + 2 * kGridWarps - 1) / (2 * kGridWarps)));
-  }
-  if (const char *env = getenv("YALPS_GRID_CTAS")) grid = std::max(1, std::min(atoi(env), ctx->prop.multiProcessorCount * occ));
-  if (max_ctas > 0) grid = std::max(1, std::min(grid, max_ctas));  // several K4 launches sharing the GPU (node waves)
-  GridArgs a{};
-  a.M = d_M;
-  a.H = H;
-  a.W = W;
-  a.status = d_status;
-  a.value = d_value;
-  a.pivots = d_pivots;
-  a.rhs_out = d_rhs;
-  a.pos_out = d_pos;
-  a.red_out = d_red;
-  a.precision = opt->precision;
-  a.max_pivots = opt->max_pivots;
-  a.check_cycles = opt->check_cycles ? 1 : 0;
-  a.hist_cap = hist_capacity(opt);
-  void *p = nullptr;
-  if (!d_var) {
-    if (int rc = dev_ensure(ctx, "grid_var" + slot, (size_t)(W + H) * 4, &p)) return rc;
-    d_var = (int *)p;
-  }
-  a.var = d_var;
-  a.init_var = d_init_var;
-  a.init_n = init_n;
-  a.rows_out = d_rows ? d_rows : ((ctx->d_rows && !ctx->rows_per_lp) ? ctx->d_rows : nullptr);
-  if (int rc = dev_ensure(ctx, "grid_flags" + slot, 64, &p)) return rc;
-  a.flags = (int *)p;
-  a.barrier = (unsigned long long *)((char *)p + 32);
-  CU(ctx, cudaMemsetAsync(p, 0, 64, stream));
-  if (a.check_cycles) {
-    if (int rc = dev_ensure(ctx, "grid_hist" + slot, (size_t)2 * a.hist_cap * sizeof(int), &p)) return rc;
-    a.hist = (int *)p;
-  }
-  void *params[] = {&a};
-  CU(ctx, cudaLaunchCooperativeKernel((void *)k_simplex_grid, dim3(grid), dim3(kGridThreads), params, L.total, stream));
-  ctx->launches++;
-  return 0;
-}
-
 // ---------------------------------------------------------------------------------------------------------
 // `slot` names the pooled scratch (LP queue counter, cycle history, cluster scratch) of this launch: calls that may be in
 // flight at the same time on different streams of one ctx must use different slots.
@@ -901,31 +947,10 @@ static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, in
   fill_options(a, opt);
   a.rows_out = ctx->d_rows ? ctx->d_rows + (ctx->rows_per_lp ? rows_base : 0) : nullptr;
   a.rows_per_lp = ctx->rows_per_lp;
-  if (int rc = maybe_cluster(ctx, n, height, width, nullptr, a, slot, (cudaStream_t)stream)) return rc < 0 ? rc : 0;
-  LaunchPlan plan;
-  if (int rc = plan_launch(ctx, n, height, width, opt->check_cycles != 0, &plan, density, true)) return rc;
-  if (int rc = maybe_cluster(ctx, n, height, width, &plan, a, slot, (cudaStream_t)stream)) return rc < 0 ? rc : 0;
-  if (use_grid_path(ctx, n, plan)) {
-    if (!d_work) return fail(ctx, YALPS_ERR_ARGUMENT, "d_work is required for the grid path");
-    cudaStream_t st = (cudaStream_t)stream;
-    const size_t cells = (size_t)height * width;
-    if (d_work != d_matrices)
-      CU(ctx, cudaMemcpyAsync(d_work, d_matrices, (size_t)n * cells * 8, cudaMemcpyDeviceToDevice, st));
-    for (int64_t i = 0; i < n; i++) {
-      if (int rc = launch_grid(ctx, height, width, d_work + i * cells, opt, d_status ? d_status + i : nullptr,
-                               d_value ? d_value + i : nullptr, d_pivots ? (long long *)d_pivots + 2 * i : nullptr,
-                               d_rhs_out ? d_rhs_out + i * height : nullptr,
-                               d_pos_out ? d_pos_out + i * (width + height) : nullptr,
-                               d_var_out ? d_var_out + i * (width + height) : nullptr, st, nullptr, 0, 0, slot,
-                               ctx->d_rows ? ctx->d_rows + (ctx->rows_per_lp ? rows_base + i : 0) : nullptr,
-                               d_red_out ? d_red_out + i * (width + height) : nullptr))
-        return rc;
-    }
-    if (d_matrices_out && d_matrices_out != d_work)
-      CU(ctx, cudaMemcpyAsync(d_matrices_out, d_work, (size_t)n * cells * 8, cudaMemcpyDeviceToDevice, st));
-    return 0;
-  }
-  if (!plan.resident) {
+  Route route;
+  if (int rc = choose_route(ctx, {n, height, width, density, opt->check_cycles != 0, true}, &route)) return rc;
+  if (route.kind == ROUTE_GRID && !d_work) return fail(ctx, YALPS_ERR_ARGUMENT, "d_work is required for the grid path");
+  if (route.kind == ROUTE_SIMPLEX && !route.resident) {
     if (!d_work) return fail(ctx, YALPS_ERR_ARGUMENT, "d_work is required for the HBM-resident path");
     if (!d_pos_out || !d_var_out) {
       void *p = nullptr;
@@ -934,7 +959,7 @@ static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, in
       if (!a.var_out) a.var_out = (int *)p + (size_t)n * (width + height);
     }
   }
-  return launch_simplex(ctx, plan, a, slot, (cudaStream_t)stream);
+  return launch_route(ctx, route, a, slot, (cudaStream_t)stream);
 }
 
 int yalps_solve_batch_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
@@ -1016,6 +1041,16 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     }
   }
 
+  // density of (a sample of) the first tableau: the path policy distinguishes dense from very sparse LPs
+  auto first_density = [&]() {
+    const double *m0 = matrices + (ragged ? mat_offsets[0] : 0);
+    const long long c0 = ragged ? (long long)heights[0] * widths[0] : (long long)height * width;
+    const long long step = std::max(1LL, c0 / 4096);
+    long long seen = 0, nz = 0;
+    for (long long k = 0; k < c0; k += step, seen++) nz += m0[k] != 0.0;
+    return seen ? (double)nz / (double)seen : 1.0;
+  };
+
   // ---- small calls (a single LP, a handful of models): latency-bound.  Stage through one mapped pinned buffer,
   // let the kernel read the tableaus and write the results zero-copy: launch + synchronise, no memcpy calls.
   {
@@ -1023,19 +1058,10 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     const size_t red_b = reduced_out ? 2 * pv_b : 0;  // doubles, packed like pos_out
     const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (matrices_out ? in_b : 0) + (red_b ? red_b + 16 : 0);
     const size_t desc_b = (ragged ? (size_t)n * 32 + 64 : 0) + (var_in ? pv_b + 16 : 0);
-    LaunchPlan plan;
-    // density of (a sample of) the first tableau: the latency-mode policy distinguishes dense from very sparse LPs
-    double small_density = -1.0;
-    if (ctx->coo_nnz < 0 && n > 0 && in_b + out_b + desc_b <= ((size_t)768 << 10)) {
-      const double *m0 = matrices + (ragged ? mat_offsets[0] : 0);
-      const long long c0 = ragged ? (long long)heights[0] * widths[0] : (long long)height * width;
-      const long long step = std::max(1LL, c0 / 4096);
-      long long seen = 0, nz = 0;
-      for (long long k = 0; k < c0; k += step, seen++) nz += m0[k] != 0.0;
-      small_density = seen ? (double)nz / (double)seen : 1.0;
-    }
-    if (!ctx->keep_final && ctx->coo_nnz < 0 && in_b + out_b + desc_b <= ((size_t)768 << 10) && ctx->tune_path != YALPS_PATH_GRID && ctx->tune_path != YALPS_PATH_CLUSTER && ctx->tune_path != YALPS_PATH_GRID_RESIDENT &&
-        plan_launch(ctx, n, Hcap, Wcap, opt->check_cycles != 0, &plan, small_density, true) == 0 && (plan.k || plan.tmem) && plan.resident) {
+    Route route;
+    if (!ctx->keep_final && ctx->coo_nnz < 0 && in_b + out_b + desc_b <= ((size_t)768 << 10) &&
+        choose_route(ctx, {n, Hcap, Wcap, first_density(), opt->check_cycles != 0, true}, &route) == 0 &&
+        (route.kind == ROUTE_K1T || (route.kind == ROUTE_SIMPLEX && route.resident))) {
       auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
       size_t o = 0;
       const size_t o_in = o; o += up16(in_b);
@@ -1097,7 +1123,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       }
       fill_options(a, opt);
       cudaStream_t st = ctx->streams[0];
-      if ((rc = launch_simplex(ctx, plan, a, "small", st))) return rc;
+      if ((rc = launch_route(ctx, route, a, "small", st))) return rc;
       CU(ctx, cudaStreamSynchronize(st));
       if (status) std::memcpy(status, h + o_st, (size_t)n * 4);
       if (value) std::memcpy(value, h + o_val, (size_t)n * 8);
@@ -1146,18 +1172,13 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
         cwcap = std::max(cwcap, widths[i]);
       }
     }
-    LaunchPlan plan;
     const bool from_cells = ctx->coo_nnz >= 0 && n == 1 && !ragged;
     if (from_cells) density = (double)ctx->coo_nnz / (double)((long long)height * width);
-    if (density < 0.0) {  // sample the first tableau once
-      const double *m0 = matrices + (ragged ? mat_offsets[0] : 0);
-      const long long c0 = ragged ? (long long)heights[0] * widths[0] : (long long)height * width;
-      const long long step = std::max(1LL, c0 / 4096);
-      long long seen = 0, nz = 0;
-      for (long long k = 0; k < c0; k += step, seen++) nz += m0[k] != 0.0;
-      density = seen ? (double)nz / (double)seen : 1.0;
-    }
-    if ((rc = plan_launch(ctx, cn, chcap, cwcap, opt->check_cycles != 0, &plan, density, true))) return rc;
+    if (density < 0.0) density = first_density();  // sampled once
+    // a uniform chunk is one launch, routed before its buffers are set up (the route decides where its final tableaus
+    // go); a ragged chunk is routed group by group below
+    Route route;
+    if (!ragged && (rc = choose_route(ctx, {cn, chcap, cwcap, density, opt->check_cycles != 0, true}, &route))) return rc;
 
     void *d_in, *d_status, *d_value, *d_piv, *d_rhs, *d_pos, *d_var;
     if ((rc = dev_ensure(ctx, "in" + s, ccells * 8, &d_in))) return rc;
@@ -1176,7 +1197,9 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     }
     void *d_out = nullptr;
     const bool want_mat = matrices_out != nullptr || (ctx->keep_final && n == 1 && !ragged);
-    if (want_mat && (plan.resident || ragged))
+    // K1t and K1/K1s write the final tableaus apart; the others leave them in the working copy d_in
+    const bool out_apart = ragged || (route.resident && route.kind != ROUTE_GRID);
+    if (want_mat && out_apart)
       if ((rc = dev_ensure(ctx, "matout" + s, ccells * 8, &d_out))) return rc;
 
     const double *src = matrices + (ragged ? mat_offsets[begin] : cells_upto(begin));
@@ -1229,7 +1252,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     a.Wcap = cwcap;
     a.in = (const double *)d_in;
     a.work = (double *)d_in;  // K2 works in place on the device copy
-    a.mat_out = want_mat ? (plan.resident ? (double *)d_out : (double *)d_in) : nullptr;
+    a.mat_out = want_mat ? (out_apart ? (double *)d_out : (double *)d_in) : nullptr;
     a.status = (int *)d_status;
     a.value = (double *)d_value;
     a.pivots = (long long *)d_piv;
@@ -1238,9 +1261,10 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     a.var_out = (int *)d_var;
     a.var_in = (const int *)d_vin;
     a.red_out = (double *)d_red;
+    std::vector<long long> lm, lr, lpv;  // chunk-local offsets of a ragged chunk
     if (ragged) {
       void *d_h, *d_w, *d_mo, *d_ro, *d_po;
-      std::vector<long long> lm(cn), lr(cn), lpv(cn);
+      lm.resize(cn), lr.resize(cn), lpv.resize(cn);
       for (int64_t i = 0; i < cn; i++) {
         lm[i] = moff[begin + i] - moff[begin];
         lr[i] = roff[begin + i] - roff[begin];
@@ -1256,7 +1280,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       CU(ctx, cudaMemcpyAsync(d_mo, lm.data(), (size_t)cn * 8, cudaMemcpyHostToDevice, st));
       CU(ctx, cudaMemcpyAsync(d_ro, lr.data(), (size_t)cn * 8, cudaMemcpyHostToDevice, st));
       CU(ctx, cudaMemcpyAsync(d_po, lpv.data(), (size_t)cn * 8, cudaMemcpyHostToDevice, st));
-      CU(ctx, cudaStreamSynchronize(st));  // the staging vectors die at the end of this scope
+      CU(ctx, cudaStreamSynchronize(st));  // the staging vectors die at the end of the chunk
       a.heights = (const int *)d_h;
       a.widths = (const int *)d_w;
       a.mat_off = (const long long *)d_mo;
@@ -1264,34 +1288,12 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       a.pos_off = (const long long *)d_po;
     }
     fill_options(a, opt);
-    int on_cluster = 0;
     if (!ragged) {
-      if ((on_cluster = maybe_cluster(ctx, cn, chcap, cwcap, nullptr, a, s, st)) < 0) return on_cluster;
-      if (!on_cluster && (on_cluster = maybe_cluster(ctx, cn, chcap, cwcap, &plan, a, s, st)) < 0) return on_cluster;
-    }
-    if (on_cluster) {
-      // launched: one LP per thread-block cluster
-    } else if (!ragged) {
-      if (use_grid_path(ctx, cn, plan)) {
-        for (int64_t i = 0; i < cn; i++) {
-          const long long mo = (long long)i * height * width;
-          if ((rc = launch_grid(ctx, height, width, (double *)d_in + mo, opt, (int *)d_status + i, (double *)d_value + i,
-                                (long long *)d_piv + 2 * i, (double *)d_rhs + (size_t)i * height,
-                                (int *)d_pos + (size_t)i * (width + height), (int *)d_var + (size_t)i * (width + height),
-                                st, d_vin ? (const int *)d_vin + (size_t)i * (width + height) : nullptr,
-                                d_vin ? width + height : 0, 0, "", nullptr,
-                                d_red ? (double *)d_red + (size_t)i * (width + height) : nullptr)))
-            return rc;
-        }
-        a.mat_out = want_mat ? (double *)d_in : nullptr;
-      } else if ((rc = launch_simplex(ctx, plan, a, s, st))) {
-        return rc;
-      }
+      if ((rc = launch_route(ctx, route, a, s, st))) return rc;
     } else {
       // Ragged chunk: LPs of very different sizes must not share one launch configuration (one large model would
       // push a thousand small ones onto the HBM-resident kernel).  Group by (fits in shared memory, CTA width) and
-      // launch each group with its own plan through an index indirection.
-      if (matrices_out) a.mat_out = (double *)d_out;
+      // route each group on its own through an index indirection.
       std::vector<std::vector<int>> groups;
       std::vector<std::pair<int, int>> caps;  // (Hcap, Wcap) per group
       std::unordered_map<int, int> group_of;
@@ -1315,45 +1317,24 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       if ((rc = dev_ensure(ctx, "rg_index" + s, flat.size() * 4, &d_index))) return rc;
       CU(ctx, cudaMemcpyAsync(d_index, flat.data(), flat.size() * 4, cudaMemcpyHostToDevice, st));
       CU(ctx, cudaStreamSynchronize(st));
+      BatchArgs h{};  // host-side copies of the shape, offset and index arrays (K4 reads them on the host)
+      h.heights = heights + begin;
+      h.widths = widths + begin;
+      h.mat_off = lm.data();
+      h.rhs_off = lr.data();
+      h.pos_off = lpv.data();
       size_t at = 0;
       for (size_t g = 0; g < groups.size(); g++) {
-        const long long gn = (long long)groups[g].size();
-        LaunchPlan gp;
-        if ((rc = plan_launch(ctx, gn, caps[g].first, caps[g].second, opt->check_cycles != 0, &gp,
-                              groups.size() == 1 ? density : -1.0, true)))
+        BatchArgs ga = a;
+        ga.n = (long long)groups[g].size();
+        ga.Hcap = caps[g].first;
+        ga.Wcap = caps[g].second;
+        ga.index = (const int *)d_index + at;
+        h.index = flat.data() + at;
+        if ((rc = choose_route(ctx, {ga.n, ga.Hcap, ga.Wcap, groups.size() == 1 ? density : -1.0, opt->check_cycles != 0, true},
+                               &route)))
           return rc;
-        BatchArgs ca = a;
-        ca.n = gn;
-        ca.Hcap = caps[g].first;
-        ca.Wcap = caps[g].second;
-        ca.index = (const int *)d_index + at;
-        int g_cluster = maybe_cluster(ctx, gn, caps[g].first, caps[g].second, nullptr, ca, s, st);
-        if (g_cluster == 0) g_cluster = maybe_cluster(ctx, gn, caps[g].first, caps[g].second, &gp, ca, s, st);
-        if (g_cluster < 0) return g_cluster;
-        if (g_cluster) {
-          // launched on the cluster path
-        } else if (use_grid_path(ctx, gn, gp)) {
-          for (int id : groups[g]) {
-            const int hi = heights[begin + id], wi = widths[begin + id];
-            const long long mo = moff[begin + id] - moff[begin], ro = roff[begin + id] - roff[begin],
-                            po = poff[begin + id] - poff[begin];
-            if ((rc = launch_grid(ctx, hi, wi, (double *)d_in + mo, opt, (int *)d_status + id, (double *)d_value + id,
-                                  (long long *)d_piv + 2 * id, (double *)d_rhs + ro, (int *)d_pos + po, (int *)d_var + po,
-                                  st, d_vin ? (const int *)d_vin + po : nullptr, d_vin ? wi + hi : 0, 0, "", nullptr,
-                                  d_red ? (double *)d_red + po : nullptr)))
-              return rc;
-            if (matrices_out)
-              CU(ctx, cudaMemcpyAsync((double *)d_out + mo, (double *)d_in + mo, (size_t)hi * wi * 8,
-                                      cudaMemcpyDeviceToDevice, st));
-          }
-        } else {
-          BatchArgs ga = a;
-          ga.n = gn;
-          ga.Hcap = caps[g].first;
-          ga.Wcap = caps[g].second;
-          ga.index = (const int *)d_index + at;
-          if ((rc = launch_simplex(ctx, gp, ga, s, st))) return rc;
-        }
+        if ((rc = launch_route(ctx, route, ga, s, st, &h))) return rc;
         at += groups[g].size();
       }
     }
@@ -1463,9 +1444,11 @@ static int replica_leader_trace(yalps_ctx *ctx, int H, int W, const double *base
   long long cap = (long long)std::min(2.0 * std::ceil(budget), 4096.0);
   cap = std::min<long long>(cap, (long long)(((size_t)512 << 20) / (cells * 8)) - 1);
   if (cap < 8) return 0;
-  LaunchPlan plan;
-  if (int rc = plan_launch(ctx, 1, H, W, false, &plan, -1.0, false)) return rc;
-  if (plan.tmem || !plan.k || plan.k->nwr < 2) return 0;  // only the row-split kernels record a trace
+  Route route;
+  RouteRequest q{1, H, W};
+  q.table_only = true;
+  if (int rc = choose_route(ctx, q, &route)) return rc;
+  if (route.kind != ROUTE_SIMPLEX || route.k->nwr < 2) return 0;  // only the row-split kernels record a trace
   size_t nz = 0;
   for (size_t i = 0; i < cells; i++) nz += base_host[i] != 0.0;
   tr->density = (double)nz / (double)cells;
@@ -1513,7 +1496,7 @@ static int replica_leader_trace(yalps_ctx *ctx, int H, int W, const double *base
   a.tr_var = tr->var;
   a.tr_hp = tr->Hp;
   a.tr_cap = tr->cap;
-  if ((rc = launch_simplex(ctx, plan, a, "rs_lead", st))) return rc;
+  if ((rc = launch_route(ctx, route, a, "rs_lead", st))) return rc;
   struct {
     int status, pad;
     double value;
@@ -1614,15 +1597,13 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
     CU(ctx, cudaGetLastError());
     ctx->launches++;
   }
-  LaunchPlan plan;
-  if ((rc = plan_launch(ctx, nf, H, W, false, &plan, tr.density, false))) return rc;
-  if (use_grid_path(ctx, nf, plan) || plan.tmem || !plan.k) {  // few large forks: one CTA per LP on the HBM-resident kernel
-    const int keep = ctx->tune_path;
-    ctx->tune_path = YALPS_PATH_GMEM;
-    rc = plan_launch(ctx, nf, H, W, false, &plan, tr.density, false);
-    ctx->tune_path = keep;
-    if (rc) return rc;
-  }
+  // one CTA per fork, also where K4 would take a batch of this size: a plan that K4 would replace is already the
+  // HBM-resident kernel
+  Route route;
+  RouteRequest q{nf, H, W, tr.density};
+  q.table_only = true;
+  if ((rc = choose_route(ctx, q, &route))) return rc;
+  if (route.kind != ROUTE_SIMPLEX) return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau width %d exceeds the widest kernel", W);
   BatchArgs a{};
   a.n = nf;
   a.mode = kModeBatch;
@@ -1640,7 +1621,7 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   a.red_out = c_red;
   a.resume = c_resume;
   fill_options(a, opt);
-  if ((rc = launch_simplex(ctx, plan, a, "rs_fork" + s, st))) return rc;
+  if ((rc = launch_route(ctx, route, a, "rs_fork" + s, st))) return rc;
   k_replica_scatter<<<(unsigned)std::min(nf, ctx->prop.multiProcessorCount * 8), 128, 0, st>>>(
       0, nf, H, W, d_fids, c_status, c_value, c_piv, c_rhs, c_pos, c_var, c_red, d_status, d_value, d_piv, d_rhs, d_pos,
       d_var, d_red);
