@@ -295,6 +295,7 @@ int yalps_solve_sparse(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nn
  *     d result / d x_j   =  sign * reduced_out[j]           (structural variable j)
  *     d result / d rhs_r = -sign * reduced_out[width + r]   (right-hand side of row r)
  * e.g. max 3x s.t. x <= 4 ends with row 0 = [-12, -3]: sign = 1, the shadow price of the row is 3.
+ * How far each of these values holds is what the *_ranging entry points below report ("sensitivity ranging").
  */
 /* yalps_solve_batch_basis + reduced_out (pos_in = var_in = NULL: yalps_solve_batch) */
 int yalps_solve_batch_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
@@ -321,6 +322,54 @@ int yalps_solve_batch_device_duals(yalps_ctx *ctx, int64_t n, int32_t height, in
 int yalps_solve_sparse_duals(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nnz, const int32_t *cell,
                              const double *val, const yalps_options *opt, int32_t *status, double *value, int64_t *pivots,
                              double *rhs_out, int32_t *pos_out, int32_t *var_out, double *reduced_out);
+
+/* ---- sensitivity ranging: how far the optimal basis holds ---------------------------------------------------
+ * A shadow price or reduced cost is valid while the optimal basis stays the same.  Ranging reports, per variable id
+ * (packed like pos_out, width + height doubles per LP), the interval [range_lo, range_hi] of shifts over which it does:
+ *   structural j (1 <= j < width):  shifts of the initial objective cell M0[0,j] (= sign * c_j) that keep the final
+ *                                   basis optimal;
+ *   slack of row k (id width + k):  shifts of row k's initial right-hand side that keep it primal feasible.
+ * With b+_r = max(M[r,0], +0), g_c = min(M[0,c], +0) and a cell counting when |cell| > opt->precision:
+ *   structural j non-basic at column c:  (-inf, -g_c)
+ *   structural j basic at row r:         (max g_c / M[r,c] over counting M[r,c] > 0, min over M[r,c] < 0), c >= 1
+ *   slack of row k:                      (max -b+_r / d[r] over counting d[r] > 0, min over d[r] < 0), r >= 1
+ * where d is dir(width + k), or dir(width + k) - dir(width + pairs[k]) when the row has a pair, and dir(u) is the final
+ * tableau's column pos[u] when u is non-basic, else the unit vector of u's basic row.  A pair is the other row of the
+ * same constraint (the lower row of a key whose upper row is k, or the other way round): its right-hand side moves by
+ * -t when row k's moves by +t, which is how a key with two finite bounds (a range or an equality) shifts as one;
+ * ranging its rows one by one would give the wrong interval.  pairs is packed like rhs_out: pairs[0] = -1, every
+ * other entry -1 (none) or a row 1..height-1 whose entry points back (YALPS_ERR_ARGUMENT otherwise).
+ * An empty max is -inf, an empty min +inf, zeros are +0.0 and lo <= 0 <= hi.  Ids 0 and width, and every id of an LP
+ * that is not optimal, are NaN.  Every value is one IEEE division followed by a max or min: bit-exact, whatever the
+ * kernel path.  e.g. max 3x s.t. x <= 4: the row ranges over [-4, inf), the objective cell of x over [-3, inf).
+ * k_ranging computes the ranges on the device from the final tableaus after the solve; the tableaus are copied to the
+ * host only when matrices_out is given, and the ranges cost 16*(width+height) bytes of device-to-host copy per LP.
+ *
+ * yalps_solve_{batch,ragged}_ranging: the *_duals sibling's arguments plus pairs (NULL: no pairs), range_lo and
+ * range_hi (both NULL: the *_duals call exactly; one without the other is YALPS_ERR_ARGUMENT).
+ */
+int yalps_solve_batch_ranging(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
+                              const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt, int32_t *status,
+                              double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                              double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                              double *range_hi);
+int yalps_solve_ragged_ranging(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
+                               const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                               const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                               double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                               double *range_hi);
+/* yalps_solve_sparse_duals + pairs, range_lo, range_hi */
+int yalps_solve_sparse_ranging(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nnz, const int32_t *cell,
+                               const double *val, const yalps_options *opt, int32_t *status, double *value,
+                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out, double *reduced_out,
+                               const int32_t *pairs, double *range_lo, double *range_hi);
+/* Ranges of n final tableaus already in device memory (e.g. d_matrices_out of yalps_solve_batch_device_duals), with
+ * their positionOfVariable d_pos and status d_status (NULL: every LP is optimal); d_pairs NULL: no pairs.  Every pointer
+ * is device memory; the kernel is enqueued on `stream`.  d_pairs is not validated here. */
+int yalps_ranging_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                         const int32_t *d_pos, const int32_t *d_status, const int32_t *d_pairs, double precision,
+                         double *d_range_lo, double *d_range_hi, void *stream);
 
 /* ---- one process, several GPUs (SURVEY 8b/8e) ------------------------------------------------------------
  * The reference is single-process and synchronous (src/YALPS.ts:73-92); a Node addon cannot use torchrun.  A
@@ -360,6 +409,18 @@ int yalps_multi_solve_replicas_duals(yalps_multi *m, int64_t n, int32_t height, 
                                      const double *rhs, const yalps_options *opt, int32_t *status, double *value,
                                      int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                                      double *reduced_out);
+/* the batch and ragged *_duals entries + pairs, range_lo, range_hi (see "sensitivity ranging"), sharded like rhs_out
+ * and pos_out */
+int yalps_multi_solve_batch_ranging(yalps_multi *m, int64_t n, int32_t height, int32_t width, const double *matrices,
+                                    const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt,
+                                    int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
+                                    int32_t *var_out, double *matrices_out, double *reduced_out, const int32_t *pairs,
+                                    double *range_lo, double *range_hi);
+int yalps_multi_solve_ragged_ranging(yalps_multi *m, int64_t n, const int32_t *heights, const int32_t *widths,
+                                     const int64_t *mat_offsets, const double *matrices, const yalps_options *opt,
+                                     int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
+                                     int32_t *var_out, double *matrices_out, double *reduced_out, const int32_t *pairs,
+                                     double *range_lo, double *range_hi);
 /*
  * incumbent_allreduce (SURVEY 8b, north_star): min-allreduce of one fp64 per rank -- the incumbent objective of a
  * branch-and-bound search, lower is better internally (src/branchAndCut.ts:124,130).  local[ndev] in, agreed[ndev]

@@ -33,6 +33,7 @@
 #include "cluster_kernel.cuh"
 #include "grid_kernel.cuh"
 #include "multigrid_kernel.cuh"
+#include "ranging_kernel.cuh"
 #include "tmem_launch.h"
 #include "bnb_launch.h"
 
@@ -778,6 +779,55 @@ int check_device_status(yalps_ctx *ctx, const int32_t *status, long long n) {
   return 0;
 }
 
+// k_ranging over the LPs of `a` (device pointers, shape or ragged fields and caps filled in by the caller).  Small
+// tableaus take warp mode (one launch), the others tile mode (two launches; the inverse of pos goes to per-slot scratch
+// of pv_total ints, the size of the pos layout the launch's offsets index into).
+int launch_ranging(yalps_ctx *ctx, RangingArgs a, size_t pv_total, const std::string &slot, cudaStream_t stream) {
+  if (a.n <= 0) return 0;
+  const long long sms = ctx->prop.multiProcessorCount;
+  if (a.Wcap <= 128 && a.Hcap <= 256) {
+    a.warp_smem = (((size_t)(a.Hcap + a.Wcap) * 4 + 15) & ~(size_t)15) + (size_t)16 * a.Hcap;
+    const long long blocks = std::min<long long>((a.n + kRngWarps - 1) / kRngWarps, sms * 64);
+    k_ranging<<<(unsigned)blocks, kRngWarps * 32, kRngWarps * a.warp_smem, stream>>>(a, kRngWarp);
+    CU(ctx, cudaGetLastError());
+    ctx->launches++;
+    return 0;
+  }
+  void *p;
+  if (int rc = dev_ensure(ctx, "rng_var" + slot, pv_total * 4, &p)) return rc;
+  a.var = (int *)p;
+  a.tiles_r = std::max(1, (a.Hcap - 1 + kRngTileRows - 1) / kRngTileRows);
+  a.tiles_c = (a.Wcap + kRngTileCols - 1) / kRngTileCols;
+  k_ranging<<<(unsigned)std::min<long long>(a.n, sms * 16), kRngTileCols, 0, stream>>>(a, kRngInit);
+  CU(ctx, cudaGetLastError());
+  const long long tiles = a.n * a.tiles_r * a.tiles_c;
+  k_ranging<<<(unsigned)std::min<long long>(tiles, sms * 64), kRngTileCols, 0, stream>>>(a, kRngTiles);
+  CU(ctx, cudaGetLastError());
+  ctx->launches += 2;
+  return 0;
+}
+
+// pairs (packed like rhs_out, one LP after another): pairs[0] = -1, every other entry -1 or another row 1..H-1 of the
+// same LP that points back
+int check_pairs(yalps_ctx *ctx, const int32_t *pairs, long long n, int32_t height, const int32_t *heights) {
+  if (!pairs) return 0;
+  long long ro = 0;
+  for (long long i = 0; i < n; i++) {
+    const int H = heights ? heights[i] : height;
+    const int32_t *pr = pairs + ro;
+    if (pr[0] != -1) return fail(ctx, YALPS_ERR_ARGUMENT, "LP %lld: pairs[0] must be -1 (row 0 is the objective)", i);
+    for (int r = 1; r < H; r++) {
+      const int q = pr[r];
+      if (q == -1) continue;
+      if (q < 1 || q >= H || q == r || pr[q] != r)
+        return fail(ctx, YALPS_ERR_ARGUMENT, "LP %lld: pairs[%d] = %d is not a symmetric pair of two rows 1..%d", i, r,
+                    q, H - 1);
+    }
+    ro += H;
+  }
+  return 0;
+}
+
 }  // namespace
 
 // =========================================================================================================
@@ -978,16 +1028,45 @@ int yalps_solve_batch_device_duals(yalps_ctx *ctx, int64_t n, int32_t height, in
                                  d_pos_out, d_var_out, d_matrices_out, stream, "dev", 0, d_reduced_out);
 }
 
+int yalps_ranging_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                         const int32_t *d_pos, const int32_t *d_status, const int32_t *d_pairs, double precision,
+                         double *d_range_lo, double *d_range_hi, void *stream) {
+  if (!ctx) return YALPS_ERR_ARGUMENT;
+  if (n < 0 || height < 1 || width < 1 || (n > 0 && (!d_matrices || !d_pos || !d_range_lo || !d_range_hi)))
+    return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", (long long)n, height, width);
+  if ((long long)height * width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
+  if (n == 0) return 0;
+  CU(ctx, cudaSetDevice(ctx->device));
+  RangingArgs a{};
+  a.n = n;
+  a.H = a.Hcap = height;
+  a.W = a.Wcap = width;
+  a.M = d_matrices;
+  a.pos = d_pos;
+  a.status = d_status;
+  a.pairs = d_pairs;
+  a.precision = precision;
+  a.lo = d_range_lo;
+  a.hi = d_range_hi;
+  return launch_ranging(ctx, a, (size_t)n * (width + height), "dev", (cudaStream_t)stream);
+}
+
 // Shared host-side pipeline for uniform and ragged batches.
 static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const int32_t *heights,
                       const int32_t *widths, const int64_t *mat_offsets, const double *matrices,
                       const yalps_options *opt, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
                       int32_t *pos_out, int32_t *var_out, double *matrices_out, const int32_t *pos_in = nullptr,
-                      const int32_t *var_in = nullptr, double *reduced_out = nullptr) {
+                      const int32_t *var_in = nullptr, double *reduced_out = nullptr, const int32_t *pairs = nullptr,
+                      double *range_lo = nullptr, double *range_hi = nullptr) {
   if (!ctx) return YALPS_ERR_ARGUMENT;
   if (n < 0 || !opt || (n > 0 && !matrices)) return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments");
   if ((pos_in == nullptr) != (var_in == nullptr))
     return fail(ctx, YALPS_ERR_ARGUMENT, "pos_in and var_in must be given together (or both null for the identity)");
+  if ((range_lo == nullptr) != (range_hi == nullptr))
+    return fail(ctx, YALPS_ERR_ARGUMENT, "range_lo and range_hi must be given together (or both null)");
+  // ranging: k_ranging runs over the final tableaus after the solve, which therefore stay in device memory
+  const bool want_rng = range_lo != nullptr;
+  if (!want_rng) pairs = nullptr;
   if (n == 0) return 0;
   CU(ctx, cudaSetDevice(ctx->device));
   const bool ragged = heights != nullptr;
@@ -1021,6 +1100,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     if (height < 1 || width < 1) return fail(ctx, YALPS_ERR_ARGUMENT, "bad shape %dx%d", height, width);
     if ((long long)height * width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
   }
+  if (int rc = check_pairs(ctx, pairs, n, height, heights)) return rc;
 
   auto cells_upto = [&](int64_t i) -> long long { return ragged ? moff[i] : (long long)i * height * width; };
   auto rows_upto = [&](int64_t i) -> long long { return ragged ? roff[i] : (long long)i * height; };
@@ -1056,8 +1136,11 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
   {
     const size_t in_b = (size_t)cells_upto(n) * 8, rows_b = (size_t)rows_upto(n) * 8, pv_b = (size_t)pv_upto(n) * 4;
     const size_t red_b = reduced_out ? 2 * pv_b : 0;  // doubles, packed like pos_out
-    const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (matrices_out ? in_b : 0) + (red_b ? red_b + 16 : 0);
-    const size_t desc_b = (ragged ? (size_t)n * 32 + 64 : 0) + (var_in ? pv_b + 16 : 0);
+    const size_t rng_b = want_rng ? 2 * pv_b : 0;     // range_lo, range_hi: doubles, packed like pos_out
+    const size_t pair_b = pairs ? rows_b / 2 : 0;      // int32, packed like rhs_out
+    const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (matrices_out ? in_b : 0) + (red_b ? red_b + 16 : 0) +
+                         (rng_b ? 2 * rng_b + 32 : 0);
+    const size_t desc_b = (ragged ? (size_t)n * 32 + 64 : 0) + (var_in ? pv_b + 16 : 0) + (pair_b ? pair_b + 16 : 0);
     Route route;
     if (!ctx->keep_final && ctx->coo_nnz < 0 && in_b + out_b + desc_b <= ((size_t)768 << 10) &&
         choose_route(ctx, {n, Hcap, Wcap, first_density(), opt->check_cycles != 0, true}, &route) == 0 &&
@@ -1079,11 +1162,18 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       const size_t o_var = o; o += up16(pv_b);
       const size_t o_mat = o; o += matrices_out ? up16(in_b) : 0;
       const size_t o_red = o; o += up16(red_b);
+      const size_t o_rlo = o; o += up16(rng_b);
+      const size_t o_rhi = o; o += up16(rng_b);
+      const size_t o_pair = o; o += up16(pair_b);
       void *hb, *db;
       int rc;
       if ((rc = pin_ensure(ctx, "small_io", o + 16, &hb))) return rc;
       if ((rc = pin_device_ptr(ctx, hb, &db))) return rc;
       char *h = (char *)hb, *d = (char *)db;
+      // ranging reads the final tableaus from device scratch, not over PCIe from the mapped buffer
+      void *d_fin = nullptr;
+      if (want_rng && (rc = dev_ensure(ctx, "small_final", in_b, &d_fin))) return rc;
+      if (pairs) std::memcpy(h + o_pair, pairs, pair_b);
       if (ragged) {
         for (int64_t i = 0; i < n; i++)
           std::memcpy(h + o_in + (size_t)moff[i] * 8, matrices + mat_offsets[i], (size_t)heights[i] * widths[i] * 8);
@@ -1105,7 +1195,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       a.Wcap = Wcap;
       a.in = (const double *)(d + o_in);
       a.work = nullptr;
-      a.mat_out = matrices_out ? (double *)(d + o_mat) : nullptr;
+      a.mat_out = want_rng ? (double *)d_fin : matrices_out ? (double *)(d + o_mat) : nullptr;
       a.status = (int *)(d + o_st);
       a.value = (double *)(d + o_val);
       a.pivots = (long long *)(d + o_piv);
@@ -1124,6 +1214,28 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       fill_options(a, opt);
       cudaStream_t st = ctx->streams[0];
       if ((rc = launch_route(ctx, route, a, "small", st))) return rc;
+      if (want_rng) {
+        RangingArgs g{};
+        g.n = n;
+        g.H = height;
+        g.W = width;
+        g.Hcap = Hcap;
+        g.Wcap = Wcap;
+        g.M = (const double *)d_fin;
+        g.heights = a.heights;
+        g.widths = a.widths;
+        g.mat_off = a.mat_off;
+        g.rhs_off = a.rhs_off;
+        g.pos_off = a.pos_off;
+        g.pos = a.pos_out;
+        g.status = a.status;
+        g.pairs = pairs ? (const int *)(d + o_pair) : nullptr;
+        g.precision = opt->precision;
+        g.lo = (double *)(d + o_rlo);
+        g.hi = (double *)(d + o_rhi);
+        if ((rc = launch_ranging(ctx, g, (size_t)pv_upto(n), "small", st))) return rc;
+        if (matrices_out) CU(ctx, cudaMemcpyAsync(h + o_mat, d_fin, in_b, cudaMemcpyDeviceToHost, st));
+      }
       CU(ctx, cudaStreamSynchronize(st));
       if (status) std::memcpy(status, h + o_st, (size_t)n * 4);
       if (value) std::memcpy(value, h + o_val, (size_t)n * 8);
@@ -1132,6 +1244,10 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       if (pos_out) std::memcpy(pos_out, h + o_pos, pv_b);
       if (var_out) std::memcpy(var_out, h + o_var, pv_b);
       if (reduced_out) std::memcpy(reduced_out, h + o_red, red_b);
+      if (want_rng) {
+        std::memcpy(range_lo, h + o_rlo, rng_b);
+        std::memcpy(range_hi, h + o_rhi, rng_b);
+      }
       if (matrices_out) {
         if (ragged)
           for (int64_t i = 0; i < n; i++)
@@ -1190,13 +1306,22 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     if ((rc = dev_ensure(ctx, "var" + s, cpv * 4, &d_var))) return rc;
     void *d_red = nullptr;
     if (reduced_out && (rc = dev_ensure(ctx, "red" + s, cpv * 8, &d_red))) return rc;
+    void *d_rlo = nullptr, *d_rhi = nullptr, *d_pairs = nullptr;
+    if (want_rng) {
+      if ((rc = dev_ensure(ctx, "rlo" + s, cpv * 8, &d_rlo))) return rc;
+      if ((rc = dev_ensure(ctx, "rhi" + s, cpv * 8, &d_rhi))) return rc;
+      if (pairs) {
+        if ((rc = dev_ensure(ctx, "pairs" + s, crows * 4, &d_pairs))) return rc;
+        CU(ctx, cudaMemcpyAsync(d_pairs, pairs + rows_upto(begin), crows * 4, cudaMemcpyHostToDevice, st));
+      }
+    }
     void *d_vin = nullptr;
     if (var_in) {
       if ((rc = dev_ensure(ctx, "varin" + s, cpv * 4, &d_vin))) return rc;
       CU(ctx, cudaMemcpyAsync(d_vin, var_in + pv_upto(begin), cpv * 4, cudaMemcpyHostToDevice, st));
     }
     void *d_out = nullptr;
-    const bool want_mat = matrices_out != nullptr || (ctx->keep_final && n == 1 && !ragged);
+    const bool want_mat = matrices_out != nullptr || want_rng || (ctx->keep_final && n == 1 && !ragged);
     // K1t and K1/K1s write the final tableaus apart; the others leave them in the working copy d_in
     const bool out_apart = ragged || (route.resident && route.kind != ROUTE_GRID);
     if (want_mat && out_apart)
@@ -1288,8 +1413,33 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       a.pos_off = (const long long *)d_po;
     }
     fill_options(a, opt);
+    // k_ranging over LPs of this chunk (all of them, or one ragged group through its index), after their route
+    auto ranging = [&](long long rn, int rh, int rw, const int *rindex) -> int {
+      if (!want_rng) return 0;
+      RangingArgs g{};
+      g.n = rn;
+      g.H = height;
+      g.W = width;
+      g.Hcap = rh;
+      g.Wcap = rw;
+      g.M = a.mat_out;
+      g.heights = a.heights;
+      g.widths = a.widths;
+      g.mat_off = a.mat_off;
+      g.rhs_off = a.rhs_off;
+      g.pos_off = a.pos_off;
+      g.index = rindex;
+      g.pos = a.pos_out;
+      g.status = a.status;
+      g.pairs = (const int *)d_pairs;
+      g.precision = opt->precision;
+      g.lo = (double *)d_rlo;
+      g.hi = (double *)d_rhi;
+      return launch_ranging(ctx, g, cpv, s, st);
+    };
     if (!ragged) {
       if ((rc = launch_route(ctx, route, a, s, st))) return rc;
+      if ((rc = ranging(cn, chcap, cwcap, nullptr))) return rc;
     } else {
       // Ragged chunk: LPs of very different sizes must not share one launch configuration (one large model would
       // push a thousand small ones onto the HBM-resident kernel).  Group by (fits in shared memory, CTA width) and
@@ -1335,6 +1485,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
                                &route)))
           return rc;
         if ((rc = launch_route(ctx, route, ga, s, st, &h))) return rc;
+        if ((rc = ranging(ga.n, ga.Hcap, ga.Wcap, ga.index))) return rc;
         at += groups[g].size();
       }
     }
@@ -1347,6 +1498,10 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     if (var_out) CU(ctx, cudaMemcpyAsync(var_out + pv_upto(begin), d_var, cpv * 4, cudaMemcpyDeviceToHost, st));
     if (reduced_out)
       CU(ctx, cudaMemcpyAsync(reduced_out + pv_upto(begin), d_red, cpv * 8, cudaMemcpyDeviceToHost, st));
+    if (want_rng) {
+      CU(ctx, cudaMemcpyAsync(range_lo + pv_upto(begin), d_rlo, cpv * 8, cudaMemcpyDeviceToHost, st));
+      CU(ctx, cudaMemcpyAsync(range_hi + pv_upto(begin), d_rhi, cpv * 8, cudaMemcpyDeviceToHost, st));
+    }
     if (ctx->keep_final && n == 1 && !ragged) ctx->kept_final = a.mat_out;
     if (matrices_out) {
       if (ragged) {
@@ -1417,6 +1572,26 @@ int yalps_solve_ragged_duals(yalps_ctx *ctx, int64_t n, const int32_t *heights, 
   if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
   return solve_host(ctx, n, 0, 0, heights, widths, mat_offsets, matrices, opt, status, value, pivots, rhs_out,
                     pos_out, var_out, matrices_out, pos_in, var_in, reduced_out);
+}
+
+int yalps_solve_batch_ranging(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
+                              const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt, int32_t *status,
+                              double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                              double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                              double *range_hi) {
+  return solve_host(ctx, n, height, width, nullptr, nullptr, nullptr, matrices, opt, status, value, pivots, rhs_out,
+                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out, pairs, range_lo, range_hi);
+}
+
+int yalps_solve_ragged_ranging(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
+                               const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                               const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                               double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                               double *range_hi) {
+  if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
+  return solve_host(ctx, n, 0, 0, heights, widths, mat_offsets, matrices, opt, status, value, pivots, rhs_out,
+                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out, pairs, range_lo, range_hi);
 }
 
 // ---- replica path sharing (aux_kernels.cuh: k_replica_follow) ------------------------------------------------------

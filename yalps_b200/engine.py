@@ -33,6 +33,19 @@ def _basis_in(pos_in, var_in, size: int) -> tuple:
     return p, v
 
 
+def _pairs_in(pairs, n: int, rows: int):
+    """pairs as int32 (n*rows for n uniform LPs of `rows` rows, or the packed rows of a ragged batch); a single LP's
+    (rows,) array applies to every LP of a uniform batch."""
+    if pairs is None:
+        return None
+    p = np.ascontiguousarray(pairs, np.int32).reshape(-1)
+    if p.size == rows and n > 1:
+        p = np.tile(p, n)
+    if p.size != n * rows:
+        raise ValueError("pairs needs one entry per tableau row (packed like rhs)")
+    return p
+
+
 def make_options(precision=1e-8, max_pivots=8192, check_cycles=False, tolerance=0.0, timeout_ms=math.inf,
                  max_iterations=32768) -> Options:
     o = Options()
@@ -131,13 +144,16 @@ class Engine:
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, want_basis: bool = True, out: Optional[dict] = None,
                     pos_in: Optional[np.ndarray] = None, var_in: Optional[np.ndarray] = None,
-                    want_duals: bool = False) -> dict:
+                    want_duals: bool = False, want_ranges: bool = False, pairs: Optional[np.ndarray] = None) -> dict:
         """n same-shape tableaus, `matrices` float64 of n*height*width values (not modified).
         `out` may be a dict from batch_outputs() to reuse (pinned) result buffers.
         pos_in / var_in (int32, n*(width+height)): the basis bookkeeping the tableaus arrive with (the node LPs of
         src/branchAndCut.ts:127); None = the identity of a fresh tableau (src/tableau.ts:95-98).
         want_duals: also out["reduced"] (n, width+height), row 0 of the final tableau per variable id
-        (yalps_solve_batch_duals; yalps_b200.sensitivity turns it into shadow prices and reduced costs)."""
+        (yalps_solve_batch_duals; yalps_b200.sensitivity turns it into shadow prices and reduced costs).
+        want_ranges: also out["range_lo"], out["range_hi"] (n, width+height), the sensitivity ranges computed on the
+        device from the final tableaus (yalps_solve_batch_ranging); `pairs` (int32 per row, -1 = none; one LP's
+        (height,) array or n*height values) pairs the two rows of a key (yalps_b200.sensitivity.row_pairs)."""
         opt = options or make_options()
         m = np.ascontiguousarray(matrices, dtype=np.float64).reshape(-1)
         cells = height * width
@@ -150,6 +166,18 @@ class Engine:
             raise ValueError("out was allocated for a different batch size")
         if want_duals and out.get("reduced") is None:
             out["reduced"] = np.empty((n, width + height), np.float64)
+        if want_ranges:
+            for k in ("range_lo", "range_hi"):
+                if out.get(k) is None:
+                    out[k] = np.empty((n, width + height), np.float64)
+            p, v = _basis_in(pos_in, var_in, n * (width + height))
+            pr = _pairs_in(pairs, n, height)
+            self._check(self._lib.yalps_solve_batch_ranging(
+                self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
+                _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
+                _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None, _ptr(pr), _ptr(out["range_lo"]),
+                _ptr(out["range_hi"])))
+            return out
         if want_duals:
             p, v = _basis_in(pos_in, var_in, n * (width + height))
             self._check(self._lib.yalps_solve_batch_duals(self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v),
@@ -225,9 +253,11 @@ class Engine:
         return int(self._lib.yalps_replica_forks(self._ctx))
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
-                     want_matrices: bool = False, want_duals: bool = False) -> list:
+                     want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,
+                     pairs: Optional[Sequence] = None) -> list:
         """LPs of different shapes in one call.  tableaus[i] is float64 of height_i*width_i values.
-        want_duals: every result also has "reduced" (width_i+height_i values, as solve_batch)."""
+        want_duals: every result also has "reduced" (width_i+height_i values, as solve_batch).
+        want_ranges: every result also has "range_lo", "range_hi" (as solve_batch); pairs[i] (height_i int32) or None."""
         opt = options or make_options()
         n = len(tableaus)
         if n == 0:
@@ -251,8 +281,16 @@ class Engine:
         pos = np.empty(int(poffs[-1]), np.int32)
         var = np.empty(int(poffs[-1]), np.int32)
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
-        if want_duals:
-            red = np.empty(int(poffs[-1]), np.float64)
+        red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
+        if want_ranges:
+            rlo, rhi = np.empty(int(poffs[-1]), np.float64), np.empty(int(poffs[-1]), np.float64)
+            pr = None if pairs is None else _pairs_in(np.concatenate([np.asarray(p, np.int32).reshape(-1) for p in pairs]),
+                                                      1, int(roffs[-1]))
+            self._check(self._lib.yalps_solve_ragged_ranging(
+                self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
+                _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
+                _ptr(rlo), _ptr(rhi)))
+        elif want_duals:
             self._check(self._lib.yalps_solve_ragged_duals(self._ctx, n, _ptr(heights), _ptr(widths),
                                                            _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
                                                            _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos),
@@ -270,6 +308,8 @@ class Engine:
             })
             if want_duals:
                 res[i]["reduced"] = red[poffs[i]:poffs[i + 1]]
+            if want_ranges:
+                res[i]["range_lo"], res[i]["range_hi"] = rlo[poffs[i]:poffs[i + 1]], rhi[poffs[i]:poffs[i + 1]]
         return res
 
     def solve_batch_device(self, n: int, height: int, width: int, d_matrices: int, options: Optional[Options] = None,
@@ -289,6 +329,16 @@ class Engine:
         self._check(self._lib.yalps_solve_batch_device(self._ctx, n, height, width, z(d_matrices), z(d_work),
                                                        C.byref(opt), z(d_status), z(d_value), z(d_pivots), z(d_rhs),
                                                        z(d_pos), z(d_var), z(d_matrices_out), z(stream)))
+
+    def ranging_device(self, n: int, height: int, width: int, d_matrices: int, d_pos: int, d_range_lo: int,
+                       d_range_hi: int, precision: float = 1e-8, d_status: int = 0, d_pairs: int = 0, stream: int = 0):
+        """Sensitivity ranges of n final tableaus already in device memory (yalps_ranging_device, raw pointers):
+        d_pos int32 n*(width+height), d_status int32 n (0: all optimal), d_pairs int32 n*height (0: none); writes
+        float64 n*(width+height) to d_range_lo / d_range_hi.  Enqueues on `stream` and returns."""
+        z = lambda p: C.c_void_p(p) if p else None
+        self._check(self._lib.yalps_ranging_device(self._ctx, n, height, width, z(d_matrices), z(d_pos), z(d_status),
+                                                   z(d_pairs), float(precision), z(d_range_lo), z(d_range_hi),
+                                                   z(stream)))
 
     def generate_synthetic_device(self, first: int, n: int, m: int, nvars: int, d_out: int, neg_rows: int = 0,
                                   salt: int = 0x5BD1E995, stream: int = 0):
@@ -350,9 +400,11 @@ class Engine:
         return self.solve_tableau(values, height, width, integers, sign, options, cells=cells)
 
     def solve_lp_sparse(self, cells: np.ndarray, values: np.ndarray, height: int, width: int,
-                        options: Optional[Options] = None) -> dict:
+                        options: Optional[Options] = None, want_ranges: bool = False,
+                        pairs: Optional[np.ndarray] = None) -> dict:
         """One LP given as ordered (cell, value) stores into a zero matrix (yalps_solve_sparse_duals): status, value,
-        pivots, rhs, pos, var and reduced, as solve_batch with n = 1 and want_duals."""
+        pivots, rhs, pos, var and reduced, as solve_batch with n = 1 and want_duals; want_ranges adds range_lo and
+        range_hi (yalps_solve_sparse_ranging, `pairs` as solve_batch)."""
         opt = options or make_options()
         cells = np.ascontiguousarray(cells, np.int32).reshape(-1)
         values = np.ascontiguousarray(values, np.float64).reshape(-1)
@@ -362,6 +414,16 @@ class Engine:
         piv = np.zeros(2, np.int64)
         rhs, pos, var = np.empty(height), np.empty(width + height, np.int32), np.empty(width + height, np.int32)
         red = np.empty(width + height, np.float64)
+        if want_ranges:
+            rlo, rhi = np.empty(width + height, np.float64), np.empty(width + height, np.float64)
+            self._check(self._lib.yalps_solve_sparse_ranging(self._ctx, height, width, int(cells.size),
+                                                             _ptr(cells) if cells.size else None,
+                                                             _ptr(values) if values.size else None, C.byref(opt),
+                                                             C.byref(status), C.byref(value), _ptr(piv), _ptr(rhs),
+                                                             _ptr(pos), _ptr(var), _ptr(red), _ptr(_pairs_in(pairs, 1, height)),
+                                                             _ptr(rlo), _ptr(rhi)))
+            return {"status": status.value, "value": value.value, "pivots": (int(piv[0]), int(piv[1])), "rhs": rhs,
+                    "pos": pos, "var": var, "reduced": red, "range_lo": rlo, "range_hi": rhi}
         self._check(self._lib.yalps_solve_sparse_duals(self._ctx, height, width, int(cells.size),
                                                        _ptr(cells) if cells.size else None,
                                                        _ptr(values) if values.size else None, C.byref(opt),
@@ -528,13 +590,25 @@ class MultiEngine:
 
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, pos_in=None, var_in=None, out: Optional[dict] = None,
-                    want_duals: bool = False) -> dict:
+                    want_duals: bool = False, want_ranges: bool = False, pairs=None) -> dict:
         opt = options or make_options()
         m = np.ascontiguousarray(matrices, np.float64).reshape(-1)
         n = m.size // (height * width)
         out = out or self._outputs(n, height, width, want_matrices, want_duals)
         p = None if pos_in is None else np.ascontiguousarray(pos_in, np.int32).reshape(-1)
         v = None if var_in is None else np.ascontiguousarray(var_in, np.int32).reshape(-1)
+        if want_ranges:
+            for k in ("range_lo", "range_hi"):
+                if out.get(k) is None:
+                    out[k] = np.empty((n, width + height), np.float64)
+            if want_duals and out.get("reduced") is None:
+                out["reduced"] = np.empty((n, width + height), np.float64)
+            self._check(self._lib.yalps_multi_solve_batch_ranging(
+                self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
+                _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
+                _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None, _ptr(_pairs_in(pairs, n, height)),
+                _ptr(out["range_lo"]), _ptr(out["range_hi"])))
+            return out
         if want_duals:
             if out.get("reduced") is None:
                 out["reduced"] = np.empty((n, width + height), np.float64)
@@ -569,7 +643,8 @@ class MultiEngine:
         return out
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
-                     want_matrices: bool = False, want_duals: bool = False) -> list:
+                     want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,
+                     pairs: Optional[Sequence] = None) -> list:
         opt = options or make_options()
         n = len(tableaus)
         if n == 0:
@@ -586,8 +661,16 @@ class MultiEngine:
         status, value, pivots = np.empty(n, np.int32), np.empty(n, np.float64), np.empty((n, 2), np.int64)
         rhs, pos, var = np.empty(int(roffs[-1])), np.empty(int(poffs[-1]), np.int32), np.empty(int(poffs[-1]), np.int32)
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
-        if want_duals:
-            red = np.empty(int(poffs[-1]), np.float64)
+        red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
+        if want_ranges:
+            rlo, rhi = np.empty(int(poffs[-1]), np.float64), np.empty(int(poffs[-1]), np.float64)
+            pr = None if pairs is None else _pairs_in(np.concatenate([np.asarray(p, np.int32).reshape(-1) for p in pairs]),
+                                                      1, int(roffs[-1]))
+            self._check(self._lib.yalps_multi_solve_ragged_ranging(
+                self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
+                _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
+                _ptr(rlo), _ptr(rhi)))
+        elif want_duals:
             self._check(self._lib.yalps_multi_solve_ragged_duals(
                 self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
                 _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red)))
@@ -601,6 +684,9 @@ class MultiEngine:
         if want_duals:
             for i in range(n):
                 res[i]["reduced"] = red[poffs[i]:poffs[i + 1]]
+        if want_ranges:
+            for i in range(n):
+                res[i]["range_lo"], res[i]["range_hi"] = rlo[poffs[i]:poffs[i + 1]], rhi[poffs[i]:poffs[i + 1]]
         return res
 
     def solve_large(self, matrix: np.ndarray, height: int, width: int, options: Optional[Options] = None,

@@ -13,10 +13,27 @@ A constraint key owns at most two rows (tableau.constraint_rows): an upper row `
 `-a.x <= -min`.  Shifting every finite bound of the key by t moves rhs(upper) by +t and rhs(lower) by -t, so the key's
 shadow price is y(upper) - y(lower): d result / d max for a lessEq, d / d min for a greaterEq, d / d value for an
 equalTo (one of its two slacks is basic, so the sum is valid in both directions).
+
+Ranging (how far the optimal basis holds) is one interval [lo, hi] per variable id, packed like `reduced`, with
+b+_r = max(M[r,0], +0.0), g_c = min(M[0,c], +0.0), and a cell counting when |cell| > precision (ranges_from_tableau):
+
+    structural j, non-basic at column c:  (-inf, -g_c)
+    structural j, basic at row r:         (max g_c / M[r,c] over counting M[r,c] > 0, min over M[r,c] < 0), c = 1..W-1
+    slack of row k:                       (max -b+_r / d[r] over counting d[r] > 0, min over d[r] < 0), r = 1..H-1
+
+where [lo, hi] bounds the shift of the initial objective cell M0[0,j] = sign * c_j (structural) or of row k's initial
+RHS (slack) that keeps the final basis optimal, resp. primal feasible.  d is the column of the final tableau that
+shifting row k's RHS moves column 0 along (-d per unit), dir(W+k): the non-basic column M[:, pos], or the unit vector
+of the basic row.  With a pair (the other row of the same constraint key, whose RHS moves by -t when row k's moves by
++t) d = dir(W+k) - dir(W+pair): a key with two finite bounds must be ranged as one, its two slacks always sum to a
+constant.  An empty max is -inf, an empty min +inf, a zero is +0.0, and lo <= 0 <= hi.  Ids 0 and W and every id of a
+non-optimal LP are NaN.
 """
 from __future__ import annotations
 
 import numpy as np
+
+_CHUNK = 256  # slack ids per vectorised step of ranges_from_tableau (bounds its H x _CHUNK temporaries)
 
 
 def reduced_from_tableau(matrix: np.ndarray, width: int, height: int, pos: np.ndarray) -> np.ndarray:
@@ -54,3 +71,103 @@ def model_sensitivity(variables: list, rows: list, reduced: np.ndarray, width: i
             v = v - float(y[lo])
         shadow.append([key, v])
     return reduced_costs, shadow
+
+
+def _z(x):
+    """+0.0 for either zero (x + 0.0 rounds -0.0 to +0.0 and leaves everything else as it is)."""
+    return x + 0.0
+
+
+def ranges_from_tableau(matrix: np.ndarray, width: int, height: int, pos: np.ndarray, precision: float,
+                        pairs: np.ndarray = None, optimal: bool = True) -> tuple:
+    """What the kernels write into `range_lo` / `range_hi` (one value per variable id, packed like `reduced`),
+    computed from a final tableau, its positionOfVariable and the row pairs (int per row, -1 = none; row_pairs).
+    Reference definition: every value is one IEEE division followed by a max or min (module docstring)."""
+    W, H = int(width), int(height)
+    lo = np.full(W + H, -np.inf)
+    hi = np.full(W + H, np.inf)
+    if not optimal:
+        lo[:] = hi[:] = np.nan
+        return lo, hi
+    M = np.asarray(matrix, np.float64).reshape(-1)[:H * W].reshape(H, W)
+    p = np.asarray(pos, np.int64).reshape(-1)[:W + H]
+    prec = float(precision)
+    g = np.minimum(M[0], 0.0)
+    bplus = np.maximum(M[:, 0], 0.0)
+    nonbasic = (p >= 1) & (p < W)
+    rows = np.arange(H)
+    with np.errstate(divide="ignore", invalid="ignore", over="ignore"):
+        # structural variables
+        js = np.arange(1, W)
+        nb = nonbasic[js]
+        hi[js[nb]] = -g[p[js[nb]]]
+        bj = js[~nb]
+        r = p[bj] - W
+        ok = (r >= 1) & (r < H)
+        bj, r = bj[ok], r[ok]
+        if bj.size:
+            A = M[r][:, 1:]
+            Q = g[None, 1:] / A
+            cnt = np.abs(A) > prec
+            lo[bj] = np.where(cnt & (A > 0), Q, -np.inf).max(axis=1)
+            hi[bj] = np.where(cnt & (A < 0), Q, np.inf).min(axis=1)
+
+        # slacks: d = dir(W+k) [- dir(W+pair)]
+        def direction(ids):
+            q = p[ids]
+            nbq = (q >= 1) & (q < W)
+            D = M[:, np.where(nbq, q, 0)]
+            return np.where(nbq[None, :], D, (rows[:, None] == (q - W)[None, :]).astype(np.float64))
+
+        pr = None if pairs is None else np.asarray(pairs, np.int64).reshape(-1)[:H]
+        for k0 in range(1, H, _CHUNK):
+            ks = np.arange(k0, min(H, k0 + _CHUNK))
+            d = direction(W + ks)
+            if pr is not None:
+                has = pr[ks] >= 0
+                if has.any():
+                    dq = direction(W + np.where(has, pr[ks], ks))
+                    d = np.where(has[None, :], d - dq, d)
+            d = d[1:]
+            Q = -bplus[1:, None] / d
+            cnt = np.abs(d) > prec
+            lo[W + ks] = np.where(cnt & (d > 0), Q, -np.inf).max(axis=0)
+            hi[W + ks] = np.where(cnt & (d < 0), Q, np.inf).min(axis=0)
+    lo, hi = _z(lo), _z(hi)
+    lo[[0, W]] = np.nan
+    hi[[0, W]] = np.nan
+    return lo, hi
+
+
+def row_pairs(rows: list, height: int) -> np.ndarray:
+    """pairs for ranges_from_tableau / the `_ranging` entries: upper <-> lower row of every key that has both, from
+    the (key, upper row | -1, lower row | -1) list of tableau.constraint_rows; -1 elsewhere (int32, one per row)."""
+    out = np.full(int(height), -1, np.int32)
+    for _, up, lo in rows:
+        if up >= 0 and lo >= 0:
+            out[up], out[lo] = lo, up
+    return out
+
+
+def model_ranges(variables: list, rows: list, range_lo: np.ndarray, range_hi: np.ndarray, width: int,
+                 sign: float) -> tuple:
+    """Model level: (costRanges, rhsRanges) of one optimal LP from ranges computed with row_pairs(rows).
+    costRanges [[variable, lo, hi]]: allowable shifts of the variable's objective coefficient.  rhsRanges
+    [[key, lo, hi]]: allowable shift of all the key's finite bounds together (the shift its shadow price is the
+    derivative for): the upper row's range, else the lower row's negated and swapped (its RHS is -min)."""
+    lo = np.asarray(range_lo, np.float64).reshape(-1)
+    hi = np.asarray(range_hi, np.float64).reshape(-1)
+    W = int(width)
+    cost = []
+    for j, (key, _) in enumerate(variables):
+        a, b = float(lo[j + 1]), float(hi[j + 1])
+        cost.append([key, _z(a), _z(b)] if sign > 0 else [key, _z(-b), _z(-a)])
+    rhs = []
+    for key, up, lw in rows:
+        if up >= 0:
+            rhs.append([key, _z(float(lo[W + up])), _z(float(hi[W + up]))])
+        elif lw >= 0:
+            rhs.append([key, _z(-float(hi[W + lw])), _z(-float(lo[W + lw]))])
+        else:
+            rhs.append([key, -np.inf, np.inf])
+    return cost, rhs

@@ -10,6 +10,10 @@ One option goes beyond the reference: `sensitivity` (default False).  When it is
 Solution also has "reducedCosts" ([[variable, d result / d variable], ...], model order) and "shadowPrices"
 ([[constraint key, d result / d bound], ...], first-seen order): raw doubles for an optimal LP, empty lists
 otherwise (yalps_b200.sensitivity has the conventions).
+A second one, `ranging` (default False), implies `sensitivity` and adds "costRanges" ([[variable, lo, hi], ...]: the
+allowable shifts of the variable's objective coefficient that keep the optimal basis) and "rhsRanges" ([[constraint
+key, lo, hi], ...]: the allowable shifts of all of the key's finite bounds together over which its shadow price holds),
+computed on the GPU from the final tableau; empty lists unless optimal.
 The tableau is built on the host (tableau.py), the simplex and branch-and-cut numerics run on the GPU
 through the C ABI; there is no CPU solve path.
 """
@@ -21,7 +25,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
-from .sensitivity import model_sensitivity
+from .sensitivity import model_ranges, model_sensitivity, row_pairs
 from .tableau import SPARSE_OVER_BYTES, TableauModel, constraint_rows, entries, tableau_model
 
 # src/YALPS.ts:52-60
@@ -97,13 +101,23 @@ def _check_lp(tabmod: TableauModel):
         raise ValueError("sensitivity: duals are defined for LP models only (this model has integer or binary variables)")
 
 
-def _with_sensitivity(sol: dict, tabmod: TableauModel, model: dict, reduced) -> dict:
-    """Solution + reducedCosts / shadowPrices (empty unless optimal)."""
+def _rows(model: dict) -> list:
+    return constraint_rows(list(entries(model["constraints"])))
+
+
+def _with_sensitivity(sol: dict, tabmod: TableauModel, model: dict, reduced, ranges: Optional[tuple] = None) -> dict:
+    """Solution + reducedCosts / shadowPrices, and costRanges / rhsRanges when `ranges` = (range_lo, range_hi) is
+    given (all empty unless optimal)."""
     if sol["status"] != "optimal":
-        return {**sol, "reducedCosts": [], "shadowPrices": []}
-    rows = constraint_rows(list(entries(model["constraints"])))
+        out = {**sol, "reducedCosts": [], "shadowPrices": []}
+        return out if ranges is None else {**out, "costRanges": [], "rhsRanges": []}
+    rows = _rows(model)
     rc, sp = model_sensitivity(tabmod.variables, rows, reduced, tabmod.tableau.width, tabmod.sign)
-    return {**sol, "reducedCosts": rc, "shadowPrices": sp}
+    out = {**sol, "reducedCosts": rc, "shadowPrices": sp}
+    if ranges is None:
+        return out
+    cr, rr = model_ranges(tabmod.variables, rows, ranges[0], ranges[1], tabmod.tableau.width, tabmod.sign)
+    return {**out, "costRanges": cr, "rhsRanges": rr}
 
 
 def solve(model: dict, options: Optional[dict] = None, *, engine: Optional[Engine] = None,
@@ -115,26 +129,32 @@ def solve(model: dict, options: Optional[dict] = None, *, engine: Optional[Engin
     sparse_ok = hasattr(engine, "solve_tableau_sparse") if engine is not None else True
     tabmod = tableau_model(model, SPARSE_OVER_BYTES if sparse_ok else None)
     t = tabmod.tableau
-    if opt.get("sensitivity"):
+    rng = bool(opt.get("ranging"))
+    if opt.get("sensitivity") or rng:
         _check_lp(tabmod)
     eng = engine or get_engine()
-    if opt.get("sensitivity"):
-        # the root LP is the whole solve: one LP with its reduced-cost row (dense batch of one, or the cell pairs)
+    if opt.get("sensitivity") or rng:
+        # the root LP is the whole solve: one LP with its reduced-cost row (dense batch of one, or the cell pairs), and
+        # its ranges when asked for
+        pairs = row_pairs(_rows(model), t.height) if rng else None
         if t.matrix is None:
-            r = eng.solve_lp_sparse(t.cells, t.values, t.height, t.width, _c_options(opt))
+            r = eng.solve_lp_sparse(t.cells, t.values, t.height, t.width, _c_options(opt), want_ranges=rng, pairs=pairs)
             status, value, rhs, pos, var, red = (r["status"], r["value"], r["rhs"], r["pos"], r["var"], r["reduced"])
             piv = r["pivots"]
+            ranges = (r["range_lo"], r["range_hi"]) if rng else None
         else:
-            r = eng.solve_batch(t.matrix, t.height, t.width, _c_options(opt), want_duals=True)
+            r = eng.solve_batch(t.matrix, t.height, t.width, _c_options(opt), want_duals=True, want_ranges=rng,
+                                pairs=pairs)
             status, value = int(r["status"][0]), float(r["value"][0])
             rhs, pos, var, red = r["rhs"][0], r["pos"][0], r["var"][0], r["reduced"][0]
             piv = (int(r["pivots"][0, 0]), int(r["pivots"][0, 1]))
+            ranges = (r["range_lo"][0], r["range_hi"][0]) if rng else None
         if info is not None:
             info.update(nodes=0, node_pivots=0, max_cuts=0, max_heap=0, waves=0, device_nodes=0, wave_us=0, bnb_us=0,
                         root_status=STATUS_NAMES[status], root_value=value, root_pivots=piv, height=t.height,
                         width=t.width, final_rhs=rhs, final_pos=pos, final_var=var)
         sol = _solution(tabmod, STATUS_NAMES[status], value, rhs, pos, var, opt)
-        return _with_sensitivity(sol, tabmod, model, red)
+        return _with_sensitivity(sol, tabmod, model, red, ranges)
     if t.matrix is None:
         r = eng.solve_tableau_sparse(t.cells, t.values, t.height, t.width, tabmod.integers, tabmod.sign, _c_options(opt))
     else:
@@ -169,17 +189,21 @@ def solve_many(models: Sequence[dict], options: Optional[dict] = None, *, engine
     opt = {**_DEFAULTS, **(options or {})}
     copt = _c_options(opt)
     tabmods = [tableau_model(m) for m in models]
-    if opt.get("sensitivity"):
+    rng = bool(opt.get("ranging"))
+    if opt.get("sensitivity") or rng:
         for tm in tabmods:
             _check_lp(tm)
     eng = engine or get_engine()
     if not tabmods:
         return []
-    if opt.get("sensitivity"):  # LP models only: the ragged root batch is the whole solve (one GPU or sharded)
+    if opt.get("sensitivity") or rng:  # LP models only: the ragged root batch is the whole solve (one GPU or sharded)
+        pairs = [row_pairs(_rows(m), tm.tableau.height) for tm, m in zip(tabmods, models)] if rng else None
         roots = eng.solve_ragged([tm.tableau.matrix for tm in tabmods],
-                                 [(tm.tableau.height, tm.tableau.width) for tm in tabmods], copt, want_duals=True)
+                                 [(tm.tableau.height, tm.tableau.width) for tm in tabmods], copt, want_duals=True,
+                                 want_ranges=rng, pairs=pairs)
         return [_with_sensitivity(_solution(tm, STATUS_NAMES[r["status"]], r["value"], r["rhs"], r["pos"], r["var"], opt),
-                                  tm, m, r["reduced"]) for tm, m, r in zip(tabmods, models, roots)]
+                                  tm, m, r["reduced"], (r["range_lo"], r["range_hi"]) if rng else None)
+                for tm, m, r in zip(tabmods, models, roots)]
     if isinstance(eng, MultiEngine):  # one C-ABI call: roots sharded over the GPUs, searches dealt to worker contexts
         res = eng.solve_many_tableaus(tabmods, copt, searches_per_device=milp_workers)
         return [_solution(tm, STATUS_NAMES[r["status"]], r["result"], r["rhs"], r["pos"], r["var"], opt)
