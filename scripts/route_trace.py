@@ -40,6 +40,46 @@ def tableaus(n, H, W, sparse, seed):
     return np.ascontiguousarray(m)
 
 
+def random_pairs(n, H, seed):
+    """Row pairs of n LPs of H rows (sensitivity ranging): random disjoint pairs of rows 1..H-1, -1 elsewhere."""
+    rng = np.random.default_rng(seed)
+    out = np.full((n, H), -1, np.int32)
+    for i in range(n):
+        rows = rng.permutation(np.arange(1, H))
+        for j in range(0, len(rows) - 1, 2):
+            if rng.random() < 0.5:
+                out[i, rows[j]], out[i, rows[j + 1]] = rows[j + 1], rows[j]
+    return out
+
+
+def duplicated_stores(cells, values):
+    """The stores with every tenth one preceded by a store of another value to the same cell (the last store wins)."""
+    dc, dv = [], []
+    for k, (c, v) in enumerate(zip(cells.tolist(), values.tolist())):
+        if k % 10 == 0:
+            dc.append(c)
+            dv.append(v + 1.5)
+        dc.append(c)
+        dv.append(v)
+    return np.asarray(dc, np.int32), np.asarray(dv, np.float64)
+
+
+def tableau_outputs(r):
+    """solve_tableau's result without its timings"""
+    return {k: np.asarray(v) for k, v in r.items() if k != "stats"} | {
+        "nodes": np.array([r["stats"]["nodes"], r["stats"]["node_pivots"], r["stats"]["max_cuts"]])}
+
+
+def node_outputs(r, nodes, H, W):
+    """bnb_solve_nodes' result without the rows past each node's own height, which it leaves as they were"""
+    out = {k: r[k] for k in ("status", "value", "pivots")}
+    for j, cuts in enumerate(nodes):
+        h = H + len(cuts)
+        out |= {f"{j}:rhs": r["rhs"][j, :h], f"{j}:pos": r["pos"][j, :W + h], f"{j}:var": r["var"][j, :W + h],
+                f"{j}:matrix": r["matrices"][j, :h * W]}
+    return out
+
+
 def digest(outs):
     h = hashlib.sha256()
     for k in sorted(outs):
@@ -87,9 +127,9 @@ def main():
     seen_library_kernel = False
     out = open(args.out, "w")
 
-    def emit(case, fn):
+    def emit(case, fn, who=None):
         nonlocal seen_library_kernel
-        k, c, dc, err, hsh = trace(eng, fn)
+        k, c, dc, err, hsh = trace(who or eng, fn)
         seen_library_kernel |= any("k_simplex" in x[0] for x in k)
         out.write(json.dumps({**case, "kernels": k, "copies": c, "launches": dc, "error": err, "hash": hsh}) + "\n")
         out.flush()
@@ -142,6 +182,52 @@ def main():
                              | {"forks": np.array([eng.replica_forks])})
                     eng.set_replica_sharing(True)
                 del d_in
+    eng.set_tuning(E.PATH_AUTO, 0)
+    # ranges with paired rows, one engine and two ranks on one GPU; the zero-copy small call and the chunk pipeline
+    multi = yalps_b200.MultiEngine([0, 0])
+    for (H, W) in [(9, 17), (33, 65), (120, 200)]:
+        for n in (1, 17, 2 * sms + 1):
+            m = tableaus(n, H, W, True, seed=H + n)
+            pairs = random_pairs(n, H, seed=n)
+            rag_shapes = [[(H, W), (9, 17)][i % 2] for i in range(n)]
+            rag = [tableaus(1, h, w, True, seed=i)[0].reshape(-1) for i, (h, w) in enumerate(rag_shapes)]
+            rag_pairs = [random_pairs(1, h, seed=i)[0] for i, (h, _) in enumerate(rag_shapes)]
+            rhs = m[:, :, 0].copy()
+            case = {"shape": [H, W], "n": n}
+            for who, x in (("engine", eng), ("multi", multi)):
+                emit({"entry": "batch_ranges", "on": who, **case}, lambda: x.solve_batch(
+                    m, H, W, want_matrices=True, want_duals=True, want_ranges=True, pairs=pairs), x)
+                emit({"entry": "ragged_ranges", "on": who, **case}, lambda: {
+                    f"{i}:{k}": np.asarray(v) for i, r in enumerate(x.solve_ragged(
+                        rag, rag_shapes, want_matrices=True, want_duals=True, want_ranges=True, pairs=rag_pairs))
+                    for k, v in r.items() if v is not None}, x)
+            emit({"entry": "replicas", "on": "multi", **case},
+                 lambda: multi.solve_replicas(m[0], rhs, H, W, want_duals=True), multi)
+    multi.close()
+    # tableaus given as (cell, value) stores, below and above the 768 KB zero-copy limit, with and without duplicate
+    # cells; a MILP whose root (above 256 KB) stays on the device for branch and cut
+    cases = {c["name"]: c for c in load_cases()}
+    for name in ["Monster Problem", "Monster 2"]:
+        tm = yalps_b200.tableau_model(cases[name]["model"], 0)
+        t = tm.tableau
+        stores = {"plain": (t.cells, t.values), "duplicates": duplicated_stores(t.cells, t.values)}
+        dense = np.zeros(t.height * t.width)
+        for c, v in zip(t.cells.tolist(), t.values.tolist()):
+            dense[c] = v
+        emit({"entry": "tableau", "model": name}, lambda: tableau_outputs(
+            eng.solve_tableau(dense, t.height, t.width, tm.integers, tm.sign)))
+        for kind, (c, v) in stores.items():
+            for limit in ("below", "above") if not tm.integers else ("above",):
+                h, w = (t.height, t.width) if limit == "above" else (t.height // 4, t.width // 4)  # a corner
+                keep = ((c // t.width) < h) & ((c % t.width) < w)
+                cs, vs = ((c // t.width) * w + c % t.width)[keep].astype(np.int32), v[keep]
+                case = {"model": name, "stores": kind, "limit": limit}
+                emit({"entry": "tableau_sparse", **case}, lambda: tableau_outputs(
+                    eng.solve_tableau_sparse(cs, vs, h, w, tm.integers, tm.sign)))
+                if not tm.integers:
+                    emit({"entry": "lp_sparse", **case}, lambda: eng.solve_lp_sparse(
+                        cs, vs, h, w, want_ranges=True, pairs=random_pairs(1, h, seed=h)[0]))
+                    emit({"entry": "lp_sparse", "ranges": False, **case}, lambda: eng.solve_lp_sparse(cs, vs, h, w))
     # node waves: synthetic roots (solved by the oracle) and the big sparse Monster 2 root
     roots = []
     for (H, W) in shapes[:8]:
@@ -163,7 +249,7 @@ def main():
             for pname in paths:
                 eng.set_tuning(PATHS[pname], 0)
                 emit({"entry": "nodes", "root": name, "n": n, "path": pname},
-                     lambda: {k: v for k, v in eng.bnb_solve_nodes(nodes, want_matrices=True).items() if k != "stride_h"})
+                     lambda: node_outputs(eng.bnb_solve_nodes(nodes, want_matrices=True), nodes, H, W))
     eng.set_tuning(E.PATH_AUTO, 0)
     out.close()
     eng.close()

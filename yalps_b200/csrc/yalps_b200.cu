@@ -86,14 +86,6 @@ struct yalps_ctx {
   std::vector<cudaStream_t> aux_streams;  // concurrent K4 launches of one node wave
   std::vector<cudaEvent_t> aux_events;
   cudaEvent_t fork_event = nullptr;
-  bool keep_final = false;         // solve_host (n == 1): leave the final tableau on the device, no D2H copy of it
-  double *kept_final = nullptr;    // ... and where it is (valid until the next batch call on this ctx)
-  // yalps_solve_sparse: solve_host (n == 1) builds its device tableau from these (cell, value) pairs instead of copying
-  // a dense host matrix (coo_nnz < 0: not in use); coo_dup reports that duplicates with different values were seen
-  const int32_t *coo_cell = nullptr;
-  const double *coo_val = nullptr;
-  int64_t coo_nnz = -1;
-  int coo_dup = 0;
   // YALPS_BNB_DEBUG: where the host spends a node wave (ns): before the first CUDA call, enqueueing, waiting, copying out
   int64_t wave_ns[4] = {0, 0, 0, 0};
   int wave = 256;  // upper bound of the adaptive look-ahead of the branch-and-cut driver
@@ -1051,217 +1043,304 @@ int yalps_ranging_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t widt
   return launch_ranging(ctx, a, (size_t)n * (width + height), "dev", (cudaStream_t)stream);
 }
 
-// Shared host-side pipeline for uniform and ragged batches.
-static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const int32_t *heights,
-                      const int32_t *widths, const int64_t *mat_offsets, const double *matrices,
-                      const yalps_options *opt, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
-                      int32_t *pos_out, int32_t *var_out, double *matrices_out, const int32_t *pos_in = nullptr,
-                      const int32_t *var_in = nullptr, double *reduced_out = nullptr, const int32_t *pairs = nullptr,
-                      double *range_lo = nullptr, double *range_hi = nullptr) {
-  if (!ctx) return YALPS_ERR_ARGUMENT;
-  if (n < 0 || !opt || (n > 0 && !matrices)) return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments");
-  if ((pos_in == nullptr) != (var_in == nullptr))
-    return fail(ctx, YALPS_ERR_ARGUMENT, "pos_in and var_in must be given together (or both null for the identity)");
-  if ((range_lo == nullptr) != (range_hi == nullptr))
-    return fail(ctx, YALPS_ERR_ARGUMENT, "range_lo and range_hi must be given together (or both null)");
-  // ranging: k_ranging runs over the final tableaus after the solve, which therefore stay in device memory
-  const bool want_rng = range_lo != nullptr;
-  if (!want_rng) pairs = nullptr;
-  if (n == 0) return 0;
-  CU(ctx, cudaSetDevice(ctx->device));
-  const bool ragged = heights != nullptr;
+}  // extern "C"
 
-  // per-LP prefix offsets (ragged) and caps
-  std::vector<long long> moff, roff, poff;
-  int Hcap = height, Wcap = width;
-  if (ragged) {
-    if (!widths || !mat_offsets) return fail(ctx, YALPS_ERR_ARGUMENT, "ragged batch needs widths and mat_offsets");
-    moff.resize(n + 1);
-    roff.resize(n + 1);
-    poff.resize(n + 1);
-    long long r = 0, p = 0, m = 0;
-    Hcap = Wcap = 1;
-    for (int64_t i = 0; i < n; i++) {
-      if (heights[i] < 1 || widths[i] < 1) return fail(ctx, YALPS_ERR_ARGUMENT, "LP %lld has empty shape", (long long)i);
-      if ((long long)heights[i] * widths[i] >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
-      moff[i] = m;
-      roff[i] = r;
-      poff[i] = p;
-      m += (long long)heights[i] * widths[i];
-      r += heights[i];
-      p += heights[i] + widths[i];
-      Hcap = std::max(Hcap, heights[i]);
-      Wcap = std::max(Wcap, widths[i]);
-    }
-    moff[n] = m;
-    roff[n] = r;
-    poff[n] = p;
-  } else {
-    if (height < 1 || width < 1) return fail(ctx, YALPS_ERR_ARGUMENT, "bad shape %dx%d", height, width);
-    if ((long long)height * width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
+// ---- host batches --------------------------------------------------------------------------------------------------
+namespace {
+
+// One host batch solve: the shape, where the tableaus come from, the optional inputs and every output (null: not
+// wanted).  The yalps_solve_{batch,ragged}_ranging entries, yalps_solve's root LP and the sparse entries fill one in.
+struct HostBatch {
+  int64_t n = 0;
+  int32_t height = 0, width = 0;                        // a uniform batch, or
+  const int32_t *heights = nullptr, *widths = nullptr;  // a ragged one (heights given)
+  const int64_t *mat_offsets = nullptr;
+  const double *matrices = nullptr;  // dense host tableaus, or (n == 1, uniform, nnz >= 0) the (cell, value) stores
+  const int32_t *cell = nullptr;     // into a zero tableau, scattered on the device (yalps_solve_sparse)
+  const double *val = nullptr;
+  int64_t nnz = -1;
+  const int32_t *pos_in = nullptr, *var_in = nullptr;  // the basis the tableaus arrive with (both null: the identity)
+  const int32_t *pairs = nullptr;                       // ranging: the other row of each row's key
+  const yalps_options *opt = nullptr;
+  int32_t *status = nullptr;
+  double *value = nullptr;
+  int64_t *pivots = nullptr;
+  double *rhs_out = nullptr;
+  int32_t *pos_out = nullptr, *var_out = nullptr;
+  double *matrices_out = nullptr, *reduced_out = nullptr, *range_lo = nullptr, *range_hi = nullptr;
+  bool keep_final = false;  // (n == 1, uniform) leave the final tableau on the device, no D2H copy of it
+  // results
+  double *kept_final = nullptr;  // keep_final: where the final tableau is (valid until the next batch call on the ctx)
+  int32_t dup_cells = 0;         // nnz >= 0: the device found duplicate cells with different values
+};
+
+// The per-LP outputs of a host batch, described once: pool name, host array (null: not wanted), element size and
+// packing.  The kernels write the first six whether they are wanted or not, so those always get a device buffer.
+enum OutPack { PER_LP, PER_ROW, PER_VAR };  // per LP (times k), per row like rhs_out, per variable id like pos_out
+struct OutSpec {
+  const char *name;
+  void *host;
+  size_t elem;
+  OutPack pack;
+  int k;
+  bool always;
+  bool used() const { return always || host; }
+  // bytes for `lps` LPs of `rows` rows and `pvs` variable ids in all
+  size_t bytes(long long lps, long long rows, long long pvs) const {
+    return elem * (size_t)(pack == PER_LP ? lps * k : pack == PER_ROW ? rows : pvs);
   }
-  if (int rc = check_pairs(ctx, pairs, n, height, heights)) return rc;
+};
+enum { O_STATUS, O_VALUE, O_PIVOTS, O_RHS, O_POS, O_VAR, O_RED, O_RLO, O_RHI, O_COUNT };
+struct Outputs {
+  OutSpec t[O_COUNT];
+  Outputs(int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+          double *reduced_out, double *range_lo, double *range_hi)
+      : t{{"status", status, 4, PER_LP, 1, true},     {"value", value, 8, PER_LP, 1, true},
+          {"pivots", pivots, 8, PER_LP, 2, true},     {"rhs", rhs_out, 8, PER_ROW, 1, true},
+          {"pos", pos_out, 4, PER_VAR, 1, true},      {"var", var_out, 4, PER_VAR, 1, true},
+          {"red", reduced_out, 8, PER_VAR, 1, false}, {"rlo", range_lo, 8, PER_VAR, 1, false},
+          {"rhi", range_hi, 8, PER_VAR, 1, false}} {}
+  explicit Outputs(const HostBatch &b)
+      : Outputs(b.status, b.value, b.pivots, b.rhs_out, b.pos_out, b.var_out, b.reduced_out, b.range_lo, b.range_hi) {}
 
-  auto cells_upto = [&](int64_t i) -> long long { return ragged ? moff[i] : (long long)i * height * width; };
-  auto rows_upto = [&](int64_t i) -> long long { return ragged ? roff[i] : (long long)i * height; };
-  auto pv_upto = [&](int64_t i) -> long long { return ragged ? poff[i] : (long long)i * (height + width); };
+  // device buffers "<name><slot>" for a chunk of `lps` LPs (`rows` rows, `pvs` variable ids); null where not used
+  int ensure(yalps_ctx *ctx, const std::string &slot, long long lps, long long rows, long long pvs, void **dev) const {
+    for (int i = 0; i < O_COUNT; i++) {
+      dev[i] = nullptr;
+      if (t[i].used())
+        if (int rc = dev_ensure(ctx, t[i].name + slot, t[i].bytes(lps, rows, pvs), &dev[i])) return rc;
+    }
+    return 0;
+  }
+  // D2H copies of the wanted outputs of a chunk that starts after lp0 LPs (row0 rows, pv0 variable ids)
+  int copy_out(yalps_ctx *ctx, void *const *dev, long long lp0, long long row0, long long pv0, long long lps,
+               long long rows, long long pvs, cudaStream_t st) const {
+    for (const OutSpec &o : t)
+      if (o.host)
+        CU(ctx, cudaMemcpyAsync((char *)o.host + o.bytes(lp0, row0, pv0), dev[&o - t], o.bytes(lps, rows, pvs),
+                                cudaMemcpyDeviceToHost, st));
+    return 0;
+  }
+};
 
+void set_outputs(BatchArgs &a, void *const *dev) {
+  a.status = (int *)dev[O_STATUS];
+  a.value = (double *)dev[O_VALUE];
+  a.pivots = (long long *)dev[O_PIVOTS];
+  a.rhs_out = (double *)dev[O_RHS];
+  a.pos_out = (int *)dev[O_POS];
+  a.var_out = (int *)dev[O_VAR];
+  a.red_out = (double *)dev[O_RED];
+}
+
+// What solve_host derives from a valid request: the caps and the per-LP prefix counts of cells, rows and variable ids.
+struct BatchLayout {
+  bool ragged = false;
+  int32_t height = 0, width = 0, Hcap = 0, Wcap = 0;
+  std::vector<long long> moff, roff, poff;  // ragged only
+  const int32_t *pairs = nullptr;           // the request's pairs when ranges are wanted, else null
+  long long cells_upto(int64_t i) const { return ragged ? moff[i] : (long long)i * height * width; }
+  long long rows_upto(int64_t i) const { return ragged ? roff[i] : (long long)i * height; }
+  long long pv_upto(int64_t i) const { return ragged ? poff[i] : (long long)i * (height + width); }
+};
+
+// Validates a request and lays it out (nothing more when b.n == 0).
+int batch_layout(yalps_ctx *ctx, const HostBatch &b, BatchLayout *L) {
+  const int64_t n = b.n;
+  if (n < 0 || !b.opt || (n > 0 && !b.matrices && b.nnz < 0)) return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments");
+  if ((b.pos_in == nullptr) != (b.var_in == nullptr))
+    return fail(ctx, YALPS_ERR_ARGUMENT, "pos_in and var_in must be given together (or both null for the identity)");
+  if ((b.range_lo == nullptr) != (b.range_hi == nullptr))
+    return fail(ctx, YALPS_ERR_ARGUMENT, "range_lo and range_hi must be given together (or both null)");
+  if (n == 0) return 0;
+  L->ragged = b.heights != nullptr;
+  L->height = L->Hcap = b.height;
+  L->width = L->Wcap = b.width;
+  // ranging: k_ranging runs over the final tableaus after the solve, which therefore stay in device memory
+  L->pairs = b.range_lo ? b.pairs : nullptr;
+  if (L->ragged) {
+    if (!b.widths || !b.mat_offsets) return fail(ctx, YALPS_ERR_ARGUMENT, "ragged batch needs widths and mat_offsets");
+    L->moff.resize(n + 1);
+    L->roff.resize(n + 1);
+    L->poff.resize(n + 1);
+    long long r = 0, p = 0, m = 0;
+    L->Hcap = L->Wcap = 1;
+    for (int64_t i = 0; i < n; i++) {
+      const int32_t h = b.heights[i], w = b.widths[i];
+      if (h < 1 || w < 1) return fail(ctx, YALPS_ERR_ARGUMENT, "LP %lld has empty shape", (long long)i);
+      if ((long long)h * w >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
+      L->moff[i] = m;
+      L->roff[i] = r;
+      L->poff[i] = p;
+      m += (long long)h * w;
+      r += h;
+      p += h + w;
+      L->Hcap = std::max(L->Hcap, h);
+      L->Wcap = std::max(L->Wcap, w);
+    }
+    L->moff[n] = m;
+    L->roff[n] = r;
+    L->poff[n] = p;
+  } else {
+    if (b.height < 1 || b.width < 1) return fail(ctx, YALPS_ERR_ARGUMENT, "bad shape %dx%d", b.height, b.width);
+    if ((long long)b.height * b.width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
+  }
+  if (int rc = check_pairs(ctx, L->pairs, n, b.height, b.heights)) return rc;
   // caller-supplied basis: the two arrays must be inverse permutations of 0..W+H-1 (src/tableau.ts:9-15); the kernels
   // carry variableAtPosition and rebuild positionOfVariable on output, so an inconsistent pair would silently
   // change meaning instead of behaving like the reference
-  if (var_in) {
+  if (b.var_in) {
     for (int64_t i = 0; i < n; i++) {
-      const long long o = pv_upto(i), len = pv_upto(i + 1) - o;
+      const long long o = L->pv_upto(i), len = L->pv_upto(i + 1) - o;
       for (long long k = 0; k < len; k++) {
-        const int32_t v = var_in[o + k];
-        if (v < 0 || v >= len || pos_in[o + v] != (int32_t)k)
+        const int32_t v = b.var_in[o + k];
+        if (v < 0 || v >= len || b.pos_in[o + v] != (int32_t)k)
           return fail(ctx, YALPS_ERR_ARGUMENT, "LP %lld: pos_in/var_in are not inverse permutations at position %lld",
                       (long long)i, k);
       }
     }
   }
+  return 0;
+}
 
-  // density of (a sample of) the first tableau: the path policy distinguishes dense from very sparse LPs
-  auto first_density = [&]() {
-    const double *m0 = matrices + (ragged ? mat_offsets[0] : 0);
-    const long long c0 = ragged ? (long long)heights[0] * widths[0] : (long long)height * width;
-    const long long step = std::max(1LL, c0 / 4096);
-    long long seen = 0, nz = 0;
-    for (long long k = 0; k < c0; k += step, seen++) nz += m0[k] != 0.0;
-    return seen ? (double)nz / (double)seen : 1.0;
-  };
+// density of (a sample of) the first tableau: the path policy distinguishes dense from very sparse LPs
+double first_density(const HostBatch &b) {
+  const bool ragged = b.heights != nullptr;
+  const double *m0 = b.matrices + (ragged ? b.mat_offsets[0] : 0);
+  const long long c0 = ragged ? (long long)b.heights[0] * b.widths[0] : (long long)b.height * b.width;
+  const long long step = std::max(1LL, c0 / 4096);
+  long long seen = 0, nz = 0;
+  for (long long k = 0; k < c0; k += step, seen++) nz += m0[k] != 0.0;
+  return seen ? (double)nz / (double)seen : 1.0;
+}
 
-  // ---- small calls (a single LP, a handful of models): latency-bound.  Stage through one mapped pinned buffer,
-  // let the kernel read the tableaus and write the results zero-copy: launch + synchronise, no memcpy calls.
-  {
-    const size_t in_b = (size_t)cells_upto(n) * 8, rows_b = (size_t)rows_upto(n) * 8, pv_b = (size_t)pv_upto(n) * 4;
-    const size_t red_b = reduced_out ? 2 * pv_b : 0;  // doubles, packed like pos_out
-    const size_t rng_b = want_rng ? 2 * pv_b : 0;     // range_lo, range_hi: doubles, packed like pos_out
-    const size_t pair_b = pairs ? rows_b / 2 : 0;      // int32, packed like rhs_out
-    const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (matrices_out ? in_b : 0) + (red_b ? red_b + 16 : 0) +
-                         (rng_b ? 2 * rng_b + 32 : 0);
-    const size_t desc_b = (ragged ? (size_t)n * 32 + 64 : 0) + (var_in ? pv_b + 16 : 0) + (pair_b ? pair_b + 16 : 0);
-    Route route;
-    if (!ctx->keep_final && ctx->coo_nnz < 0 && in_b + out_b + desc_b <= ((size_t)768 << 10) &&
-        choose_route(ctx, {n, Hcap, Wcap, first_density(), opt->check_cycles != 0, true}, &route) == 0 &&
-        (route.kind == ROUTE_K1T || (route.kind == ROUTE_SIMPLEX && route.resident))) {
-      auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
-      size_t o = 0;
-      const size_t o_in = o; o += up16(in_b);
-      const size_t o_h = o; o += ragged ? up16((size_t)n * 4) : 0;
-      const size_t o_w = o; o += ragged ? up16((size_t)n * 4) : 0;
-      const size_t o_mo = o; o += ragged ? up16((size_t)n * 8) : 0;
-      const size_t o_ro = o; o += ragged ? up16((size_t)n * 8) : 0;
-      const size_t o_po = o; o += ragged ? up16((size_t)n * 8) : 0;
-      const size_t o_vin = o; o += var_in ? up16(pv_b) : 0;
-      const size_t o_st = o; o += up16((size_t)n * 4);
-      const size_t o_val = o; o += up16((size_t)n * 8);
-      const size_t o_piv = o; o += up16((size_t)n * 16);
-      const size_t o_rhs = o; o += up16(rows_b);
-      const size_t o_pos = o; o += up16(pv_b);
-      const size_t o_var = o; o += up16(pv_b);
-      const size_t o_mat = o; o += matrices_out ? up16(in_b) : 0;
-      const size_t o_red = o; o += up16(red_b);
-      const size_t o_rlo = o; o += up16(rng_b);
-      const size_t o_rhi = o; o += up16(rng_b);
-      const size_t o_pair = o; o += up16(pair_b);
-      void *hb, *db;
-      int rc;
-      if ((rc = pin_ensure(ctx, "small_io", o + 16, &hb))) return rc;
-      if ((rc = pin_device_ptr(ctx, hb, &db))) return rc;
-      char *h = (char *)hb, *d = (char *)db;
-      // ranging reads the final tableaus from device scratch, not over PCIe from the mapped buffer
-      void *d_fin = nullptr;
-      if (want_rng && (rc = dev_ensure(ctx, "small_final", in_b, &d_fin))) return rc;
-      if (pairs) std::memcpy(h + o_pair, pairs, pair_b);
-      if (ragged) {
-        for (int64_t i = 0; i < n; i++)
-          std::memcpy(h + o_in + (size_t)moff[i] * 8, matrices + mat_offsets[i], (size_t)heights[i] * widths[i] * 8);
-        std::memcpy(h + o_h, heights, (size_t)n * 4);
-        std::memcpy(h + o_w, widths, (size_t)n * 4);
-        std::memcpy(h + o_mo, moff.data(), (size_t)n * 8);
-        std::memcpy(h + o_ro, roff.data(), (size_t)n * 8);
-        std::memcpy(h + o_po, poff.data(), (size_t)n * 8);
-      } else {
-        std::memcpy(h + o_in, matrices, in_b);
-      }
-      if (var_in) std::memcpy(h + o_vin, var_in, pv_b);
-      BatchArgs a{};
-      a.n = n;
-      a.mode = kModeBatch;
-      a.H = height;
-      a.W = width;
-      a.Hcap = Hcap;
-      a.Wcap = Wcap;
-      a.in = (const double *)(d + o_in);
-      a.work = nullptr;
-      a.mat_out = want_rng ? (double *)d_fin : matrices_out ? (double *)(d + o_mat) : nullptr;
-      a.status = (int *)(d + o_st);
-      a.value = (double *)(d + o_val);
-      a.pivots = (long long *)(d + o_piv);
-      a.rhs_out = (double *)(d + o_rhs);
-      a.pos_out = (int *)(d + o_pos);
-      a.var_out = (int *)(d + o_var);
-      a.var_in = var_in ? (const int *)(d + o_vin) : nullptr;
-      a.red_out = reduced_out ? (double *)(d + o_red) : nullptr;
-      if (ragged) {
-        a.heights = (const int *)(d + o_h);
-        a.widths = (const int *)(d + o_w);
-        a.mat_off = (const long long *)(d + o_mo);
-        a.rhs_off = (const long long *)(d + o_ro);
-        a.pos_off = (const long long *)(d + o_po);
-      }
-      fill_options(a, opt);
-      cudaStream_t st = ctx->streams[0];
-      if ((rc = launch_route(ctx, route, a, "small", st))) return rc;
-      if (want_rng) {
-        RangingArgs g{};
-        g.n = n;
-        g.H = height;
-        g.W = width;
-        g.Hcap = Hcap;
-        g.Wcap = Wcap;
-        g.M = (const double *)d_fin;
-        g.heights = a.heights;
-        g.widths = a.widths;
-        g.mat_off = a.mat_off;
-        g.rhs_off = a.rhs_off;
-        g.pos_off = a.pos_off;
-        g.pos = a.pos_out;
-        g.status = a.status;
-        g.pairs = pairs ? (const int *)(d + o_pair) : nullptr;
-        g.precision = opt->precision;
-        g.lo = (double *)(d + o_rlo);
-        g.hi = (double *)(d + o_rhi);
-        if ((rc = launch_ranging(ctx, g, (size_t)pv_upto(n), "small", st))) return rc;
-        if (matrices_out) CU(ctx, cudaMemcpyAsync(h + o_mat, d_fin, in_b, cudaMemcpyDeviceToHost, st));
-      }
-      CU(ctx, cudaStreamSynchronize(st));
-      if (status) std::memcpy(status, h + o_st, (size_t)n * 4);
-      if (value) std::memcpy(value, h + o_val, (size_t)n * 8);
-      if (pivots) std::memcpy(pivots, h + o_piv, (size_t)n * 16);
-      if (rhs_out) std::memcpy(rhs_out, h + o_rhs, rows_b);
-      if (pos_out) std::memcpy(pos_out, h + o_pos, pv_b);
-      if (var_out) std::memcpy(var_out, h + o_var, pv_b);
-      if (reduced_out) std::memcpy(reduced_out, h + o_red, red_b);
-      if (want_rng) {
-        std::memcpy(range_lo, h + o_rlo, rng_b);
-        std::memcpy(range_hi, h + o_rhi, rng_b);
-      }
-      if (matrices_out) {
-        if (ragged)
-          for (int64_t i = 0; i < n; i++)
-            std::memcpy(matrices_out + mat_offsets[i], h + o_mat + (size_t)moff[i] * 8, (size_t)heights[i] * widths[i] * 8);
-        else
-          std::memcpy(matrices_out, h + o_mat, in_b);
-      }
-      return check_device_status(ctx, status, n);
-    }
+// Small calls (a single LP, a handful of models) are latency-bound.  Stage through one mapped pinned buffer, let the
+// kernel read the tableaus and write the results zero-copy: launch + synchronise, no memcpy calls.  *taken is false
+// (and nothing was done) when the batch does not qualify.
+int solve_small(yalps_ctx *ctx, const HostBatch &b, const BatchLayout &L, bool *taken) {
+  *taken = false;
+  const int64_t n = b.n;
+  const bool ragged = L.ragged, want_rng = b.range_lo != nullptr;
+  const long long rows = L.rows_upto(n), pvs = L.pv_upto(n);
+  const size_t in_b = (size_t)L.cells_upto(n) * 8, rows_b = (size_t)rows * 8, pv_b = (size_t)pvs * 4;
+  const size_t red_b = b.reduced_out ? 2 * pv_b : 0;  // doubles, packed like pos_out
+  const size_t rng_b = want_rng ? 2 * pv_b : 0;       // range_lo, range_hi: doubles, packed like pos_out
+  const size_t pair_b = L.pairs ? rows_b / 2 : 0;     // int32, packed like rhs_out
+  const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (b.matrices_out ? in_b : 0) + (red_b ? red_b + 16 : 0) +
+                       (rng_b ? 2 * rng_b + 32 : 0);
+  const size_t desc_b = (ragged ? (size_t)n * 32 + 64 : 0) + (b.var_in ? pv_b + 16 : 0) + (pair_b ? pair_b + 16 : 0);
+  Route route;
+  if (b.keep_final || b.nnz >= 0 || in_b + out_b + desc_b > ((size_t)768 << 10) ||
+      choose_route(ctx, {n, L.Hcap, L.Wcap, first_density(b), b.opt->check_cycles != 0, true}, &route) != 0 ||
+      !(route.kind == ROUTE_K1T || (route.kind == ROUTE_SIMPLEX && route.resident)))
+    return 0;
+  *taken = true;
+  const Outputs outs(b);
+  auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+  size_t o = 0;
+  const size_t o_in = o; o += up16(in_b);
+  const size_t o_h = o; o += ragged ? up16((size_t)n * 4) : 0;
+  const size_t o_w = o; o += ragged ? up16((size_t)n * 4) : 0;
+  const size_t o_mo = o; o += ragged ? up16((size_t)n * 8) : 0;
+  const size_t o_ro = o; o += ragged ? up16((size_t)n * 8) : 0;
+  const size_t o_po = o; o += ragged ? up16((size_t)n * 8) : 0;
+  const size_t o_vin = o; o += b.var_in ? up16(pv_b) : 0;
+  size_t o_out[O_COUNT];
+  for (int i = 0; i < O_COUNT; i++) {
+    o_out[i] = o;
+    o += outs.t[i].used() ? up16(outs.t[i].bytes(n, rows, pvs)) : 0;
   }
+  const size_t o_mat = o; o += b.matrices_out ? up16(in_b) : 0;
+  const size_t o_pair = o; o += up16(pair_b);
+  void *hb, *db;
+  int rc;
+  if ((rc = pin_ensure(ctx, "small_io", o + 16, &hb))) return rc;
+  if ((rc = pin_device_ptr(ctx, hb, &db))) return rc;
+  char *h = (char *)hb, *d = (char *)db;
+  // ranging reads the final tableaus from device scratch, not over PCIe from the mapped buffer
+  void *d_fin = nullptr;
+  if (want_rng && (rc = dev_ensure(ctx, "small_final", in_b, &d_fin))) return rc;
+  if (L.pairs) std::memcpy(h + o_pair, L.pairs, pair_b);
+  if (ragged) {
+    for (int64_t i = 0; i < n; i++)
+      std::memcpy(h + o_in + (size_t)L.moff[i] * 8, b.matrices + b.mat_offsets[i], (size_t)b.heights[i] * b.widths[i] * 8);
+    std::memcpy(h + o_h, b.heights, (size_t)n * 4);
+    std::memcpy(h + o_w, b.widths, (size_t)n * 4);
+    std::memcpy(h + o_mo, L.moff.data(), (size_t)n * 8);
+    std::memcpy(h + o_ro, L.roff.data(), (size_t)n * 8);
+    std::memcpy(h + o_po, L.poff.data(), (size_t)n * 8);
+  } else {
+    std::memcpy(h + o_in, b.matrices, in_b);
+  }
+  if (b.var_in) std::memcpy(h + o_vin, b.var_in, pv_b);
+  void *dev[O_COUNT];
+  for (int i = 0; i < O_COUNT; i++) dev[i] = outs.t[i].used() ? d + o_out[i] : nullptr;
+  BatchArgs a{};
+  a.n = n;
+  a.mode = kModeBatch;
+  a.H = L.height;
+  a.W = L.width;
+  a.Hcap = L.Hcap;
+  a.Wcap = L.Wcap;
+  a.in = (const double *)(d + o_in);
+  a.work = nullptr;
+  a.mat_out = want_rng ? (double *)d_fin : b.matrices_out ? (double *)(d + o_mat) : nullptr;
+  set_outputs(a, dev);
+  a.var_in = b.var_in ? (const int *)(d + o_vin) : nullptr;
+  if (ragged) {
+    a.heights = (const int *)(d + o_h);
+    a.widths = (const int *)(d + o_w);
+    a.mat_off = (const long long *)(d + o_mo);
+    a.rhs_off = (const long long *)(d + o_ro);
+    a.pos_off = (const long long *)(d + o_po);
+  }
+  fill_options(a, b.opt);
+  cudaStream_t st = ctx->streams[0];
+  if ((rc = launch_route(ctx, route, a, "small", st))) return rc;
+  if (want_rng) {
+    RangingArgs g{};
+    g.n = n;
+    g.H = L.height;
+    g.W = L.width;
+    g.Hcap = L.Hcap;
+    g.Wcap = L.Wcap;
+    g.M = (const double *)d_fin;
+    g.heights = a.heights;
+    g.widths = a.widths;
+    g.mat_off = a.mat_off;
+    g.rhs_off = a.rhs_off;
+    g.pos_off = a.pos_off;
+    g.pos = a.pos_out;
+    g.status = a.status;
+    g.pairs = L.pairs ? (const int *)(d + o_pair) : nullptr;
+    g.precision = b.opt->precision;
+    g.lo = (double *)dev[O_RLO];
+    g.hi = (double *)dev[O_RHI];
+    if ((rc = launch_ranging(ctx, g, (size_t)pvs, "small", st))) return rc;
+    if (b.matrices_out) CU(ctx, cudaMemcpyAsync(h + o_mat, d_fin, in_b, cudaMemcpyDeviceToHost, st));
+  }
+  CU(ctx, cudaStreamSynchronize(st));
+  for (int i = 0; i < O_COUNT; i++)
+    if (outs.t[i].host) std::memcpy(outs.t[i].host, h + o_out[i], outs.t[i].bytes(n, rows, pvs));
+  if (b.matrices_out) {
+    if (ragged)
+      for (int64_t i = 0; i < n; i++)
+        std::memcpy(b.matrices_out + b.mat_offsets[i], h + o_mat + (size_t)L.moff[i] * 8,
+                    (size_t)b.heights[i] * b.widths[i] * 8);
+    else
+      std::memcpy(b.matrices_out, h + o_mat, in_b);
+  }
+  return check_device_status(ctx, b.status, n);
+}
 
-  // chunking: two pipeline slots; a large batch is cut into ~8 chunks (64 MiB .. 1.5 GiB each) so that the
-  // H2D copy of chunk k+1 overlaps the kernel and the D2H copies of chunk k
-  const size_t total_bytes = (size_t)cells_upto(n) * 8;
+// The pipelined path: two slots; a large batch is cut into ~8 chunks (64 MiB .. 1.5 GiB each) so that the H2D copy of
+// chunk k+1 overlaps the kernel and the D2H copies of chunk k.
+int solve_chunks(yalps_ctx *ctx, HostBatch &b, const BatchLayout &L) {
+  const int64_t n = b.n;
+  const bool ragged = L.ragged, want_rng = b.range_lo != nullptr;
+  const yalps_options *opt = b.opt;
+  const Outputs outs(b);
+  const size_t total_bytes = (size_t)L.cells_upto(n) * 8;
   const size_t kSlotBytes = std::min((size_t)1536 << 20, std::max((size_t)64 << 20, total_bytes / 8 + 4096));
 
   int64_t begin = 0;
@@ -1271,85 +1350,74 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
   bool used[2] = {false, false};
   while (begin < n) {
     int64_t end = begin + 1;
-    while (end < n && (size_t)(cells_upto(end + 1) - cells_upto(begin)) * 8 <= kSlotBytes) end++;
+    while (end < n && (size_t)(L.cells_upto(end + 1) - L.cells_upto(begin)) * 8 <= kSlotBytes) end++;
     const int64_t cn = end - begin;
-    const size_t ccells = (size_t)(cells_upto(end) - cells_upto(begin));
-    const size_t crows = (size_t)(rows_upto(end) - rows_upto(begin));
-    const size_t cpv = (size_t)(pv_upto(end) - pv_upto(begin));
+    const size_t ccells = (size_t)(L.cells_upto(end) - L.cells_upto(begin));
+    const size_t crows = (size_t)(L.rows_upto(end) - L.rows_upto(begin));
+    const size_t cpv = (size_t)(L.pv_upto(end) - L.pv_upto(begin));
     const std::string s = std::to_string(slot);
     cudaStream_t st = ctx->streams[slot];
     if (used[slot]) CU(ctx, cudaEventSynchronize(ctx->events[slot]));
 
-    int chcap = Hcap, cwcap = Wcap;
+    int chcap = L.Hcap, cwcap = L.Wcap;
     if (ragged) {
       chcap = cwcap = 1;
       for (int64_t i = begin; i < end; i++) {
-        chcap = std::max(chcap, heights[i]);
-        cwcap = std::max(cwcap, widths[i]);
+        chcap = std::max(chcap, b.heights[i]);
+        cwcap = std::max(cwcap, b.widths[i]);
       }
     }
-    const bool from_cells = ctx->coo_nnz >= 0 && n == 1 && !ragged;
-    if (from_cells) density = (double)ctx->coo_nnz / (double)((long long)height * width);
-    if (density < 0.0) density = first_density();  // sampled once
+    const bool from_cells = b.nnz >= 0;
+    if (from_cells) density = (double)b.nnz / (double)((long long)b.height * b.width);
+    if (density < 0.0) density = first_density(b);  // sampled once
     // a uniform chunk is one launch, routed before its buffers are set up (the route decides where its final tableaus
     // go); a ragged chunk is routed group by group below
     Route route;
     if (!ragged && (rc = choose_route(ctx, {cn, chcap, cwcap, density, opt->check_cycles != 0, true}, &route))) return rc;
 
-    void *d_in, *d_status, *d_value, *d_piv, *d_rhs, *d_pos, *d_var;
+    void *d_in, *dev[O_COUNT];
     if ((rc = dev_ensure(ctx, "in" + s, ccells * 8, &d_in))) return rc;
-    if ((rc = dev_ensure(ctx, "status" + s, (size_t)cn * 4, &d_status))) return rc;
-    if ((rc = dev_ensure(ctx, "value" + s, (size_t)cn * 8, &d_value))) return rc;
-    if ((rc = dev_ensure(ctx, "pivots" + s, (size_t)cn * 16, &d_piv))) return rc;
-    if ((rc = dev_ensure(ctx, "rhs" + s, crows * 8, &d_rhs))) return rc;
-    if ((rc = dev_ensure(ctx, "pos" + s, cpv * 4, &d_pos))) return rc;
-    if ((rc = dev_ensure(ctx, "var" + s, cpv * 4, &d_var))) return rc;
-    void *d_red = nullptr;
-    if (reduced_out && (rc = dev_ensure(ctx, "red" + s, cpv * 8, &d_red))) return rc;
-    void *d_rlo = nullptr, *d_rhi = nullptr, *d_pairs = nullptr;
-    if (want_rng) {
-      if ((rc = dev_ensure(ctx, "rlo" + s, cpv * 8, &d_rlo))) return rc;
-      if ((rc = dev_ensure(ctx, "rhi" + s, cpv * 8, &d_rhi))) return rc;
-      if (pairs) {
-        if ((rc = dev_ensure(ctx, "pairs" + s, crows * 4, &d_pairs))) return rc;
-        CU(ctx, cudaMemcpyAsync(d_pairs, pairs + rows_upto(begin), crows * 4, cudaMemcpyHostToDevice, st));
-      }
+    if ((rc = outs.ensure(ctx, s, cn, crows, cpv, dev))) return rc;
+    void *d_pairs = nullptr;
+    if (L.pairs) {
+      if ((rc = dev_ensure(ctx, "pairs" + s, crows * 4, &d_pairs))) return rc;
+      CU(ctx, cudaMemcpyAsync(d_pairs, L.pairs + L.rows_upto(begin), crows * 4, cudaMemcpyHostToDevice, st));
     }
     void *d_vin = nullptr;
-    if (var_in) {
+    if (b.var_in) {
       if ((rc = dev_ensure(ctx, "varin" + s, cpv * 4, &d_vin))) return rc;
-      CU(ctx, cudaMemcpyAsync(d_vin, var_in + pv_upto(begin), cpv * 4, cudaMemcpyHostToDevice, st));
+      CU(ctx, cudaMemcpyAsync(d_vin, b.var_in + L.pv_upto(begin), cpv * 4, cudaMemcpyHostToDevice, st));
     }
     void *d_out = nullptr;
-    const bool want_mat = matrices_out != nullptr || want_rng || (ctx->keep_final && n == 1 && !ragged);
+    const bool want_mat = b.matrices_out != nullptr || want_rng || b.keep_final;
     // K1t and K1/K1s write the final tableaus apart; the others leave them in the working copy d_in
     const bool out_apart = ragged || (route.resident && route.kind != ROUTE_GRID);
     if (want_mat && out_apart)
       if ((rc = dev_ensure(ctx, "matout" + s, ccells * 8, &d_out))) return rc;
 
-    const double *src = matrices + (ragged ? mat_offsets[begin] : cells_upto(begin));
+    const double *src = b.matrices + (ragged ? b.mat_offsets[begin] : L.cells_upto(begin));
     if (ragged) {
       // caller offsets may be non-contiguous: copy LP by LP when they are
       bool contiguous = true;
       for (int64_t i = begin; i < end && contiguous; i++)
-        contiguous = (mat_offsets[i] - mat_offsets[begin]) == (moff[i] - moff[begin]);
+        contiguous = (b.mat_offsets[i] - b.mat_offsets[begin]) == (L.moff[i] - L.moff[begin]);
       if (contiguous) {
         CU(ctx, cudaMemcpyAsync(d_in, src, ccells * 8, cudaMemcpyHostToDevice, st));
       } else {
         for (int64_t i = begin; i < end; i++)
-          CU(ctx, cudaMemcpyAsync((double *)d_in + (moff[i] - moff[begin]), matrices + mat_offsets[i],
-                                  (size_t)heights[i] * widths[i] * 8, cudaMemcpyHostToDevice, st));
+          CU(ctx, cudaMemcpyAsync((double *)d_in + (L.moff[i] - L.moff[begin]), b.matrices + b.mat_offsets[i],
+                                  (size_t)b.heights[i] * b.widths[i] * 8, cudaMemcpyHostToDevice, st));
       }
     } else if (from_cells) {
       // the (cell, value) pairs cross PCIe, the zeros are written by the device
-      const size_t nnz = (size_t)ctx->coo_nnz, val_off = (nnz * 4 + 15) & ~(size_t)15;
+      const size_t nnz = (size_t)b.nnz, val_off = (nnz * 4 + 15) & ~(size_t)15;
       void *h_coo, *d_coo, *d_flag;
       if ((rc = pin_ensure(ctx, "coo", val_off + nnz * 8 + 16, &h_coo))) return rc;
       if ((rc = dev_ensure(ctx, "coo", val_off + nnz * 8 + 16, &d_coo))) return rc;
       if ((rc = dev_ensure(ctx, "coo_flag", 4, &d_flag))) return rc;
       if (nnz) {
-        std::memcpy(h_coo, ctx->coo_cell, nnz * 4);
-        std::memcpy((char *)h_coo + val_off, ctx->coo_val, nnz * 8);
+        std::memcpy(h_coo, b.cell, nnz * 4);
+        std::memcpy((char *)h_coo + val_off, b.val, nnz * 8);
         CU(ctx, cudaMemcpyAsync(d_coo, h_coo, val_off + nnz * 8, cudaMemcpyHostToDevice, st));
       }
       CU(ctx, cudaMemsetAsync(d_in, 0, ccells * 8, st));
@@ -1363,7 +1431,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
         ctx->launches += 2;
         CU(ctx, cudaGetLastError());
       }
-      CU(ctx, cudaMemcpyAsync(&ctx->coo_dup, d_flag, 4, cudaMemcpyDeviceToHost, st));
+      CU(ctx, cudaMemcpyAsync(&b.dup_cells, d_flag, 4, cudaMemcpyDeviceToHost, st));
     } else {
       CU(ctx, cudaMemcpyAsync(d_in, src, ccells * 8, cudaMemcpyHostToDevice, st));
     }
@@ -1371,37 +1439,31 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
     BatchArgs a{};
     a.n = cn;
     a.mode = kModeBatch;
-    a.H = height;
-    a.W = width;
+    a.H = L.height;
+    a.W = L.width;
     a.Hcap = chcap;
     a.Wcap = cwcap;
     a.in = (const double *)d_in;
     a.work = (double *)d_in;  // K2 works in place on the device copy
     a.mat_out = want_mat ? (out_apart ? (double *)d_out : (double *)d_in) : nullptr;
-    a.status = (int *)d_status;
-    a.value = (double *)d_value;
-    a.pivots = (long long *)d_piv;
-    a.rhs_out = (double *)d_rhs;
-    a.pos_out = (int *)d_pos;
-    a.var_out = (int *)d_var;
+    set_outputs(a, dev);
     a.var_in = (const int *)d_vin;
-    a.red_out = (double *)d_red;
     std::vector<long long> lm, lr, lpv;  // chunk-local offsets of a ragged chunk
     if (ragged) {
       void *d_h, *d_w, *d_mo, *d_ro, *d_po;
       lm.resize(cn), lr.resize(cn), lpv.resize(cn);
       for (int64_t i = 0; i < cn; i++) {
-        lm[i] = moff[begin + i] - moff[begin];
-        lr[i] = roff[begin + i] - roff[begin];
-        lpv[i] = poff[begin + i] - poff[begin];
+        lm[i] = L.moff[begin + i] - L.moff[begin];
+        lr[i] = L.roff[begin + i] - L.roff[begin];
+        lpv[i] = L.poff[begin + i] - L.poff[begin];
       }
       if ((rc = dev_ensure(ctx, "rg_h" + s, (size_t)cn * 4, &d_h))) return rc;
       if ((rc = dev_ensure(ctx, "rg_w" + s, (size_t)cn * 4, &d_w))) return rc;
       if ((rc = dev_ensure(ctx, "rg_mo" + s, (size_t)cn * 8, &d_mo))) return rc;
       if ((rc = dev_ensure(ctx, "rg_ro" + s, (size_t)cn * 8, &d_ro))) return rc;
       if ((rc = dev_ensure(ctx, "rg_po" + s, (size_t)cn * 8, &d_po))) return rc;
-      CU(ctx, cudaMemcpyAsync(d_h, heights + begin, (size_t)cn * 4, cudaMemcpyHostToDevice, st));
-      CU(ctx, cudaMemcpyAsync(d_w, widths + begin, (size_t)cn * 4, cudaMemcpyHostToDevice, st));
+      CU(ctx, cudaMemcpyAsync(d_h, b.heights + begin, (size_t)cn * 4, cudaMemcpyHostToDevice, st));
+      CU(ctx, cudaMemcpyAsync(d_w, b.widths + begin, (size_t)cn * 4, cudaMemcpyHostToDevice, st));
       CU(ctx, cudaMemcpyAsync(d_mo, lm.data(), (size_t)cn * 8, cudaMemcpyHostToDevice, st));
       CU(ctx, cudaMemcpyAsync(d_ro, lr.data(), (size_t)cn * 8, cudaMemcpyHostToDevice, st));
       CU(ctx, cudaMemcpyAsync(d_po, lpv.data(), (size_t)cn * 8, cudaMemcpyHostToDevice, st));
@@ -1418,8 +1480,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       if (!want_rng) return 0;
       RangingArgs g{};
       g.n = rn;
-      g.H = height;
-      g.W = width;
+      g.H = L.height;
+      g.W = L.width;
       g.Hcap = rh;
       g.Wcap = rw;
       g.M = a.mat_out;
@@ -1433,8 +1495,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       g.status = a.status;
       g.pairs = (const int *)d_pairs;
       g.precision = opt->precision;
-      g.lo = (double *)d_rlo;
-      g.hi = (double *)d_rhi;
+      g.lo = (double *)dev[O_RLO];
+      g.hi = (double *)dev[O_RHI];
       return launch_ranging(ctx, g, cpv, s, st);
     };
     if (!ragged) {
@@ -1448,7 +1510,7 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       std::vector<std::pair<int, int>> caps;  // (Hcap, Wcap) per group
       std::unordered_map<int, int> group_of;
       for (int64_t i = 0; i < cn; i++) {
-        const int hi = heights[begin + i], wi = widths[begin + i];
+        const int hi = b.heights[begin + i], wi = b.widths[begin + i];
         const bool res = SmemLayout(hi, wi, true, 32).total <= (size_t)ctx->smem_optin;
         const int key = (res ? 0 : 64) + default_warps((long long)hi * wi, res);
         auto it = group_of.find(key);
@@ -1468,8 +1530,8 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       CU(ctx, cudaMemcpyAsync(d_index, flat.data(), flat.size() * 4, cudaMemcpyHostToDevice, st));
       CU(ctx, cudaStreamSynchronize(st));
       BatchArgs h{};  // host-side copies of the shape, offset and index arrays (K4 reads them on the host)
-      h.heights = heights + begin;
-      h.widths = widths + begin;
+      h.heights = b.heights + begin;
+      h.widths = b.widths + begin;
       h.mat_off = lm.data();
       h.rhs_off = lr.data();
       h.pos_off = lpv.data();
@@ -1490,26 +1552,15 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
       }
     }
 
-    if (status) CU(ctx, cudaMemcpyAsync(status + begin, d_status, (size_t)cn * 4, cudaMemcpyDeviceToHost, st));
-    if (value) CU(ctx, cudaMemcpyAsync(value + begin, d_value, (size_t)cn * 8, cudaMemcpyDeviceToHost, st));
-    if (pivots) CU(ctx, cudaMemcpyAsync(pivots + 2 * begin, d_piv, (size_t)cn * 16, cudaMemcpyDeviceToHost, st));
-    if (rhs_out) CU(ctx, cudaMemcpyAsync(rhs_out + rows_upto(begin), d_rhs, crows * 8, cudaMemcpyDeviceToHost, st));
-    if (pos_out) CU(ctx, cudaMemcpyAsync(pos_out + pv_upto(begin), d_pos, cpv * 4, cudaMemcpyDeviceToHost, st));
-    if (var_out) CU(ctx, cudaMemcpyAsync(var_out + pv_upto(begin), d_var, cpv * 4, cudaMemcpyDeviceToHost, st));
-    if (reduced_out)
-      CU(ctx, cudaMemcpyAsync(reduced_out + pv_upto(begin), d_red, cpv * 8, cudaMemcpyDeviceToHost, st));
-    if (want_rng) {
-      CU(ctx, cudaMemcpyAsync(range_lo + pv_upto(begin), d_rlo, cpv * 8, cudaMemcpyDeviceToHost, st));
-      CU(ctx, cudaMemcpyAsync(range_hi + pv_upto(begin), d_rhi, cpv * 8, cudaMemcpyDeviceToHost, st));
-    }
-    if (ctx->keep_final && n == 1 && !ragged) ctx->kept_final = a.mat_out;
-    if (matrices_out) {
+    if ((rc = outs.copy_out(ctx, dev, begin, L.rows_upto(begin), L.pv_upto(begin), cn, crows, cpv, st))) return rc;
+    if (b.keep_final) b.kept_final = a.mat_out;
+    if (b.matrices_out) {
       if (ragged) {
         for (int64_t i = begin; i < end; i++)
-          CU(ctx, cudaMemcpyAsync(matrices_out + mat_offsets[i], (double *)a.mat_out + (moff[i] - moff[begin]),
-                                  (size_t)heights[i] * widths[i] * 8, cudaMemcpyDeviceToHost, st));
+          CU(ctx, cudaMemcpyAsync(b.matrices_out + b.mat_offsets[i], (double *)a.mat_out + (L.moff[i] - L.moff[begin]),
+                                  (size_t)b.heights[i] * b.widths[i] * 8, cudaMemcpyDeviceToHost, st));
       } else {
-        CU(ctx, cudaMemcpyAsync(matrices_out + cells_upto(begin), a.mat_out, ccells * 8, cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaMemcpyAsync(b.matrices_out + L.cells_upto(begin), a.mat_out, ccells * 8, cudaMemcpyDeviceToHost, st));
       }
     }
     CU(ctx, cudaEventRecord(ctx->events[slot], st));
@@ -1519,31 +1570,47 @@ static int solve_host(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, 
   }
   for (int i = 0; i < 2; i++)
     if (used[i]) CU(ctx, cudaStreamSynchronize(ctx->streams[i]));
-  return check_device_status(ctx, status, n);
+  return check_device_status(ctx, b.status, n);
 }
+
+// Shared host-side solve of uniform and ragged batches: the zero-copy small call when the batch qualifies, else the
+// pipelined chunks.
+int solve_host(yalps_ctx *ctx, HostBatch &b) {
+  if (!ctx) return YALPS_ERR_ARGUMENT;
+  BatchLayout L;
+  if (int rc = batch_layout(ctx, b, &L)) return rc;
+  if (b.n == 0) return 0;
+  CU(ctx, cudaSetDevice(ctx->device));
+  bool taken;
+  if (int rc = solve_small(ctx, b, L, &taken)) return rc;
+  return taken ? 0 : solve_chunks(ctx, b, L);
+}
+
+}  // namespace
+
+extern "C" {
 
 int yalps_solve_batch(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
                       const yalps_options *opt, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
                       int32_t *pos_out, int32_t *var_out, double *matrices_out) {
-  return solve_host(ctx, n, height, width, nullptr, nullptr, nullptr, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out);
+  return yalps_solve_batch_ranging(ctx, n, height, width, matrices, nullptr, nullptr, opt, status, value, pivots, rhs_out,
+                                   pos_out, var_out, matrices_out, nullptr, nullptr, nullptr, nullptr);
 }
 
 int yalps_solve_ragged(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
                        const int64_t *mat_offsets, const double *matrices, const yalps_options *opt, int32_t *status,
                        double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                        double *matrices_out) {
-  if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
-  return solve_host(ctx, n, 0, 0, heights, widths, mat_offsets, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out);
+  return yalps_solve_ragged_ranging(ctx, n, heights, widths, mat_offsets, matrices, nullptr, nullptr, opt, status, value,
+                                    pivots, rhs_out, pos_out, var_out, matrices_out, nullptr, nullptr, nullptr, nullptr);
 }
 
 int yalps_solve_batch_basis(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
                             const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt, int32_t *status,
                             double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                             double *matrices_out) {
-  return solve_host(ctx, n, height, width, nullptr, nullptr, nullptr, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out, pos_in, var_in);
+  return yalps_solve_batch_ranging(ctx, n, height, width, matrices, pos_in, var_in, opt, status, value, pivots, rhs_out,
+                                   pos_out, var_out, matrices_out, nullptr, nullptr, nullptr, nullptr);
 }
 
 int yalps_solve_ragged_basis(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
@@ -1551,17 +1618,16 @@ int yalps_solve_ragged_basis(yalps_ctx *ctx, int64_t n, const int32_t *heights, 
                              const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
                              int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                              double *matrices_out) {
-  if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
-  return solve_host(ctx, n, 0, 0, heights, widths, mat_offsets, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out, pos_in, var_in);
+  return yalps_solve_ragged_ranging(ctx, n, heights, widths, mat_offsets, matrices, pos_in, var_in, opt, status, value,
+                                    pivots, rhs_out, pos_out, var_out, matrices_out, nullptr, nullptr, nullptr, nullptr);
 }
 
 int yalps_solve_batch_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
                             const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt, int32_t *status,
                             double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                             double *matrices_out, double *reduced_out) {
-  return solve_host(ctx, n, height, width, nullptr, nullptr, nullptr, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out);
+  return yalps_solve_batch_ranging(ctx, n, height, width, matrices, pos_in, var_in, opt, status, value, pivots, rhs_out,
+                                   pos_out, var_out, matrices_out, reduced_out, nullptr, nullptr, nullptr);
 }
 
 int yalps_solve_ragged_duals(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
@@ -1569,9 +1635,9 @@ int yalps_solve_ragged_duals(yalps_ctx *ctx, int64_t n, const int32_t *heights, 
                              const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
                              int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                              double *matrices_out, double *reduced_out) {
-  if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
-  return solve_host(ctx, n, 0, 0, heights, widths, mat_offsets, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out);
+  return yalps_solve_ragged_ranging(ctx, n, heights, widths, mat_offsets, matrices, pos_in, var_in, opt, status, value,
+                                    pivots, rhs_out, pos_out, var_out, matrices_out, reduced_out, nullptr, nullptr,
+                                    nullptr);
 }
 
 int yalps_solve_batch_ranging(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
@@ -1579,8 +1645,26 @@ int yalps_solve_batch_ranging(yalps_ctx *ctx, int64_t n, int32_t height, int32_t
                               double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                               double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
                               double *range_hi) {
-  return solve_host(ctx, n, height, width, nullptr, nullptr, nullptr, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out, pairs, range_lo, range_hi);
+  HostBatch b;
+  b.n = n;
+  b.height = height;
+  b.width = width;
+  b.matrices = matrices;
+  b.pos_in = pos_in;
+  b.var_in = var_in;
+  b.pairs = pairs;
+  b.opt = opt;
+  b.status = status;
+  b.value = value;
+  b.pivots = pivots;
+  b.rhs_out = rhs_out;
+  b.pos_out = pos_out;
+  b.var_out = var_out;
+  b.matrices_out = matrices_out;
+  b.reduced_out = reduced_out;
+  b.range_lo = range_lo;
+  b.range_hi = range_hi;
+  return solve_host(ctx, b);
 }
 
 int yalps_solve_ragged_ranging(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
@@ -1590,8 +1674,27 @@ int yalps_solve_ragged_ranging(yalps_ctx *ctx, int64_t n, const int32_t *heights
                                double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
                                double *range_hi) {
   if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
-  return solve_host(ctx, n, 0, 0, heights, widths, mat_offsets, matrices, opt, status, value, pivots, rhs_out,
-                    pos_out, var_out, matrices_out, pos_in, var_in, reduced_out, pairs, range_lo, range_hi);
+  HostBatch b;
+  b.n = n;
+  b.heights = heights;
+  b.widths = widths;
+  b.mat_offsets = mat_offsets;
+  b.matrices = matrices;
+  b.pos_in = pos_in;
+  b.var_in = var_in;
+  b.pairs = pairs;
+  b.opt = opt;
+  b.status = status;
+  b.value = value;
+  b.pivots = pivots;
+  b.rhs_out = rhs_out;
+  b.pos_out = pos_out;
+  b.var_out = var_out;
+  b.matrices_out = matrices_out;
+  b.reduced_out = reduced_out;
+  b.range_lo = range_lo;
+  b.range_hi = range_hi;
+  return solve_host(ctx, b);
 }
 
 // ---- replica path sharing (aux_kernels.cuh: k_replica_follow) ------------------------------------------------------
@@ -1829,6 +1932,7 @@ int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_
   // D2H of chunk k-1's results overlap the solve of chunk k
   const int64_t per_chunk = std::max<int64_t>(1, std::min<int64_t>((n + 1) / 2 > 4096 ? (n + 7) / 8 : n,
                                                                   (int64_t)(((size_t)1536 << 20) / (cells * 8))));
+  const Outputs outs(status, value, pivots, rhs_out, pos_out, var_out, reduced_out, nullptr, nullptr);
   bool used[2] = {false, false};
   int slot = 0;
   for (int64_t begin = 0; begin < n; begin += per_chunk, slot ^= 1) {
@@ -1836,22 +1940,16 @@ int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_
     const std::string s = "rp" + std::to_string(slot);
     cudaStream_t st = ctx->streams[slot];
     if (used[slot]) CU(ctx, cudaEventSynchronize(ctx->events[slot]));
-    void *d_rin, *d_work, *d_status, *d_value, *d_piv, *d_rhs, *d_pos, *d_var;
+    void *d_rin, *d_work, *dev[O_COUNT];
     if ((rc = dev_ensure(ctx, "rin" + s, (size_t)cn * height * 8, &d_rin))) return rc;
     if ((rc = dev_ensure(ctx, "work" + s, (size_t)cn * cells * 8, &d_work))) return rc;
-    if ((rc = dev_ensure(ctx, "status" + s, (size_t)cn * 4, &d_status))) return rc;
-    if ((rc = dev_ensure(ctx, "value" + s, (size_t)cn * 8, &d_value))) return rc;
-    if ((rc = dev_ensure(ctx, "pivots" + s, (size_t)cn * 16, &d_piv))) return rc;
-    if ((rc = dev_ensure(ctx, "rhs" + s, (size_t)cn * height * 8, &d_rhs))) return rc;
-    if ((rc = dev_ensure(ctx, "pos" + s, (size_t)cn * pv * 4, &d_pos))) return rc;
-    if ((rc = dev_ensure(ctx, "var" + s, (size_t)cn * pv * 4, &d_var))) return rc;
-    void *d_red = nullptr;
-    if (reduced_out && (rc = dev_ensure(ctx, "red" + s, (size_t)cn * pv * 8, &d_red))) return rc;
+    if ((rc = outs.ensure(ctx, s, cn, cn * height, cn * (long long)pv, dev))) return rc;
     CU(ctx, cudaMemcpyAsync(d_rin, rhs + (size_t)begin * height, (size_t)cn * height * 8, cudaMemcpyHostToDevice, st));
     if (trace.ok) {
-      if ((rc = replica_chunk_shared(ctx, trace, cn, height, width, (const double *)d_rin, (double *)d_work, opt, (int *)d_status,
-                                     (double *)d_value, (long long *)d_piv, (double *)d_rhs, (int *)d_pos, (int *)d_var,
-                                     (double *)d_red, st, s, &ctx->replica_forks)))
+      if ((rc = replica_chunk_shared(ctx, trace, cn, height, width, (const double *)d_rin, (double *)d_work, opt,
+                                     (int *)dev[O_STATUS], (double *)dev[O_VALUE], (long long *)dev[O_PIVOTS],
+                                     (double *)dev[O_RHS], (int *)dev[O_POS], (int *)dev[O_VAR], (double *)dev[O_RED],
+                                     st, s, &ctx->replica_forks)))
         return rc;
     } else {
       const size_t total = (size_t)cn * cells;
@@ -1860,18 +1958,13 @@ int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_
       CU(ctx, cudaGetLastError());
       ctx->launches++;
       if ((rc = solve_batch_device_impl(ctx, cn, height, width, (const double *)d_work, (double *)d_work, opt,
-                                        (int32_t *)d_status, (double *)d_value, (int64_t *)d_piv, (double *)d_rhs,
-                                        (int32_t *)d_pos, (int32_t *)d_var, nullptr, st, s, begin, (double *)d_red)))
+                                        (int32_t *)dev[O_STATUS], (double *)dev[O_VALUE], (int64_t *)dev[O_PIVOTS],
+                                        (double *)dev[O_RHS], (int32_t *)dev[O_POS], (int32_t *)dev[O_VAR], nullptr, st,
+                                        s, begin, (double *)dev[O_RED])))
         return rc;
     }
-    if (status) CU(ctx, cudaMemcpyAsync(status + begin, d_status, (size_t)cn * 4, cudaMemcpyDeviceToHost, st));
-    if (value) CU(ctx, cudaMemcpyAsync(value + begin, d_value, (size_t)cn * 8, cudaMemcpyDeviceToHost, st));
-    if (pivots) CU(ctx, cudaMemcpyAsync(pivots + 2 * begin, d_piv, (size_t)cn * 16, cudaMemcpyDeviceToHost, st));
-    if (rhs_out) CU(ctx, cudaMemcpyAsync(rhs_out + (size_t)begin * height, d_rhs, (size_t)cn * height * 8, cudaMemcpyDeviceToHost, st));
-    if (pos_out) CU(ctx, cudaMemcpyAsync(pos_out + (size_t)begin * pv, d_pos, (size_t)cn * pv * 4, cudaMemcpyDeviceToHost, st));
-    if (var_out) CU(ctx, cudaMemcpyAsync(var_out + (size_t)begin * pv, d_var, (size_t)cn * pv * 4, cudaMemcpyDeviceToHost, st));
-    if (reduced_out)
-      CU(ctx, cudaMemcpyAsync(reduced_out + (size_t)begin * pv, d_red, (size_t)cn * pv * 8, cudaMemcpyDeviceToHost, st));
+    if ((rc = outs.copy_out(ctx, dev, begin, begin * height, begin * (long long)pv, cn, cn * height, cn * (long long)pv, st)))
+      return rc;
     CU(ctx, cudaEventRecord(ctx->events[slot], st));
     used[slot] = true;
   }

@@ -46,6 +46,36 @@ def _pairs_in(pairs, n: int, rows: int):
     return p
 
 
+def _batch_outputs(n: int, height: int, width: int, want_matrices: bool = False, want_basis: bool = True,
+                   want_duals: bool = False, mk=np.empty) -> dict:
+    return {
+        "status": mk((n,), np.int32),
+        "value": mk((n,), np.float64),
+        "pivots": mk((n, 2), np.int64),
+        "rhs": mk((n, height), np.float64),
+        "pos": mk((n, width + height), np.int32) if want_basis else None,
+        "var": mk((n, width + height), np.int32) if want_basis else None,
+        "matrices": mk((n, height * width), np.float64) if want_matrices else None,
+        "reduced": mk((n, width + height), np.float64) if want_duals else None,
+    }
+
+
+def _add_outputs(out: dict, n: int, pv: int, want_duals: bool, want_ranges: bool = False):
+    """The reduced costs and ranges a call wants, added to a reused `out` that lacks them."""
+    for k, want in (("reduced", want_duals), ("range_lo", want_ranges), ("range_hi", want_ranges)):
+        if want and out.get(k) is None:
+            out[k] = np.empty((n, pv), np.float64)
+
+
+def _ragged_ranges(want_ranges: bool, pairs, rows: int, pvs: int) -> tuple:
+    """(range_lo, range_hi, packed pairs) of a ragged call, all None when no ranges are wanted."""
+    if not want_ranges:
+        return None, None, None
+    pr = None if pairs is None else _pairs_in(np.concatenate([np.asarray(p, np.int32).reshape(-1) for p in pairs]),
+                                              1, rows)
+    return np.empty(pvs, np.float64), np.empty(pvs, np.float64), pr
+
+
 def make_options(precision=1e-8, max_pivots=8192, check_cycles=False, tolerance=0.0, timeout_ms=math.inf,
                  max_iterations=32768) -> Options:
     o = Options()
@@ -129,17 +159,8 @@ class Engine:
     def batch_outputs(self, n: int, height: int, width: int, want_matrices: bool = False, want_basis: bool = True,
                       pinned: bool = False, want_duals: bool = False) -> dict:
         """Output buffers for solve_batch; pinned=True allocates them page-locked (reusable across calls)."""
-        mk = self.pinned_empty if pinned else (lambda shape, dtype: np.empty(shape, dtype))
-        return {
-            "status": mk((n,), np.int32),
-            "value": mk((n,), np.float64),
-            "pivots": mk((n, 2), np.int64),
-            "rhs": mk((n, height), np.float64),
-            "pos": mk((n, width + height), np.int32) if want_basis else None,
-            "var": mk((n, width + height), np.int32) if want_basis else None,
-            "matrices": mk((n, height * width), np.float64) if want_matrices else None,
-            "reduced": mk((n, width + height), np.float64) if want_duals else None,
-        }
+        return _batch_outputs(n, height, width, want_matrices, want_basis, want_duals,
+                              self.pinned_empty if pinned else np.empty)
 
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, want_basis: bool = True, out: Optional[dict] = None,
@@ -164,38 +185,14 @@ class Engine:
             out = self.batch_outputs(n, height, width, want_matrices, want_basis, want_duals=want_duals)
         elif out["status"].shape[0] != n:
             raise ValueError("out was allocated for a different batch size")
-        if want_duals and out.get("reduced") is None:
-            out["reduced"] = np.empty((n, width + height), np.float64)
-        if want_ranges:
-            for k in ("range_lo", "range_hi"):
-                if out.get(k) is None:
-                    out[k] = np.empty((n, width + height), np.float64)
-            p, v = _basis_in(pos_in, var_in, n * (width + height))
-            pr = _pairs_in(pairs, n, height)
-            self._check(self._lib.yalps_solve_batch_ranging(
-                self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
-                _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None, _ptr(pr), _ptr(out["range_lo"]),
-                _ptr(out["range_hi"])))
-            return out
-        if want_duals:
-            p, v = _basis_in(pos_in, var_in, n * (width + height))
-            self._check(self._lib.yalps_solve_batch_duals(self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v),
-                                                          C.byref(opt), _ptr(out["status"]), _ptr(out["value"]),
-                                                          _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]),
-                                                          _ptr(out["var"]), _ptr(out["matrices"]), _ptr(out["reduced"])))
-            return out
-        if pos_in is None and var_in is None:
-            self._check(self._lib.yalps_solve_batch(self._ctx, n, height, width, _ptr(m), C.byref(opt),
-                                                    _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
-                                                    _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                                                    _ptr(out["matrices"])))
-            return out
+        _add_outputs(out, n, width + height, want_duals, want_ranges)
         p, v = _basis_in(pos_in, var_in, n * (width + height))
-        self._check(self._lib.yalps_solve_batch_basis(self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt),
-                                                      _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
-                                                      _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                                                      _ptr(out["matrices"])))
+        pr = _pairs_in(pairs, n, height) if want_ranges else None
+        self._check(self._lib.yalps_solve_batch_ranging(
+            self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
+            _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
+            _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None, _ptr(pr),
+            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None))
         return out
 
     def simplex(self, tableau, options: Optional[Options] = None) -> tuple:
@@ -230,17 +227,11 @@ class Engine:
         n = r.size // height
         if out is None:
             out = self.batch_outputs(n, height, width, False, want_basis, want_duals=want_duals)
-        if not want_duals:
-            self._check(self._lib.yalps_solve_replicas(self._ctx, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
-                                                       _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
-                                                       _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"])))
-            return out
-        if out.get("reduced") is None:
-            out["reduced"] = np.empty((n, width + height), np.float64)
+        _add_outputs(out, n, width + height, want_duals)
         self._check(self._lib.yalps_solve_replicas_duals(self._ctx, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
                                                          _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
                                                          _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                                                         _ptr(out["reduced"])))
+                                                         _ptr(out["reduced"]) if want_duals else None))
         return out
 
     def set_replica_sharing(self, on: bool = True):
@@ -282,23 +273,11 @@ class Engine:
         var = np.empty(int(poffs[-1]), np.int32)
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
         red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
-        if want_ranges:
-            rlo, rhi = np.empty(int(poffs[-1]), np.float64), np.empty(int(poffs[-1]), np.float64)
-            pr = None if pairs is None else _pairs_in(np.concatenate([np.asarray(p, np.int32).reshape(-1) for p in pairs]),
-                                                      1, int(roffs[-1]))
-            self._check(self._lib.yalps_solve_ragged_ranging(
-                self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
-                _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
-                _ptr(rlo), _ptr(rhi)))
-        elif want_duals:
-            self._check(self._lib.yalps_solve_ragged_duals(self._ctx, n, _ptr(heights), _ptr(widths),
-                                                           _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
-                                                           _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos),
-                                                           _ptr(var), _ptr(mats), _ptr(red)))
-        else:
-            self._check(self._lib.yalps_solve_ragged(self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()),
-                                                     _ptr(packed), C.byref(opt), _ptr(status), _ptr(value), _ptr(pivots),
-                                                     _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats)))
+        rlo, rhi, pr = _ragged_ranges(want_ranges, pairs, int(roffs[-1]), int(poffs[-1]))
+        self._check(self._lib.yalps_solve_ragged_ranging(
+            self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
+            _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
+            _ptr(rlo), _ptr(rhi)))
         res = []
         for i in range(n):
             res.append({
@@ -320,15 +299,10 @@ class Engine:
         d_reduced (float64, n*(width+height)): reduced costs per variable id, as solve_batch's out["reduced"]."""
         opt = options or make_options()
         z = lambda p: C.c_void_p(p) if p else None
-        if d_reduced:
-            self._check(self._lib.yalps_solve_batch_device_duals(self._ctx, n, height, width, z(d_matrices), z(d_work),
-                                                                 C.byref(opt), z(d_status), z(d_value), z(d_pivots),
-                                                                 z(d_rhs), z(d_pos), z(d_var), z(d_matrices_out),
-                                                                 z(stream), z(d_reduced)))
-            return
-        self._check(self._lib.yalps_solve_batch_device(self._ctx, n, height, width, z(d_matrices), z(d_work),
-                                                       C.byref(opt), z(d_status), z(d_value), z(d_pivots), z(d_rhs),
-                                                       z(d_pos), z(d_var), z(d_matrices_out), z(stream)))
+        self._check(self._lib.yalps_solve_batch_device_duals(self._ctx, n, height, width, z(d_matrices), z(d_work),
+                                                             C.byref(opt), z(d_status), z(d_value), z(d_pivots),
+                                                             z(d_rhs), z(d_pos), z(d_var), z(d_matrices_out),
+                                                             z(stream), z(d_reduced)))
 
     def ranging_device(self, n: int, height: int, width: int, d_matrices: int, d_pos: int, d_range_lo: int,
                        d_range_hi: int, precision: float = 1e-8, d_status: int = 0, d_pairs: int = 0, stream: int = 0):
@@ -580,47 +554,22 @@ class MultiEngine:
             if self._lib.yalps_set_tuning(ctx, path, threads_per_lp) or self._lib.yalps_set_row_groups(ctx, row_groups):
                 raise YalpsError(-2, (self._lib.yalps_last_error(ctx) or b"").decode())
 
-    @staticmethod
-    def _outputs(n, height, width, want_matrices, want_duals=False):
-        return {"status": np.empty(n, np.int32), "value": np.empty(n, np.float64), "pivots": np.empty((n, 2), np.int64),
-                "rhs": np.empty((n, height), np.float64), "pos": np.empty((n, width + height), np.int32),
-                "var": np.empty((n, width + height), np.int32),
-                "matrices": np.empty((n, height * width), np.float64) if want_matrices else None,
-                "reduced": np.empty((n, width + height), np.float64) if want_duals else None}
-
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, pos_in=None, var_in=None, out: Optional[dict] = None,
                     want_duals: bool = False, want_ranges: bool = False, pairs=None) -> dict:
         opt = options or make_options()
         m = np.ascontiguousarray(matrices, np.float64).reshape(-1)
         n = m.size // (height * width)
-        out = out or self._outputs(n, height, width, want_matrices, want_duals)
+        out = out or _batch_outputs(n, height, width, want_matrices, want_duals=want_duals)
         p = None if pos_in is None else np.ascontiguousarray(pos_in, np.int32).reshape(-1)
         v = None if var_in is None else np.ascontiguousarray(var_in, np.int32).reshape(-1)
-        if want_ranges:
-            for k in ("range_lo", "range_hi"):
-                if out.get(k) is None:
-                    out[k] = np.empty((n, width + height), np.float64)
-            if want_duals and out.get("reduced") is None:
-                out["reduced"] = np.empty((n, width + height), np.float64)
-            self._check(self._lib.yalps_multi_solve_batch_ranging(
-                self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
-                _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None, _ptr(_pairs_in(pairs, n, height)),
-                _ptr(out["range_lo"]), _ptr(out["range_hi"])))
-            return out
-        if want_duals:
-            if out.get("reduced") is None:
-                out["reduced"] = np.empty((n, width + height), np.float64)
-            self._check(self._lib.yalps_multi_solve_batch_duals(
-                self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
-                _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                _ptr(out["matrices"]), _ptr(out["reduced"])))
-            return out
-        self._check(self._lib.yalps_multi_solve_batch(self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt),
-                                                      _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
-                                                      _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                                                      _ptr(out["matrices"])))
+        _add_outputs(out, n, width + height, want_duals, want_ranges)
+        self._check(self._lib.yalps_multi_solve_batch_ranging(
+            self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
+            _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
+            _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None,
+            _ptr(_pairs_in(pairs, n, height)) if want_ranges else None,
+            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None))
         return out
 
     def solve_replicas(self, base: np.ndarray, rhs: np.ndarray, height: int, width: int,
@@ -629,17 +578,12 @@ class MultiEngine:
         b = np.ascontiguousarray(base, np.float64).reshape(-1)
         r = np.ascontiguousarray(rhs, np.float64).reshape(-1)
         n = r.size // height
-        out = out or self._outputs(n, height, width, False, want_duals)
-        if want_duals:
-            if out.get("reduced") is None:
-                out["reduced"] = np.empty((n, width + height), np.float64)
-            self._check(self._lib.yalps_multi_solve_replicas_duals(
-                self._m, n, height, width, _ptr(b), _ptr(r), C.byref(opt), _ptr(out["status"]), _ptr(out["value"]),
-                _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]), _ptr(out["reduced"])))
-            return out
-        self._check(self._lib.yalps_multi_solve_replicas(self._m, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
-                                                         _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
-                                                         _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"])))
+        out = out or _batch_outputs(n, height, width, want_duals=want_duals)
+        _add_outputs(out, n, width + height, want_duals)
+        self._check(self._lib.yalps_multi_solve_replicas_duals(
+            self._m, n, height, width, _ptr(b), _ptr(r), C.byref(opt), _ptr(out["status"]), _ptr(out["value"]),
+            _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
+            _ptr(out["reduced"]) if want_duals else None))
         return out
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
@@ -662,22 +606,11 @@ class MultiEngine:
         rhs, pos, var = np.empty(int(roffs[-1])), np.empty(int(poffs[-1]), np.int32), np.empty(int(poffs[-1]), np.int32)
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
         red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
-        if want_ranges:
-            rlo, rhi = np.empty(int(poffs[-1]), np.float64), np.empty(int(poffs[-1]), np.float64)
-            pr = None if pairs is None else _pairs_in(np.concatenate([np.asarray(p, np.int32).reshape(-1) for p in pairs]),
-                                                      1, int(roffs[-1]))
-            self._check(self._lib.yalps_multi_solve_ragged_ranging(
-                self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
-                _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
-                _ptr(rlo), _ptr(rhi)))
-        elif want_duals:
-            self._check(self._lib.yalps_multi_solve_ragged_duals(
-                self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
-                _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red)))
-        else:
-            self._check(self._lib.yalps_multi_solve_ragged(self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()),
-                                                           _ptr(packed), C.byref(opt), _ptr(status), _ptr(value),
-                                                           _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats)))
+        rlo, rhi, pr = _ragged_ranges(want_ranges, pairs, int(roffs[-1]), int(poffs[-1]))
+        self._check(self._lib.yalps_multi_solve_ragged_ranging(
+            self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
+            _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
+            _ptr(rlo), _ptr(rhi)))
         res = [{"status": int(status[i]), "value": float(value[i]), "pivots": (int(pivots[i, 0]), int(pivots[i, 1])),
                 "rhs": rhs[roffs[i]:roffs[i + 1]], "pos": pos[poffs[i]:poffs[i + 1]], "var": var[poffs[i]:poffs[i + 1]],
                 "matrix": mats[offs[i]:offs[i + 1]] if want_matrices else None} for i in range(n)]
