@@ -371,6 +371,52 @@ int yalps_ranging_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t widt
                          const int32_t *d_pos, const int32_t *d_status, const int32_t *d_pairs, double precision,
                          double *d_range_lo, double *d_range_hi, void *stream);
 
+/* ---- certificates: why an LP is infeasible or unbounded ----------------------------------------------------
+ * One double per variable id (packed like pos_out, width + height per LP), read from the final tableau M, its
+ * positionOfVariable pos, and the status and value the call reports:
+ *   infeasible (status 1), a Farkas certificate.  r is the row phase 1 chose: the lowest r in 1..height-1 whose
+ *     M[r,0] is the minimum over the rows with M[r,0] < -opt->precision (NaN never qualifies, -inf does).  Phase 1
+ *     stops there without a pivot, so the final tableau is the tableau of that choice.
+ *       cert[0] = M[r,0], cert[width] = +0.0, and for every other id v:
+ *       cert[v] = M[r, pos[v]] if 1 <= pos[v] < width (bits as they are), 1.0 if pos[v] == width + r, +0.0 otherwise.
+ *     cert[width + k] is the multiplier y_k >= -precision of original row k (a_k.x <= b_k); the structural entries
+ *     equal sum_k y_k a_kj >= -precision and cert[0] = sum_k y_k b_k < 0, so no x >= 0 satisfies every row.
+ *   unbounded (status 2), a ray.  c = (int)value is the entering column.
+ *       cert[0] = M[0,c] (d result / dt = sign * cert[0], the convention of reduced_out), cert[width] = +0.0, and
+ *       cert[v] = 1.0 if pos[v] == c, -M[pos[v] - width, c] if width < pos[v] < width + height (the sign bit
+ *       flipped), +0.0 otherwise.
+ *     Moving every variable by t * cert[v] keeps every row feasible and improves the objective without bound.
+ *   Every other status, an infeasible LP with no qualifying row and an unbounded LP with c outside 1..width-1: NaN.
+ * The values are raw tableau cells (nothing below precision is cleaned), bit-exact whatever the kernel path.
+ * k_certificate computes them on the device from the final tableaus after the solve, like k_ranging; they cost
+ * 8*(width+height) bytes of device-to-host copy per LP.  e.g. max p with c: x <= -1 and p = x: infeasible,
+ * cert = [-1, 1, +0, 1].
+ *
+ * Each *_certificate entry takes its *_ranging sibling's arguments plus a trailing cert_out (NULL: the sibling
+ * exactly).
+ */
+int yalps_solve_batch_certificate(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
+                                  const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt,
+                                  int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
+                                  int32_t *var_out, double *matrices_out, double *reduced_out, const int32_t *pairs,
+                                  double *range_lo, double *range_hi, double *cert_out);
+int yalps_solve_ragged_certificate(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
+                                   const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                                   const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                                   int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                                   double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                                   double *range_hi, double *cert_out);
+int yalps_solve_sparse_certificate(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nnz, const int32_t *cell,
+                                   const double *val, const yalps_options *opt, int32_t *status, double *value,
+                                   int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                                   double *reduced_out, const int32_t *pairs, double *range_lo, double *range_hi,
+                                   double *cert_out);
+/* Certificates of n final tableaus already in device memory, with their positionOfVariable d_pos, status d_status and
+ * value d_value as a solve reported them.  Every pointer is device memory; the kernel is enqueued on `stream`. */
+int yalps_certificate_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                             const int32_t *d_pos, const int32_t *d_status, const double *d_value, double precision,
+                             double *d_cert_out, void *stream);
+
 /* ---- one process, several GPUs (SURVEY 8b/8e) ------------------------------------------------------------
  * The reference is single-process and synchronous (src/YALPS.ts:73-92); a Node addon cannot use torchrun.  A
  * yalps_multi owns one ctx (plus worker ctxs for concurrent branch-and-cut searches) per entry of `devices` and one
@@ -421,6 +467,18 @@ int yalps_multi_solve_ragged_ranging(yalps_multi *m, int64_t n, const int32_t *h
                                      int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
                                      int32_t *var_out, double *matrices_out, double *reduced_out, const int32_t *pairs,
                                      double *range_lo, double *range_hi);
+/* the two above + cert_out (see "certificates"), sharded like pos_out */
+int yalps_multi_solve_batch_certificate(yalps_multi *m, int64_t n, int32_t height, int32_t width,
+                                        const double *matrices, const int32_t *pos_in, const int32_t *var_in,
+                                        const yalps_options *opt, int32_t *status, double *value, int64_t *pivots,
+                                        double *rhs_out, int32_t *pos_out, int32_t *var_out, double *matrices_out,
+                                        double *reduced_out, const int32_t *pairs, double *range_lo, double *range_hi,
+                                        double *cert_out);
+int yalps_multi_solve_ragged_certificate(yalps_multi *m, int64_t n, const int32_t *heights, const int32_t *widths,
+                                         const int64_t *mat_offsets, const double *matrices, const yalps_options *opt,
+                                         int32_t *status, double *value, int64_t *pivots, double *rhs_out,
+                                         int32_t *pos_out, int32_t *var_out, double *matrices_out, double *reduced_out,
+                                         const int32_t *pairs, double *range_lo, double *range_hi, double *cert_out);
 /*
  * incumbent_allreduce (SURVEY 8b, north_star): min-allreduce of one fp64 per rank -- the incumbent objective of a
  * branch-and-bound search, lower is better internally (src/branchAndCut.ts:124,130).  local[ndev] in, agreed[ndev]

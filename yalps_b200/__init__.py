@@ -9,8 +9,8 @@ from .constraint import equal_to, equalTo, greater_eq, greaterEq, in_range, inRa
 from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
 from .solver import default_options, defaultOptions, get_engine, solve, solve_many, solveMany
 from .mps import apply_bounds, model_from_mps, netlib_model
-from .sensitivity import (model_ranges, model_sensitivity, ranges_from_tableau, reduced_from_tableau, row_pairs,
-                          split_reduced)
+from .sensitivity import (certificate_from_tableau, model_certificate, model_ranges, model_sensitivity,
+                          ranges_from_tableau, reduced_from_tableau, row_pairs, split_reduced)
 from .tableau import Tableau, TableauModel, constraint_rows, tableau_model
 
 __all__ = [
@@ -18,5 +18,5 @@ __all__ = [
     "in_range", "lessEq", "greaterEq", "equalTo", "inRange", "Engine", "MultiEngine", "make_options", "STATUS_NAMES",
     "tableau_model", "Tableau", "TableauModel", "get_engine", "model_from_mps", "netlib_model", "apply_bounds",
     "constraint_rows", "split_reduced", "model_sensitivity", "reduced_from_tableau", "ranges_from_tableau", "row_pairs",
-    "model_ranges",
+    "model_ranges", "certificate_from_tableau", "model_certificate",
 ]

@@ -41,16 +41,42 @@ constexpr int kRngTileCols = 256;   // tile mode: threads per CTA, one column ea
 constexpr int kRngTileRows = 128;   // tile mode: rows per tile
 constexpr int kRngBatch = 4;        // rows whose loads are issued together
 
-struct RangingArgs {
+// The LPs a post-pass over final tableaus visits (k_ranging, k_certificate): uniform or ragged, optionally through the
+// `index` of a ragged group, packed like the solve's outputs.
+struct PostArgs {
   long long n;
   int H, W;                                       // uniform shape (heights == nullptr)
-  int Hcap, Wcap;                                 // largest LP of the launch (warp-mode shared memory, tile grid)
+  int Hcap, Wcap;                                 // largest LP of the launch (warp or CTA decomposition)
   const double *M;                                // final tableaus, packed like mat_out
   const int *heights, *widths;                    // ragged (nullable)
   const long long *mat_off, *rhs_off, *pos_off;
   const int *index;                               // launch-local LP -> LP id (nullable)
   const int *pos;                                 // positionOfVariable, packed like pos_out
-  const int *status;                              // nullable: every LP is optimal
+  const int *status;                              // nullable (k_ranging: every LP is optimal)
+};
+
+// one warp per LP for tableaus up to 256 x 128, else a wider decomposition
+inline bool post_warp_mode(const PostArgs &a) { return a.Wcap <= 128 && a.Hcap <= 256; }
+
+// LP i of a post-pass launch: its id, shape and the offsets of its tableau, rows and variable ids
+struct PostLP {
+  long long id, mo, ro, po;
+  int H, W;
+};
+
+__device__ __forceinline__ PostLP post_lp(const PostArgs &a, long long i) {
+  PostLP P;
+  P.id = a.index ? a.index[i] : i;
+  const bool ragged = a.heights != nullptr;
+  P.H = ragged ? a.heights[P.id] : a.H;
+  P.W = ragged ? a.widths[P.id] : a.W;
+  P.mo = ragged ? a.mat_off[P.id] : P.id * (long long)a.H * a.W;
+  P.ro = ragged ? a.rhs_off[P.id] : P.id * (long long)a.H;
+  P.po = ragged ? a.pos_off[P.id] : P.id * (long long)(a.H + a.W);
+  return P;
+}
+
+struct RangingArgs : PostArgs {
   const int *pairs;                               // nullable: per row, the other row of its key or -1 (like rhs_out)
   double precision;
   double *lo, *hi;                                // outputs, packed like pos_out
@@ -69,21 +95,17 @@ struct RngLP {
 };
 
 __device__ __forceinline__ RngLP rng_lp(const RangingArgs &a, long long i) {
-  const long long id = a.index ? a.index[i] : i;
-  const bool ragged = a.heights != nullptr;
+  const PostLP P = post_lp(a, i);
   RngLP L;
-  L.H = ragged ? a.heights[id] : a.H;
-  L.W = ragged ? a.widths[id] : a.W;
-  const long long mo = ragged ? a.mat_off[id] : id * (long long)a.H * a.W;
-  const long long ro = ragged ? a.rhs_off[id] : id * (long long)a.H;
-  const long long po = ragged ? a.pos_off[id] : id * (long long)(a.H + a.W);
-  L.M = a.M + mo;
-  L.pos = a.pos + po;
-  L.pairs = a.pairs ? a.pairs + ro : nullptr;
-  L.lo = a.lo + po;
-  L.hi = a.hi + po;
-  L.var = a.var ? a.var + po : nullptr;
-  L.optimal = !a.status || a.status[id] == ST_OPTIMAL;
+  L.H = P.H;
+  L.W = P.W;
+  L.M = a.M + P.mo;
+  L.pos = a.pos + P.po;
+  L.pairs = a.pairs ? a.pairs + P.ro : nullptr;
+  L.lo = a.lo + P.po;
+  L.hi = a.hi + P.po;
+  L.var = a.var ? a.var + P.po : nullptr;
+  L.optimal = !a.status || a.status[P.id] == ST_OPTIMAL;
   return L;
 }
 

@@ -33,6 +33,7 @@
 #include "cluster_kernel.cuh"
 #include "grid_kernel.cuh"
 #include "multigrid_kernel.cuh"
+#include "certificate_kernel.cuh"
 #include "ranging_kernel.cuh"
 #include "tmem_launch.h"
 #include "bnb_launch.h"
@@ -777,7 +778,7 @@ int check_device_status(yalps_ctx *ctx, const int32_t *status, long long n) {
 int launch_ranging(yalps_ctx *ctx, RangingArgs a, size_t pv_total, const std::string &slot, cudaStream_t stream) {
   if (a.n <= 0) return 0;
   const long long sms = ctx->prop.multiProcessorCount;
-  if (a.Wcap <= 128 && a.Hcap <= 256) {
+  if (post_warp_mode(a)) {
     a.warp_smem = (((size_t)(a.Hcap + a.Wcap) * 4 + 15) & ~(size_t)15) + (size_t)16 * a.Hcap;
     const long long blocks = std::min<long long>((a.n + kRngWarps - 1) / kRngWarps, sms * 64);
     k_ranging<<<(unsigned)blocks, kRngWarps * 32, kRngWarps * a.warp_smem, stream>>>(a, kRngWarp);
@@ -796,6 +797,18 @@ int launch_ranging(yalps_ctx *ctx, RangingArgs a, size_t pv_total, const std::st
   k_ranging<<<(unsigned)std::min<long long>(tiles, sms * 64), kRngTileCols, 0, stream>>>(a, kRngTiles);
   CU(ctx, cudaGetLastError());
   ctx->launches += 2;
+  return 0;
+}
+
+// k_certificate over the LPs of `a`: one warp per LP when post_warp_mode allows it, else one CTA per LP.
+int launch_certificate(yalps_ctx *ctx, const CertArgs &a, cudaStream_t stream) {
+  if (a.n <= 0) return 0;
+  const bool warp = post_warp_mode(a);
+  const long long per_block = warp ? kCertThreads / 32 : 1;
+  const long long blocks = std::min<long long>((a.n + per_block - 1) / per_block, ctx->prop.multiProcessorCount * 64LL);
+  k_certificate<<<(unsigned)blocks, kCertThreads, 0, stream>>>(a, warp ? 1 : 0);
+  CU(ctx, cudaGetLastError());
+  ctx->launches++;
   return 0;
 }
 
@@ -1043,13 +1056,36 @@ int yalps_ranging_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t widt
   return launch_ranging(ctx, a, (size_t)n * (width + height), "dev", (cudaStream_t)stream);
 }
 
+int yalps_certificate_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                             const int32_t *d_pos, const int32_t *d_status, const double *d_value, double precision,
+                             double *d_cert_out, void *stream) {
+  if (!ctx) return YALPS_ERR_ARGUMENT;
+  if (n < 0 || height < 1 || width < 1 ||
+      (n > 0 && (!d_matrices || !d_pos || !d_status || !d_value || !d_cert_out)))
+    return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", (long long)n, height, width);
+  if ((long long)height * width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
+  if (n == 0) return 0;
+  CU(ctx, cudaSetDevice(ctx->device));
+  CertArgs a{};
+  a.n = n;
+  a.H = a.Hcap = height;
+  a.W = a.Wcap = width;
+  a.M = d_matrices;
+  a.pos = d_pos;
+  a.status = d_status;
+  a.value = d_value;
+  a.precision = precision;
+  a.cert = d_cert_out;
+  return launch_certificate(ctx, a, (cudaStream_t)stream);
+}
+
 }  // extern "C"
 
 // ---- host batches --------------------------------------------------------------------------------------------------
 namespace {
 
 // One host batch solve: the shape, where the tableaus come from, the optional inputs and every output (null: not
-// wanted).  The yalps_solve_{batch,ragged}_ranging entries, yalps_solve's root LP and the sparse entries fill one in.
+// wanted).  The yalps_solve_{batch,ragged}_certificate entries, yalps_solve's root LP and the sparse entries fill one in.
 struct HostBatch {
   int64_t n = 0;
   int32_t height = 0, width = 0;                        // a uniform batch, or
@@ -1068,10 +1104,13 @@ struct HostBatch {
   double *rhs_out = nullptr;
   int32_t *pos_out = nullptr, *var_out = nullptr;
   double *matrices_out = nullptr, *reduced_out = nullptr, *range_lo = nullptr, *range_hi = nullptr;
+  double *cert_out = nullptr;
   bool keep_final = false;  // (n == 1, uniform) leave the final tableau on the device, no D2H copy of it
   // results
   double *kept_final = nullptr;  // keep_final: where the final tableau is (valid until the next batch call on the ctx)
   int32_t dup_cells = 0;         // nnz >= 0: the device found duplicate cells with different values
+  // a post-pass (k_ranging, k_certificate) reads the final tableaus, which therefore stay in device memory
+  bool post_pass() const { return range_lo != nullptr || cert_out != nullptr; }
 };
 
 // The per-LP outputs of a host batch, described once: pool name, host array (null: not wanted), element size and
@@ -1090,18 +1129,19 @@ struct OutSpec {
     return elem * (size_t)(pack == PER_LP ? lps * k : pack == PER_ROW ? rows : pvs);
   }
 };
-enum { O_STATUS, O_VALUE, O_PIVOTS, O_RHS, O_POS, O_VAR, O_RED, O_RLO, O_RHI, O_COUNT };
+enum { O_STATUS, O_VALUE, O_PIVOTS, O_RHS, O_POS, O_VAR, O_RED, O_RLO, O_RHI, O_CERT, O_COUNT };
 struct Outputs {
   OutSpec t[O_COUNT];
   Outputs(int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
-          double *reduced_out, double *range_lo, double *range_hi)
+          double *reduced_out, double *range_lo, double *range_hi, double *cert_out)
       : t{{"status", status, 4, PER_LP, 1, true},     {"value", value, 8, PER_LP, 1, true},
           {"pivots", pivots, 8, PER_LP, 2, true},     {"rhs", rhs_out, 8, PER_ROW, 1, true},
           {"pos", pos_out, 4, PER_VAR, 1, true},      {"var", var_out, 4, PER_VAR, 1, true},
           {"red", reduced_out, 8, PER_VAR, 1, false}, {"rlo", range_lo, 8, PER_VAR, 1, false},
-          {"rhi", range_hi, 8, PER_VAR, 1, false}} {}
+          {"rhi", range_hi, 8, PER_VAR, 1, false},    {"cert", cert_out, 8, PER_VAR, 1, false}} {}
   explicit Outputs(const HostBatch &b)
-      : Outputs(b.status, b.value, b.pivots, b.rhs_out, b.pos_out, b.var_out, b.reduced_out, b.range_lo, b.range_hi) {}
+      : Outputs(b.status, b.value, b.pivots, b.rhs_out, b.pos_out, b.var_out, b.reduced_out, b.range_lo, b.range_hi,
+                b.cert_out) {}
 
   // device buffers "<name><slot>" for a chunk of `lps` LPs (`rows` rows, `pvs` variable ids); null where not used
   int ensure(yalps_ctx *ctx, const std::string &slot, long long lps, long long rows, long long pvs, void **dev) const {
@@ -1133,6 +1173,46 @@ void set_outputs(BatchArgs &a, void *const *dev) {
   a.red_out = (double *)dev[O_RED];
 }
 
+// The post-passes `b` wants (k_ranging, then k_certificate) over the final tableaus M of the LPs `a` solved (all LPs
+// of a launch, or one ragged group through a.index), on the solve's stream before the copies back.  pairs: device
+// copy of the request's pairs, or null; pv_total: the variable ids of the layout a's offsets index into.
+int post_passes(yalps_ctx *ctx, const HostBatch &b, const BatchArgs &a, const double *M, const int *pairs,
+                void *const *dev, size_t pv_total, const std::string &slot, cudaStream_t st) {
+  PostArgs p{};
+  p.n = a.n;
+  p.H = a.H;
+  p.W = a.W;
+  p.Hcap = a.Hcap;
+  p.Wcap = a.Wcap;
+  p.M = M;
+  p.heights = a.heights;
+  p.widths = a.widths;
+  p.mat_off = a.mat_off;
+  p.rhs_off = a.rhs_off;
+  p.pos_off = a.pos_off;
+  p.index = a.index;
+  p.pos = a.pos_out;
+  p.status = a.status;
+  if (b.range_lo) {
+    RangingArgs g{};
+    static_cast<PostArgs &>(g) = p;
+    g.pairs = pairs;
+    g.precision = b.opt->precision;
+    g.lo = (double *)dev[O_RLO];
+    g.hi = (double *)dev[O_RHI];
+    if (int rc = launch_ranging(ctx, g, pv_total, slot, st)) return rc;
+  }
+  if (b.cert_out) {
+    CertArgs g{};
+    static_cast<PostArgs &>(g) = p;
+    g.value = a.value;
+    g.precision = b.opt->precision;
+    g.cert = (double *)dev[O_CERT];
+    if (int rc = launch_certificate(ctx, g, st)) return rc;
+  }
+  return 0;
+}
+
 // What solve_host derives from a valid request: the caps and the per-LP prefix counts of cells, rows and variable ids.
 struct BatchLayout {
   bool ragged = false;
@@ -1156,7 +1236,6 @@ int batch_layout(yalps_ctx *ctx, const HostBatch &b, BatchLayout *L) {
   L->ragged = b.heights != nullptr;
   L->height = L->Hcap = b.height;
   L->width = L->Wcap = b.width;
-  // ranging: k_ranging runs over the final tableaus after the solve, which therefore stay in device memory
   L->pairs = b.range_lo ? b.pairs : nullptr;
   if (L->ragged) {
     if (!b.widths || !b.mat_offsets) return fail(ctx, YALPS_ERR_ARGUMENT, "ragged batch needs widths and mat_offsets");
@@ -1220,14 +1299,15 @@ double first_density(const HostBatch &b) {
 int solve_small(yalps_ctx *ctx, const HostBatch &b, const BatchLayout &L, bool *taken) {
   *taken = false;
   const int64_t n = b.n;
-  const bool ragged = L.ragged, want_rng = b.range_lo != nullptr;
+  const bool ragged = L.ragged, post = b.post_pass();
   const long long rows = L.rows_upto(n), pvs = L.pv_upto(n);
   const size_t in_b = (size_t)L.cells_upto(n) * 8, rows_b = (size_t)rows * 8, pv_b = (size_t)pvs * 4;
   const size_t red_b = b.reduced_out ? 2 * pv_b : 0;  // doubles, packed like pos_out
-  const size_t rng_b = want_rng ? 2 * pv_b : 0;       // range_lo, range_hi: doubles, packed like pos_out
+  const size_t rng_b = b.range_lo ? 2 * pv_b : 0;     // range_lo, range_hi: doubles, packed like pos_out
+  const size_t cert_b = b.cert_out ? 2 * pv_b : 0;    // doubles, packed like pos_out
   const size_t pair_b = L.pairs ? rows_b / 2 : 0;     // int32, packed like rhs_out
   const size_t out_b = (size_t)n * 32 + rows_b + 2 * pv_b + 64 + (b.matrices_out ? in_b : 0) + (red_b ? red_b + 16 : 0) +
-                       (rng_b ? 2 * rng_b + 32 : 0);
+                       (rng_b ? 2 * rng_b + 32 : 0) + (cert_b ? cert_b + 16 : 0);
   const size_t desc_b = (ragged ? (size_t)n * 32 + 64 : 0) + (b.var_in ? pv_b + 16 : 0) + (pair_b ? pair_b + 16 : 0);
   Route route;
   if (b.keep_final || b.nnz >= 0 || in_b + out_b + desc_b > ((size_t)768 << 10) ||
@@ -1257,9 +1337,9 @@ int solve_small(yalps_ctx *ctx, const HostBatch &b, const BatchLayout &L, bool *
   if ((rc = pin_ensure(ctx, "small_io", o + 16, &hb))) return rc;
   if ((rc = pin_device_ptr(ctx, hb, &db))) return rc;
   char *h = (char *)hb, *d = (char *)db;
-  // ranging reads the final tableaus from device scratch, not over PCIe from the mapped buffer
+  // the post-passes read the final tableaus from device scratch, not over PCIe from the mapped buffer
   void *d_fin = nullptr;
-  if (want_rng && (rc = dev_ensure(ctx, "small_final", in_b, &d_fin))) return rc;
+  if (post && (rc = dev_ensure(ctx, "small_final", in_b, &d_fin))) return rc;
   if (L.pairs) std::memcpy(h + o_pair, L.pairs, pair_b);
   if (ragged) {
     for (int64_t i = 0; i < n; i++)
@@ -1284,7 +1364,7 @@ int solve_small(yalps_ctx *ctx, const HostBatch &b, const BatchLayout &L, bool *
   a.Wcap = L.Wcap;
   a.in = (const double *)(d + o_in);
   a.work = nullptr;
-  a.mat_out = want_rng ? (double *)d_fin : b.matrices_out ? (double *)(d + o_mat) : nullptr;
+  a.mat_out = post ? (double *)d_fin : b.matrices_out ? (double *)(d + o_mat) : nullptr;
   set_outputs(a, dev);
   a.var_in = b.var_in ? (const int *)(d + o_vin) : nullptr;
   if (ragged) {
@@ -1297,26 +1377,9 @@ int solve_small(yalps_ctx *ctx, const HostBatch &b, const BatchLayout &L, bool *
   fill_options(a, b.opt);
   cudaStream_t st = ctx->streams[0];
   if ((rc = launch_route(ctx, route, a, "small", st))) return rc;
-  if (want_rng) {
-    RangingArgs g{};
-    g.n = n;
-    g.H = L.height;
-    g.W = L.width;
-    g.Hcap = L.Hcap;
-    g.Wcap = L.Wcap;
-    g.M = (const double *)d_fin;
-    g.heights = a.heights;
-    g.widths = a.widths;
-    g.mat_off = a.mat_off;
-    g.rhs_off = a.rhs_off;
-    g.pos_off = a.pos_off;
-    g.pos = a.pos_out;
-    g.status = a.status;
-    g.pairs = L.pairs ? (const int *)(d + o_pair) : nullptr;
-    g.precision = b.opt->precision;
-    g.lo = (double *)dev[O_RLO];
-    g.hi = (double *)dev[O_RHI];
-    if ((rc = launch_ranging(ctx, g, (size_t)pvs, "small", st))) return rc;
+  if (post) {
+    const int *pairs = L.pairs ? (const int *)(d + o_pair) : nullptr;
+    if ((rc = post_passes(ctx, b, a, (const double *)d_fin, pairs, dev, (size_t)pvs, "small", st))) return rc;
     if (b.matrices_out) CU(ctx, cudaMemcpyAsync(h + o_mat, d_fin, in_b, cudaMemcpyDeviceToHost, st));
   }
   CU(ctx, cudaStreamSynchronize(st));
@@ -1337,7 +1400,7 @@ int solve_small(yalps_ctx *ctx, const HostBatch &b, const BatchLayout &L, bool *
 // chunk k+1 overlaps the kernel and the D2H copies of chunk k.
 int solve_chunks(yalps_ctx *ctx, HostBatch &b, const BatchLayout &L) {
   const int64_t n = b.n;
-  const bool ragged = L.ragged, want_rng = b.range_lo != nullptr;
+  const bool ragged = L.ragged;
   const yalps_options *opt = b.opt;
   const Outputs outs(b);
   const size_t total_bytes = (size_t)L.cells_upto(n) * 8;
@@ -1389,7 +1452,7 @@ int solve_chunks(yalps_ctx *ctx, HostBatch &b, const BatchLayout &L) {
       CU(ctx, cudaMemcpyAsync(d_vin, b.var_in + L.pv_upto(begin), cpv * 4, cudaMemcpyHostToDevice, st));
     }
     void *d_out = nullptr;
-    const bool want_mat = b.matrices_out != nullptr || want_rng || b.keep_final;
+    const bool want_mat = b.matrices_out != nullptr || b.post_pass() || b.keep_final;
     // K1t and K1/K1s write the final tableaus apart; the others leave them in the working copy d_in
     const bool out_apart = ragged || (route.resident && route.kind != ROUTE_GRID);
     if (want_mat && out_apart)
@@ -1475,33 +1538,9 @@ int solve_chunks(yalps_ctx *ctx, HostBatch &b, const BatchLayout &L) {
       a.pos_off = (const long long *)d_po;
     }
     fill_options(a, opt);
-    // k_ranging over LPs of this chunk (all of them, or one ragged group through its index), after their route
-    auto ranging = [&](long long rn, int rh, int rw, const int *rindex) -> int {
-      if (!want_rng) return 0;
-      RangingArgs g{};
-      g.n = rn;
-      g.H = L.height;
-      g.W = L.width;
-      g.Hcap = rh;
-      g.Wcap = rw;
-      g.M = a.mat_out;
-      g.heights = a.heights;
-      g.widths = a.widths;
-      g.mat_off = a.mat_off;
-      g.rhs_off = a.rhs_off;
-      g.pos_off = a.pos_off;
-      g.index = rindex;
-      g.pos = a.pos_out;
-      g.status = a.status;
-      g.pairs = (const int *)d_pairs;
-      g.precision = opt->precision;
-      g.lo = (double *)dev[O_RLO];
-      g.hi = (double *)dev[O_RHI];
-      return launch_ranging(ctx, g, cpv, s, st);
-    };
     if (!ragged) {
       if ((rc = launch_route(ctx, route, a, s, st))) return rc;
-      if ((rc = ranging(cn, chcap, cwcap, nullptr))) return rc;
+      if (b.post_pass() && (rc = post_passes(ctx, b, a, a.mat_out, (const int *)d_pairs, dev, cpv, s, st))) return rc;
     } else {
       // Ragged chunk: LPs of very different sizes must not share one launch configuration (one large model would
       // push a thousand small ones onto the HBM-resident kernel).  Group by (fits in shared memory, CTA width) and
@@ -1547,7 +1586,7 @@ int solve_chunks(yalps_ctx *ctx, HostBatch &b, const BatchLayout &L) {
                                &route)))
           return rc;
         if ((rc = launch_route(ctx, route, ga, s, st, &h))) return rc;
-        if ((rc = ranging(ga.n, ga.Hcap, ga.Wcap, ga.index))) return rc;
+        if (b.post_pass() && (rc = post_passes(ctx, b, ga, a.mat_out, (const int *)d_pairs, dev, cpv, s, st))) return rc;
         at += groups[g].size();
       }
     }
@@ -1645,6 +1684,27 @@ int yalps_solve_batch_ranging(yalps_ctx *ctx, int64_t n, int32_t height, int32_t
                               double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                               double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
                               double *range_hi) {
+  return yalps_solve_batch_certificate(ctx, n, height, width, matrices, pos_in, var_in, opt, status, value, pivots,
+                                       rhs_out, pos_out, var_out, matrices_out, reduced_out, pairs, range_lo, range_hi,
+                                       nullptr);
+}
+
+int yalps_solve_ragged_ranging(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
+                               const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                               const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                               double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                               double *range_hi) {
+  return yalps_solve_ragged_certificate(ctx, n, heights, widths, mat_offsets, matrices, pos_in, var_in, opt, status,
+                                        value, pivots, rhs_out, pos_out, var_out, matrices_out, reduced_out, pairs,
+                                        range_lo, range_hi, nullptr);
+}
+
+int yalps_solve_batch_certificate(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *matrices,
+                                  const int32_t *pos_in, const int32_t *var_in, const yalps_options *opt,
+                                  int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
+                                  int32_t *var_out, double *matrices_out, double *reduced_out, const int32_t *pairs,
+                                  double *range_lo, double *range_hi, double *cert_out) {
   HostBatch b;
   b.n = n;
   b.height = height;
@@ -1664,15 +1724,16 @@ int yalps_solve_batch_ranging(yalps_ctx *ctx, int64_t n, int32_t height, int32_t
   b.reduced_out = reduced_out;
   b.range_lo = range_lo;
   b.range_hi = range_hi;
+  b.cert_out = cert_out;
   return solve_host(ctx, b);
 }
 
-int yalps_solve_ragged_ranging(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
-                               const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
-                               const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
-                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
-                               double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
-                               double *range_hi) {
+int yalps_solve_ragged_certificate(yalps_ctx *ctx, int64_t n, const int32_t *heights, const int32_t *widths,
+                                   const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                                   const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                                   int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                                   double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                                   double *range_hi, double *cert_out) {
   if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
   HostBatch b;
   b.n = n;
@@ -1694,6 +1755,7 @@ int yalps_solve_ragged_ranging(yalps_ctx *ctx, int64_t n, const int32_t *heights
   b.reduced_out = reduced_out;
   b.range_lo = range_lo;
   b.range_hi = range_hi;
+  b.cert_out = cert_out;
   return solve_host(ctx, b);
 }
 
@@ -1932,7 +1994,7 @@ int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_
   // D2H of chunk k-1's results overlap the solve of chunk k
   const int64_t per_chunk = std::max<int64_t>(1, std::min<int64_t>((n + 1) / 2 > 4096 ? (n + 7) / 8 : n,
                                                                   (int64_t)(((size_t)1536 << 20) / (cells * 8))));
-  const Outputs outs(status, value, pivots, rhs_out, pos_out, var_out, reduced_out, nullptr, nullptr);
+  const Outputs outs(status, value, pivots, rhs_out, pos_out, var_out, reduced_out, nullptr, nullptr, nullptr);
   bool used[2] = {false, false};
   int slot = 0;
   for (int64_t begin = 0; begin < n; begin += per_chunk, slot ^= 1) {

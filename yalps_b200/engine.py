@@ -60,9 +60,11 @@ def _batch_outputs(n: int, height: int, width: int, want_matrices: bool = False,
     }
 
 
-def _add_outputs(out: dict, n: int, pv: int, want_duals: bool, want_ranges: bool = False):
-    """The reduced costs and ranges a call wants, added to a reused `out` that lacks them."""
-    for k, want in (("reduced", want_duals), ("range_lo", want_ranges), ("range_hi", want_ranges)):
+def _add_outputs(out: dict, n: int, pv: int, want_duals: bool, want_ranges: bool = False,
+                 want_certificates: bool = False):
+    """The reduced costs, ranges and certificates a call wants, added to a reused `out` that lacks them."""
+    for k, want in (("reduced", want_duals), ("range_lo", want_ranges), ("range_hi", want_ranges),
+                    ("certificate", want_certificates)):
         if want and out.get(k) is None:
             out[k] = np.empty((n, pv), np.float64)
 
@@ -165,7 +167,8 @@ class Engine:
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, want_basis: bool = True, out: Optional[dict] = None,
                     pos_in: Optional[np.ndarray] = None, var_in: Optional[np.ndarray] = None,
-                    want_duals: bool = False, want_ranges: bool = False, pairs: Optional[np.ndarray] = None) -> dict:
+                    want_duals: bool = False, want_ranges: bool = False, pairs: Optional[np.ndarray] = None,
+                    want_certificates: bool = False) -> dict:
         """n same-shape tableaus, `matrices` float64 of n*height*width values (not modified).
         `out` may be a dict from batch_outputs() to reuse (pinned) result buffers.
         pos_in / var_in (int32, n*(width+height)): the basis bookkeeping the tableaus arrive with (the node LPs of
@@ -174,7 +177,10 @@ class Engine:
         (yalps_solve_batch_duals; yalps_b200.sensitivity turns it into shadow prices and reduced costs).
         want_ranges: also out["range_lo"], out["range_hi"] (n, width+height), the sensitivity ranges computed on the
         device from the final tableaus (yalps_solve_batch_ranging); `pairs` (int32 per row, -1 = none; one LP's
-        (height,) array or n*height values) pairs the two rows of a key (yalps_b200.sensitivity.row_pairs)."""
+        (height,) array or n*height values) pairs the two rows of a key (yalps_b200.sensitivity.row_pairs).
+        want_certificates: also out["certificate"] (n, width+height), the Farkas certificate of an infeasible LP or the
+        ray of an unbounded one, computed on the device from the final tableaus (yalps_solve_batch_certificate; NaN
+        for every other status)."""
         opt = options or make_options()
         m = np.ascontiguousarray(matrices, dtype=np.float64).reshape(-1)
         cells = height * width
@@ -185,14 +191,15 @@ class Engine:
             out = self.batch_outputs(n, height, width, want_matrices, want_basis, want_duals=want_duals)
         elif out["status"].shape[0] != n:
             raise ValueError("out was allocated for a different batch size")
-        _add_outputs(out, n, width + height, want_duals, want_ranges)
+        _add_outputs(out, n, width + height, want_duals, want_ranges, want_certificates)
         p, v = _basis_in(pos_in, var_in, n * (width + height))
         pr = _pairs_in(pairs, n, height) if want_ranges else None
-        self._check(self._lib.yalps_solve_batch_ranging(
+        self._check(self._lib.yalps_solve_batch_certificate(
             self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
             _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
             _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None, _ptr(pr),
-            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None))
+            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None,
+            _ptr(out["certificate"]) if want_certificates else None))
         return out
 
     def simplex(self, tableau, options: Optional[Options] = None) -> tuple:
@@ -245,10 +252,11 @@ class Engine:
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
                      want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,
-                     pairs: Optional[Sequence] = None) -> list:
+                     pairs: Optional[Sequence] = None, want_certificates: bool = False) -> list:
         """LPs of different shapes in one call.  tableaus[i] is float64 of height_i*width_i values.
         want_duals: every result also has "reduced" (width_i+height_i values, as solve_batch).
-        want_ranges: every result also has "range_lo", "range_hi" (as solve_batch); pairs[i] (height_i int32) or None."""
+        want_ranges: every result also has "range_lo", "range_hi" (as solve_batch); pairs[i] (height_i int32) or None.
+        want_certificates: every result also has "certificate" (width_i+height_i values, as solve_batch)."""
         opt = options or make_options()
         n = len(tableaus)
         if n == 0:
@@ -274,10 +282,11 @@ class Engine:
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
         red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
         rlo, rhi, pr = _ragged_ranges(want_ranges, pairs, int(roffs[-1]), int(poffs[-1]))
-        self._check(self._lib.yalps_solve_ragged_ranging(
+        cert = np.empty(int(poffs[-1]), np.float64) if want_certificates else None
+        self._check(self._lib.yalps_solve_ragged_certificate(
             self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
             _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
-            _ptr(rlo), _ptr(rhi)))
+            _ptr(rlo), _ptr(rhi), _ptr(cert)))
         res = []
         for i in range(n):
             res.append({
@@ -289,6 +298,8 @@ class Engine:
                 res[i]["reduced"] = red[poffs[i]:poffs[i + 1]]
             if want_ranges:
                 res[i]["range_lo"], res[i]["range_hi"] = rlo[poffs[i]:poffs[i + 1]], rhi[poffs[i]:poffs[i + 1]]
+            if want_certificates:
+                res[i]["certificate"] = cert[poffs[i]:poffs[i + 1]]
         return res
 
     def solve_batch_device(self, n: int, height: int, width: int, d_matrices: int, options: Optional[Options] = None,
@@ -313,6 +324,16 @@ class Engine:
         self._check(self._lib.yalps_ranging_device(self._ctx, n, height, width, z(d_matrices), z(d_pos), z(d_status),
                                                    z(d_pairs), float(precision), z(d_range_lo), z(d_range_hi),
                                                    z(stream)))
+
+    def certificate_device(self, n: int, height: int, width: int, d_matrices: int, d_pos: int, d_status: int,
+                           d_value: int, d_cert: int, precision: float = 1e-8, stream: int = 0):
+        """Certificates of n final tableaus already in device memory (yalps_certificate_device, raw pointers): d_pos
+        int32 n*(width+height), d_status int32 n, d_value float64 n, as a solve reported them; writes float64
+        n*(width+height) to d_cert.  Enqueues on `stream` and returns."""
+        z = lambda p: C.c_void_p(p) if p else None
+        self._check(self._lib.yalps_certificate_device(self._ctx, n, height, width, z(d_matrices), z(d_pos),
+                                                       z(d_status), z(d_value), float(precision), z(d_cert),
+                                                       z(stream)))
 
     def generate_synthetic_device(self, first: int, n: int, m: int, nvars: int, d_out: int, neg_rows: int = 0,
                                   salt: int = 0x5BD1E995, stream: int = 0):
@@ -375,10 +396,10 @@ class Engine:
 
     def solve_lp_sparse(self, cells: np.ndarray, values: np.ndarray, height: int, width: int,
                         options: Optional[Options] = None, want_ranges: bool = False,
-                        pairs: Optional[np.ndarray] = None) -> dict:
+                        pairs: Optional[np.ndarray] = None, want_certificates: bool = False) -> dict:
         """One LP given as ordered (cell, value) stores into a zero matrix (yalps_solve_sparse_duals): status, value,
         pivots, rhs, pos, var and reduced, as solve_batch with n = 1 and want_duals; want_ranges adds range_lo and
-        range_hi (yalps_solve_sparse_ranging, `pairs` as solve_batch)."""
+        range_hi (`pairs` as solve_batch), want_certificates adds certificate (yalps_solve_sparse_certificate)."""
         opt = options or make_options()
         cells = np.ascontiguousarray(cells, np.int32).reshape(-1)
         values = np.ascontiguousarray(values, np.float64).reshape(-1)
@@ -387,24 +408,19 @@ class Engine:
         status, value = C.c_int32(), C.c_double()
         piv = np.zeros(2, np.int64)
         rhs, pos, var = np.empty(height), np.empty(width + height, np.int32), np.empty(width + height, np.int32)
-        red = np.empty(width + height, np.float64)
-        if want_ranges:
-            rlo, rhi = np.empty(width + height, np.float64), np.empty(width + height, np.float64)
-            self._check(self._lib.yalps_solve_sparse_ranging(self._ctx, height, width, int(cells.size),
+        out = {"reduced": np.empty(width + height, np.float64)}
+        wanted = (("range_lo", want_ranges), ("range_hi", want_ranges), ("certificate", want_certificates))
+        out.update({k: np.empty(width + height, np.float64) for k, want in wanted if want})
+        pr = _pairs_in(pairs, 1, height) if want_ranges else None
+        self._check(self._lib.yalps_solve_sparse_certificate(self._ctx, height, width, int(cells.size),
                                                              _ptr(cells) if cells.size else None,
                                                              _ptr(values) if values.size else None, C.byref(opt),
                                                              C.byref(status), C.byref(value), _ptr(piv), _ptr(rhs),
-                                                             _ptr(pos), _ptr(var), _ptr(red), _ptr(_pairs_in(pairs, 1, height)),
-                                                             _ptr(rlo), _ptr(rhi)))
-            return {"status": status.value, "value": value.value, "pivots": (int(piv[0]), int(piv[1])), "rhs": rhs,
-                    "pos": pos, "var": var, "reduced": red, "range_lo": rlo, "range_hi": rhi}
-        self._check(self._lib.yalps_solve_sparse_duals(self._ctx, height, width, int(cells.size),
-                                                       _ptr(cells) if cells.size else None,
-                                                       _ptr(values) if values.size else None, C.byref(opt),
-                                                       C.byref(status), C.byref(value), _ptr(piv), _ptr(rhs), _ptr(pos),
-                                                       _ptr(var), _ptr(red)))
+                                                             _ptr(pos), _ptr(var), _ptr(out["reduced"]), _ptr(pr),
+                                                             _ptr(out.get("range_lo")), _ptr(out.get("range_hi")),
+                                                             _ptr(out.get("certificate"))))
         return {"status": status.value, "value": value.value, "pivots": (int(piv[0]), int(piv[1])), "rhs": rhs,
-                "pos": pos, "var": var, "reduced": red}
+                "pos": pos, "var": var, **out}
 
     def solve_tableau(self, matrix: np.ndarray, height: int, width: int, integers: Sequence[int], sign: float,
                       options: Optional[Options] = None, cells: Optional[np.ndarray] = None) -> dict:
@@ -556,20 +572,22 @@ class MultiEngine:
 
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, pos_in=None, var_in=None, out: Optional[dict] = None,
-                    want_duals: bool = False, want_ranges: bool = False, pairs=None) -> dict:
+                    want_duals: bool = False, want_ranges: bool = False, pairs=None,
+                    want_certificates: bool = False) -> dict:
         opt = options or make_options()
         m = np.ascontiguousarray(matrices, np.float64).reshape(-1)
         n = m.size // (height * width)
         out = out or _batch_outputs(n, height, width, want_matrices, want_duals=want_duals)
         p = None if pos_in is None else np.ascontiguousarray(pos_in, np.int32).reshape(-1)
         v = None if var_in is None else np.ascontiguousarray(var_in, np.int32).reshape(-1)
-        _add_outputs(out, n, width + height, want_duals, want_ranges)
-        self._check(self._lib.yalps_multi_solve_batch_ranging(
+        _add_outputs(out, n, width + height, want_duals, want_ranges, want_certificates)
+        self._check(self._lib.yalps_multi_solve_batch_certificate(
             self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
             _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
             _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None,
             _ptr(_pairs_in(pairs, n, height)) if want_ranges else None,
-            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None))
+            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None,
+            _ptr(out["certificate"]) if want_certificates else None))
         return out
 
     def solve_replicas(self, base: np.ndarray, rhs: np.ndarray, height: int, width: int,
@@ -588,7 +606,7 @@ class MultiEngine:
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
                      want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,
-                     pairs: Optional[Sequence] = None) -> list:
+                     pairs: Optional[Sequence] = None, want_certificates: bool = False) -> list:
         opt = options or make_options()
         n = len(tableaus)
         if n == 0:
@@ -607,10 +625,11 @@ class MultiEngine:
         mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
         red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
         rlo, rhi, pr = _ragged_ranges(want_ranges, pairs, int(roffs[-1]), int(poffs[-1]))
-        self._check(self._lib.yalps_multi_solve_ragged_ranging(
+        cert = np.empty(int(poffs[-1]), np.float64) if want_certificates else None
+        self._check(self._lib.yalps_multi_solve_ragged_certificate(
             self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
             _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
-            _ptr(rlo), _ptr(rhi)))
+            _ptr(rlo), _ptr(rhi), _ptr(cert)))
         res = [{"status": int(status[i]), "value": float(value[i]), "pivots": (int(pivots[i, 0]), int(pivots[i, 1])),
                 "rhs": rhs[roffs[i]:roffs[i + 1]], "pos": pos[poffs[i]:poffs[i + 1]], "var": var[poffs[i]:poffs[i + 1]],
                 "matrix": mats[offs[i]:offs[i + 1]] if want_matrices else None} for i in range(n)]
@@ -620,6 +639,9 @@ class MultiEngine:
         if want_ranges:
             for i in range(n):
                 res[i]["range_lo"], res[i]["range_hi"] = rlo[poffs[i]:poffs[i + 1]], rhi[poffs[i]:poffs[i + 1]]
+        if want_certificates:
+            for i in range(n):
+                res[i]["certificate"] = cert[poffs[i]:poffs[i + 1]]
         return res
 
     def solve_large(self, matrix: np.ndarray, height: int, width: int, options: Optional[Options] = None,

@@ -28,6 +28,28 @@ of the basic row.  With a pair (the other row of the same constraint key, whose 
 +t) d = dir(W+k) - dir(W+pair): a key with two finite bounds must be ranged as one, its two slacks always sum to a
 constant.  An empty max is -inf, an empty min +inf, a zero is +0.0, and lo <= 0 <= hi.  Ids 0 and W and every id of a
 non-optimal LP are NaN.
+
+Certificates explain the other two outcomes, one float64 per variable id packed like `reduced`
+(certificate_from_tableau):
+
+    infeasible (status 1): r = the row phase 1 chose, the lowest r in 1..H-1 whose M[r,0] is the minimum over the rows
+        with M[r,0] < -precision (the reference's strict-< scan: NaN never qualifies, -inf does).  Phase 1 returns
+        `infeasible` on that row without pivoting (src/simplex.ts:106-142), so the final tableau is that tableau.
+        cert[0] = M[r,0], cert[W] = +0.0, and for every other id v: M[r, pos[v]] if 1 <= pos[v] < W (bits as they
+        are), 1.0 if pos[v] == W + r, +0.0 otherwise.
+    unbounded (status 2): c = int(value), the entering column.  cert[0] = M[0,c], cert[W] = +0.0, and for every other
+        id v: 1.0 if pos[v] == c, -M[pos[v] - W, c] if W < pos[v] < W + H (the sign bit flipped), +0.0 otherwise.
+    every other status, an infeasible LP without a qualifying row, an unbounded LP with c outside 1..W-1: NaN.
+
+Row r of the final tableau is sum_k y_k (original row k), where original row k reads a_k.x + s_k = b_k: the slack
+entries cert[W + k] are the multipliers y_k (>= -precision, or the row would have had an entering column), the
+structural entries equal sum_k y_k a_kj (>= -precision) and cert[0] = sum_k y_k b_k < 0.  So no x >= 0 satisfies every
+row: a Farkas certificate.  A column c with no leaving row is a direction d >= 0 (cert[1..]) that keeps every row
+feasible while the objective moves at rate d result / dt = sign * cert[0], the convention of reducedCosts.  Candidates
+whose ratio was NaN or +-inf were rejected by the reference too, and the certificate is still its row or column; the
+values are raw cells, nothing below precision is cleaned.  At model level (model_certificate) a key's multiplier is
+cert[W + upper] - cert[W + lower], the sign convention of shadowPrices: m > 0 means its `max` takes part, m < 0 its
+`min`.
 """
 from __future__ import annotations
 
@@ -171,3 +193,61 @@ def model_ranges(variables: list, rows: list, range_lo: np.ndarray, range_hi: np
         else:
             rhs.append([key, -np.inf, np.inf])
     return cost, rhs
+
+
+_SIGN = np.uint64(0x8000000000000000)
+
+
+def certificate_from_tableau(matrix: np.ndarray, width: int, height: int, pos: np.ndarray, status: int, value: float,
+                             precision: float) -> np.ndarray:
+    """What the kernels write into `cert` (one value per variable id, packed like `reduced`), computed from a final
+    tableau, its positionOfVariable and the status and value the solve reported (module docstring)."""
+    W, H = int(width), int(height)
+    out = np.full(W + H, np.nan)
+    M = np.asarray(matrix, np.float64).reshape(-1)[:H * W].reshape(H, W)
+    p = np.asarray(pos, np.int64).reshape(-1)[:W + H]
+    prec = float(precision)
+    if status == 1:
+        b = M[1:, 0]
+        ok = b < -prec  # NaN never qualifies
+        if not ok.any():
+            return out
+        r = 1 + int(np.flatnonzero(ok & (b == b[ok].min()))[0])
+        nonbasic = (p >= 1) & (p < W)
+        out[:] = np.where(nonbasic, M[r][np.where(nonbasic, p, 0)], np.where(p == W + r, 1.0, 0.0))
+        out[0] = M[r, 0]
+    elif status == 2:
+        x = float(value)
+        if not (1.0 <= x < W):
+            return out
+        c = int(x)
+        basic = (p > W) & (p < W + H)
+        col = M[:, c].copy()
+        col.view(np.uint64)[:] ^= _SIGN
+        out[:] = np.where(p == c, 1.0, np.where(basic, col[np.where(basic, p - W, 0)], 0.0))
+        out[0] = M[0, c]
+    else:
+        return out
+    out[W] = 0.0
+    return out
+
+
+def model_certificate(variables: list, rows: list, cert: np.ndarray, width: int, status: int) -> tuple:
+    """Model level: (infeasibilityCertificate, unboundedRay) of one LP from its certificate_from_tableau values, both
+    empty unless the status matches.  infeasibilityCertificate [[key, m]] in first-seen order, m = cert[W + upper] -
+    cert[W + lower] (a missing row counts as 0; m > 0: the key's max takes part, m < 0: its min).  unboundedRay
+    [[variable, d]] in model order, d = cert[j + 1]."""
+    c = np.asarray(cert, np.float64).reshape(-1)
+    W = int(width)
+    farkas, ray = [], []
+    if status == 1 and not np.isnan(c[0]):
+        for key, up, lw in rows:
+            m = 0.0
+            if up >= 0:
+                m = float(c[W + up])
+            if lw >= 0:
+                m = m - float(c[W + lw])
+            farkas.append([key, m])
+    elif status == 2 and not np.isnan(c[0]):
+        ray = [[key, float(c[j + 1])] for j, (key, _) in enumerate(variables)]
+    return farkas, ray

@@ -14,6 +14,11 @@ A second one, `ranging` (default False), implies `sensitivity` and adds "costRan
 allowable shifts of the variable's objective coefficient that keep the optimal basis) and "rhsRanges" ([[constraint
 key, lo, hi], ...]: the allowable shifts of all of the key's finite bounds together over which its shadow price holds),
 computed on the GPU from the final tableau; empty lists unless optimal.
+A third one, `certificate` (default False), adds "infeasibilityCertificate" ([[constraint key, multiplier], ...],
+first-seen order: non-negative combinations of the keys' max rows and min rows that read 0 <= negative, the Farkas
+proof that no solution exists) and "unboundedRay" ([[variable, direction], ...], model order: a direction that keeps
+every constraint satisfied while the result moves toward the reported +-inf), computed on the GPU from the final
+tableau; each is an empty list unless the status is infeasible, resp. unbounded.
 The tableau is built on the host (tableau.py), the simplex and branch-and-cut numerics run on the GPU
 through the C ABI; there is no CPU solve path.
 """
@@ -25,7 +30,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
-from .sensitivity import model_ranges, model_sensitivity, row_pairs
+from .sensitivity import model_certificate, model_ranges, model_sensitivity, row_pairs
 from .tableau import SPARSE_OVER_BYTES, TableauModel, constraint_rows, entries, tableau_model
 
 # src/YALPS.ts:52-60
@@ -101,6 +106,20 @@ def _check_lp(tabmod: TableauModel):
         raise ValueError("sensitivity: duals are defined for LP models only (this model has integer or binary variables)")
 
 
+def _wants(opt: dict) -> tuple:
+    """(duals, ranges, certificate): what the options ask of the root LP."""
+    rng = bool(opt.get("ranging"))
+    return bool(opt.get("sensitivity")) or rng, rng, bool(opt.get("certificate"))
+
+
+def _with_certificate(sol: dict, tabmod: TableauModel, model: dict, cert) -> dict:
+    """Solution + infeasibilityCertificate / unboundedRay (both empty unless the status matches)."""
+    status = {"infeasible": 1, "unbounded": 2}.get(sol["status"], 0)
+    rows = _rows(model) if status == 1 else []
+    farkas, ray = model_certificate(tabmod.variables, rows, cert, tabmod.tableau.width, status)
+    return {**sol, "infeasibilityCertificate": farkas, "unboundedRay": ray}
+
+
 def _rows(model: dict) -> list:
     return constraint_rows(list(entries(model["constraints"])))
 
@@ -129,32 +148,38 @@ def solve(model: dict, options: Optional[dict] = None, *, engine: Optional[Engin
     sparse_ok = hasattr(engine, "solve_tableau_sparse") if engine is not None else True
     tabmod = tableau_model(model, SPARSE_OVER_BYTES if sparse_ok else None)
     t = tabmod.tableau
-    rng = bool(opt.get("ranging"))
-    if opt.get("sensitivity") or rng:
+    duals, rng, cert = _wants(opt)
+    if duals or cert:
         _check_lp(tabmod)
     eng = engine or get_engine()
-    if opt.get("sensitivity") or rng:
+    if duals or cert:
         # the root LP is the whole solve: one LP with its reduced-cost row (dense batch of one, or the cell pairs), and
-        # its ranges when asked for
+        # its ranges and certificate when asked for
         pairs = row_pairs(_rows(model), t.height) if rng else None
         if t.matrix is None:
-            r = eng.solve_lp_sparse(t.cells, t.values, t.height, t.width, _c_options(opt), want_ranges=rng, pairs=pairs)
+            r = eng.solve_lp_sparse(t.cells, t.values, t.height, t.width, _c_options(opt), want_ranges=rng, pairs=pairs,
+                                    want_certificates=cert)
             status, value, rhs, pos, var, red = (r["status"], r["value"], r["rhs"], r["pos"], r["var"], r["reduced"])
             piv = r["pivots"]
             ranges = (r["range_lo"], r["range_hi"]) if rng else None
+            c = r["certificate"] if cert else None
         else:
-            r = eng.solve_batch(t.matrix, t.height, t.width, _c_options(opt), want_duals=True, want_ranges=rng,
-                                pairs=pairs)
+            r = eng.solve_batch(t.matrix, t.height, t.width, _c_options(opt), want_duals=duals, want_ranges=rng,
+                                pairs=pairs, want_certificates=cert)
             status, value = int(r["status"][0]), float(r["value"][0])
-            rhs, pos, var, red = r["rhs"][0], r["pos"][0], r["var"][0], r["reduced"][0]
+            rhs, pos, var = r["rhs"][0], r["pos"][0], r["var"][0]
+            red = r["reduced"][0] if duals else None
             piv = (int(r["pivots"][0, 0]), int(r["pivots"][0, 1]))
             ranges = (r["range_lo"][0], r["range_hi"][0]) if rng else None
+            c = r["certificate"][0] if cert else None
         if info is not None:
             info.update(nodes=0, node_pivots=0, max_cuts=0, max_heap=0, waves=0, device_nodes=0, wave_us=0, bnb_us=0,
                         root_status=STATUS_NAMES[status], root_value=value, root_pivots=piv, height=t.height,
                         width=t.width, final_rhs=rhs, final_pos=pos, final_var=var)
         sol = _solution(tabmod, STATUS_NAMES[status], value, rhs, pos, var, opt)
-        return _with_sensitivity(sol, tabmod, model, red, ranges)
+        if duals:
+            sol = _with_sensitivity(sol, tabmod, model, red, ranges)
+        return _with_certificate(sol, tabmod, model, c) if cert else sol
     if t.matrix is None:
         r = eng.solve_tableau_sparse(t.cells, t.values, t.height, t.width, tabmod.integers, tabmod.sign, _c_options(opt))
     else:
@@ -189,21 +214,25 @@ def solve_many(models: Sequence[dict], options: Optional[dict] = None, *, engine
     opt = {**_DEFAULTS, **(options or {})}
     copt = _c_options(opt)
     tabmods = [tableau_model(m) for m in models]
-    rng = bool(opt.get("ranging"))
-    if opt.get("sensitivity") or rng:
+    duals, rng, cert = _wants(opt)
+    if duals or cert:
         for tm in tabmods:
             _check_lp(tm)
     eng = engine or get_engine()
     if not tabmods:
         return []
-    if opt.get("sensitivity") or rng:  # LP models only: the ragged root batch is the whole solve (one GPU or sharded)
+    if duals or cert:  # LP models only: the ragged root batch is the whole solve (one GPU or sharded)
         pairs = [row_pairs(_rows(m), tm.tableau.height) for tm, m in zip(tabmods, models)] if rng else None
         roots = eng.solve_ragged([tm.tableau.matrix for tm in tabmods],
-                                 [(tm.tableau.height, tm.tableau.width) for tm in tabmods], copt, want_duals=True,
-                                 want_ranges=rng, pairs=pairs)
-        return [_with_sensitivity(_solution(tm, STATUS_NAMES[r["status"]], r["value"], r["rhs"], r["pos"], r["var"], opt),
-                                  tm, m, r["reduced"], (r["range_lo"], r["range_hi"]) if rng else None)
-                for tm, m, r in zip(tabmods, models, roots)]
+                                 [(tm.tableau.height, tm.tableau.width) for tm in tabmods], copt, want_duals=duals,
+                                 want_ranges=rng, pairs=pairs, want_certificates=cert)
+        out = []
+        for tm, m, r in zip(tabmods, models, roots):
+            sol = _solution(tm, STATUS_NAMES[r["status"]], r["value"], r["rhs"], r["pos"], r["var"], opt)
+            if duals:
+                sol = _with_sensitivity(sol, tm, m, r["reduced"], (r["range_lo"], r["range_hi"]) if rng else None)
+            out.append(_with_certificate(sol, tm, m, r["certificate"]) if cert else sol)
+        return out
     if isinstance(eng, MultiEngine):  # one C-ABI call: roots sharded over the GPUs, searches dealt to worker contexts
         res = eng.solve_many_tableaus(tabmods, copt, searches_per_device=milp_workers)
         return [_solution(tm, STATUS_NAMES[r["status"]], r["result"], r["rhs"], r["pos"], r["var"], opt)
