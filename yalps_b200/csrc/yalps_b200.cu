@@ -58,6 +58,22 @@ cudaError_t raise_smem_limit(int device, const void *fn, int bytes) {
   return e;
 }
 
+// The dynamic shared memory a launch of fn can have: the per-block opt-in limit less fn's static shared memory
+// (k_simplex and the cluster kernels: 16 bytes).  A carve-up is checked against this, not the opt-in limit itself --
+// at the tallest tableau of a kernel the difference decides between a launch and a failing cudaFuncSetAttribute.
+size_t dynamic_smem_limit(int device, int optin, const void *fn) {
+  std::lock_guard<std::mutex> lock(g_attr_mutex);
+  static std::unordered_map<std::string, int> static_bytes;
+  const std::string key = std::to_string(device) + ":" + std::to_string((size_t)fn);
+  auto it = static_bytes.find(key);
+  if (it == static_bytes.end()) {
+    cudaFuncAttributes a{};
+    const int s = cudaFuncGetAttributes(&a, fn) == cudaSuccess ? (int)a.sharedSizeBytes : 0;
+    it = static_bytes.emplace(key, s).first;
+  }
+  return (size_t)std::max(0, optin - it->second);
+}
+
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
@@ -377,11 +393,19 @@ int choose_route(yalps_ctx *ctx, const RouteRequest &q, Route *r) {
   const KernelEntry *k = nullptr;
   if (staged && nwr > 1) {
     k = pick_kernel(std::max(1, nw / nwr), nwr, Wcap, resident);
-    if (k && SmemLayout(Hcap, Wcap, resident, k->nw * k->nwr, true).total > (size_t)ctx->smem_optin) k = nullptr;
+    if (k && SmemLayout(Hcap, Wcap, resident, k->nw * k->nwr, true).total >
+                 dynamic_smem_limit(ctx->device, ctx->smem_optin, (const void *)(resident ? k->resident : k->global)))
+      k = nullptr;
   }
   if (staged && !k) {
     nwr = 1;
     k = pick_kernel(nw, 1, Wcap, resident);
+    // (the staging checks above use the 32-warp carve-up; the kernel's own static shared memory comes on top)
+    if (k && SmemLayout(Hcap, Wcap, resident, k->nw, false).total >
+                 dynamic_smem_limit(ctx->device, ctx->smem_optin, (const void *)(resident ? k->resident : k->global))) {
+      if (!grid_ok) return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau %dx%d does not fit in shared memory", Hcap, Wcap);
+      k = nullptr;
+    }
   }
   if (!k && !grid_ok) return fail(ctx, YALPS_ERR_TOO_LARGE, "tableau width %d exceeds the widest kernel", Wcap);
   if (k) {
@@ -439,7 +463,7 @@ int choose_route(yalps_ctx *ctx, const RouteRequest &q, Route *r) {
     if (const KernelEntry *k = pick_kernel(split_nwc, split_nwr, Wcap, false)) {
       if (k->nwr == split_nwr) {
         const size_t smem_k = SmemLayout(Hcap, Wcap, false, k->nw * k->nwr, true).total;
-        if (smem_k <= (size_t)ctx->smem_optin) {
+        if (smem_k <= dynamic_smem_limit(ctx->device, ctx->smem_optin, (const void *)k->global)) {
           CU(ctx, raise_smem_limit(ctx->device, (const void *)k->global, (int)smem_k));
           int occ = 0;
           CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k->global, k->nw * k->nwr * 32, smem_k));
@@ -512,7 +536,7 @@ int plan_cluster(yalps_ctx *ctx, int Hcap, int Wcap, Route *r) {
   if (!k) return 0;
   for (int C = 2; C <= kMaxCluster; C *= 2) {
     const ClusterSmem L(Hcap, Wcap, C);
-    if (L.total > (size_t)ctx->smem_optin) continue;
+    if (L.total > dynamic_smem_limit(ctx->device, ctx->smem_optin, (const void *)k->resident)) continue;
     // more CTAs than the capacity needs when a CTA would otherwise own many rows (dense updates are row-parallel)
     if (L.Hloc > 40 && C < kMaxCluster) continue;
     const std::string key = "cl:" + std::to_string((size_t)(void *)k->resident) + ":" + std::to_string(C) + ":" + std::to_string(L.total);
@@ -609,7 +633,7 @@ int plan_gridres(yalps_ctx *ctx, int Hcap, int Wcap, Route *r) {
   int C = std::max(1, std::min(std::min(ctx->prop.multiProcessorCount, 160), Hcap - 1));  // (grid_select: 5 slots per lane)
   if (const char *env = getenv("YALPS_KG_CTAS")) C = std::max(1, std::min(C, atoi(env)));
   const ClusterSmem L(Hcap, Wcap, C);
-  if (L.total > (size_t)ctx->smem_optin) return 0;
+  if (L.total > dynamic_smem_limit(ctx->device, ctx->smem_optin, (const void *)k->global)) return 0;
   CU(ctx, raise_smem_limit(ctx->device, (const void *)k->global, (int)L.total));
   const std::string key = "kg:" + std::to_string((size_t)(void *)k->global) + ":" + std::to_string(L.total);
   int occ = 0;
