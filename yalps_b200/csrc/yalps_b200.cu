@@ -1187,6 +1187,39 @@ struct Outputs {
   }
 };
 
+// The LPs [lo, hi) of request b, after row0 rows and pv0 variable ids.  A uniform batch moves its tableaus by cells; a
+// ragged one moves its shapes and offsets by LPs and keeps matrices and matrices_out, which those offsets index
+// absolutely.  The basis moves by variable ids, the pairs by rows, the outputs as the Outputs table packs them.
+HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long row0, long long pv0) {
+  HostBatch s = b;
+  s.n = hi - lo;
+  if (b.heights) {
+    s.heights += lo;
+    s.widths += lo;
+    s.mat_offsets += lo;
+  } else {
+    const size_t cells = (size_t)lo * b.height * b.width;
+    if (s.matrices) s.matrices += cells;
+    if (s.matrices_out) s.matrices_out += cells;
+  }
+  if (s.pos_in) s.pos_in += pv0;
+  if (s.var_in) s.var_in += pv0;
+  if (s.pairs) s.pairs += row0;
+  const Outputs o(b);
+  auto at = [&](int i) -> void * { return o.t[i].host ? (char *)o.t[i].host + o.t[i].bytes(lo, row0, pv0) : nullptr; };
+  s.status = (int32_t *)at(O_STATUS);
+  s.value = (double *)at(O_VALUE);
+  s.pivots = (int64_t *)at(O_PIVOTS);
+  s.rhs_out = (double *)at(O_RHS);
+  s.pos_out = (int32_t *)at(O_POS);
+  s.var_out = (int32_t *)at(O_VAR);
+  s.reduced_out = (double *)at(O_RED);
+  s.range_lo = (double *)at(O_RLO);
+  s.range_hi = (double *)at(O_RHI);
+  s.cert_out = (double *)at(O_CERT);
+  return s;
+}
+
 void set_outputs(BatchArgs &a, void *const *dev) {
   a.status = (int *)dev[O_STATUS];
   a.value = (double *)dev[O_VALUE];
@@ -1649,6 +1682,39 @@ int solve_host(yalps_ctx *ctx, HostBatch &b) {
   return taken ? 0 : solve_chunks(ctx, b, L);
 }
 
+// The request of a yalps_solve_{batch,ragged}_certificate call (heights null: a uniform batch of height x width).
+HostBatch batch_request(int64_t n, int32_t height, int32_t width, const int32_t *heights, const int32_t *widths,
+                        const int64_t *mat_offsets, const double *matrices, const int32_t *pos_in,
+                        const int32_t *var_in, const yalps_options *opt, int32_t *status, double *value,
+                        int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out, double *matrices_out,
+                        double *reduced_out, const int32_t *pairs, double *range_lo, double *range_hi,
+                        double *cert_out) {
+  HostBatch b;
+  b.n = n;
+  b.height = height;
+  b.width = width;
+  b.heights = heights;
+  b.widths = widths;
+  b.mat_offsets = mat_offsets;
+  b.matrices = matrices;
+  b.pos_in = pos_in;
+  b.var_in = var_in;
+  b.pairs = pairs;
+  b.opt = opt;
+  b.status = status;
+  b.value = value;
+  b.pivots = pivots;
+  b.rhs_out = rhs_out;
+  b.pos_out = pos_out;
+  b.var_out = var_out;
+  b.matrices_out = matrices_out;
+  b.reduced_out = reduced_out;
+  b.range_lo = range_lo;
+  b.range_hi = range_hi;
+  b.cert_out = cert_out;
+  return b;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1729,26 +1795,9 @@ int yalps_solve_batch_certificate(yalps_ctx *ctx, int64_t n, int32_t height, int
                                   int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out,
                                   int32_t *var_out, double *matrices_out, double *reduced_out, const int32_t *pairs,
                                   double *range_lo, double *range_hi, double *cert_out) {
-  HostBatch b;
-  b.n = n;
-  b.height = height;
-  b.width = width;
-  b.matrices = matrices;
-  b.pos_in = pos_in;
-  b.var_in = var_in;
-  b.pairs = pairs;
-  b.opt = opt;
-  b.status = status;
-  b.value = value;
-  b.pivots = pivots;
-  b.rhs_out = rhs_out;
-  b.pos_out = pos_out;
-  b.var_out = var_out;
-  b.matrices_out = matrices_out;
-  b.reduced_out = reduced_out;
-  b.range_lo = range_lo;
-  b.range_hi = range_hi;
-  b.cert_out = cert_out;
+  HostBatch b = batch_request(n, height, width, nullptr, nullptr, nullptr, matrices, pos_in, var_in, opt, status, value,
+                              pivots, rhs_out, pos_out, var_out, matrices_out, reduced_out, pairs, range_lo, range_hi,
+                              cert_out);
   return solve_host(ctx, b);
 }
 
@@ -1759,27 +1808,9 @@ int yalps_solve_ragged_certificate(yalps_ctx *ctx, int64_t n, const int32_t *hei
                                    double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
                                    double *range_hi, double *cert_out) {
   if (!heights) return fail(ctx, YALPS_ERR_ARGUMENT, "heights is null");
-  HostBatch b;
-  b.n = n;
-  b.heights = heights;
-  b.widths = widths;
-  b.mat_offsets = mat_offsets;
-  b.matrices = matrices;
-  b.pos_in = pos_in;
-  b.var_in = var_in;
-  b.pairs = pairs;
-  b.opt = opt;
-  b.status = status;
-  b.value = value;
-  b.pivots = pivots;
-  b.rhs_out = rhs_out;
-  b.pos_out = pos_out;
-  b.var_out = var_out;
-  b.matrices_out = matrices_out;
-  b.reduced_out = reduced_out;
-  b.range_lo = range_lo;
-  b.range_hi = range_hi;
-  b.cert_out = cert_out;
+  HostBatch b = batch_request(n, 0, 0, heights, widths, mat_offsets, matrices, pos_in, var_in, opt, status, value,
+                              pivots, rhs_out, pos_out, var_out, matrices_out, reduced_out, pairs, range_lo, range_hi,
+                              cert_out);
   return solve_host(ctx, b);
 }
 

@@ -46,36 +46,158 @@ def _pairs_in(pairs, n: int, rows: int):
     return p
 
 
-def _batch_outputs(n: int, height: int, width: int, want_matrices: bool = False, want_basis: bool = True,
-                   want_duals: bool = False, mk=np.empty) -> dict:
-    return {
-        "status": mk((n,), np.int32),
-        "value": mk((n,), np.float64),
-        "pivots": mk((n, 2), np.int64),
-        "rhs": mk((n, height), np.float64),
-        "pos": mk((n, width + height), np.int32) if want_basis else None,
-        "var": mk((n, width + height), np.int32) if want_basis else None,
-        "matrices": mk((n, height * width), np.float64) if want_matrices else None,
-        "reduced": mk((n, width + height), np.float64) if want_duals else None,
-    }
+# The per-LP outputs of a batch call, as the C Outputs table (csrc/yalps_b200.cu) describes them, in the order the
+# widest entries take them: key, dtype, packing and the want_* flag that turns the output on (None: always on).
+# Packing: a tuple is the shape of one LP's values; "row" is one value per tableau row (like rhs), "var" one per
+# variable id (like pos) and "cell" one per cell of the final tableau.
+_OUTPUTS = (
+    ("status", np.int32, (), None),
+    ("value", np.float64, (), None),
+    ("pivots", np.int64, (2,), None),
+    ("rhs", np.float64, "row", None),
+    ("pos", np.int32, "var", "want_basis"),
+    ("var", np.int32, "var", "want_basis"),
+    ("matrices", np.float64, "cell", "want_matrices"),
+    ("reduced", np.float64, "var", "want_duals"),
+    ("range_lo", np.float64, "var", "want_ranges"),
+    ("range_hi", np.float64, "var", "want_ranges"),
+    ("certificate", np.float64, "var", "want_certificates"),
+)
+# Outputs a call passes only when it asks for them (else NULL), and adds to a reused `out` that lacks them.  The other
+# outputs are passed as `out` holds them.
+_EXTRAS = ("want_duals", "want_ranges", "want_certificates")
 
 
-def _add_outputs(out: dict, n: int, pv: int, want_duals: bool, want_ranges: bool = False,
-                 want_certificates: bool = False):
-    """The reduced costs, ranges and certificates a call wants, added to a reused `out` that lacks them."""
-    for k, want in (("reduced", want_duals), ("range_lo", want_ranges), ("range_hi", want_ranges),
-                    ("certificate", want_certificates)):
-        if want and out.get(k) is None:
-            out[k] = np.empty((n, pv), np.float64)
+def _shape(n: int, pack, height: int, width: int) -> tuple:
+    """The shape of one output of n uniform LPs."""
+    if isinstance(pack, tuple):
+        return (n,) + pack
+    return (n, {"row": height, "var": height + width, "cell": height * width}[pack])
 
 
-def _ragged_ranges(want_ranges: bool, pairs, rows: int, pvs: int) -> tuple:
-    """(range_lo, range_hi, packed pairs) of a ragged call, all None when no ranges are wanted."""
-    if not want_ranges:
-        return None, None, None
-    pr = None if pairs is None else _pairs_in(np.concatenate([np.asarray(p, np.int32).reshape(-1) for p in pairs]),
-                                              1, rows)
-    return np.empty(pvs, np.float64), np.empty(pvs, np.float64), pr
+def _batch_outputs(n: int, height: int, width: int, want: dict, mk=np.empty) -> dict:
+    """Fresh buffers of n uniform LPs: a key for every output up to the reduced costs, None where its flag is off (the
+    ranges and certificates are keys only when asked for, see _add_outputs)."""
+    return {key: mk(_shape(n, pack, height, width), dtype) if flag is None or want.get(flag) else None
+            for key, dtype, pack, flag in _OUTPUTS if flag not in ("want_ranges", "want_certificates")}
+
+
+def _add_outputs(out: dict, n: int, height: int, width: int, want: dict):
+    """The extras a call wants, added to `out` where it lacks them."""
+    for key, dtype, pack, flag in _OUTPUTS:
+        if flag in _EXTRAS and want.get(flag) and out.get(key) is None:
+            out[key] = np.empty(_shape(n, pack, height, width), dtype)
+
+
+def _out_args(out: dict, want: dict, pairs=None, omit: tuple = ()) -> list:
+    """The output arguments of a widest entry in table order, with the input `pairs` before range_lo; `omit`: the flags
+    of outputs a narrower entry does not take."""
+    args = []
+    for key, _, _, flag in _OUTPUTS:
+        if flag in omit:
+            continue
+        if key == "range_lo":
+            args.append(_ptr(pairs))
+        args.append(_ptr(out[key]) if flag not in _EXTRAS or want[flag] else None)
+    return args
+
+
+def _offsets(counts) -> np.ndarray:
+    """n + 1 int64 prefix sums of per-LP counts."""
+    offs = np.zeros(len(counts) + 1, np.int64)
+    np.cumsum(counts, out=offs[1:])
+    return offs
+
+
+def _pack_ragged(tableaus: Sequence, heights: np.ndarray, widths: np.ndarray) -> tuple:
+    """(cell offsets, n + 1 int64; the float64 tableaus back to back) of LPs of the given shapes."""
+    offs = _offsets(heights.astype(np.int64) * widths)
+    packed = np.empty(int(offs[-1]), np.float64)
+    for i, t in enumerate(tableaus):
+        packed[offs[i]:offs[i + 1]] = np.asarray(t, np.float64).reshape(-1)
+    return offs, packed
+
+
+def _solve_uniform(check, fn, handle, matrices, height: int, width: int, options, out, pos_in, var_in, pairs,
+                   want: dict) -> dict:
+    """Engine/MultiEngine.solve_batch through fn, a yalps_*solve_batch_certificate entry, on handle (ctx or multi)."""
+    opt = options or make_options()
+    m = np.ascontiguousarray(matrices, dtype=np.float64).reshape(-1)
+    cells = height * width
+    if cells <= 0 or m.size % cells:
+        raise ValueError(f"matrices has {m.size} values, not a multiple of {height}x{width}")
+    n = m.size // cells
+    if out is None:
+        out = _batch_outputs(n, height, width, want)
+    elif out["status"].shape[0] != n:
+        raise ValueError("out was allocated for a different batch size")
+    _add_outputs(out, n, height, width, want)
+    p, v = _basis_in(pos_in, var_in, n * (width + height))
+    pr = _pairs_in(pairs, n, height) if want["want_ranges"] else None
+    check(fn(handle, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), *_out_args(out, want, pr)))
+    return out
+
+
+def _solve_replicas(check, fn, handle, base, rhs, height: int, width: int, options, out, want: dict) -> dict:
+    """Engine/MultiEngine.solve_replicas through fn, a yalps_*solve_replicas_duals entry, on handle."""
+    opt = options or make_options()
+    b = np.ascontiguousarray(base, np.float64).reshape(-1)
+    r = np.ascontiguousarray(rhs, np.float64).reshape(-1)
+    if b.size != height * width or r.size % height:
+        raise ValueError("base must hold height*width values and rhs n*height")
+    n = r.size // height
+    if out is None:
+        out = _batch_outputs(n, height, width, want)
+    _add_outputs(out, n, height, width, want)
+    check(fn(handle, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
+             *_out_args(out, want, omit=("want_matrices", "want_ranges", "want_certificates"))))
+    return out
+
+
+def _solve_ragged(check, fn, handle, tableaus, shapes, options, pairs, want: dict, basis_in: bool) -> list:
+    """Engine/MultiEngine.solve_ragged through fn, a yalps_*solve_ragged_certificate entry, on handle; basis_in: fn
+    takes pos_in / var_in (passed as NULL)."""
+    opt = options or make_options()
+    n = len(tableaus)
+    if n == 0:
+        return []
+    heights = np.asarray([s[0] for s in shapes], np.int32)
+    widths = np.asarray([s[1] for s in shapes], np.int32)
+    offs, packed = _pack_ragged(tableaus, heights, widths)
+    at = {"row": _offsets(heights), "var": _offsets(heights.astype(np.int64) + widths), "cell": offs}
+    out = {key: np.empty((n,) + pack if isinstance(pack, tuple) else int(at[pack][-1]), dtype)
+           if flag is None or want[flag] else None for key, dtype, pack, flag in _OUTPUTS}
+    pr = None if not want["want_ranges"] or pairs is None else _pairs_in(
+        np.concatenate([np.asarray(p, np.int32).reshape(-1) for p in pairs]), 1, int(at["row"][-1]))
+    check(fn(handle, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed),
+             *((None, None) if basis_in else ()), C.byref(opt), *_out_args(out, want, pr)))
+    res = []
+    for i in range(n):
+        r = {"status": int(out["status"][i]), "value": float(out["value"][i]),
+             "pivots": (int(out["pivots"][i, 0]), int(out["pivots"][i, 1]))}
+        for key, _, pack, flag in _OUTPUTS:
+            if isinstance(pack, str) and (flag not in _EXTRAS or want[flag]):
+                a, o = out[key], at[pack]
+                r["matrix" if key == "matrices" else key] = None if a is None else a[o[i]:o[i + 1]]
+        res.append(r)
+    return res
+
+
+_STATS = ("nodes", "node_pivots", "max_cuts", "max_heap", "waves", "device_nodes", "wave_us", "bnb_us",
+          "sharded_waves", "allreduces")
+
+
+def _search_result(width: int, status, result, out_h, rhs, pos, var, stats, root: Optional[tuple] = None) -> dict:
+    """The dict of a branch-and-cut call from its C outputs; root: (status, value, pivots) of the root LP, if reported.
+    stats names its first len(stats) counters."""
+    h = out_h.value
+    res = {"status": status.value, "result": result.value, "height": h, "rhs": rhs[:h], "pos": pos[:width + h],
+           "var": var[:width + h]}
+    if root is not None:
+        res.update(root_status=root[0].value, root_value=root[1].value,
+                   root_pivots=(int(root[2][0]), int(root[2][1])))
+    res["stats"] = {k: int(v) for k, v in zip(_STATS, stats)}
+    return res
 
 
 def make_options(precision=1e-8, max_pivots=8192, check_cycles=False, tolerance=0.0, timeout_ms=math.inf,
@@ -161,8 +283,8 @@ class Engine:
     def batch_outputs(self, n: int, height: int, width: int, want_matrices: bool = False, want_basis: bool = True,
                       pinned: bool = False, want_duals: bool = False) -> dict:
         """Output buffers for solve_batch; pinned=True allocates them page-locked (reusable across calls)."""
-        return _batch_outputs(n, height, width, want_matrices, want_basis, want_duals,
-                              self.pinned_empty if pinned else np.empty)
+        return _batch_outputs(n, height, width, {"want_matrices": want_matrices, "want_basis": want_basis,
+                                                 "want_duals": want_duals}, self.pinned_empty if pinned else np.empty)
 
     def solve_batch(self, matrices: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrices: bool = False, want_basis: bool = True, out: Optional[dict] = None,
@@ -181,26 +303,10 @@ class Engine:
         want_certificates: also out["certificate"] (n, width+height), the Farkas certificate of an infeasible LP or the
         ray of an unbounded one, computed on the device from the final tableaus (yalps_solve_batch_certificate; NaN
         for every other status)."""
-        opt = options or make_options()
-        m = np.ascontiguousarray(matrices, dtype=np.float64).reshape(-1)
-        cells = height * width
-        if cells <= 0 or m.size % cells:
-            raise ValueError(f"matrices has {m.size} values, not a multiple of {height}x{width}")
-        n = m.size // cells
-        if out is None:
-            out = self.batch_outputs(n, height, width, want_matrices, want_basis, want_duals=want_duals)
-        elif out["status"].shape[0] != n:
-            raise ValueError("out was allocated for a different batch size")
-        _add_outputs(out, n, width + height, want_duals, want_ranges, want_certificates)
-        p, v = _basis_in(pos_in, var_in, n * (width + height))
-        pr = _pairs_in(pairs, n, height) if want_ranges else None
-        self._check(self._lib.yalps_solve_batch_certificate(
-            self._ctx, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
-            _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-            _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None, _ptr(pr),
-            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None,
-            _ptr(out["certificate"]) if want_certificates else None))
-        return out
+        return _solve_uniform(self._check, self._lib.yalps_solve_batch_certificate, self._ctx, matrices, height, width,
+                              options, out, pos_in, var_in, pairs,
+                              {"want_matrices": want_matrices, "want_basis": want_basis, "want_duals": want_duals,
+                               "want_ranges": want_ranges, "want_certificates": want_certificates})
 
     def simplex(self, tableau, options: Optional[Options] = None) -> tuple:
         """simplex(tableau, options) -> (status, number), src/simplex.ts:144, with the reference's in-place contract:
@@ -226,20 +332,8 @@ class Engine:
                        want_duals: bool = False) -> dict:
         """n replicas of `base` (height*width) that differ only in column 0: rhs is float64 (n, height).
         want_duals: also out["reduced"] (n, width+height), as solve_batch."""
-        opt = options or make_options()
-        b = np.ascontiguousarray(base, np.float64).reshape(-1)
-        r = np.ascontiguousarray(rhs, np.float64).reshape(-1)
-        if b.size != height * width or r.size % height:
-            raise ValueError("base must hold height*width values and rhs n*height")
-        n = r.size // height
-        if out is None:
-            out = self.batch_outputs(n, height, width, False, want_basis, want_duals=want_duals)
-        _add_outputs(out, n, width + height, want_duals)
-        self._check(self._lib.yalps_solve_replicas_duals(self._ctx, n, height, width, _ptr(b), _ptr(r), C.byref(opt),
-                                                         _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
-                                                         _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-                                                         _ptr(out["reduced"]) if want_duals else None))
-        return out
+        return _solve_replicas(self._check, self._lib.yalps_solve_replicas_duals, self._ctx, base, rhs, height, width,
+                               options, out, {"want_basis": want_basis, "want_duals": want_duals})
 
     def set_replica_sharing(self, on: bool = True):
         """solve_replicas: follow the base tableau's pivot path while a replica makes the same choices (default on)."""
@@ -257,50 +351,10 @@ class Engine:
         want_duals: every result also has "reduced" (width_i+height_i values, as solve_batch).
         want_ranges: every result also has "range_lo", "range_hi" (as solve_batch); pairs[i] (height_i int32) or None.
         want_certificates: every result also has "certificate" (width_i+height_i values, as solve_batch)."""
-        opt = options or make_options()
-        n = len(tableaus)
-        if n == 0:
-            return []
-        heights = np.asarray([s[0] for s in shapes], np.int32)
-        widths = np.asarray([s[1] for s in shapes], np.int32)
-        cells = heights.astype(np.int64) * widths
-        offs = np.zeros(n + 1, np.int64)
-        np.cumsum(cells, out=offs[1:])
-        packed = np.empty(int(offs[-1]), np.float64)
-        for i, t in enumerate(tableaus):
-            packed[offs[i]:offs[i + 1]] = np.asarray(t, np.float64).reshape(-1)
-        roffs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights, out=roffs[1:])
-        poffs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights.astype(np.int64) + widths, out=poffs[1:])
-        status = np.empty(n, np.int32)
-        value = np.empty(n, np.float64)
-        pivots = np.empty((n, 2), np.int64)
-        rhs = np.empty(int(roffs[-1]), np.float64)
-        pos = np.empty(int(poffs[-1]), np.int32)
-        var = np.empty(int(poffs[-1]), np.int32)
-        mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
-        red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
-        rlo, rhi, pr = _ragged_ranges(want_ranges, pairs, int(roffs[-1]), int(poffs[-1]))
-        cert = np.empty(int(poffs[-1]), np.float64) if want_certificates else None
-        self._check(self._lib.yalps_solve_ragged_certificate(
-            self._ctx, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), None, None, C.byref(opt),
-            _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
-            _ptr(rlo), _ptr(rhi), _ptr(cert)))
-        res = []
-        for i in range(n):
-            res.append({
-                "status": int(status[i]), "value": float(value[i]), "pivots": (int(pivots[i, 0]), int(pivots[i, 1])),
-                "rhs": rhs[roffs[i]:roffs[i + 1]], "pos": pos[poffs[i]:poffs[i + 1]], "var": var[poffs[i]:poffs[i + 1]],
-                "matrix": mats[offs[i]:offs[i + 1]] if want_matrices else None,
-            })
-            if want_duals:
-                res[i]["reduced"] = red[poffs[i]:poffs[i + 1]]
-            if want_ranges:
-                res[i]["range_lo"], res[i]["range_hi"] = rlo[poffs[i]:poffs[i + 1]], rhi[poffs[i]:poffs[i + 1]]
-            if want_certificates:
-                res[i]["certificate"] = cert[poffs[i]:poffs[i + 1]]
-        return res
+        return _solve_ragged(self._check, self._lib.yalps_solve_ragged_certificate, self._ctx, tableaus, shapes,
+                             options, pairs, {"want_basis": True, "want_matrices": want_matrices,
+                                              "want_duals": want_duals, "want_ranges": want_ranges,
+                                              "want_certificates": want_certificates}, basis_in=True)
 
     def solve_batch_device(self, n: int, height: int, width: int, d_matrices: int, options: Optional[Options] = None,
                            d_work: int = 0, d_status: int = 0, d_value: int = 0, d_pivots: int = 0, d_rhs: int = 0,
@@ -405,22 +459,18 @@ class Engine:
         values = np.ascontiguousarray(values, np.float64).reshape(-1)
         if cells.size != values.size:
             raise ValueError("cells and values must have the same length")
-        status, value = C.c_int32(), C.c_double()
-        piv = np.zeros(2, np.int64)
-        rhs, pos, var = np.empty(height), np.empty(width + height, np.int32), np.empty(width + height, np.int32)
-        out = {"reduced": np.empty(width + height, np.float64)}
-        wanted = (("range_lo", want_ranges), ("range_hi", want_ranges), ("certificate", want_certificates))
-        out.update({k: np.empty(width + height, np.float64) for k, want in wanted if want})
+        want = {"want_basis": True, "want_duals": True, "want_ranges": want_ranges,
+                "want_certificates": want_certificates}
+        out = _batch_outputs(1, height, width, want)
+        _add_outputs(out, 1, height, width, want)
         pr = _pairs_in(pairs, 1, height) if want_ranges else None
         self._check(self._lib.yalps_solve_sparse_certificate(self._ctx, height, width, int(cells.size),
                                                              _ptr(cells) if cells.size else None,
                                                              _ptr(values) if values.size else None, C.byref(opt),
-                                                             C.byref(status), C.byref(value), _ptr(piv), _ptr(rhs),
-                                                             _ptr(pos), _ptr(var), _ptr(out["reduced"]), _ptr(pr),
-                                                             _ptr(out.get("range_lo")), _ptr(out.get("range_hi")),
-                                                             _ptr(out.get("certificate"))))
-        return {"status": status.value, "value": value.value, "pivots": (int(piv[0]), int(piv[1])), "rhs": rhs,
-                "pos": pos, "var": var, **out}
+                                                             *_out_args(out, want, pr, omit=("want_matrices",))))
+        return {"status": int(out.pop("status")[0]), "value": float(out.pop("value")[0]),
+                "pivots": tuple(int(p) for p in out.pop("pivots")[0]),
+                **{k: a[0] for k, a in out.items() if a is not None}}
 
     def solve_tableau(self, matrix: np.ndarray, height: int, width: int, integers: Sequence[int], sign: float,
                       options: Optional[Options] = None, cells: Optional[np.ndarray] = None) -> dict:
@@ -449,15 +499,7 @@ class Engine:
                                                      C.byref(opt), C.byref(status), C.byref(result), C.byref(out_h),
                                                      _ptr(rhs), _ptr(pos), _ptr(var), C.byref(root_status),
                                                      C.byref(root_value), _ptr(root_piv), _ptr(stats)))
-        h = out_h.value
-        return {
-            "status": status.value, "result": result.value, "height": h, "rhs": rhs[:h], "pos": pos[:width + h],
-            "var": var[:width + h], "root_status": root_status.value, "root_value": root_value.value,
-            "root_pivots": (int(root_piv[0]), int(root_piv[1])),
-            "stats": {"nodes": int(stats[0]), "node_pivots": int(stats[1]), "max_cuts": int(stats[2]),
-                      "max_heap": int(stats[3]), "waves": int(stats[4]), "device_nodes": int(stats[5]),
-                      "wave_us": int(stats[6]), "bnb_us": int(stats[7])},
-        }
+        return _search_result(width, status, result, out_h, rhs, pos, var, stats, (root_status, root_value, root_piv))
 
     def branch_and_cut(self, integers: Sequence[int], sign: float, init_result: float,
                        options: Optional[Options] = None) -> dict:
@@ -475,12 +517,7 @@ class Engine:
         self._check(self._lib.yalps_branch_and_cut(self._ctx, _ptr(ints), int(ints.size), float(sign),
                                                    float(init_result), C.byref(opt), C.byref(status), C.byref(result),
                                                    C.byref(out_h), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(stats)))
-        h = out_h.value
-        return {"status": status.value, "result": result.value, "height": h, "rhs": rhs[:h], "pos": pos[:W + h],
-                "var": var[:W + h],
-                "stats": {"nodes": int(stats[0]), "node_pivots": int(stats[1]), "max_cuts": int(stats[2]),
-                          "max_heap": int(stats[3]), "waves": int(stats[4]), "device_nodes": int(stats[5]),
-                          "wave_us": int(stats[6]), "bnb_us": int(stats[7])}}
+        return _search_result(W, status, result, out_h, rhs, pos, var, stats)
 
     # ------------------------------------------------------------------ probes
     def round_to_precision(self, x: np.ndarray, precision: float) -> np.ndarray:
@@ -574,75 +611,23 @@ class MultiEngine:
                     want_matrices: bool = False, pos_in=None, var_in=None, out: Optional[dict] = None,
                     want_duals: bool = False, want_ranges: bool = False, pairs=None,
                     want_certificates: bool = False) -> dict:
-        opt = options or make_options()
-        m = np.ascontiguousarray(matrices, np.float64).reshape(-1)
-        n = m.size // (height * width)
-        out = out or _batch_outputs(n, height, width, want_matrices, want_duals=want_duals)
-        p = None if pos_in is None else np.ascontiguousarray(pos_in, np.int32).reshape(-1)
-        v = None if var_in is None else np.ascontiguousarray(var_in, np.int32).reshape(-1)
-        _add_outputs(out, n, width + height, want_duals, want_ranges, want_certificates)
-        self._check(self._lib.yalps_multi_solve_batch_certificate(
-            self._m, n, height, width, _ptr(m), _ptr(p), _ptr(v), C.byref(opt), _ptr(out["status"]),
-            _ptr(out["value"]), _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-            _ptr(out["matrices"]), _ptr(out["reduced"]) if want_duals else None,
-            _ptr(_pairs_in(pairs, n, height)) if want_ranges else None,
-            _ptr(out["range_lo"]) if want_ranges else None, _ptr(out["range_hi"]) if want_ranges else None,
-            _ptr(out["certificate"]) if want_certificates else None))
-        return out
+        return _solve_uniform(self._check, self._lib.yalps_multi_solve_batch_certificate, self._m, matrices, height,
+                              width, options, out, pos_in, var_in, pairs,
+                              {"want_matrices": want_matrices, "want_basis": True, "want_duals": want_duals,
+                               "want_ranges": want_ranges, "want_certificates": want_certificates})
 
     def solve_replicas(self, base: np.ndarray, rhs: np.ndarray, height: int, width: int,
                        options: Optional[Options] = None, out: Optional[dict] = None, want_duals: bool = False) -> dict:
-        opt = options or make_options()
-        b = np.ascontiguousarray(base, np.float64).reshape(-1)
-        r = np.ascontiguousarray(rhs, np.float64).reshape(-1)
-        n = r.size // height
-        out = out or _batch_outputs(n, height, width, want_duals=want_duals)
-        _add_outputs(out, n, width + height, want_duals)
-        self._check(self._lib.yalps_multi_solve_replicas_duals(
-            self._m, n, height, width, _ptr(b), _ptr(r), C.byref(opt), _ptr(out["status"]), _ptr(out["value"]),
-            _ptr(out["pivots"]), _ptr(out["rhs"]), _ptr(out["pos"]), _ptr(out["var"]),
-            _ptr(out["reduced"]) if want_duals else None))
-        return out
+        return _solve_replicas(self._check, self._lib.yalps_multi_solve_replicas_duals, self._m, base, rhs, height,
+                               width, options, out, {"want_basis": True, "want_duals": want_duals})
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
                      want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,
                      pairs: Optional[Sequence] = None, want_certificates: bool = False) -> list:
-        opt = options or make_options()
-        n = len(tableaus)
-        if n == 0:
-            return []
-        heights = np.asarray([s[0] for s in shapes], np.int32)
-        widths = np.asarray([s[1] for s in shapes], np.int32)
-        offs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights.astype(np.int64) * widths, out=offs[1:])
-        packed = np.concatenate([np.asarray(t, np.float64).reshape(-1) for t in tableaus])
-        roffs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights, out=roffs[1:])
-        poffs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights.astype(np.int64) + widths, out=poffs[1:])
-        status, value, pivots = np.empty(n, np.int32), np.empty(n, np.float64), np.empty((n, 2), np.int64)
-        rhs, pos, var = np.empty(int(roffs[-1])), np.empty(int(poffs[-1]), np.int32), np.empty(int(poffs[-1]), np.int32)
-        mats = np.empty(int(offs[-1]), np.float64) if want_matrices else None
-        red = np.empty(int(poffs[-1]), np.float64) if want_duals else None
-        rlo, rhi, pr = _ragged_ranges(want_ranges, pairs, int(roffs[-1]), int(poffs[-1]))
-        cert = np.empty(int(poffs[-1]), np.float64) if want_certificates else None
-        self._check(self._lib.yalps_multi_solve_ragged_certificate(
-            self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()), _ptr(packed), C.byref(opt),
-            _ptr(status), _ptr(value), _ptr(pivots), _ptr(rhs), _ptr(pos), _ptr(var), _ptr(mats), _ptr(red), _ptr(pr),
-            _ptr(rlo), _ptr(rhi), _ptr(cert)))
-        res = [{"status": int(status[i]), "value": float(value[i]), "pivots": (int(pivots[i, 0]), int(pivots[i, 1])),
-                "rhs": rhs[roffs[i]:roffs[i + 1]], "pos": pos[poffs[i]:poffs[i + 1]], "var": var[poffs[i]:poffs[i + 1]],
-                "matrix": mats[offs[i]:offs[i + 1]] if want_matrices else None} for i in range(n)]
-        if want_duals:
-            for i in range(n):
-                res[i]["reduced"] = red[poffs[i]:poffs[i + 1]]
-        if want_ranges:
-            for i in range(n):
-                res[i]["range_lo"], res[i]["range_hi"] = rlo[poffs[i]:poffs[i + 1]], rhi[poffs[i]:poffs[i + 1]]
-        if want_certificates:
-            for i in range(n):
-                res[i]["certificate"] = cert[poffs[i]:poffs[i + 1]]
-        return res
+        return _solve_ragged(self._check, self._lib.yalps_multi_solve_ragged_certificate, self._m, tableaus, shapes,
+                             options, pairs, {"want_basis": True, "want_matrices": want_matrices,
+                                              "want_duals": want_duals, "want_ranges": want_ranges,
+                                              "want_certificates": want_certificates}, basis_in=False)
 
     def solve_large(self, matrix: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrix: bool = False) -> dict:
@@ -688,14 +673,7 @@ class MultiEngine:
                                                 C.byref(status), C.byref(result), C.byref(out_h), _ptr(rhs), _ptr(pos),
                                                 _ptr(var), C.byref(root_status), C.byref(root_value), _ptr(root_piv),
                                                 _ptr(stats)))
-        h = out_h.value
-        return {"status": status.value, "result": result.value, "height": h, "rhs": rhs[:h], "pos": pos[:width + h],
-                "var": var[:width + h], "root_status": root_status.value, "root_value": root_value.value,
-                "root_pivots": (int(root_piv[0]), int(root_piv[1])),
-                "stats": {"nodes": int(stats[0]), "node_pivots": int(stats[1]), "max_cuts": int(stats[2]),
-                          "max_heap": int(stats[3]), "waves": int(stats[4]), "device_nodes": int(stats[5]),
-                          "wave_us": int(stats[6]), "bnb_us": int(stats[7]), "sharded_waves": int(stats[8]),
-                          "allreduces": int(stats[9])}}
+        return _search_result(width, status, result, out_h, rhs, pos, var, stats, (root_status, root_value, root_piv))
 
     def solve_many_tableaus(self, tabmods: Sequence, options: Optional[Options] = None,
                             searches_per_device: int = 4) -> list:
@@ -707,17 +685,12 @@ class MultiEngine:
         heights = np.asarray([tm.tableau.height for tm in tabmods], np.int32)
         widths = np.asarray([tm.tableau.width for tm in tabmods], np.int32)
         nints = np.asarray([len(tm.integers) for tm in tabmods], np.int64)
-        offs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights.astype(np.int64) * widths, out=offs[1:])
-        packed = np.concatenate([np.asarray(tm.tableau.matrix, np.float64).reshape(-1) for tm in tabmods])
-        ioffs = np.zeros(n + 1, np.int64)
-        np.cumsum(nints, out=ioffs[1:])
+        offs, packed = _pack_ragged([tm.tableau.matrix for tm in tabmods], heights, widths)
+        ioffs = _offsets(nints)
         ints = np.asarray([v for tm in tabmods for v in tm.integers], np.int32) if ioffs[-1] else np.zeros(1, np.int32)
         signs = np.asarray([tm.sign for tm in tabmods], np.float64)
-        roffs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights + 2 * nints, out=roffs[1:])
-        poffs = np.zeros(n + 1, np.int64)
-        np.cumsum(heights.astype(np.int64) + widths + 2 * nints, out=poffs[1:])
+        roffs = _offsets(heights + 2 * nints)
+        poffs = _offsets(heights.astype(np.int64) + widths + 2 * nints)
         status, result, out_h = np.empty(n, np.int32), np.empty(n, np.float64), np.empty(n, np.int32)
         rhs, pos, var = np.empty(int(roffs[-1])), np.empty(int(poffs[-1]), np.int32), np.empty(int(poffs[-1]), np.int32)
         self._check(self._lib.yalps_multi_solve_many(self._m, n, _ptr(heights), _ptr(widths), _ptr(offs[:-1].copy()),
