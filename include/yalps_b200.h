@@ -417,6 +417,41 @@ int yalps_certificate_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t 
                              const int32_t *d_pos, const int32_t *d_status, const double *d_value, double precision,
                              double *d_cert_out, void *stream);
 
+/* ---- irreducible infeasible subsets: which constraints conflict ------------------------------------------------
+ * For a row set S of 1..height-1, T_S is the tableau with every row outside S set to +0.0 (column 0 included); row 0,
+ * the objective, always stays.  With precision >= 0 the simplex never picks a zero row in phase 1 (its RHS is not
+ * < -precision), never in the ratio test (its cell is not > precision) and never changes it in a pivot (its cells are
+ * not above 1e-16): status, value, pivot counts and every other row are those of the model without the removed rows,
+ * bit for bit.  Variables keep their implicit x >= 0 in every subset.
+ * supp(cert) of an infeasible LP is the set of rows k with cert[width + k] > +0.0 (the raw value: NaN and both zeros
+ * do not count), the rows its Farkas certificate combines.  Words of a row mask: words = (height + 31) / 32, bit r of
+ * word r / 32 is row r.
+ *
+ * n LPs = base restricted to row subsets (keep: n*words uint32, bit r = row r; row 0 always kept, bit 0 ignored, bits
+ * >= height must be clear), expanded on the device; outputs as yalps_solve_batch plus cert_out[n*(width+height)] and
+ * support_out[n*words] (zero words unless infeasible), each may be NULL.  A negative or NaN precision is
+ * YALPS_ERR_ARGUMENT. */
+int yalps_solve_row_subsets(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
+                            const uint32_t *keep, const yalps_options *opt, int32_t *status, double *value,
+                            int64_t *pivots, double *cert_out, uint32_t *support_out);
+/* An IIS: a row set S whose T_S the solver finds infeasible while every T_{S \ {r}} it finds optimal or unbounded, by
+ * deletion rounds on the GPU.  Round 0 solves the whole tableau; if it is not infeasible that status is returned with
+ * *count = 0.  Otherwise S = supp(cert), and each round solves T_S and every T_{S \ {u}}, u in S, as one batch: when
+ * T_S is not infeasible S falls back to the last set solved infeasible; when no T_{S \ {u}} is infeasible S is the
+ * result; else S becomes the support of the infeasible T_{S \ {u}} with the smallest support (lowest u on ties).
+ * S strictly shrinks, so there are at most height rounds.  opt->max_pivots and check_cycles apply to every subset LP;
+ * opt->timeout_ms (+inf: none) is checked between rounds and returns the last set solved infeasible.
+ * status = the model's own status, rows_out[height] ascending, *count rows; stats[5] (may be NULL): rounds (round 0
+ * included), LPs solved, their pivots (both phases), undecided rows (u whose T_{S \ {u}} ended `cycled` in the final
+ * round), timed out (0/1).  S is irreducible when the last two are 0.  A negative or NaN precision is
+ * YALPS_ERR_ARGUMENT. */
+int yalps_iis(yalps_ctx *ctx, int32_t height, int32_t width, const double *matrix, const yalps_options *opt,
+              int32_t *status, int32_t *rows_out, int32_t *count, int64_t *stats);
+/* yalps_iis with the tableau given as (cell, value) stores into a zero matrix, as yalps_solve_sparse */
+int yalps_iis_sparse(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nnz, const int32_t *cell,
+                     const double *val, const yalps_options *opt, int32_t *status, int32_t *rows_out,
+                     int32_t *count, int64_t *stats);
+
 /* ---- one process, several GPUs (SURVEY 8b/8e) ------------------------------------------------------------
  * The reference is single-process and synchronous (src/YALPS.ts:73-92); a Node addon cannot use torchrun.  A
  * yalps_multi owns one ctx (plus worker ctxs for concurrent branch-and-cut searches) per entry of `devices` and one

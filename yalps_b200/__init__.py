@@ -7,6 +7,7 @@ it without a CUDA device, raises.
 """
 from .constraint import equal_to, equalTo, greater_eq, greaterEq, in_range, inRange, less_eq, lessEq
 from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
+from .iis import model_iis
 from .solver import default_options, defaultOptions, get_engine, solve, solve_many, solveMany
 from .mps import apply_bounds, model_from_mps, netlib_model
 from .sensitivity import (certificate_from_tableau, model_certificate, model_ranges, model_sensitivity,
@@ -18,5 +19,5 @@ __all__ = [
     "in_range", "lessEq", "greaterEq", "equalTo", "inRange", "Engine", "MultiEngine", "make_options", "STATUS_NAMES",
     "tableau_model", "Tableau", "TableauModel", "get_engine", "model_from_mps", "netlib_model", "apply_bounds",
     "constraint_rows", "split_reduced", "model_sensitivity", "reduced_from_tableau", "ranges_from_tableau", "row_pairs",
-    "model_ranges", "certificate_from_tableau", "model_certificate",
+    "model_ranges", "certificate_from_tableau", "model_certificate", "model_iis",
 ]

@@ -142,6 +142,11 @@ SIGNATURES = {
                                                       _vp, _vp, _vp]),
     "yalps_multi_solve_ragged_certificate": (C.c_int, [_vp, C.c_int64, _vp, _vp, _vp, _vp, C.POINTER(Options), _vp, _vp,
                                                        _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "yalps_solve_row_subsets": (C.c_int, [_vp, C.c_int64, C.c_int32, C.c_int32, _vp, _vp, C.POINTER(Options), _vp, _vp,
+                                          _vp, _vp, _vp]),
+    "yalps_iis": (C.c_int, [_vp, C.c_int32, C.c_int32, _vp, C.POINTER(Options), _ip, _vp, _ip, _vp]),
+    "yalps_iis_sparse": (C.c_int, [_vp, C.c_int32, C.c_int32, C.c_int64, _vp, _vp, C.POINTER(Options), _ip, _vp, _ip,
+                                   _vp]),
     "yalps_round_to_precision": (C.c_int, [_vp, C.c_int64, _vp, C.c_double, _vp]),
     "yalps_measure_smem_bandwidth": (C.c_int, [_vp, _dp, _dp]),
     "yalps_measure_tmem_bandwidth": (C.c_int, [_vp, _dp, _dp]),

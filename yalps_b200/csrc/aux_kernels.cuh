@@ -108,6 +108,36 @@ __global__ void k_expand_replicas(long long n, int H, int W, const double *base,
   }
 }
 
+// Row subsets of one base tableau (yalps_solve_row_subsets): LP i is `base` with every row r >= 1 whose bit is clear in
+// keep[i*words + r/32] set to +0.0 in every cell, column 0 included.  The simplex then follows the trajectory of the
+// model without those rows (DESIGN §3), so the caller ships the base once and H/8 bytes of mask per LP.  Write-bound:
+// one warp per (LP, row), whose keep word lane 0 reads once; a zeroed row does not read the base; a row is stored as
+// 16-byte pairs from its first 16-byte aligned cell (consecutive tableaus, and the rows of an odd width, are only
+// 8-byte aligned).  Cells move as 64-bit integers, so NaN payloads and signed zeros keep their bits.
+__global__ void k_expand_subsets(long long n, int H, int W, int words, const double *base, const unsigned *keep,
+                                 double *out) {
+  const int lane = threadIdx.x & 31;
+  const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+  const long long *src0 = reinterpret_cast<const long long *>(base);
+  for (long long item = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); item < n * H; item += warps) {
+    const long long i = item / H;
+    const int r = (int)(item - i * H);
+    unsigned w = 0;
+    if (lane == 0) w = keep[i * words + (r >> 5)];
+    w = __shfl_sync(0xffffffffu, w, 0);
+    const bool kept = r == 0 || ((w >> (r & 31)) & 1u);
+    long long *dst = reinterpret_cast<long long *>(out) + item * W;
+    const long long *src = src0 + (size_t)r * W;
+    const int head = min((int)((reinterpret_cast<uintptr_t>(dst) >> 3) & 1), W);  // 1: dst is 8 mod 16
+    const int pairs = (W - head) >> 1;
+    if (lane == 0 && head) dst[0] = kept ? src[0] : 0;
+    longlong2 *d2 = reinterpret_cast<longlong2 *>(dst + head);
+    for (int k = lane; k < pairs; k += 32)
+      d2[k] = kept ? make_longlong2(src[head + 2 * k], src[head + 2 * k + 1]) : make_longlong2(0, 0);
+    if (lane == 0 && head + 2 * pairs < W) dst[W - 1] = kept ? src[W - 1] : 0;
+  }
+}
+
 // ---- replica path sharing (yalps_solve_replicas) -----------------------------------------------------------------
 // n replicas of one tableau differ only in column 0.  Everything else of the tableau -- objective row, pivot rows and
 // columns, the basis bookkeeping -- evolves identically for every replica that makes the same pivot choices, and those

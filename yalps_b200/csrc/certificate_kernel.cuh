@@ -93,4 +93,26 @@ __global__ void __launch_bounds__(kCertThreads) k_certificate(CertArgs a, int wa
   }
 }
 
+// The rows a Farkas certificate uses (yalps_solve_row_subsets, the IIS search): bit r of support[i*words + r/32] is
+// set when LP i is infeasible and cert[i*(W+H) + W + r] > +0.0, rows 1..H-1 (the raw value: NaN and both zeros do not
+// count, noise above zero does); count[i] is the number of bits set.  Every other LP gets zero words.  Uniform batches
+// only.  One warp per LP: lane l reads row 32k + l, the ballot is word k.
+__global__ void k_cert_support(long long n, int H, int W, int words, const int *status, const double *cert,
+                               unsigned *support, int *count) {
+  const int lane = threadIdx.x & 31;
+  const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+  for (long long i = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += warps) {
+    const bool inf = status[i] == ST_INFEASIBLE;
+    const double *y = cert + i * (long long)(W + H) + W;
+    int total = 0;
+    for (int k = 0; k < words; k++) {
+      const int r = 32 * k + lane;
+      const unsigned m = __ballot_sync(0xffffffffu, inf && r >= 1 && r < H && y[r] > 0.0);
+      if (lane == 0) support[i * words + k] = m;
+      total += __popc(m);
+    }
+    if (lane == 0) count[i] = total;
+  }
+}
+
 }  // namespace yalps

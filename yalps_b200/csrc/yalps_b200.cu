@@ -1453,6 +1453,35 @@ int solve_small(yalps_ctx *ctx, const HostBatch &b, const BatchLayout &L, bool *
   return check_device_status(ctx, b.status, n);
 }
 
+// The (cell, value) stores of request b (b.nnz >= 0) into the tableau d_M of `cells` cells, on stream st: the pairs
+// cross PCIe, the zeros are written by the device.  b.dup_cells is valid once st has reached this point.
+int scatter_cells(yalps_ctx *ctx, HostBatch &b, double *d_M, size_t cells, cudaStream_t st) {
+  const size_t nnz = (size_t)b.nnz, val_off = (nnz * 4 + 15) & ~(size_t)15;
+  void *h_coo, *d_coo, *d_flag;
+  int rc;
+  if ((rc = pin_ensure(ctx, "coo", val_off + nnz * 8 + 16, &h_coo))) return rc;
+  if ((rc = dev_ensure(ctx, "coo", val_off + nnz * 8 + 16, &d_coo))) return rc;
+  if ((rc = dev_ensure(ctx, "coo_flag", 4, &d_flag))) return rc;
+  if (nnz) {
+    std::memcpy(h_coo, b.cell, nnz * 4);
+    std::memcpy((char *)h_coo + val_off, b.val, nnz * 8);
+    CU(ctx, cudaMemcpyAsync(d_coo, h_coo, val_off + nnz * 8, cudaMemcpyHostToDevice, st));
+  }
+  CU(ctx, cudaMemsetAsync(d_M, 0, cells * 8, st));
+  CU(ctx, cudaMemsetAsync(d_flag, 0, 4, st));
+  if (nnz) {
+    const int blocks = (int)std::min<size_t>((nnz + 255) / 256, (size_t)ctx->prop.multiProcessorCount * 8);
+    const int *d_cell = (const int *)d_coo;
+    const double *d_val = (const double *)((char *)d_coo + val_off);
+    k_scatter_cells<<<blocks, 256, 0, st>>>((long long)nnz, d_cell, d_val, d_M);
+    k_verify_cells<<<blocks, 256, 0, st>>>((long long)nnz, d_cell, d_val, (const double *)d_M, (int *)d_flag);
+    ctx->launches += 2;
+    CU(ctx, cudaGetLastError());
+  }
+  CU(ctx, cudaMemcpyAsync(&b.dup_cells, d_flag, 4, cudaMemcpyDeviceToHost, st));
+  return 0;
+}
+
 // The pipelined path: two slots; a large batch is cut into ~8 chunks (64 MiB .. 1.5 GiB each) so that the H2D copy of
 // chunk k+1 overlaps the kernel and the D2H copies of chunk k.
 int solve_chunks(yalps_ctx *ctx, HostBatch &b, const BatchLayout &L) {
@@ -1529,29 +1558,7 @@ int solve_chunks(yalps_ctx *ctx, HostBatch &b, const BatchLayout &L) {
                                   (size_t)b.heights[i] * b.widths[i] * 8, cudaMemcpyHostToDevice, st));
       }
     } else if (from_cells) {
-      // the (cell, value) pairs cross PCIe, the zeros are written by the device
-      const size_t nnz = (size_t)b.nnz, val_off = (nnz * 4 + 15) & ~(size_t)15;
-      void *h_coo, *d_coo, *d_flag;
-      if ((rc = pin_ensure(ctx, "coo", val_off + nnz * 8 + 16, &h_coo))) return rc;
-      if ((rc = dev_ensure(ctx, "coo", val_off + nnz * 8 + 16, &d_coo))) return rc;
-      if ((rc = dev_ensure(ctx, "coo_flag", 4, &d_flag))) return rc;
-      if (nnz) {
-        std::memcpy(h_coo, b.cell, nnz * 4);
-        std::memcpy((char *)h_coo + val_off, b.val, nnz * 8);
-        CU(ctx, cudaMemcpyAsync(d_coo, h_coo, val_off + nnz * 8, cudaMemcpyHostToDevice, st));
-      }
-      CU(ctx, cudaMemsetAsync(d_in, 0, ccells * 8, st));
-      CU(ctx, cudaMemsetAsync(d_flag, 0, 4, st));
-      if (nnz) {
-        const int blocks = (int)std::min<size_t>((nnz + 255) / 256, (size_t)ctx->prop.multiProcessorCount * 8);
-        const int *d_cell = (const int *)d_coo;
-        const double *d_val = (const double *)((char *)d_coo + val_off);
-        k_scatter_cells<<<blocks, 256, 0, st>>>((long long)nnz, d_cell, d_val, (double *)d_in);
-        k_verify_cells<<<blocks, 256, 0, st>>>((long long)nnz, d_cell, d_val, (const double *)d_in, (int *)d_flag);
-        ctx->launches += 2;
-        CU(ctx, cudaGetLastError());
-      }
-      CU(ctx, cudaMemcpyAsync(&b.dup_cells, d_flag, 4, cudaMemcpyDeviceToHost, st));
+      if ((rc = scatter_cells(ctx, b, (double *)d_in, ccells, st))) return rc;
     } else {
       CU(ctx, cudaMemcpyAsync(d_in, src, ccells * 8, cudaMemcpyHostToDevice, st));
     }
@@ -2312,3 +2319,4 @@ int yalps_measure_tmem_bandwidth(yalps_ctx *ctx, double *gbs, double *sm_clock_m
 
 #include "bnb.inl"
 #include "multi.inl"
+#include "iis.inl"

@@ -183,6 +183,37 @@ def _solve_ragged(check, fn, handle, tableaus, shapes, options, pairs, want: dic
     return res
 
 
+def _check_precision(opt: Options):
+    if not opt.precision >= 0.0:  # NaN fails too
+        raise ValueError(f"precision must be >= 0 for row subsets (a zeroed row is a removed row only then), "
+                         f"got {opt.precision}")
+
+
+def _iis(check, lib, ctx, height: int, width: int, options, matrix=None, cells=None, values=None) -> dict:
+    """Engine/MultiEngine.iis (matrix given) and iis_sparse (cells, values given) on ctx."""
+    opt = options or make_options()
+    _check_precision(opt)
+    rows = np.empty(max(int(height), 1), np.int32)
+    status, count = C.c_int32(), C.c_int32()
+    stats = np.zeros(5, np.int64)
+    if matrix is not None:
+        m = np.ascontiguousarray(matrix, np.float64).reshape(-1)
+        if m.size != height * width:
+            raise ValueError("matrix must hold height * width cells")
+        check(lib.yalps_iis(ctx, height, width, _ptr(m), C.byref(opt), C.byref(status), _ptr(rows), C.byref(count),
+                            _ptr(stats)))
+    else:
+        cells = np.ascontiguousarray(cells, np.int32).reshape(-1)
+        values = np.ascontiguousarray(values, np.float64).reshape(-1)
+        if cells.size != values.size:
+            raise ValueError("cells and values must have the same length")
+        check(lib.yalps_iis_sparse(ctx, height, width, int(cells.size), _ptr(cells) if cells.size else None,
+                                   _ptr(values) if values.size else None, C.byref(opt), C.byref(status), _ptr(rows),
+                                   C.byref(count), _ptr(stats)))
+    return {"status": status.value, "rows": rows[:count.value].copy(), "rounds": int(stats[0]), "lps": int(stats[1]),
+            "pivots": int(stats[2]), "irreducible": bool(status.value == 1 and stats[3] == 0 and stats[4] == 0)}
+
+
 _STATS = ("nodes", "node_pivots", "max_cuts", "max_heap", "waves", "device_nodes", "wave_us", "bnb_us",
           "sharded_waves", "allreduces")
 
@@ -388,6 +419,45 @@ class Engine:
         self._check(self._lib.yalps_certificate_device(self._ctx, n, height, width, z(d_matrices), z(d_pos),
                                                        z(d_status), z(d_value), float(precision), z(d_cert),
                                                        z(stream)))
+
+    # ------------------------------------------------------------------ row subsets and irreducible infeasible subsets
+    def solve_row_subsets(self, base: np.ndarray, keep: np.ndarray, height: int, width: int,
+                          options: Optional[Options] = None, want_certificates: bool = False) -> dict:
+        """n LPs of `base` (height*width) restricted to row subsets, expanded on the device (yalps_solve_row_subsets).
+        keep: uint32 (n, words), words = (height + 31) // 32, bit r of word r // 32 keeps row r (row 0 always stays,
+        bits of rows >= height must be clear); every other row is zeroed, which the simplex treats as removed.
+        Returns status, value, pivots (as solve_batch) and support (uint32 (n, words): the rows whose Farkas multiplier
+        is > +0.0, zero words unless infeasible); want_certificates adds certificate (n, width+height)."""
+        opt = options or make_options()
+        _check_precision(opt)
+        words = (height + 31) // 32
+        b = np.ascontiguousarray(base, np.float64).reshape(-1)
+        k = np.ascontiguousarray(keep, np.uint32).reshape(-1)
+        if b.size != height * width or k.size % words:
+            raise ValueError("base must hold height*width values and keep n*((height+31)//32) words")
+        n = k.size // words
+        if height % 32 and n and (k.reshape(n, words)[:, -1] >> np.uint32(height % 32)).any():
+            raise ValueError(f"keep has bits set for rows >= height {height}")
+        out = {"status": np.empty(n, np.int32), "value": np.empty(n, np.float64), "pivots": np.empty((n, 2), np.int64),
+               "support": np.empty((n, words), np.uint32)}
+        if want_certificates:
+            out["certificate"] = np.empty((n, width + height), np.float64)
+        self._check(self._lib.yalps_solve_row_subsets(self._ctx, n, height, width, _ptr(b), _ptr(k), C.byref(opt),
+                                                      _ptr(out["status"]), _ptr(out["value"]), _ptr(out["pivots"]),
+                                                      _ptr(out.get("certificate")), _ptr(out["support"])))
+        return out
+
+    def iis(self, matrix: np.ndarray, height: int, width: int, options: Optional[Options] = None) -> dict:
+        """An irreducible infeasible subset of the tableau's rows (yalps_iis): status (the model's own), rows (int32,
+        ascending tableau rows; empty unless infeasible), rounds, lps and pivots (the work of the search, round 0
+        included) and irreducible (False when a deletion test ended `cycled`, the timeout expired or the model is not
+        infeasible)."""
+        return _iis(self._check, self._lib, self._ctx, height, width, options, matrix=matrix)
+
+    def iis_sparse(self, cells: np.ndarray, values: np.ndarray, height: int, width: int,
+                   options: Optional[Options] = None) -> dict:
+        """iis on a tableau given as ordered (cell, value) stores into a zero matrix (yalps_iis_sparse)."""
+        return _iis(self._check, self._lib, self._ctx, height, width, options, cells=cells, values=values)
 
     def generate_synthetic_device(self, first: int, n: int, m: int, nvars: int, d_out: int, neg_rows: int = 0,
                                   salt: int = 0x5BD1E995, stream: int = 0):
@@ -628,6 +698,27 @@ class MultiEngine:
                              options, pairs, {"want_basis": True, "want_matrices": want_matrices,
                                               "want_duals": want_duals, "want_ranges": want_ranges,
                                               "want_certificates": want_certificates}, basis_in=False)
+
+    def _rank0(self):
+        """rank 0's ctx and a check that reads its error message"""
+        ctx = C.c_void_p(self._lib.yalps_multi_ctx(self._m, 0))
+
+        def check(rc: int):
+            if rc != 0:
+                msg = self._lib.yalps_last_error(ctx)
+                raise YalpsError(rc, msg.decode() if msg else "")
+        return ctx, check
+
+    def iis(self, matrix: np.ndarray, height: int, width: int, options: Optional[Options] = None) -> dict:
+        """Engine.iis on rank 0's context (the rounds of one search depend on each other)."""
+        ctx, check = self._rank0()
+        return _iis(check, self._lib, ctx, height, width, options, matrix=matrix)
+
+    def iis_sparse(self, cells: np.ndarray, values: np.ndarray, height: int, width: int,
+                   options: Optional[Options] = None) -> dict:
+        """Engine.iis_sparse on rank 0's context."""
+        ctx, check = self._rank0()
+        return _iis(check, self._lib, ctx, height, width, options, cells=cells, values=values)
 
     def solve_large(self, matrix: np.ndarray, height: int, width: int, options: Optional[Options] = None,
                     want_matrix: bool = False) -> dict:

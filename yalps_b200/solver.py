@@ -19,6 +19,10 @@ first-seen order: non-negative combinations of the keys' max rows and min rows t
 proof that no solution exists) and "unboundedRay" ([[variable, direction], ...], model order: a direction that keeps
 every constraint satisfied while the result moves toward the reported +-inf), computed on the GPU from the final
 tableau; each is an empty list unless the status is infeasible, resp. unbounded.
+A fourth one, `iis` (default False), adds "irreducibleInfeasibleSet" ([[constraint key, "max" | "min"], ...], first-seen
+order, a key's max before its min): a set of bounds that cannot hold together while any one fewer can, found by batched
+deletion rounds on the GPU (yalps_b200.iis); an empty list unless the status is infeasible.  Variables keep x >= 0
+throughout, and those bounds are never listed.
 The tableau is built on the host (tableau.py), the simplex and branch-and-cut numerics run on the GPU
 through the C ABI; there is no CPU solve path.
 """
@@ -30,6 +34,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
+from .iis import model_iis
 from .sensitivity import model_certificate, model_ranges, model_sensitivity, row_pairs
 from .tableau import SPARSE_OVER_BYTES, TableauModel, constraint_rows, entries, tableau_model
 
@@ -103,7 +108,8 @@ def _solution(tabmod: TableauModel, status: str, result: float, rhs, pos, var, o
 
 def _check_lp(tabmod: TableauModel):
     if tabmod.integers:
-        raise ValueError("sensitivity: duals are defined for LP models only (this model has integer or binary variables)")
+        raise ValueError("sensitivity, ranging, certificate and iis are defined for LP models only (this model has "
+                         "integer or binary variables)")
 
 
 def _wants(opt: dict) -> tuple:
@@ -118,6 +124,17 @@ def _with_certificate(sol: dict, tabmod: TableauModel, model: dict, cert) -> dic
     rows = _rows(model) if status == 1 else []
     farkas, ray = model_certificate(tabmod.variables, rows, cert, tabmod.tableau.width, status)
     return {**sol, "infeasibilityCertificate": farkas, "unboundedRay": ray}
+
+
+def _with_iis(sol: dict, tabmod: TableauModel, model: dict, eng, copt) -> dict:
+    """Solution + irreducibleInfeasibleSet: the search runs (on the tableau form solve built) only when infeasible."""
+    out = []
+    if sol["status"] == "infeasible":
+        t = tabmod.tableau
+        r = (eng.iis(t.matrix, t.height, t.width, copt) if t.matrix is not None
+             else eng.iis_sparse(t.cells, t.values, t.height, t.width, copt))
+        out = model_iis(_rows(model), r["rows"])
+    return {**sol, "irreducibleInfeasibleSet": out}
 
 
 def _rows(model: dict) -> list:
@@ -149,9 +166,13 @@ def solve(model: dict, options: Optional[dict] = None, *, engine: Optional[Engin
     tabmod = tableau_model(model, SPARSE_OVER_BYTES if sparse_ok else None)
     t = tabmod.tableau
     duals, rng, cert = _wants(opt)
-    if duals or cert:
+    want_iis = bool(opt.get("iis"))
+    if duals or cert or want_iis:
         _check_lp(tabmod)
     eng = engine or get_engine()
+    if want_iis:
+        sol = solve(model, {**opt, "iis": False}, engine=eng, info=info)
+        return _with_iis(sol, tabmod, model, eng, _c_options(opt))
     if duals or cert:
         # the root LP is the whole solve: one LP with its reduced-cost row (dense batch of one, or the cell pairs), and
         # its ranges and certificate when asked for
@@ -215,12 +236,16 @@ def solve_many(models: Sequence[dict], options: Optional[dict] = None, *, engine
     copt = _c_options(opt)
     tabmods = [tableau_model(m) for m in models]
     duals, rng, cert = _wants(opt)
-    if duals or cert:
+    want_iis = bool(opt.get("iis"))
+    if duals or cert or want_iis:
         for tm in tabmods:
             _check_lp(tm)
     eng = engine or get_engine()
     if not tabmods:
         return []
+    if want_iis:  # per infeasible model, one search after the other
+        sols = solve_many(models, {**opt, "iis": False}, engine=eng, milp_workers=milp_workers)
+        return [_with_iis(s, tm, m, eng, copt) for s, tm, m in zip(sols, tabmods, models)]
     if duals or cert:  # LP models only: the ragged root batch is the whole solve (one GPU or sharded)
         pairs = [row_pairs(_rows(m), tm.tableau.height) for tm, m in zip(tabmods, models)] if rng else None
         roots = eng.solve_ragged([tm.tableau.matrix for tm in tabmods],
