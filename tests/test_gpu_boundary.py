@@ -17,6 +17,7 @@ from conftest import load_cases, load_netlib, same_bits, same_value
 from oracle import lib as O, model as M
 import yalps_b200
 from yalps_b200 import engine as E
+from yalps_b200.sensitivity import reduced_from_tableau
 from yalps_b200.tableau import Tableau, tableau_model
 
 pytestmark = pytest.mark.gpu
@@ -264,6 +265,43 @@ def test_replica_path_sharing_synthetic_phase2_and_statuses(engine):
     exp = O.simplex_batch(mats.copy(), 3, 3)
     assert np.array_equal(got["status"], exp["status"]) and np.array_equal(got["pivots"], exp["pivots"])
     assert same_bits(got["rhs"], exp["rhs"]) and np.array_equal(got["pos"], exp["pos"])
+
+
+def test_replicas_across_pipeline_chunks(engine):
+    """10,000 replicas are solved in 8 pipeline chunks of 1,250 (a call of more than 8,192 LPs is cut in eighths), with
+    path sharing on and off: every output equals the batch entry on the expanded tableaus bit for bit, the LPs on each
+    side of every chunk boundary equal the oracle, and two ranks on one GPU give the same bits."""
+    g = load_netlib().get("AFIRO")
+    H, W = g["height"], g["width"]
+    base = g["matrix"]
+    n, per_chunk = 10000, (10000 + 7) // 8
+    rhs, mats = _replica_case(base, H, W, n, 1e-2, 17)
+    ref = engine.solve_batch(mats, H, W, want_duals=True)
+    edges = np.array([b + d for b in range(per_chunk, n, per_chunk) for d in (-1, 0)])
+    work = mats[edges].copy()
+    exp = O.simplex_batch(work, W, H)
+    exp["reduced"] = np.stack([reduced_from_tableau(work[i], W, H, exp["pos"][i]) for i in range(edges.size)])
+    ints, floats = ("status", "pivots", "pos", "var"), ("value", "rhs", "reduced")
+    for sharing in (True, False):
+        engine.set_replica_sharing(sharing)
+        try:
+            got = engine.solve_replicas(base, rhs, H, W, want_duals=True)
+            forks = engine.replica_forks
+        finally:
+            engine.set_replica_sharing(True)
+        assert forks >= 0 if sharing else forks == -1
+        for k in ints:
+            assert np.array_equal(got[k], ref[k]) and np.array_equal(got[k][edges], exp[k]), (sharing, k)
+        for k in floats:
+            assert same_bits(got[k], ref[k]), (sharing, k)
+        assert same_bits(got["rhs"][edges], exp["rhs"]) and same_bits(got["reduced"][edges], exp["reduced"]), sharing
+        assert all(same_value(a, b) for a, b in zip(got["value"][edges], exp["value"])), sharing
+    with yalps_b200.MultiEngine([0, 0]) as me:
+        many = me.solve_replicas(base, rhs, H, W, want_duals=True)
+    for k in ints:
+        assert np.array_equal(many[k], got[k]), k
+    for k in floats:
+        assert same_bits(many[k], got[k]), k
 
 
 # ------------------------------------------------------------------------------------------------ several GPUs, one process

@@ -972,23 +972,24 @@ int yalps_host_free(yalps_ctx *ctx, void *ptr) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// `slot` names the pooled scratch (LP queue counter, cycle history, cluster scratch) of this launch: calls that may be in
-// flight at the same time on different streams of one ctx must use different slots.
-static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
-                                   double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
-                                   int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
-                                   double *d_matrices_out, void *stream, const std::string &slot, int64_t rows_base = 0,
-                                   double *d_red_out = nullptr) {
+// `a` holds the shape (n, H, W), the input, the work buffer, the final-tableau output and the outputs, all in device
+// memory; the rest is filled in here.  `slot` names the pooled scratch (LP queue counter, cycle history, cluster
+// scratch) of this launch: calls that may be in flight at the same time on different streams of one ctx must use
+// different slots.
+static int solve_batch_device_impl(yalps_ctx *ctx, BatchArgs a, const yalps_options *opt, const std::string &slot,
+                                   cudaStream_t stream, int64_t rows_base = 0) {
   if (!ctx) return YALPS_ERR_ARGUMENT;
-  if (n < 0 || height < 1 || width < 1 || !opt || (n > 0 && !d_matrices))
-    return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", (long long)n, height, width);
+  const long long n = a.n;
+  const int height = a.H, width = a.W;
+  if (n < 0 || height < 1 || width < 1 || !opt || (n > 0 && !a.in))
+    return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", n, height, width);
   if ((long long)height * width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
   if (n == 0) return 0;
   CU(ctx, cudaSetDevice(ctx->device));
   // density probe for the path policy, once per (buffer, shape): synchronises `stream` the first time only
   double density = -1.0;
-  if (ctx->tune_path == YALPS_PATH_AUTO && n > 64 && d_work) {
-    const std::string key = std::to_string((size_t)d_matrices) + ":" + std::to_string(height) + "x" + std::to_string(width);
+  if (ctx->tune_path == YALPS_PATH_AUTO && n > 64 && a.work) {
+    const std::string key = std::to_string((size_t)a.in) + ":" + std::to_string(height) + "x" + std::to_string(width);
     auto it = ctx->density_cache.find(key);
     if (it == ctx->density_cache.end()) {
       void *hp, *dp;
@@ -996,9 +997,9 @@ static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, in
       if (int rc = pin_device_ptr(ctx, hp, &dp)) return rc;
       ((int *)hp)[0] = ((int *)hp)[1] = 0;
       const long long cells = (long long)height * width;
-      k_sample_density<<<1, 256, 0, (cudaStream_t)stream>>>(d_matrices, cells, std::max(1LL, cells / 4096), (int *)dp);
+      k_sample_density<<<1, 256, 0, stream>>>(a.in, cells, std::max(1LL, cells / 4096), (int *)dp);
       CU(ctx, cudaGetLastError());
-      CU(ctx, cudaStreamSynchronize((cudaStream_t)stream));
+      CU(ctx, cudaStreamSynchronize(stream));
       ctx->launches++;
       const int seen = ((int *)hp)[0], nz = ((int *)hp)[1];
       density = seen ? (double)nz / seen : 1.0;
@@ -1008,11 +1009,43 @@ static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, in
       density = it->second;
     }
   }
+  a.mode = kModeBatch;
+  a.Hcap = height;
+  a.Wcap = width;
+  fill_options(a, opt);
+  a.rows_out = ctx->d_rows ? ctx->d_rows + (ctx->rows_per_lp ? rows_base : 0) : nullptr;
+  a.rows_per_lp = ctx->rows_per_lp;
+  Route route;
+  if (int rc = choose_route(ctx, {n, height, width, density, opt->check_cycles != 0, true}, &route)) return rc;
+  if (route.kind == ROUTE_GRID && !a.work) return fail(ctx, YALPS_ERR_ARGUMENT, "d_work is required for the grid path");
+  if (route.kind == ROUTE_SIMPLEX && !route.resident) {
+    if (!a.work) return fail(ctx, YALPS_ERR_ARGUMENT, "d_work is required for the HBM-resident path");
+    if (!a.pos_out || !a.var_out) {
+      void *p = nullptr;
+      if (int rc = dev_ensure(ctx, "posvar_scratch" + slot, (size_t)n * (width + height) * 2 * sizeof(int), &p)) return rc;
+      if (!a.pos_out) a.pos_out = (int *)p;
+      if (!a.var_out) a.var_out = (int *)p + (size_t)n * (width + height);
+    }
+  }
+  return launch_route(ctx, route, a, slot, stream);
+}
+
+int yalps_solve_batch_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                             double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
+                             int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
+                             double *d_matrices_out, void *stream) {
+  return yalps_solve_batch_device_duals(ctx, n, height, width, d_matrices, d_work, opt, d_status, d_value, d_pivots,
+                                        d_rhs_out, d_pos_out, d_var_out, d_matrices_out, stream, nullptr);
+}
+
+int yalps_solve_batch_device_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
+                                   double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
+                                   int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
+                                   double *d_matrices_out, void *stream, double *d_reduced_out) {
   BatchArgs a{};
   a.n = n;
-  a.mode = kModeBatch;
-  a.H = a.Hcap = height;
-  a.W = a.Wcap = width;
+  a.H = height;
+  a.W = width;
   a.in = d_matrices;
   a.work = d_work;
   a.mat_out = d_matrices_out;
@@ -1022,39 +1055,8 @@ static int solve_batch_device_impl(yalps_ctx *ctx, int64_t n, int32_t height, in
   a.rhs_out = d_rhs_out;
   a.pos_out = d_pos_out;
   a.var_out = d_var_out;
-  a.red_out = d_red_out;
-  fill_options(a, opt);
-  a.rows_out = ctx->d_rows ? ctx->d_rows + (ctx->rows_per_lp ? rows_base : 0) : nullptr;
-  a.rows_per_lp = ctx->rows_per_lp;
-  Route route;
-  if (int rc = choose_route(ctx, {n, height, width, density, opt->check_cycles != 0, true}, &route)) return rc;
-  if (route.kind == ROUTE_GRID && !d_work) return fail(ctx, YALPS_ERR_ARGUMENT, "d_work is required for the grid path");
-  if (route.kind == ROUTE_SIMPLEX && !route.resident) {
-    if (!d_work) return fail(ctx, YALPS_ERR_ARGUMENT, "d_work is required for the HBM-resident path");
-    if (!d_pos_out || !d_var_out) {
-      void *p = nullptr;
-      if (int rc = dev_ensure(ctx, "posvar_scratch" + slot, (size_t)n * (width + height) * 2 * sizeof(int), &p)) return rc;
-      if (!a.pos_out) a.pos_out = (int *)p;
-      if (!a.var_out) a.var_out = (int *)p + (size_t)n * (width + height);
-    }
-  }
-  return launch_route(ctx, route, a, slot, (cudaStream_t)stream);
-}
-
-int yalps_solve_batch_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
-                             double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
-                             int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
-                             double *d_matrices_out, void *stream) {
-  return solve_batch_device_impl(ctx, n, height, width, d_matrices, d_work, opt, d_status, d_value, d_pivots, d_rhs_out,
-                                 d_pos_out, d_var_out, d_matrices_out, stream, "dev");
-}
-
-int yalps_solve_batch_device_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
-                                   double *d_work, const yalps_options *opt, int32_t *d_status, double *d_value,
-                                   int64_t *d_pivots, double *d_rhs_out, int32_t *d_pos_out, int32_t *d_var_out,
-                                   double *d_matrices_out, void *stream, double *d_reduced_out) {
-  return solve_batch_device_impl(ctx, n, height, width, d_matrices, d_work, opt, d_status, d_value, d_pivots, d_rhs_out,
-                                 d_pos_out, d_var_out, d_matrices_out, stream, "dev", 0, d_reduced_out);
+  a.red_out = d_reduced_out;
+  return solve_batch_device_impl(ctx, a, opt, "dev", (cudaStream_t)stream);
 }
 
 int yalps_ranging_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *d_matrices,
@@ -1109,7 +1111,8 @@ int yalps_certificate_device(yalps_ctx *ctx, int64_t n, int32_t height, int32_t 
 namespace {
 
 // One host batch solve: the shape, where the tableaus come from, the optional inputs and every output (null: not
-// wanted).  The yalps_solve_{batch,ragged}_certificate entries, yalps_solve's root LP and the sparse entries fill one in.
+// wanted).  The yalps_solve_{batch,ragged}_certificate entries, yalps_solve's root LP, the sparse entries, the replica
+// entries and the row-subset entries fill one in.
 struct HostBatch {
   int64_t n = 0;
   int32_t height = 0, width = 0;                        // a uniform batch, or
@@ -1119,6 +1122,9 @@ struct HostBatch {
   const int32_t *cell = nullptr;     // into a zero tableau, scattered on the device (yalps_solve_sparse)
   const double *val = nullptr;
   int64_t nnz = -1;
+  const double *d_base = nullptr;  // or (uniform) LPs derived on the device from this base tableau in device memory
+  const double *rhs_in = nullptr;  // by their own column 0 (n x height values: replicas), or
+  const uint32_t *keep = nullptr;  // by their own row mask (n x words, words = (height + 31) / 32: row subsets)
   const int32_t *pos_in = nullptr, *var_in = nullptr;  // the basis the tableaus arrive with (both null: the identity)
   const int32_t *pairs = nullptr;                       // ranging: the other row of each row's key
   const yalps_options *opt = nullptr;
@@ -1129,16 +1135,21 @@ struct HostBatch {
   int32_t *pos_out = nullptr, *var_out = nullptr;
   double *matrices_out = nullptr, *reduced_out = nullptr, *range_lo = nullptr, *range_hi = nullptr;
   double *cert_out = nullptr;
+  uint32_t *support_out = nullptr;  // the rows each certificate uses (a mask, packed like keep) and their number
+  int32_t *count_out = nullptr;
   bool keep_final = false;  // (n == 1, uniform) leave the final tableau on the device, no D2H copy of it
   // results
   double *kept_final = nullptr;  // keep_final: where the final tableau is (valid until the next batch call on the ctx)
   int32_t dup_cells = 0;         // nnz >= 0: the device found duplicate cells with different values
+  // the supports are read from the certificates, wanted or not
+  bool want_support() const { return support_out != nullptr || count_out != nullptr; }
   // a post-pass (k_ranging, k_certificate) reads the final tableaus, which therefore stay in device memory
-  bool post_pass() const { return range_lo != nullptr || cert_out != nullptr; }
+  bool post_pass() const { return range_lo != nullptr || cert_out != nullptr || want_support(); }
 };
 
 // The per-LP outputs of a host batch, described once: pool name, host array (null: not wanted), element size and
-// packing.  The kernels write the first six whether they are wanted or not, so those always get a device buffer.
+// packing.  The kernels write the first six whether they are wanted or not, so those always get a device buffer;
+// k_cert_support reads the certificates and writes both support and count when either is wanted.
 enum OutPack { PER_LP, PER_ROW, PER_VAR };  // per LP (times k), per row like rhs_out, per variable id like pos_out
 struct OutSpec {
   const char *name;
@@ -1153,19 +1164,17 @@ struct OutSpec {
     return elem * (size_t)(pack == PER_LP ? lps * k : pack == PER_ROW ? rows : pvs);
   }
 };
-enum { O_STATUS, O_VALUE, O_PIVOTS, O_RHS, O_POS, O_VAR, O_RED, O_RLO, O_RHI, O_CERT, O_COUNT };
+enum { O_STATUS, O_VALUE, O_PIVOTS, O_RHS, O_POS, O_VAR, O_RED, O_RLO, O_RHI, O_CERT, O_SUP, O_CNT, O_COUNT };
 struct Outputs {
   OutSpec t[O_COUNT];
-  Outputs(int32_t *status, double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
-          double *reduced_out, double *range_lo, double *range_hi, double *cert_out)
-      : t{{"status", status, 4, PER_LP, 1, true},     {"value", value, 8, PER_LP, 1, true},
-          {"pivots", pivots, 8, PER_LP, 2, true},     {"rhs", rhs_out, 8, PER_ROW, 1, true},
-          {"pos", pos_out, 4, PER_VAR, 1, true},      {"var", var_out, 4, PER_VAR, 1, true},
-          {"red", reduced_out, 8, PER_VAR, 1, false}, {"rlo", range_lo, 8, PER_VAR, 1, false},
-          {"rhi", range_hi, 8, PER_VAR, 1, false},    {"cert", cert_out, 8, PER_VAR, 1, false}} {}
   explicit Outputs(const HostBatch &b)
-      : Outputs(b.status, b.value, b.pivots, b.rhs_out, b.pos_out, b.var_out, b.reduced_out, b.range_lo, b.range_hi,
-                b.cert_out) {}
+      : t{{"status", b.status, 4, PER_LP, 1, true},     {"value", b.value, 8, PER_LP, 1, true},
+          {"pivots", b.pivots, 8, PER_LP, 2, true},     {"rhs", b.rhs_out, 8, PER_ROW, 1, true},
+          {"pos", b.pos_out, 4, PER_VAR, 1, true},      {"var", b.var_out, 4, PER_VAR, 1, true},
+          {"red", b.reduced_out, 8, PER_VAR, 1, false}, {"rlo", b.range_lo, 8, PER_VAR, 1, false},
+          {"rhi", b.range_hi, 8, PER_VAR, 1, false},    {"cert", b.cert_out, 8, PER_VAR, 1, b.want_support()},
+          {"support", b.support_out, 4, PER_LP, (b.height + 31) / 32, b.want_support()},
+          {"count", b.count_out, 4, PER_LP, 1, b.want_support()}} {}
 
   // device buffers "<name><slot>" for a chunk of `lps` LPs (`rows` rows, `pvs` variable ids); null where not used
   int ensure(yalps_ctx *ctx, const std::string &slot, long long lps, long long rows, long long pvs, void **dev) const {
@@ -1189,7 +1198,8 @@ struct Outputs {
 
 // The LPs [lo, hi) of request b, after row0 rows and pv0 variable ids.  A uniform batch moves its tableaus by cells; a
 // ragged one moves its shapes and offsets by LPs and keeps matrices and matrices_out, which those offsets index
-// absolutely.  The basis moves by variable ids, the pairs by rows, the outputs as the Outputs table packs them.
+// absolutely.  The basis moves by variable ids, the pairs and right-hand sides by rows, the row masks by LPs, the
+// outputs as the Outputs table packs them.
 HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long row0, long long pv0) {
   HostBatch s = b;
   s.n = hi - lo;
@@ -1205,6 +1215,8 @@ HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long ro
   if (s.pos_in) s.pos_in += pv0;
   if (s.var_in) s.var_in += pv0;
   if (s.pairs) s.pairs += row0;
+  if (s.rhs_in) s.rhs_in += row0;
+  if (s.keep) s.keep += lo * ((b.height + 31) / 32);
   const Outputs o(b);
   auto at = [&](int i) -> void * { return o.t[i].host ? (char *)o.t[i].host + o.t[i].bytes(lo, row0, pv0) : nullptr; };
   s.status = (int32_t *)at(O_STATUS);
@@ -1217,6 +1229,8 @@ HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long ro
   s.range_lo = (double *)at(O_RLO);
   s.range_hi = (double *)at(O_RHI);
   s.cert_out = (double *)at(O_CERT);
+  s.support_out = (uint32_t *)at(O_SUP);
+  s.count_out = (int32_t *)at(O_CNT);
   return s;
 }
 
@@ -1259,7 +1273,7 @@ int post_passes(yalps_ctx *ctx, const HostBatch &b, const BatchArgs &a, const do
     g.hi = (double *)dev[O_RHI];
     if (int rc = launch_ranging(ctx, g, pv_total, slot, st)) return rc;
   }
-  if (b.cert_out) {
+  if (b.cert_out || b.want_support()) {
     CertArgs g{};
     static_cast<PostArgs &>(g) = p;
     g.value = a.value;
@@ -1916,12 +1930,12 @@ static int replica_leader_trace(yalps_ctx *ctx, int H, int W, const double *base
   return 0;
 }
 
-// One chunk of replicas whose right-hand sides are in d_rin: followers first, then the replicas that left the path
-// (tableau = the leader's snapshot of the fork step + their own column 0) through the ordinary batch kernels.
-static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t cn, int H, int W, const double *d_rin,
-                                double *d_work, const yalps_options *opt, int *d_status, double *d_value, long long *d_piv,
-                                double *d_rhs, int *d_pos, int *d_var, double *d_red, cudaStream_t st,
-                                const std::string &s, int64_t *forks_out) {
+// One chunk of replicas whose right-hand sides are in d_rin, results into the chunk's outputs dev (outs.ensure):
+// followers first, then the replicas that left the path (tableau = the leader's snapshot of the fork step + their own
+// column 0) through the ordinary batch kernels, into compact outputs of their own scattered back into dev.
+static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, const Outputs &outs, int64_t cn, int H, int W,
+                                const double *d_rin, double *d_work, const yalps_options *opt, void *const *dev,
+                                cudaStream_t st, const std::string &s, int64_t *forks_out) {
   const size_t cells = (size_t)H * W, pv = (size_t)H + W;
   void *p, *hp;
   int rc;
@@ -1935,6 +1949,8 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   long long *d_fres = (long long *)p;
   if ((rc = pin_ensure(ctx, "rs_fcount_h" + s, 64, &hp))) return rc;
   CU(ctx, cudaMemsetAsync(d_fcount, 0, 4, st));
+  BatchArgs d{};  // the chunk's outputs, typed
+  set_outputs(d, dev);
   FollowArgs fa{};
   fa.n = cn;
   fa.H = H;
@@ -1950,17 +1966,17 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   fa.leader_status = tr.leader_status;
   fa.precision = opt->precision;
   fa.max_pivots = opt->max_pivots;
-  fa.status = d_status;
-  fa.value = d_value;
-  fa.pivots = d_piv;
-  fa.rhs_out = d_rhs;
-  fa.pos_out = d_pos;
-  fa.var_out = d_var;
+  fa.status = d.status;
+  fa.value = d.value;
+  fa.pivots = d.pivots;
+  fa.rhs_out = d.rhs_out;
+  fa.pos_out = d.pos_out;
+  fa.var_out = d.var_out;
   fa.fork_count = d_fcount;
   fa.fork_ids = d_fids;
   fa.fork_step = d_fstep;
   fa.fork_resume = d_fres;
-  fa.red_out = d_red;
+  fa.red_out = d.red_out;
   fa.leader_red = tr.red;
   const int grid = (int)std::min<int64_t>((cn + kFollowWarps - 1) / kFollowWarps, (int64_t)ctx->prop.multiProcessorCount * 8);
   k_replica_follow<<<grid, kFollowWarps * 32, (size_t)kFollowWarps * tr.Hp * 8, st>>>(fa);
@@ -1971,31 +1987,18 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   const int nf = *(int *)hp;
   if (forks_out) *forks_out += nf;
   if (nf == 0) return 0;
-  // compact buffers of the forked replicas
+  // compact buffers of the forked replicas: their resume state and basis in, their outputs
   if ((rc = dev_ensure(ctx, "rs_cvin" + s, (size_t)nf * pv * 4, &p))) return rc;
   int *c_vin = (int *)p;
   if ((rc = dev_ensure(ctx, "rs_cres" + s, (size_t)nf * 24, &p))) return rc;
   long long *c_resume = (long long *)p;
-  if ((rc = dev_ensure(ctx, "rs_cstatus" + s, (size_t)nf * 4, &p))) return rc;
-  int *c_status = (int *)p;
-  if ((rc = dev_ensure(ctx, "rs_cvalue" + s, (size_t)nf * 8, &p))) return rc;
-  double *c_value = (double *)p;
-  if ((rc = dev_ensure(ctx, "rs_cpiv" + s, (size_t)nf * 16, &p))) return rc;
-  long long *c_piv = (long long *)p;
-  if ((rc = dev_ensure(ctx, "rs_crhs" + s, (size_t)nf * H * 8, &p))) return rc;
-  double *c_rhs = (double *)p;
-  if ((rc = dev_ensure(ctx, "rs_cpos" + s, (size_t)nf * pv * 4, &p))) return rc;
-  int *c_pos = (int *)p;
-  if ((rc = dev_ensure(ctx, "rs_cvar" + s, (size_t)nf * pv * 4, &p))) return rc;
-  int *c_var = (int *)p;
-  double *c_red = nullptr;
-  if (d_red) {
-    if ((rc = dev_ensure(ctx, "rs_cred" + s, (size_t)nf * pv * 8, &p))) return rc;
-    c_red = (double *)p;
-  }
+  const std::string fs = "rs_fork" + s;
+  void *cdev[O_COUNT];
+  if ((rc = outs.ensure(ctx, fs, nf, (long long)nf * H, (long long)nf * pv, cdev))) return rc;
   {
     const dim3 g((unsigned)std::min<size_t>((cells + 255) / 256, 64), (unsigned)std::min(nf, 32768));
-    k_replica_materialise<<<g, 256, 0, st>>>(0, nf, H, W, d_fids, d_fstep, d_fres, d_rhs, tr.snap, tr.var, d_work, c_vin, c_resume);
+    k_replica_materialise<<<g, 256, 0, st>>>(0, nf, H, W, d_fids, d_fstep, d_fres, d.rhs_out, tr.snap, tr.var, d_work,
+                                             c_vin, c_resume);
     CU(ctx, cudaGetLastError());
     ctx->launches++;
   }
@@ -2013,88 +2016,124 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, int64_t 
   a.W = a.Wcap = W;
   a.in = d_work;
   a.work = d_work;
-  a.status = c_status;
-  a.value = c_value;
-  a.pivots = c_piv;
-  a.rhs_out = c_rhs;
-  a.pos_out = c_pos;
-  a.var_out = c_var;
+  set_outputs(a, cdev);
   a.var_in = c_vin;
-  a.red_out = c_red;
   a.resume = c_resume;
   fill_options(a, opt);
-  if ((rc = launch_route(ctx, route, a, "rs_fork" + s, st))) return rc;
+  if ((rc = launch_route(ctx, route, a, fs, st))) return rc;
   k_replica_scatter<<<(unsigned)std::min(nf, ctx->prop.multiProcessorCount * 8), 128, 0, st>>>(
-      0, nf, H, W, d_fids, c_status, c_value, c_piv, c_rhs, c_pos, c_var, c_red, d_status, d_value, d_piv, d_rhs, d_pos,
-      d_var, d_red);
+      0, nf, H, W, d_fids, a.status, a.value, a.pivots, a.rhs_out, a.pos_out, a.var_out, a.red_out, d.status, d.value,
+      d.pivots, d.rhs_out, d.pos_out, d.var_out, d.red_out);
   CU(ctx, cudaGetLastError());
   ctx->launches++;
   return 0;
 }
 
-int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
-                               const double *rhs, const yalps_options *opt, int32_t *status, double *value,
-                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
-                               double *reduced_out) {
-  if (!ctx) return YALPS_ERR_ARGUMENT;
-  if (n < 0 || height < 1 || width < 1 || !opt || (n > 0 && (!base || !rhs)))
-    return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", (long long)n, height, width);
-  if ((long long)height * width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
-  if (n == 0) return 0;
-  CU(ctx, cudaSetDevice(ctx->device));
-  const size_t cells = (size_t)height * width, pv = (size_t)height + width;
-  void *d_base;
-  int rc;
-  if ((rc = dev_ensure(ctx, "rep_base", cells * 8, &d_base))) return rc;
-  CU(ctx, cudaMemcpy(d_base, base, cells * 8, cudaMemcpyHostToDevice));
-  ReplicaTrace trace;
-  if ((rc = replica_leader_trace(ctx, height, width, base, (const double *)d_base, opt, ctx->streams[0], &trace,
-                                 reduced_out != nullptr)))
-    return rc;
-  ctx->replica_forks = trace.ok ? 0 : -1;
-  // two pipeline slots of at most ~1.5 GiB of working copies each: the H2D of chunk k+1's right-hand sides and the
-  // D2H of chunk k-1's results overlap the solve of chunk k
+// The LPs of a request derived from b.d_base (replicas: b.rhs_in, row subsets: b.keep), in chunks of at most ~1.5 GiB
+// of working copies over two pipeline slots: the H2D of chunk k+1's inputs and the D2H of chunk k-1's results overlap
+// the solve of chunk k.  Per chunk, on its slot's stream: the per-LP inputs in; the replicas' shared path when `trace`
+// is usable, else the expand kernel and the solve in place; the post-passes, k_cert_support, the results out.
+// Returns once every copy has landed.
+static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *trace) {
+  const int64_t n = b.n;
+  const int H = b.height, W = b.width, words = (H + 31) / 32;
+  const size_t cells = (size_t)H * W, pv = (size_t)H + W, in_lp = b.keep ? (size_t)words * 4 : (size_t)H * 8;
+  const long long sms = ctx->prop.multiProcessorCount;
   const int64_t per_chunk = std::max<int64_t>(1, std::min<int64_t>((n + 1) / 2 > 4096 ? (n + 7) / 8 : n,
                                                                   (int64_t)(((size_t)1536 << 20) / (cells * 8))));
-  const Outputs outs(status, value, pivots, rhs_out, pos_out, var_out, reduced_out, nullptr, nullptr, nullptr);
+  const Outputs outs(b);
   bool used[2] = {false, false};
-  int slot = 0;
+  int slot = 0, rc;
   for (int64_t begin = 0; begin < n; begin += per_chunk, slot ^= 1) {
     const int64_t cn = std::min(per_chunk, n - begin);
-    const std::string s = "rp" + std::to_string(slot);
+    const std::string s = (b.keep ? "ss" : "rp") + std::to_string(slot);
     cudaStream_t st = ctx->streams[slot];
     if (used[slot]) CU(ctx, cudaEventSynchronize(ctx->events[slot]));
-    void *d_rin, *d_work, *dev[O_COUNT];
-    if ((rc = dev_ensure(ctx, "rin" + s, (size_t)cn * height * 8, &d_rin))) return rc;
+    void *d_in, *d_work, *dev[O_COUNT];
+    if ((rc = dev_ensure(ctx, (b.keep ? "keep" : "rin") + s, cn * in_lp, &d_in))) return rc;
     if ((rc = dev_ensure(ctx, "work" + s, (size_t)cn * cells * 8, &d_work))) return rc;
-    if ((rc = outs.ensure(ctx, s, cn, cn * height, cn * (long long)pv, dev))) return rc;
-    CU(ctx, cudaMemcpyAsync(d_rin, rhs + (size_t)begin * height, (size_t)cn * height * 8, cudaMemcpyHostToDevice, st));
-    if (trace.ok) {
-      if ((rc = replica_chunk_shared(ctx, trace, cn, height, width, (const double *)d_rin, (double *)d_work, opt,
-                                     (int *)dev[O_STATUS], (double *)dev[O_VALUE], (long long *)dev[O_PIVOTS],
-                                     (double *)dev[O_RHS], (int *)dev[O_POS], (int *)dev[O_VAR], (double *)dev[O_RED],
-                                     st, s, &ctx->replica_forks)))
+    if ((rc = outs.ensure(ctx, s, cn, cn * H, cn * (long long)pv, dev))) return rc;
+    const char *in = b.keep ? (const char *)b.keep : (const char *)b.rhs_in;
+    CU(ctx, cudaMemcpyAsync(d_in, in + begin * in_lp, cn * in_lp, cudaMemcpyHostToDevice, st));
+    BatchArgs a{};
+    a.n = cn;
+    a.H = a.Hcap = H;
+    a.W = a.Wcap = W;
+    a.work = (double *)d_work;
+    a.in = a.work;
+    // in place: every route reads an LP's tableau before it writes that LP's final one
+    a.mat_out = b.post_pass() ? a.work : nullptr;
+    set_outputs(a, dev);
+    if (trace && trace->ok) {
+      if ((rc = replica_chunk_shared(ctx, *trace, outs, cn, H, W, (const double *)d_in, a.work, b.opt, dev, st, s,
+                                     &ctx->replica_forks)))
         return rc;
     } else {
-      const size_t total = (size_t)cn * cells;
-      const int grid = (int)std::min<size_t>((total + 255) / 256, (size_t)ctx->prop.multiProcessorCount * 16);
-      k_expand_replicas<<<grid, 256, 0, st>>>(cn, height, width, (const double *)d_base, (const double *)d_rin, (double *)d_work);
+      if (b.keep) {
+        const int grid = (int)std::min<long long>((cn * H + 7) / 8, sms * 16);
+        k_expand_subsets<<<grid, 256, 0, st>>>(cn, H, W, words, b.d_base, (const unsigned *)d_in, a.work);
+      } else {
+        const int grid = (int)std::min<long long>((cn * (long long)cells + 255) / 256, sms * 16);
+        k_expand_replicas<<<grid, 256, 0, st>>>(cn, H, W, b.d_base, (const double *)d_in, a.work);
+      }
       CU(ctx, cudaGetLastError());
       ctx->launches++;
-      if ((rc = solve_batch_device_impl(ctx, cn, height, width, (const double *)d_work, (double *)d_work, opt,
-                                        (int32_t *)dev[O_STATUS], (double *)dev[O_VALUE], (int64_t *)dev[O_PIVOTS],
-                                        (double *)dev[O_RHS], (int32_t *)dev[O_POS], (int32_t *)dev[O_VAR], nullptr, st,
-                                        s, begin, (double *)dev[O_RED])))
-        return rc;
+      // The route's density probe is cached per (buffer, shape), so later calls on this pooled buffer -- the later
+      // rounds of an IIS search -- reuse the first call's route choice.  That decides speed only, never a result bit.
+      if ((rc = solve_batch_device_impl(ctx, a, b.opt, s, st, begin))) return rc;
     }
-    if ((rc = outs.copy_out(ctx, dev, begin, begin * height, begin * (long long)pv, cn, cn * height, cn * (long long)pv, st)))
+    if ((rc = post_passes(ctx, b, a, a.work, nullptr, dev, cn * pv, s, st))) return rc;
+    if (b.want_support()) {
+      const int grid = (int)std::min<long long>((cn + 7) / 8, sms * 16);
+      k_cert_support<<<grid, 256, 0, st>>>(cn, H, W, words, a.status, (const double *)dev[O_CERT],
+                                           (unsigned *)dev[O_SUP], (int *)dev[O_CNT]);
+      CU(ctx, cudaGetLastError());
+      ctx->launches++;
+    }
+    if ((rc = outs.copy_out(ctx, dev, begin, begin * H, begin * (long long)pv, cn, cn * H, cn * (long long)pv, st)))
       return rc;
     CU(ctx, cudaEventRecord(ctx->events[slot], st));
     used[slot] = true;
   }
   for (int i = 0; i < 2; i++)
     if (used[i]) CU(ctx, cudaStreamSynchronize(ctx->streams[i]));
-  return check_device_status(ctx, status, n);
+  return check_device_status(ctx, b.status, n);
+}
+
+// The replicas of request b (b.rhs_in) of the host base tableau `base`: the base crosses PCIe once, the leader's trace
+// is recorded when path sharing applies, then solve_from_base.  Every rank of a multi-GPU call runs its slice here.
+static int solve_replicas(yalps_ctx *ctx, const double *base, HostBatch &b) {
+  if (!ctx) return YALPS_ERR_ARGUMENT;
+  const int64_t n = b.n;
+  const int32_t height = b.height, width = b.width;
+  if (n < 0 || height < 1 || width < 1 || !b.opt || (n > 0 && (!base || !b.rhs_in)))
+    return fail(ctx, YALPS_ERR_ARGUMENT, "bad arguments (n=%lld, %dx%d)", (long long)n, height, width);
+  if ((long long)height * width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
+  if (n == 0) return 0;
+  CU(ctx, cudaSetDevice(ctx->device));
+  const size_t cells = (size_t)height * width;
+  void *d_base;
+  int rc;
+  if ((rc = dev_ensure(ctx, "rep_base", cells * 8, &d_base))) return rc;
+  CU(ctx, cudaMemcpy(d_base, base, cells * 8, cudaMemcpyHostToDevice));
+  b.d_base = (const double *)d_base;
+  ReplicaTrace trace;
+  if ((rc = replica_leader_trace(ctx, height, width, base, b.d_base, b.opt, ctx->streams[0], &trace,
+                                 b.reduced_out != nullptr)))
+    return rc;
+  ctx->replica_forks = trace.ok ? 0 : -1;
+  return solve_from_base(ctx, b, &trace);
+}
+
+int yalps_solve_replicas_duals(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
+                               const double *rhs, const yalps_options *opt, int32_t *status, double *value,
+                               int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                               double *reduced_out) {
+  HostBatch b = batch_request(n, height, width, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, opt, status, value,
+                              pivots, rhs_out, pos_out, var_out, nullptr, reduced_out, nullptr, nullptr, nullptr,
+                              nullptr);
+  b.rhs_in = rhs;
+  return solve_replicas(ctx, base, b);
 }
 
 int yalps_solve_replicas(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
