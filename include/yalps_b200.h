@@ -452,6 +452,50 @@ int yalps_iis_sparse(yalps_ctx *ctx, int32_t height, int32_t width, int64_t nnz,
                      const double *val, const yalps_options *opt, int32_t *status, int32_t *rows_out,
                      int32_t *count, int64_t *stats);
 
+/* ---- warm starts: variants of one LP re-optimised from its final basis ------------------------------------------
+ * A variant of the base LP keeps its constraint coefficients and has its own column 0 b' (rhs + i*height: height
+ * values, b'[0] is the new M0[0,0]) and/or its own row 0 c' (obj + i*width: width values, c'[0] ignored); rhs or obj
+ * NULL: that part is the base's.  Its start tableau T keeps the base's final basis (pos / var) and is derived on the
+ * device from the base's initial tableau M0 and final tableau F (any status) by:
+ *   dir(v): for a non-basic id (1 <= pos[v] < width) the column F[:, pos[v]], row 0 included; for a basic id the unit
+ *     vector of row pos[v] - width; for id width + 0 the unit vector of row 0 (the direction ranging uses).
+ *   1. column pass: T = F.  delta_k = b'[k] - M0[k,0] (rounded once; skipped when == 0.0).  For every row r and every
+ *      changed k in ascending order: T[r,0] = T[r,0] + delta_k * dir(width+k)[r], product and sum rounded apart (no
+ *      FMA).
+ *   2. row pass, on the result of 1.  delta_j = c'[j] - M0[0,j], j = 1..width-1 (skipped when == 0.0).  For every
+ *      column c and every changed j in ascending order: x_j non-basic: T[0,c] = T[0,c] + delta_j when c == pos[j];
+ *      x_j basic at row q = pos[j] - width: T[0,c] = T[0,c] - delta_j * T[q,c].
+ * With no change T is F bit for bit.  In exact arithmetic column 0 becomes B^-1 b' and row 0 the reduced costs and
+ * objective value of the same basis under c' (yalps_b200/warm.py has the derivation).  Each variant is then the
+ * reference's loop on T from that basis: after RHS changes phase 1 is the dual simplex from a dual-feasible basis, after
+ * objective changes phase 2 continues from the old vertex.
+ * Caveat: the results are bit-exact against the reference's loop run on T, NOT against a cold solve of the changed
+ * model: the pivot path differs.  Statuses agree and optimal values agree within the precision, but with alternative
+ * optima the reported vertex can differ.
+ *
+ * base: M0 (height*width).  final / final_pos / final_var: F and its basis (all three or none; the basis must be a pair
+ * of inverse permutations).  With none the library solves the base first with opt, keeps its final tableau on the
+ * device (it never crosses PCIe) and reports its status, value and pivots[2] in base_status / base_value /
+ * base_pivots (each may be NULL; untouched when final is given).  Per variant the outputs of
+ * yalps_solve_batch_certificate: status, value, pivots, rhs_out, pos_out, var_out, matrices_out (the final tableaus),
+ * reduced_out, pairs (n*height, packed like rhs_out) with range_lo / range_hi, and cert_out, each may be NULL.  n < 0,
+ * a bad shape, a negative or NaN precision, and rhs and obj both NULL with n > 0 are YALPS_ERR_ARGUMENT. */
+int yalps_solve_warm(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, const double *base,
+                     const double *final_m, const int32_t *final_pos, const int32_t *final_var, const double *rhs,
+                     const double *obj, const yalps_options *opt, int32_t *base_status, double *base_value,
+                     int64_t *base_pivots, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
+                     int32_t *pos_out, int32_t *var_out, double *matrices_out, double *reduced_out,
+                     const int32_t *pairs, double *range_lo, double *range_hi, double *cert_out);
+/* yalps_solve_warm with the base's initial tableau given as (cell, value) stores into a zero matrix, as
+ * yalps_solve_sparse: it is built on the device and never exists densely on the host */
+int yalps_solve_warm_sparse(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, int64_t nnz,
+                            const int32_t *cell, const double *val, const double *final_m, const int32_t *final_pos,
+                            const int32_t *final_var, const double *rhs, const double *obj, const yalps_options *opt,
+                            int32_t *base_status, double *base_value, int64_t *base_pivots, int32_t *status,
+                            double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
+                            double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
+                            double *range_hi, double *cert_out);
+
 /* ---- one process, several GPUs (SURVEY 8b/8e) ------------------------------------------------------------
  * The reference is single-process and synchronous (src/YALPS.ts:73-92); a Node addon cannot use torchrun.  A
  * yalps_multi owns one ctx (plus worker ctxs for concurrent branch-and-cut searches) per entry of `devices` and one
@@ -490,6 +534,14 @@ int yalps_multi_solve_replicas_duals(yalps_multi *m, int64_t n, int32_t height, 
                                      const double *rhs, const yalps_options *opt, int32_t *status, double *value,
                                      int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                                      double *reduced_out);
+/* yalps_solve_warm with the variants sharded as contiguous ranges; every rank solves (or uploads) the base on its own
+ * GPU, rank 0 reports it in base_status / base_value / base_pivots */
+int yalps_multi_solve_warm(yalps_multi *m, int64_t n, int32_t height, int32_t width, const double *base,
+                           const double *final_m, const int32_t *final_pos, const int32_t *final_var, const double *rhs,
+                           const double *obj, const yalps_options *opt, int32_t *base_status, double *base_value,
+                           int64_t *base_pivots, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
+                           int32_t *pos_out, int32_t *var_out, double *matrices_out, double *reduced_out,
+                           const int32_t *pairs, double *range_lo, double *range_hi, double *cert_out);
 /* the batch and ragged *_duals entries + pairs, range_lo, range_hi (see "sensitivity ranging"), sharded like rhs_out
  * and pos_out */
 int yalps_multi_solve_batch_ranging(yalps_multi *m, int64_t n, int32_t height, int32_t width, const double *matrices,

@@ -138,6 +138,113 @@ __global__ void k_expand_subsets(long long n, int H, int W, int words, const dou
   }
 }
 
+// Warm starts (yalps_solve_warm): LP i is the start tableau of a variant of the base, built from the base's final
+// tableau F (`base`), its final basis (pos, var) and its initial column 0 and row 0 (col0, row0), with the variant's own
+// column 0 (rhs + i*H, or rhs null: unchanged) and row 0 (obj + i*W, or null).  yalps_b200/warm.py states the
+// definition; this is the same arithmetic in the same order.  One CTA per LP: F is copied with the 16-byte stores of
+// k_expand_subsets, then the column pass runs one thread per row and the row pass one thread per column.  The changed
+// k (resp. j) are compacted once per LP in ascending order, a tile of blockDim at a time (ballot + per-warp counts),
+// with their delta and dir position; dir(W+k)[r] of a non-basic slack is a strided read of F, which every LP shares
+// (L2-resident for Netlib-size models).  var_in gets the base's final var.
+constexpr int kWarmThreads = 256;
+
+// Ordered compaction over the block: every thread passes its flag; the flagged threads get their rank among them in
+// thread order (*at), the return value is how many were flagged.  All threads of the block must call it.
+__device__ __forceinline__ int warm_compact(bool flag, int *wcount, int *at) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned m = __ballot_sync(0xffffffffu, flag);
+  if (lane == 0) wcount[warp] = __popc(m);
+  __syncthreads();
+  int before = 0, total = 0;
+  for (int w = 0; w < (int)(blockDim.x >> 5); w++) {
+    const int c = wcount[w];
+    before += w < warp ? c : 0;
+    total += c;
+  }
+  *at = before + __popc(m & ((1u << lane) - 1u));
+  return total;
+}
+
+__global__ void __launch_bounds__(kWarmThreads) k_expand_warm(long long n, int H, int W, const double *base,
+                                                              const int *__restrict__ pos, const int *__restrict__ var,
+                                                              const double *__restrict__ col0,
+                                                              const double *__restrict__ row0,
+                                                              const double *__restrict__ rhs,
+                                                              const double *__restrict__ obj, double *out,
+                                                              int *var_in) {
+  __shared__ int wcount[kWarmThreads / 32];
+  __shared__ int list_p[kWarmThreads];
+  __shared__ double list_d[kWarmThreads];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
+  const size_t cells = (size_t)H * W, pv = (size_t)H + W;
+  const long long *src0 = reinterpret_cast<const long long *>(base);
+  for (long long i = blockIdx.x; i < n; i += gridDim.x) {
+    double *T = out + (size_t)i * cells;
+    for (int r = warp; r < H; r += nwarps) {
+      long long *dst = reinterpret_cast<long long *>(T) + (size_t)r * W;
+      const long long *src = src0 + (size_t)r * W;
+      const int head = min((int)((reinterpret_cast<uintptr_t>(dst) >> 3) & 1), W);  // 1: dst is 8 mod 16
+      const int pairs = (W - head) >> 1;
+      if (lane == 0 && head) dst[0] = src[0];
+      longlong2 *d2 = reinterpret_cast<longlong2 *>(dst + head);
+      for (int k = lane; k < pairs; k += 32) d2[k] = make_longlong2(src[head + 2 * k], src[head + 2 * k + 1]);
+      if (lane == 0 && head + 2 * pairs < W) dst[W - 1] = src[W - 1];
+    }
+    for (size_t k = tid; k < pv; k += blockDim.x) var_in[(size_t)i * pv + k] = var[k];
+    __syncthreads();
+    if (rhs) {  // column pass: T[r,0] += delta_k * dir(W+k)[r], changed k ascending
+      const double *b = rhs + (size_t)i * H;
+      for (int k0 = 0; k0 < H; k0 += blockDim.x) {
+        const int k = k0 + tid;
+        const double d = k < H ? __dsub_rn(b[k], col0[k]) : 0.0;
+        int at;
+        const int cnt = warm_compact(d != 0.0, wcount, &at);
+        if (d != 0.0) {
+          list_d[at] = d;
+          list_p[at] = pos[W + k];
+        }
+        __syncthreads();
+        for (int r = tid; r < H; r += blockDim.x) {
+          double t = T[(size_t)r * W];
+          for (int e = 0; e < cnt; e++) {
+            const int p = list_p[e];
+            const double dr = (p >= 1 && p < W) ? base[(size_t)r * W + p] : (r == p - W ? 1.0 : 0.0);
+            t = __dadd_rn(t, __dmul_rn(list_d[e], dr));
+          }
+          T[(size_t)r * W] = t;
+        }
+        __syncthreads();  // the lists are refilled by the next tile; the row pass reads column 0
+      }
+    }
+    if (obj) {  // row pass: T[0,c] += delta_j at c == pos[j] (non-basic), -= delta_j * T[q,c] (basic at row q)
+      const double *c1 = obj + (size_t)i * W;
+      for (int j0 = 1; j0 < W; j0 += blockDim.x) {
+        const int j = j0 + tid;
+        const double d = j < W ? __dsub_rn(c1[j], row0[j]) : 0.0;
+        int at;
+        const int cnt = warm_compact(d != 0.0, wcount, &at);
+        if (d != 0.0) {
+          list_d[at] = d;
+          list_p[at] = pos[j];
+        }
+        __syncthreads();
+        for (int c = tid; c < W; c += blockDim.x) {
+          double t = T[c];
+          for (int e = 0; e < cnt; e++) {
+            const int q = list_p[e];
+            if (q < W)
+              t = c == q ? __dadd_rn(t, list_d[e]) : t;
+            else
+              t = __dsub_rn(t, __dmul_rn(list_d[e], T[(size_t)(q - W) * W + c]));
+          }
+          T[c] = t;
+        }
+        __syncthreads();
+      }
+    }
+  }
+}
+
 // ---- replica path sharing (yalps_solve_replicas) -----------------------------------------------------------------
 // n replicas of one tableau differ only in column 0.  Everything else of the tableau -- objective row, pivot rows and
 // columns, the basis bookkeeping -- evolves identically for every replica that makes the same pivot choices, and those

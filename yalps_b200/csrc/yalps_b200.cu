@@ -1124,7 +1124,12 @@ struct HostBatch {
   int64_t nnz = -1;
   const double *d_base = nullptr;  // or (uniform) LPs derived on the device from this base tableau in device memory
   const double *rhs_in = nullptr;  // by their own column 0 (n x height values: replicas), or
-  const uint32_t *keep = nullptr;  // by their own row mask (n x words, words = (height + 31) / 32: row subsets)
+  const uint32_t *keep = nullptr;  // by their own row mask (n x words, words = (height + 31) / 32: row subsets), or
+  // warm starts (d_var set): d_base is the base's final tableau, d_pos / d_var its final basis and d_col0 / d_row0 its
+  // initial column 0 and row 0 (device memory); each LP has its own column 0 (rhs_in) and/or row 0 (obj_in, n x width)
+  const int32_t *d_pos = nullptr, *d_var = nullptr;
+  const double *d_col0 = nullptr, *d_row0 = nullptr;
+  const double *obj_in = nullptr;
   const int32_t *pos_in = nullptr, *var_in = nullptr;  // the basis the tableaus arrive with (both null: the identity)
   const int32_t *pairs = nullptr;                       // ranging: the other row of each row's key
   const yalps_options *opt = nullptr;
@@ -1198,8 +1203,8 @@ struct Outputs {
 
 // The LPs [lo, hi) of request b, after row0 rows and pv0 variable ids.  A uniform batch moves its tableaus by cells; a
 // ragged one moves its shapes and offsets by LPs and keeps matrices and matrices_out, which those offsets index
-// absolutely.  The basis moves by variable ids, the pairs and right-hand sides by rows, the row masks by LPs, the
-// outputs as the Outputs table packs them.
+// absolutely.  The basis moves by variable ids, the pairs and right-hand sides by rows, the row masks and objective rows
+// by LPs, the outputs as the Outputs table packs them.
 HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long row0, long long pv0) {
   HostBatch s = b;
   s.n = hi - lo;
@@ -1216,6 +1221,7 @@ HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long ro
   if (s.var_in) s.var_in += pv0;
   if (s.pairs) s.pairs += row0;
   if (s.rhs_in) s.rhs_in += row0;
+  if (s.obj_in) s.obj_in += lo * b.width;
   if (s.keep) s.keep += lo * ((b.height + 31) / 32);
   const Outputs o(b);
   auto at = [&](int i) -> void * { return o.t[i].host ? (char *)o.t[i].host + o.t[i].bytes(lo, row0, pv0) : nullptr; };
@@ -1295,6 +1301,18 @@ struct BatchLayout {
   long long pv_upto(int64_t i) const { return ragged ? poff[i] : (long long)i * (height + width); }
 };
 
+// LP lp's basis (len variable ids) must be a pair of inverse permutations of 0..len-1 (src/tableau.ts:9-15); the
+// kernels carry variableAtPosition and rebuild positionOfVariable on output, so an inconsistent pair would silently
+// change meaning instead of behaving like the reference
+int check_basis(yalps_ctx *ctx, const int32_t *pos, const int32_t *var, long long len, long long lp) {
+  for (long long k = 0; k < len; k++) {
+    const int32_t v = var[k];
+    if (v < 0 || v >= len || pos[v] != (int32_t)k)
+      return fail(ctx, YALPS_ERR_ARGUMENT, "LP %lld: pos_in/var_in are not inverse permutations at position %lld", lp, k);
+  }
+  return 0;
+}
+
 // Validates a request and lays it out (nothing more when b.n == 0).
 int batch_layout(yalps_ctx *ctx, const HostBatch &b, BatchLayout *L) {
   const int64_t n = b.n;
@@ -1336,18 +1354,10 @@ int batch_layout(yalps_ctx *ctx, const HostBatch &b, BatchLayout *L) {
     if ((long long)b.height * b.width >= (1LL << 31)) return fail(ctx, YALPS_ERR_TOO_LARGE, "height*width must be < 2^31");
   }
   if (int rc = check_pairs(ctx, L->pairs, n, b.height, b.heights)) return rc;
-  // caller-supplied basis: the two arrays must be inverse permutations of 0..W+H-1 (src/tableau.ts:9-15); the kernels
-  // carry variableAtPosition and rebuild positionOfVariable on output, so an inconsistent pair would silently
-  // change meaning instead of behaving like the reference
   if (b.var_in) {
     for (int64_t i = 0; i < n; i++) {
-      const long long o = L->pv_upto(i), len = L->pv_upto(i + 1) - o;
-      for (long long k = 0; k < len; k++) {
-        const int32_t v = b.var_in[o + k];
-        if (v < 0 || v >= len || b.pos_in[o + v] != (int32_t)k)
-          return fail(ctx, YALPS_ERR_ARGUMENT, "LP %lld: pos_in/var_in are not inverse permutations at position %lld",
-                      (long long)i, k);
-      }
+      const long long o = L->pv_upto(i);
+      if (int rc = check_basis(ctx, b.pos_in + o, b.var_in + o, L->pv_upto(i + 1) - o, i)) return rc;
     }
   }
   return 0;
@@ -2029,14 +2039,15 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, const Ou
   return 0;
 }
 
-// The LPs of a request derived from b.d_base (replicas: b.rhs_in, row subsets: b.keep), in chunks of at most ~1.5 GiB
-// of working copies over two pipeline slots: the H2D of chunk k+1's inputs and the D2H of chunk k-1's results overlap
-// the solve of chunk k.  Per chunk, on its slot's stream: the per-LP inputs in; the replicas' shared path when `trace`
-// is usable, else the expand kernel and the solve in place; the post-passes, k_cert_support, the results out.
-// Returns once every copy has landed.
+// The LPs of a request derived from b.d_base (replicas: b.rhs_in, row subsets: b.keep, warm starts: b.d_var), in
+// chunks of at most ~1.5 GiB of working copies over two pipeline slots: the H2D of chunk k+1's inputs and the D2H of
+// chunk k-1's results overlap the solve of chunk k.  Per chunk, on its slot's stream: the per-LP inputs in; the
+// replicas' shared path when `trace` is usable, else the expand kernel and the solve in place; the post-passes,
+// k_cert_support, the results out.  Returns once every copy has landed.
 static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *trace) {
   const int64_t n = b.n;
   const int H = b.height, W = b.width, words = (H + 31) / 32;
+  const bool warm = b.d_var != nullptr;
   const size_t cells = (size_t)H * W, pv = (size_t)H + W, in_lp = b.keep ? (size_t)words * 4 : (size_t)H * 8;
   const long long sms = ctx->prop.multiProcessorCount;
   const int64_t per_chunk = std::max<int64_t>(1, std::min<int64_t>((n + 1) / 2 > 4096 ? (n + 7) / 8 : n,
@@ -2046,15 +2057,25 @@ static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *tra
   int slot = 0, rc;
   for (int64_t begin = 0; begin < n; begin += per_chunk, slot ^= 1) {
     const int64_t cn = std::min(per_chunk, n - begin);
-    const std::string s = (b.keep ? "ss" : "rp") + std::to_string(slot);
+    const std::string s = (warm ? "wm" : b.keep ? "ss" : "rp") + std::to_string(slot);
     cudaStream_t st = ctx->streams[slot];
     if (used[slot]) CU(ctx, cudaEventSynchronize(ctx->events[slot]));
-    void *d_in, *d_work, *dev[O_COUNT];
-    if ((rc = dev_ensure(ctx, (b.keep ? "keep" : "rin") + s, cn * in_lp, &d_in))) return rc;
+    void *d_in = nullptr, *d_obj = nullptr, *d_vin = nullptr, *d_pairs = nullptr, *d_work, *dev[O_COUNT];
+    if ((b.keep || b.rhs_in) && (rc = dev_ensure(ctx, (b.keep ? "keep" : "rin") + s, cn * in_lp, &d_in))) return rc;
     if ((rc = dev_ensure(ctx, "work" + s, (size_t)cn * cells * 8, &d_work))) return rc;
     if ((rc = outs.ensure(ctx, s, cn, cn * H, cn * (long long)pv, dev))) return rc;
-    const char *in = b.keep ? (const char *)b.keep : (const char *)b.rhs_in;
-    CU(ctx, cudaMemcpyAsync(d_in, in + begin * in_lp, cn * in_lp, cudaMemcpyHostToDevice, st));
+    if (d_in) {
+      const char *in = b.keep ? (const char *)b.keep : (const char *)b.rhs_in;
+      CU(ctx, cudaMemcpyAsync(d_in, in + begin * in_lp, cn * in_lp, cudaMemcpyHostToDevice, st));
+    }
+    if (b.obj_in) {
+      if ((rc = dev_ensure(ctx, "oin" + s, (size_t)cn * W * 8, &d_obj))) return rc;
+      CU(ctx, cudaMemcpyAsync(d_obj, b.obj_in + begin * W, (size_t)cn * W * 8, cudaMemcpyHostToDevice, st));
+    }
+    if (b.pairs && b.range_lo) {
+      if ((rc = dev_ensure(ctx, "pairs" + s, (size_t)cn * H * 4, &d_pairs))) return rc;
+      CU(ctx, cudaMemcpyAsync(d_pairs, b.pairs + begin * H, (size_t)cn * H * 4, cudaMemcpyHostToDevice, st));
+    }
     BatchArgs a{};
     a.n = cn;
     a.H = a.Hcap = H;
@@ -2062,14 +2083,20 @@ static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *tra
     a.work = (double *)d_work;
     a.in = a.work;
     // in place: every route reads an LP's tableau before it writes that LP's final one
-    a.mat_out = b.post_pass() ? a.work : nullptr;
+    a.mat_out = b.post_pass() || b.matrices_out ? a.work : nullptr;
     set_outputs(a, dev);
     if (trace && trace->ok) {
       if ((rc = replica_chunk_shared(ctx, *trace, outs, cn, H, W, (const double *)d_in, a.work, b.opt, dev, st, s,
                                      &ctx->replica_forks)))
         return rc;
     } else {
-      if (b.keep) {
+      if (warm) {
+        if ((rc = dev_ensure(ctx, "varin" + s, (size_t)cn * pv * 4, &d_vin))) return rc;
+        const int grid = (int)std::min<long long>(cn, sms * 8);
+        k_expand_warm<<<grid, kWarmThreads, 0, st>>>(cn, H, W, b.d_base, b.d_pos, b.d_var, b.d_col0, b.d_row0,
+                                                     (const double *)d_in, (const double *)d_obj, a.work, (int *)d_vin);
+        a.var_in = (const int *)d_vin;
+      } else if (b.keep) {
         const int grid = (int)std::min<long long>((cn * H + 7) / 8, sms * 16);
         k_expand_subsets<<<grid, 256, 0, st>>>(cn, H, W, words, b.d_base, (const unsigned *)d_in, a.work);
       } else {
@@ -2082,7 +2109,7 @@ static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *tra
       // rounds of an IIS search -- reuse the first call's route choice.  That decides speed only, never a result bit.
       if ((rc = solve_batch_device_impl(ctx, a, b.opt, s, st, begin))) return rc;
     }
-    if ((rc = post_passes(ctx, b, a, a.work, nullptr, dev, cn * pv, s, st))) return rc;
+    if ((rc = post_passes(ctx, b, a, a.work, (const int *)d_pairs, dev, cn * pv, s, st))) return rc;
     if (b.want_support()) {
       const int grid = (int)std::min<long long>((cn + 7) / 8, sms * 16);
       k_cert_support<<<grid, 256, 0, st>>>(cn, H, W, words, a.status, (const double *)dev[O_CERT],
@@ -2092,6 +2119,8 @@ static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *tra
     }
     if ((rc = outs.copy_out(ctx, dev, begin, begin * H, begin * (long long)pv, cn, cn * H, cn * (long long)pv, st)))
       return rc;
+    if (b.matrices_out)
+      CU(ctx, cudaMemcpyAsync(b.matrices_out + begin * cells, a.work, (size_t)cn * cells * 8, cudaMemcpyDeviceToHost, st));
     CU(ctx, cudaEventRecord(ctx->events[slot], st));
     used[slot] = true;
   }
@@ -2357,5 +2386,6 @@ int yalps_measure_tmem_bandwidth(yalps_ctx *ctx, double *gbs, double *sm_clock_m
 }  // extern "C"
 
 #include "bnb.inl"
+#include "warm.inl"
 #include "multi.inl"
 #include "iis.inl"

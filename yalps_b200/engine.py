@@ -183,6 +183,52 @@ def _solve_ragged(check, fn, handle, tableaus, shapes, options, pairs, want: dic
     return res
 
 
+def _solve_warm(check, fn, handle, base, height: int, width: int, rhs, obj, options, final, pairs, want: dict,
+                cells=None) -> dict:
+    """Engine/MultiEngine.solve_warm (base: the dense initial tableau) and Engine.solve_warm_sparse (cells given, base:
+    their values) through fn, a yalps_*solve_warm* entry, on handle."""
+    opt = options or make_options()
+    if not opt.precision >= 0.0:  # NaN fails too
+        raise ValueError(f"precision must be >= 0, got {opt.precision}")
+    H, W = int(height), int(width)
+    if H < 1 or W < 1:
+        raise ValueError(f"bad shape {H}x{W}")
+    b = np.ascontiguousarray(base, np.float64).reshape(-1)
+    if cells is None:
+        if b.size != H * W:
+            raise ValueError("base must hold height*width values")
+        base_args = (_ptr(b),)
+    else:
+        cells = np.ascontiguousarray(cells, np.int32).reshape(-1)
+        if cells.size != b.size:
+            raise ValueError("cells and values must have the same length")
+        base_args = (int(cells.size), _ptr(cells) if cells.size else None, _ptr(b) if b.size else None)
+    r = None if rhs is None else np.ascontiguousarray(rhs, np.float64).reshape(-1)
+    o = None if obj is None else np.ascontiguousarray(obj, np.float64).reshape(-1)
+    if r is None and o is None:
+        raise ValueError("rhs and obj may not both be None")
+    if (r is not None and r.size % H) or (o is not None and o.size % W):
+        raise ValueError("rhs must hold n*height values and obj n*width")
+    n = r.size // H if r is not None else o.size // W
+    if r is not None and o is not None and o.size // W != n:
+        raise ValueError("rhs and obj must describe the same number of variants")
+    f = fp = fv = None
+    if final is not None:
+        f = np.ascontiguousarray(final[0], np.float64).reshape(-1)
+        fp, fv = _basis_in(final[1], final[2], H + W)
+        if f.size != H * W or fp is None or fv is None:
+            raise ValueError("final is (matrix of height*width values, pos, var)")
+    out = _batch_outputs(n, H, W, want)
+    _add_outputs(out, n, H, W, want)
+    pr = _pairs_in(pairs, n, H) if want["want_ranges"] else None
+    bs, bv, bp = C.c_int32(), C.c_double(), np.zeros(2, np.int64)
+    check(fn(handle, n, H, W, *base_args, _ptr(f), _ptr(fp), _ptr(fv), _ptr(r), _ptr(o), C.byref(opt), C.byref(bs),
+             C.byref(bv), _ptr(bp), *_out_args(out, want, pr)))
+    out["base"] = None if final is not None else {"status": bs.value, "value": bv.value,
+                                                   "pivots": (int(bp[0]), int(bp[1]))}
+    return out
+
+
 def _check_precision(opt: Options):
     if not opt.precision >= 0.0:  # NaN fails too
         raise ValueError(f"precision must be >= 0 for row subsets (a zeroed row is a removed row only then), "
@@ -365,6 +411,35 @@ class Engine:
         want_duals: also out["reduced"] (n, width+height), as solve_batch."""
         return _solve_replicas(self._check, self._lib.yalps_solve_replicas_duals, self._ctx, base, rhs, height, width,
                                options, out, {"want_basis": want_basis, "want_duals": want_duals})
+
+    def solve_warm(self, base: np.ndarray, height: int, width: int, rhs: Optional[np.ndarray] = None,
+                   obj: Optional[np.ndarray] = None, options: Optional[Options] = None, final: Optional[tuple] = None,
+                   want_basis: bool = True, want_matrices: bool = False, want_duals: bool = False,
+                   want_ranges: bool = False, pairs: Optional[np.ndarray] = None,
+                   want_certificates: bool = False) -> dict:
+        """n variants of the LP whose initial tableau is `base` (height*width), each solved from the base's final
+        basis (yalps_solve_warm; yalps_b200.warm states the start tableau): rhs float64 (n, height) gives each its own
+        column 0, obj (n, width) its own row 0 (obj[:, 0] ignored); either may be None, not both.  final = (matrix, pos,
+        var) of the base's final tableau, or None: the library solves the base first and keeps that tableau on the
+        device.  Returns the outputs of solve_batch (same flags) plus out["base"]: {"status", "value", "pivots"} of the
+        base when the library solved it, else None.  Bit-exact against the reference loop on the warm tableau, not
+        against a cold solve of the changed model (the pivot path differs)."""
+        return _solve_warm(self._check, self._lib.yalps_solve_warm, self._ctx, base, height, width, rhs, obj, options,
+                           final, pairs, {"want_basis": want_basis, "want_matrices": want_matrices,
+                                          "want_duals": want_duals, "want_ranges": want_ranges,
+                                          "want_certificates": want_certificates})
+
+    def solve_warm_sparse(self, cells: np.ndarray, values: np.ndarray, height: int, width: int,
+                          rhs: Optional[np.ndarray] = None, obj: Optional[np.ndarray] = None,
+                          options: Optional[Options] = None, final: Optional[tuple] = None, want_basis: bool = True,
+                          want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,
+                          pairs: Optional[np.ndarray] = None, want_certificates: bool = False) -> dict:
+        """solve_warm with the base's initial tableau given as ordered (cell, value) stores into a zero matrix
+        (yalps_solve_warm_sparse): it is built on the device and never exists densely on the host."""
+        return _solve_warm(self._check, self._lib.yalps_solve_warm_sparse, self._ctx, values, height, width, rhs, obj,
+                           options, final, pairs, {"want_basis": want_basis, "want_matrices": want_matrices,
+                                                   "want_duals": want_duals, "want_ranges": want_ranges,
+                                                   "want_certificates": want_certificates}, cells=cells)
 
     def set_replica_sharing(self, on: bool = True):
         """solve_replicas: follow the base tableau's pivot path while a replica makes the same choices (default on)."""
@@ -690,6 +765,17 @@ class MultiEngine:
                        options: Optional[Options] = None, out: Optional[dict] = None, want_duals: bool = False) -> dict:
         return _solve_replicas(self._check, self._lib.yalps_multi_solve_replicas_duals, self._m, base, rhs, height,
                                width, options, out, {"want_basis": True, "want_duals": want_duals})
+
+    def solve_warm(self, base: np.ndarray, height: int, width: int, rhs: Optional[np.ndarray] = None,
+                   obj: Optional[np.ndarray] = None, options: Optional[Options] = None, final: Optional[tuple] = None,
+                   want_basis: bool = True, want_matrices: bool = False, want_duals: bool = False,
+                   want_ranges: bool = False, pairs: Optional[np.ndarray] = None,
+                   want_certificates: bool = False) -> dict:
+        """Engine.solve_warm with the variants sharded over the ranks; every rank solves (or uploads) the base."""
+        return _solve_warm(self._check, self._lib.yalps_multi_solve_warm, self._m, base, height, width, rhs, obj,
+                           options, final, pairs, {"want_basis": want_basis, "want_matrices": want_matrices,
+                                                   "want_duals": want_duals, "want_ranges": want_ranges,
+                                                   "want_certificates": want_certificates})
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
                      want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,

@@ -23,6 +23,8 @@ A fourth one, `iis` (default False), adds "irreducibleInfeasibleSet" ([[constrai
 order, a key's max before its min): a set of bounds that cannot hold together while any one fewer can, found by batched
 deletion rounds on the GPU (yalps_b200.iis); an empty list unless the status is infeasible.  Variables keep x >= 0
 throughout, and those bounds are never listed.
+solve_variants(model, variants, options) re-optimises variants of one LP model (changed bounds and objective
+coefficients) from the model's own final basis on the GPU (yalps_b200.warm), returning one Solution per variant.
 The tableau is built on the host (tableau.py), the simplex and branch-and-cut numerics run on the GPU
 through the C ABI; there is no CPU solve path.
 """
@@ -37,6 +39,7 @@ from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
 from .iis import model_iis
 from .sensitivity import model_certificate, model_ranges, model_sensitivity, row_pairs
 from .tableau import SPARSE_OVER_BYTES, TableauModel, constraint_rows, entries, tableau_model
+from .warm import variant_vectors
 
 # src/YALPS.ts:52-60
 _DEFAULTS = {
@@ -211,6 +214,47 @@ def solve(model: dict, options: Optional[dict] = None, *, engine: Optional[Engin
                     root_pivots=r["root_pivots"], height=t.height, width=t.width, final_rhs=r["rhs"],
                     final_pos=r["pos"], final_var=r["var"])
     return _solution(tabmod, STATUS_NAMES[r["status"]], r["result"], r["rhs"], r["pos"], r["var"], opt)
+
+
+def solve_variants(model: dict, variants: Sequence[dict], options: Optional[dict] = None, *,
+                   engine: Optional[Engine] = None) -> list:
+    """Solutions of variants of one LP model, each re-optimised from the model's final basis on the GPU
+    (Engine.solve_warm; yalps_b200.warm states the start tableau).  A variant is {"constraints": {key: {"min" | "max" |
+    "equal": value}}, "objective": {variable: coefficient}}, both parts optional: a key's `max` sets its upper row's
+    right-hand side, `min` its lower row's (to -min), `equal` both; a coefficient replaces the variable's objective
+    coefficient.  Returns one Solution per variant in order, the shape solve() returns; the options `sensitivity`,
+    `ranging` and `certificate` add their fields as in solve_many.  The results equal the reference's loop run from the
+    warm tableau: statuses agree with a cold solve of the changed model and optimal results agree within the precision,
+    but with alternative optima the reported vertex can differ.  ValueError for MILP models, the `iis` option, unknown
+    keys or variables, and a bound the base model does not have (an infinite bound has no tableau row)."""
+    opt = {**_DEFAULTS, **(options or {})}
+    if opt.get("iis"):
+        raise ValueError("solve_variants does not take the iis option (a search per variant)")
+    sparse_ok = hasattr(engine, "solve_warm_sparse") if engine is not None else True
+    tabmod = tableau_model(model, SPARSE_OVER_BYTES if sparse_ok else None)
+    if tabmod.integers:
+        raise ValueError("solve_variants is defined for LP models only (this model has integer or binary variables)")
+    t = tabmod.tableau
+    rhs, obj = variant_vectors(model, list(variants), t)
+    if not variants:
+        return []
+    duals, rng, cert = _wants(opt)
+    pairs = row_pairs(_rows(model), t.height) if rng else None
+    eng = engine or get_engine()
+    want = dict(options=_c_options(opt), want_duals=duals, want_ranges=rng, pairs=pairs, want_certificates=cert)
+    if t.matrix is None:
+        r = eng.solve_warm_sparse(t.cells, t.values, t.height, t.width, rhs, obj, **want)
+    else:
+        r = eng.solve_warm(t.matrix, t.height, t.width, rhs, obj, **want)
+    out = []
+    for i in range(len(variants)):
+        sol = _solution(tabmod, STATUS_NAMES[int(r["status"][i])], float(r["value"][i]), r["rhs"][i], r["pos"][i],
+                        r["var"][i], opt)
+        if duals:
+            sol = _with_sensitivity(sol, tabmod, model, r["reduced"][i],
+                                    (r["range_lo"][i], r["range_hi"][i]) if rng else None)
+        out.append(_with_certificate(sol, tabmod, model, r["certificate"][i]) if cert else sol)
+    return out
 
 
 def _worker_engines(device: int, count: int) -> list:
