@@ -495,6 +495,44 @@ int yalps_solve_warm_sparse(yalps_ctx *ctx, int64_t n, int32_t height, int32_t w
                             double *value, int64_t *pivots, double *rhs_out, int32_t *pos_out, int32_t *var_out,
                             double *matrices_out, double *reduced_out, const int32_t *pairs, double *range_lo,
                             double *range_hi, double *cert_out);
+/* Warm starts that also add constraints and variables.  Every variant adds K = add_rows rows and M = add_cols
+ * columns to the base (H = height, W = width): rows_in + i*K*(W+M) holds its K rows in initial-tableau form over the
+ * W+M columns (cell 0 the RHS, then the W-1 base structurals, then the M added ones; an upper row a.x <= max, a lower
+ * row -a.x <= -min), cols_in + i*M*H its M columns in initial-tableau form over the H base rows (cell 0 sign * cost,
+ * then the coefficient in each base row).  The start tableau has (H+K) x (W+M) cells; in base ids and positions:
+ *   1. column pass as above (step 1).
+ *   2. added columns: T[r, W+j] = sum over k ascending of g_j[k] * dir(W+k)[r], from +0.0, skipping g_j[k] == 0.0,
+ *      product and sum rounded apart (dir read from F, row 0 included; dir(W+0) is the unit vector of row 0).
+ *   3. row pass as above (step 2), over all W+M columns.
+ *   4. added rows, on the result of 3: row i starts as (a[0], +0.0, ...); for every structural v with a[v] != 0.0,
+ *      base ids then added ids ascending: v non-basic: t[pos(v)] += a[v]; v basic at row q: t[c] -= a[v] * T[q,c] for
+ *      every c, column 0 included.  Added variables are non-basic at column W+j.
+ *   5. the basis, relabelled: base structural v < W keeps v; added structural j is W+j, non-basic at column W+j; base
+ *      slack W+k becomes W+M+k; added row i's slack is W+M+H+i, basic at row H+i.
+ * In exact arithmetic an added column is B^-1 times the column with its reduced cost under the current costs, and an
+ * added row is the constraint with the basic variables substituted out (for a one-variable cut it equals the
+ * applyCuts row of branch and cut); it starts primal infeasible and dual feasible, so phase 1 runs the dual simplex.
+ * With K = M = 0 this is yalps_solve_warm bit for bit.  Outputs are per LP at the extended shape, packed as for a
+ * batch of (H+K) x (W+M) LPs; pairs covers the H+K rows.  rhs and obj keep the base's sizes (H and W values) and may
+ * both be NULL when K or M is positive.  K < 0, M < 0, rows_in NULL with K > 0 and cols_in NULL with M > 0 are
+ * YALPS_ERR_ARGUMENT; an extended shape of 2^31 cells or more is YALPS_ERR_TOO_LARGE. */
+int yalps_solve_warm_extend(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, int32_t add_rows,
+                            int32_t add_cols, const double *base, const double *final_m, const int32_t *final_pos,
+                            const int32_t *final_var, const double *rhs, const double *obj, const double *rows_in,
+                            const double *cols_in, const yalps_options *opt, int32_t *base_status, double *base_value,
+                            int64_t *base_pivots, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
+                            int32_t *pos_out, int32_t *var_out, double *matrices_out, double *reduced_out,
+                            const int32_t *pairs, double *range_lo, double *range_hi, double *cert_out);
+/* yalps_solve_warm_extend with the base's initial tableau given as (cell, value) stores, as yalps_solve_warm_sparse */
+int yalps_solve_warm_extend_sparse(yalps_ctx *ctx, int64_t n, int32_t height, int32_t width, int32_t add_rows,
+                                   int32_t add_cols, int64_t nnz, const int32_t *cell, const double *val,
+                                   const double *final_m, const int32_t *final_pos, const int32_t *final_var,
+                                   const double *rhs, const double *obj, const double *rows_in, const double *cols_in,
+                                   const yalps_options *opt, int32_t *base_status, double *base_value,
+                                   int64_t *base_pivots, int32_t *status, double *value, int64_t *pivots,
+                                   double *rhs_out, int32_t *pos_out, int32_t *var_out, double *matrices_out,
+                                   double *reduced_out, const int32_t *pairs, double *range_lo, double *range_hi,
+                                   double *cert_out);
 
 /* ---- one process, several GPUs (SURVEY 8b/8e) ------------------------------------------------------------
  * The reference is single-process and synchronous (src/YALPS.ts:73-92); a Node addon cannot use torchrun.  A
@@ -542,6 +580,16 @@ int yalps_multi_solve_warm(yalps_multi *m, int64_t n, int32_t height, int32_t wi
                            int64_t *base_pivots, int32_t *status, double *value, int64_t *pivots, double *rhs_out,
                            int32_t *pos_out, int32_t *var_out, double *matrices_out, double *reduced_out,
                            const int32_t *pairs, double *range_lo, double *range_hi, double *cert_out);
+/* yalps_solve_warm_extend with the variants sharded as yalps_multi_solve_warm shards them */
+int yalps_multi_solve_warm_extend(yalps_multi *m, int64_t n, int32_t height, int32_t width, int32_t add_rows,
+                                  int32_t add_cols, const double *base, const double *final_m,
+                                  const int32_t *final_pos, const int32_t *final_var, const double *rhs,
+                                  const double *obj, const double *rows_in, const double *cols_in,
+                                  const yalps_options *opt, int32_t *base_status, double *base_value,
+                                  int64_t *base_pivots, int32_t *status, double *value, int64_t *pivots,
+                                  double *rhs_out, int32_t *pos_out, int32_t *var_out, double *matrices_out,
+                                  double *reduced_out, const int32_t *pairs, double *range_lo, double *range_hi,
+                                  double *cert_out);
 /* the batch and ragged *_duals entries + pairs, range_lo, range_hi (see "sensitivity ranging"), sharded like rhs_out
  * and pos_out */
 int yalps_multi_solve_batch_ranging(yalps_multi *m, int64_t n, int32_t height, int32_t width, const double *matrices,

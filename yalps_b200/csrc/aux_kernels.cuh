@@ -138,14 +138,17 @@ __global__ void k_expand_subsets(long long n, int H, int W, int words, const dou
   }
 }
 
-// Warm starts (yalps_solve_warm): LP i is the start tableau of a variant of the base, built from the base's final
-// tableau F (`base`), its final basis (pos, var) and its initial column 0 and row 0 (col0, row0), with the variant's own
-// column 0 (rhs + i*H, or rhs null: unchanged) and row 0 (obj + i*W, or null).  yalps_b200/warm.py states the
-// definition; this is the same arithmetic in the same order.  One CTA per LP: F is copied with the 16-byte stores of
-// k_expand_subsets, then the column pass runs one thread per row and the row pass one thread per column.  The changed
-// k (resp. j) are compacted once per LP in ascending order, a tile of blockDim at a time (ballot + per-warp counts),
-// with their delta and dir position; dir(W+k)[r] of a non-basic slack is a strided read of F, which every LP shares
-// (L2-resident for Netlib-size models).  var_in gets the base's final var.
+// Warm starts (yalps_solve_warm[_extend]): LP i is the start tableau of a variant of the base (H x W), built from the
+// base's final tableau F (`base`), its final basis (pos, var) and its initial column 0 and row 0 (col0, row0), with the
+// variant's own column 0 (rhs + i*H, or rhs null: unchanged), row 0 (obj + i*W, or null), K added rows (rows +
+// i*K*(W+M), initial form over the W+M columns) and M added columns (cols + i*M*H, initial form over the H base rows).
+// yalps_b200/warm.py states the definition; this is the same arithmetic in the same order.  One CTA per LP, row stride
+// W+M: F is copied with the 16-byte stores of k_expand_subsets, then the column pass and the added columns run one
+// thread per row, the row pass and the added rows one thread per column.  The non-zero entries of each pass (changed
+// k, changed j, an added column's cells, an added row's cells) are compacted in ascending order, a tile of blockDim at
+// a time (ballot + per-warp counts), with their value and position; dir(W+k)[r] of a non-basic slack is a strided read
+// of F, which every LP shares (L2-resident for Netlib-size models).  var_in gets the base's final var, relabelled to
+// the extended ids.  With K = M = 0 this is the plain warm start.
 constexpr int kWarmThreads = 256;
 
 // Ordered compaction over the block: every thread passes its flag; the flagged threads get their rank among them in
@@ -165,23 +168,39 @@ __device__ __forceinline__ int warm_compact(bool flag, int *wcount, int *at) {
   return total;
 }
 
-__global__ void __launch_bounds__(kWarmThreads) k_expand_warm(long long n, int H, int W, const double *base,
-                                                              const int *__restrict__ pos, const int *__restrict__ var,
+// The sum over a compacted tile of entries (d, dir position p) of d * dir(p)[r] onto t, in list order: the column pass
+// and the added columns (dir read from F, row stride W).
+__device__ __forceinline__ double warm_dir_sum(double t, int cnt, const int *list_p, const double *list_d,
+                                               const double *base, int r, int W) {
+  for (int e = 0; e < cnt; e++) {
+    const int p = list_p[e];
+    const double dr = (p >= 1 && p < W) ? base[(size_t)r * W + p] : (r == p - W ? 1.0 : 0.0);
+    t = __dadd_rn(t, __dmul_rn(list_d[e], dr));
+  }
+  return t;
+}
+
+__global__ void __launch_bounds__(kWarmThreads) k_expand_warm(long long n, int H, int W, int K, int M,
+                                                              const double *base, const int *__restrict__ pos,
+                                                              const int *__restrict__ var,
                                                               const double *__restrict__ col0,
                                                               const double *__restrict__ row0,
                                                               const double *__restrict__ rhs,
-                                                              const double *__restrict__ obj, double *out,
+                                                              const double *__restrict__ obj,
+                                                              const double *__restrict__ rows,
+                                                              const double *__restrict__ cols, double *out,
                                                               int *var_in) {
   __shared__ int wcount[kWarmThreads / 32];
   __shared__ int list_p[kWarmThreads];
   __shared__ double list_d[kWarmThreads];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
-  const size_t cells = (size_t)H * W, pv = (size_t)H + W;
+  const int Wt = W + M;
+  const size_t cells = (size_t)(H + K) * Wt, pv = (size_t)H + K + Wt;
   const long long *src0 = reinterpret_cast<const long long *>(base);
   for (long long i = blockIdx.x; i < n; i += gridDim.x) {
     double *T = out + (size_t)i * cells;
     for (int r = warp; r < H; r += nwarps) {
-      long long *dst = reinterpret_cast<long long *>(T) + (size_t)r * W;
+      long long *dst = reinterpret_cast<long long *>(T) + (size_t)r * Wt;
       const long long *src = src0 + (size_t)r * W;
       const int head = min((int)((reinterpret_cast<uintptr_t>(dst) >> 3) & 1), W);  // 1: dst is 8 mod 16
       const int pairs = (W - head) >> 1;
@@ -190,7 +209,13 @@ __global__ void __launch_bounds__(kWarmThreads) k_expand_warm(long long n, int H
       for (int k = lane; k < pairs; k += 32) d2[k] = make_longlong2(src[head + 2 * k], src[head + 2 * k + 1]);
       if (lane == 0 && head + 2 * pairs < W) dst[W - 1] = src[W - 1];
     }
-    for (size_t k = tid; k < pv; k += blockDim.x) var_in[(size_t)i * pv + k] = var[k];
+    // extended ids: base structurals keep theirs, added structural j is W+j, base slack W+k becomes W+M+k, added row
+    // h's slack is W+M+H+h (each added id at the position of the same number)
+    for (size_t k = tid; k < pv; k += blockDim.x) {
+      const long long q = k < (size_t)W ? (long long)k : k >= (size_t)Wt && k < (size_t)Wt + H ? (long long)k - M : -1;
+      const int v = q < 0 ? (int)k : var[q];
+      var_in[(size_t)i * pv + k] = q >= 0 && v >= W ? v + M : v;
+    }
     __syncthreads();
     if (rhs) {  // column pass: T[r,0] += delta_k * dir(W+k)[r], changed k ascending
       const double *b = rhs + (size_t)i * H;
@@ -204,16 +229,28 @@ __global__ void __launch_bounds__(kWarmThreads) k_expand_warm(long long n, int H
           list_p[at] = pos[W + k];
         }
         __syncthreads();
-        for (int r = tid; r < H; r += blockDim.x) {
-          double t = T[(size_t)r * W];
-          for (int e = 0; e < cnt; e++) {
-            const int p = list_p[e];
-            const double dr = (p >= 1 && p < W) ? base[(size_t)r * W + p] : (r == p - W ? 1.0 : 0.0);
-            t = __dadd_rn(t, __dmul_rn(list_d[e], dr));
-          }
-          T[(size_t)r * W] = t;
-        }
+        for (int r = tid; r < H; r += blockDim.x)
+          T[(size_t)r * Wt] = warm_dir_sum(T[(size_t)r * Wt], cnt, list_p, list_d, base, r, W);
         __syncthreads();  // the lists are refilled by the next tile; the row pass reads column 0
+      }
+    }
+    for (int j = 0; j < M; j++) {  // added column j: T[r,W+j] = sum of g_j[k] * dir(W+k)[r] from +0.0, k ascending
+      const double *g = cols + ((size_t)i * M + j) * H;
+      for (int k0 = 0; k0 < H; k0 += blockDim.x) {
+        const int k = k0 + tid;
+        const double d = k < H ? g[k] : 0.0;
+        int at;
+        const int cnt = warm_compact(d != 0.0, wcount, &at);
+        if (d != 0.0) {
+          list_d[at] = d;
+          list_p[at] = pos[W + k];
+        }
+        __syncthreads();
+        for (int r = tid; r < H; r += blockDim.x) {
+          double *t = T + (size_t)r * Wt + W + j;
+          *t = warm_dir_sum(k0 == 0 ? 0.0 : *t, cnt, list_p, list_d, base, r, W);
+        }
+        __syncthreads();
       }
     }
     if (obj) {  // row pass: T[0,c] += delta_j at c == pos[j] (non-basic), -= delta_j * T[q,c] (basic at row q)
@@ -228,16 +265,46 @@ __global__ void __launch_bounds__(kWarmThreads) k_expand_warm(long long n, int H
           list_p[at] = pos[j];
         }
         __syncthreads();
-        for (int c = tid; c < W; c += blockDim.x) {
+        for (int c = tid; c < Wt; c += blockDim.x) {
           double t = T[c];
           for (int e = 0; e < cnt; e++) {
             const int q = list_p[e];
             if (q < W)
               t = c == q ? __dadd_rn(t, list_d[e]) : t;
             else
-              t = __dsub_rn(t, __dmul_rn(list_d[e], T[(size_t)(q - W) * W + c]));
+              t = __dsub_rn(t, __dmul_rn(list_d[e], T[(size_t)(q - W) * Wt + c]));
           }
           T[c] = t;
+        }
+        __syncthreads();
+      }
+    }
+    // added row h, from (a[0], +0.0, ...): a[v] added at v's column when v is non-basic (added structurals always
+    // are, at W+j), a[v] times v's row subtracted when v is basic; v ascending.  list_p: the column, or Wt + the row.
+    for (int h = 0; h < K; h++) {
+      const double *a = rows + ((size_t)i * K + h) * Wt;
+      double *dst = T + (size_t)(H + h) * Wt;
+      for (int v0 = 1; v0 < max(Wt, 2); v0 += blockDim.x) {  // at least one tile: a row of width 1 is its RHS
+        const int v = v0 + tid;
+        const double d = v < Wt ? a[v] : 0.0;
+        int at;
+        const int cnt = warm_compact(d != 0.0, wcount, &at);
+        if (d != 0.0) {
+          const int p = v < W ? pos[v] : v;
+          list_d[at] = d;
+          list_p[at] = p < W || v >= W ? p : Wt + (p - W);
+        }
+        __syncthreads();
+        for (int c = tid; c < Wt; c += blockDim.x) {
+          double t = v0 == 1 ? (c == 0 ? a[0] : 0.0) : dst[c];
+          for (int e = 0; e < cnt; e++) {
+            const int p = list_p[e];
+            if (p < Wt)
+              t = c == p ? __dadd_rn(t, list_d[e]) : t;
+            else
+              t = __dsub_rn(t, __dmul_rn(list_d[e], T[(size_t)(p - Wt) * Wt + c]));
+          }
+          dst[c] = t;
         }
         __syncthreads();
       }

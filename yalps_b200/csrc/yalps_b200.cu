@@ -1126,10 +1126,16 @@ struct HostBatch {
   const double *rhs_in = nullptr;  // by their own column 0 (n x height values: replicas), or
   const uint32_t *keep = nullptr;  // by their own row mask (n x words, words = (height + 31) / 32: row subsets), or
   // warm starts (d_var set): d_base is the base's final tableau, d_pos / d_var its final basis and d_col0 / d_row0 its
-  // initial column 0 and row 0 (device memory); each LP has its own column 0 (rhs_in) and/or row 0 (obj_in, n x width)
+  // initial column 0 and row 0 (device memory); each LP has its own column 0 (rhs_in) and/or row 0 (obj_in, n x base
+  // width), and its own add_rows rows (rows_in, n x add_rows x width) and add_cols columns (cols_in, n x add_cols x
+  // base height).  height / width are the LPs' shape; the base is add_rows rows and add_cols columns smaller.
   const int32_t *d_pos = nullptr, *d_var = nullptr;
   const double *d_col0 = nullptr, *d_row0 = nullptr;
   const double *obj_in = nullptr;
+  int32_t add_rows = 0, add_cols = 0;
+  const double *rows_in = nullptr, *cols_in = nullptr;
+  int32_t base_height() const { return height - add_rows; }
+  int32_t base_width() const { return width - add_cols; }
   const int32_t *pos_in = nullptr, *var_in = nullptr;  // the basis the tableaus arrive with (both null: the identity)
   const int32_t *pairs = nullptr;                       // ranging: the other row of each row's key
   const yalps_options *opt = nullptr;
@@ -1203,8 +1209,9 @@ struct Outputs {
 
 // The LPs [lo, hi) of request b, after row0 rows and pv0 variable ids.  A uniform batch moves its tableaus by cells; a
 // ragged one moves its shapes and offsets by LPs and keeps matrices and matrices_out, which those offsets index
-// absolutely.  The basis moves by variable ids, the pairs and right-hand sides by rows, the row masks and objective rows
-// by LPs, the outputs as the Outputs table packs them.
+// absolutely.  The basis moves by variable ids, the pairs by rows, the outputs as the Outputs table packs them, and the
+// per-LP inputs of LPs derived from a base (uniform only) by LPs: right-hand sides by base rows, objective rows by base
+// columns, row masks, added rows and added columns by their own sizes.
 HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long row0, long long pv0) {
   HostBatch s = b;
   s.n = hi - lo;
@@ -1220,8 +1227,10 @@ HostBatch slice_request(const HostBatch &b, int64_t lo, int64_t hi, long long ro
   if (s.pos_in) s.pos_in += pv0;
   if (s.var_in) s.var_in += pv0;
   if (s.pairs) s.pairs += row0;
-  if (s.rhs_in) s.rhs_in += row0;
-  if (s.obj_in) s.obj_in += lo * b.width;
+  if (s.rhs_in) s.rhs_in += lo * b.base_height();
+  if (s.obj_in) s.obj_in += lo * b.base_width();
+  if (s.rows_in) s.rows_in += lo * b.add_rows * b.width;
+  if (s.cols_in) s.cols_in += lo * b.add_cols * b.base_height();
   if (s.keep) s.keep += lo * ((b.height + 31) / 32);
   const Outputs o(b);
   auto at = [&](int i) -> void * { return o.t[i].host ? (char *)o.t[i].host + o.t[i].bytes(lo, row0, pv0) : nullptr; };
@@ -2047,8 +2056,9 @@ static int replica_chunk_shared(yalps_ctx *ctx, const ReplicaTrace &tr, const Ou
 static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *trace) {
   const int64_t n = b.n;
   const int H = b.height, W = b.width, words = (H + 31) / 32;
+  const int K = b.add_rows, M = b.add_cols, bH = b.base_height(), bW = b.base_width();
   const bool warm = b.d_var != nullptr;
-  const size_t cells = (size_t)H * W, pv = (size_t)H + W, in_lp = b.keep ? (size_t)words * 4 : (size_t)H * 8;
+  const size_t cells = (size_t)H * W, pv = (size_t)H + W, in_lp = b.keep ? (size_t)words * 4 : (size_t)bH * 8;
   const long long sms = ctx->prop.multiProcessorCount;
   const int64_t per_chunk = std::max<int64_t>(1, std::min<int64_t>((n + 1) / 2 > 4096 ? (n + 7) / 8 : n,
                                                                   (int64_t)(((size_t)1536 << 20) / (cells * 8))));
@@ -2060,7 +2070,8 @@ static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *tra
     const std::string s = (warm ? "wm" : b.keep ? "ss" : "rp") + std::to_string(slot);
     cudaStream_t st = ctx->streams[slot];
     if (used[slot]) CU(ctx, cudaEventSynchronize(ctx->events[slot]));
-    void *d_in = nullptr, *d_obj = nullptr, *d_vin = nullptr, *d_pairs = nullptr, *d_work, *dev[O_COUNT];
+    void *d_in = nullptr, *d_obj = nullptr, *d_rows = nullptr, *d_cols = nullptr, *d_vin = nullptr, *d_pairs = nullptr,
+         *d_work, *dev[O_COUNT];
     if ((b.keep || b.rhs_in) && (rc = dev_ensure(ctx, (b.keep ? "keep" : "rin") + s, cn * in_lp, &d_in))) return rc;
     if ((rc = dev_ensure(ctx, "work" + s, (size_t)cn * cells * 8, &d_work))) return rc;
     if ((rc = outs.ensure(ctx, s, cn, cn * H, cn * (long long)pv, dev))) return rc;
@@ -2069,8 +2080,18 @@ static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *tra
       CU(ctx, cudaMemcpyAsync(d_in, in + begin * in_lp, cn * in_lp, cudaMemcpyHostToDevice, st));
     }
     if (b.obj_in) {
-      if ((rc = dev_ensure(ctx, "oin" + s, (size_t)cn * W * 8, &d_obj))) return rc;
-      CU(ctx, cudaMemcpyAsync(d_obj, b.obj_in + begin * W, (size_t)cn * W * 8, cudaMemcpyHostToDevice, st));
+      if ((rc = dev_ensure(ctx, "oin" + s, (size_t)cn * bW * 8, &d_obj))) return rc;
+      CU(ctx, cudaMemcpyAsync(d_obj, b.obj_in + begin * bW, (size_t)cn * bW * 8, cudaMemcpyHostToDevice, st));
+    }
+    if (K > 0) {
+      const size_t lp_rows = (size_t)K * W;
+      if ((rc = dev_ensure(ctx, "rows" + s, cn * lp_rows * 8, &d_rows))) return rc;
+      CU(ctx, cudaMemcpyAsync(d_rows, b.rows_in + begin * lp_rows, cn * lp_rows * 8, cudaMemcpyHostToDevice, st));
+    }
+    if (M > 0) {
+      const size_t lp_cols = (size_t)M * bH;
+      if ((rc = dev_ensure(ctx, "cols" + s, cn * lp_cols * 8, &d_cols))) return rc;
+      CU(ctx, cudaMemcpyAsync(d_cols, b.cols_in + begin * lp_cols, cn * lp_cols * 8, cudaMemcpyHostToDevice, st));
     }
     if (b.pairs && b.range_lo) {
       if ((rc = dev_ensure(ctx, "pairs" + s, (size_t)cn * H * 4, &d_pairs))) return rc;
@@ -2093,8 +2114,9 @@ static int solve_from_base(yalps_ctx *ctx, HostBatch &b, const ReplicaTrace *tra
       if (warm) {
         if ((rc = dev_ensure(ctx, "varin" + s, (size_t)cn * pv * 4, &d_vin))) return rc;
         const int grid = (int)std::min<long long>(cn, sms * 8);
-        k_expand_warm<<<grid, kWarmThreads, 0, st>>>(cn, H, W, b.d_base, b.d_pos, b.d_var, b.d_col0, b.d_row0,
-                                                     (const double *)d_in, (const double *)d_obj, a.work, (int *)d_vin);
+        k_expand_warm<<<grid, kWarmThreads, 0, st>>>(cn, bH, bW, K, M, b.d_base, b.d_pos, b.d_var, b.d_col0, b.d_row0,
+                                                     (const double *)d_in, (const double *)d_obj, (const double *)d_rows,
+                                                     (const double *)d_cols, a.work, (int *)d_vin);
         a.var_in = (const int *)d_vin;
       } else if (b.keep) {
         const int grid = (int)std::min<long long>((cn * H + 7) / 8, sms * 16);

@@ -184,9 +184,10 @@ def _solve_ragged(check, fn, handle, tableaus, shapes, options, pairs, want: dic
 
 
 def _solve_warm(check, fn, handle, base, height: int, width: int, rhs, obj, options, final, pairs, want: dict,
-                cells=None) -> dict:
+                cells=None, add_rows=None, add_cols=None) -> dict:
     """Engine/MultiEngine.solve_warm (base: the dense initial tableau) and Engine.solve_warm_sparse (cells given, base:
-    their values) through fn, a yalps_*solve_warm* entry, on handle."""
+    their values) through fn, a yalps_*solve_warm* entry, on handle; a yalps_*solve_warm_extend* entry when add_rows or
+    add_cols is given."""
     opt = options or make_options()
     if not opt.precision >= 0.0:  # NaN fails too
         raise ValueError(f"precision must be >= 0, got {opt.precision}")
@@ -205,25 +206,43 @@ def _solve_warm(check, fn, handle, base, height: int, width: int, rhs, obj, opti
         base_args = (int(cells.size), _ptr(cells) if cells.size else None, _ptr(b) if b.size else None)
     r = None if rhs is None else np.ascontiguousarray(rhs, np.float64).reshape(-1)
     o = None if obj is None else np.ascontiguousarray(obj, np.float64).reshape(-1)
-    if r is None and o is None:
+    extend = add_rows is not None or add_cols is not None
+    if r is None and o is None and not extend:
         raise ValueError("rhs and obj may not both be None")
     if (r is not None and r.size % H) or (o is not None and o.size % W):
         raise ValueError("rhs must hold n*height values and obj n*width")
-    n = r.size // H if r is not None else o.size // W
-    if r is not None and o is not None and o.size // W != n:
-        raise ValueError("rhs and obj must describe the same number of variants")
+    counts = [] if r is None else [r.size // H]
+    counts += [] if o is None else [o.size // W]
+    K = M = 0
+    ext_args = ()
+    if extend:
+        g = None if add_cols is None else np.ascontiguousarray(add_cols, np.float64)
+        if g is not None and (g.ndim != 3 or g.shape[2] != H):
+            raise ValueError("add_cols must be (n, M, height): M added columns per variant over the base rows")
+        M = 0 if g is None else g.shape[1]
+        a = None if add_rows is None else np.ascontiguousarray(add_rows, np.float64)
+        if a is not None and (a.ndim != 3 or a.shape[2] != W + M):
+            raise ValueError("add_rows must be (n, K, width + M): K added rows per variant over the base and added "
+                             "columns")
+        K = 0 if a is None else a.shape[1]
+        counts += [x.shape[0] for x in (a, g) if x is not None]
+        ext_args = (_ptr(a) if K else None, _ptr(g) if M else None)
+    n = counts[0]
+    if any(c != n for c in counts):
+        raise ValueError("rhs, obj, add_rows and add_cols must describe the same number of variants")
     f = fp = fv = None
     if final is not None:
         f = np.ascontiguousarray(final[0], np.float64).reshape(-1)
         fp, fv = _basis_in(final[1], final[2], H + W)
         if f.size != H * W or fp is None or fv is None:
             raise ValueError("final is (matrix of height*width values, pos, var)")
-    out = _batch_outputs(n, H, W, want)
-    _add_outputs(out, n, H, W, want)
-    pr = _pairs_in(pairs, n, H) if want["want_ranges"] else None
+    out = _batch_outputs(n, H + K, W + M, want)
+    _add_outputs(out, n, H + K, W + M, want)
+    pr = _pairs_in(pairs, n, H + K) if want["want_ranges"] else None
     bs, bv, bp = C.c_int32(), C.c_double(), np.zeros(2, np.int64)
-    check(fn(handle, n, H, W, *base_args, _ptr(f), _ptr(fp), _ptr(fv), _ptr(r), _ptr(o), C.byref(opt), C.byref(bs),
-             C.byref(bv), _ptr(bp), *_out_args(out, want, pr)))
+    shape = (H, W, K, M) if extend else (H, W)
+    check(fn(handle, n, *shape, *base_args, _ptr(f), _ptr(fp), _ptr(fv), _ptr(r), _ptr(o), *ext_args, C.byref(opt),
+             C.byref(bs), C.byref(bv), _ptr(bp), *_out_args(out, want, pr)))
     out["base"] = None if final is not None else {"status": bs.value, "value": bv.value,
                                                    "pivots": (int(bp[0]), int(bp[1]))}
     return out
@@ -416,30 +435,40 @@ class Engine:
                    obj: Optional[np.ndarray] = None, options: Optional[Options] = None, final: Optional[tuple] = None,
                    want_basis: bool = True, want_matrices: bool = False, want_duals: bool = False,
                    want_ranges: bool = False, pairs: Optional[np.ndarray] = None,
-                   want_certificates: bool = False) -> dict:
+                   want_certificates: bool = False, add_rows: Optional[np.ndarray] = None,
+                   add_cols: Optional[np.ndarray] = None) -> dict:
         """n variants of the LP whose initial tableau is `base` (height*width), each solved from the base's final
         basis (yalps_solve_warm; yalps_b200.warm states the start tableau): rhs float64 (n, height) gives each its own
         column 0, obj (n, width) its own row 0 (obj[:, 0] ignored); either may be None, not both.  final = (matrix, pos,
         var) of the base's final tableau, or None: the library solves the base first and keeps that tableau on the
         device.  Returns the outputs of solve_batch (same flags) plus out["base"]: {"status", "value", "pivots"} of the
         base when the library solved it, else None.  Bit-exact against the reference loop on the warm tableau, not
-        against a cold solve of the changed model (the pivot path differs)."""
-        return _solve_warm(self._check, self._lib.yalps_solve_warm, self._ctx, base, height, width, rhs, obj, options,
-                           final, pairs, {"want_basis": want_basis, "want_matrices": want_matrices,
-                                          "want_duals": want_duals, "want_ranges": want_ranges,
-                                          "want_certificates": want_certificates})
+        against a cold solve of the changed model (the pivot path differs).
+        add_rows float64 (n, K, width + M) and add_cols (n, M, height), either or both (yalps_solve_warm_extend): each
+        variant also adds K constraint rows and M variable columns in initial-tableau form; rhs and obj may then both
+        be None, and the outputs and pairs have the (height + K) x (width + M) shape."""
+        extend = add_rows is not None or add_cols is not None
+        return _solve_warm(self._check, self._lib.yalps_solve_warm_extend if extend else self._lib.yalps_solve_warm,
+                           self._ctx, base, height, width, rhs, obj, options, final, pairs,
+                           {"want_basis": want_basis, "want_matrices": want_matrices, "want_duals": want_duals,
+                            "want_ranges": want_ranges, "want_certificates": want_certificates},
+                           add_rows=add_rows, add_cols=add_cols)
 
     def solve_warm_sparse(self, cells: np.ndarray, values: np.ndarray, height: int, width: int,
                           rhs: Optional[np.ndarray] = None, obj: Optional[np.ndarray] = None,
                           options: Optional[Options] = None, final: Optional[tuple] = None, want_basis: bool = True,
                           want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,
-                          pairs: Optional[np.ndarray] = None, want_certificates: bool = False) -> dict:
+                          pairs: Optional[np.ndarray] = None, want_certificates: bool = False,
+                          add_rows: Optional[np.ndarray] = None, add_cols: Optional[np.ndarray] = None) -> dict:
         """solve_warm with the base's initial tableau given as ordered (cell, value) stores into a zero matrix
-        (yalps_solve_warm_sparse): it is built on the device and never exists densely on the host."""
-        return _solve_warm(self._check, self._lib.yalps_solve_warm_sparse, self._ctx, values, height, width, rhs, obj,
-                           options, final, pairs, {"want_basis": want_basis, "want_matrices": want_matrices,
-                                                   "want_duals": want_duals, "want_ranges": want_ranges,
-                                                   "want_certificates": want_certificates}, cells=cells)
+        (yalps_solve_warm_sparse, yalps_solve_warm_extend_sparse): it is built on the device and never exists densely
+        on the host."""
+        extend = add_rows is not None or add_cols is not None
+        fn = self._lib.yalps_solve_warm_extend_sparse if extend else self._lib.yalps_solve_warm_sparse
+        return _solve_warm(self._check, fn, self._ctx, values, height, width, rhs, obj, options, final, pairs,
+                           {"want_basis": want_basis, "want_matrices": want_matrices, "want_duals": want_duals,
+                            "want_ranges": want_ranges, "want_certificates": want_certificates}, cells=cells,
+                           add_rows=add_rows, add_cols=add_cols)
 
     def set_replica_sharing(self, on: bool = True):
         """solve_replicas: follow the base tableau's pivot path while a replica makes the same choices (default on)."""
@@ -770,12 +799,15 @@ class MultiEngine:
                    obj: Optional[np.ndarray] = None, options: Optional[Options] = None, final: Optional[tuple] = None,
                    want_basis: bool = True, want_matrices: bool = False, want_duals: bool = False,
                    want_ranges: bool = False, pairs: Optional[np.ndarray] = None,
-                   want_certificates: bool = False) -> dict:
+                   want_certificates: bool = False, add_rows: Optional[np.ndarray] = None,
+                   add_cols: Optional[np.ndarray] = None) -> dict:
         """Engine.solve_warm with the variants sharded over the ranks; every rank solves (or uploads) the base."""
-        return _solve_warm(self._check, self._lib.yalps_multi_solve_warm, self._m, base, height, width, rhs, obj,
-                           options, final, pairs, {"want_basis": want_basis, "want_matrices": want_matrices,
-                                                   "want_duals": want_duals, "want_ranges": want_ranges,
-                                                   "want_certificates": want_certificates})
+        extend = add_rows is not None or add_cols is not None
+        fn = self._lib.yalps_multi_solve_warm_extend if extend else self._lib.yalps_multi_solve_warm
+        return _solve_warm(self._check, fn, self._m, base, height, width, rhs, obj, options, final, pairs,
+                           {"want_basis": want_basis, "want_matrices": want_matrices, "want_duals": want_duals,
+                            "want_ranges": want_ranges, "want_certificates": want_certificates},
+                           add_rows=add_rows, add_cols=add_cols)
 
     def solve_ragged(self, tableaus: Sequence[np.ndarray], shapes: Sequence[tuple], options: Optional[Options] = None,
                      want_matrices: bool = False, want_duals: bool = False, want_ranges: bool = False,

@@ -24,7 +24,8 @@ order, a key's max before its min): a set of bounds that cannot hold together wh
 deletion rounds on the GPU (yalps_b200.iis); an empty list unless the status is infeasible.  Variables keep x >= 0
 throughout, and those bounds are never listed.
 solve_variants(model, variants, options) re-optimises variants of one LP model (changed bounds and objective
-coefficients) from the model's own final basis on the GPU (yalps_b200.warm), returning one Solution per variant.
+coefficients, added constraints and variables) from the model's own final basis on the GPU (yalps_b200.warm), returning
+one Solution per variant.
 The tableau is built on the host (tableau.py), the simplex and branch-and-cut numerics run on the GPU
 through the C ABI; there is no CPU solve path.
 """
@@ -38,8 +39,8 @@ import numpy as np
 from .engine import Engine, MultiEngine, STATUS_NAMES, make_options
 from .iis import model_iis
 from .sensitivity import model_certificate, model_ranges, model_sensitivity, row_pairs
-from .tableau import SPARSE_OVER_BYTES, TableauModel, constraint_rows, entries, tableau_model
-from .warm import variant_vectors
+from .tableau import SPARSE_OVER_BYTES, Tableau, TableauModel, constraint_rows, entries, tableau_model
+from .warm import variant_additions, variant_vectors
 
 # src/YALPS.ts:52-60
 _DEFAULTS = {
@@ -121,10 +122,11 @@ def _wants(opt: dict) -> tuple:
     return bool(opt.get("sensitivity")) or rng, rng, bool(opt.get("certificate"))
 
 
-def _with_certificate(sol: dict, tabmod: TableauModel, model: dict, cert) -> dict:
-    """Solution + infeasibilityCertificate / unboundedRay (both empty unless the status matches)."""
+def _with_certificate(sol: dict, tabmod: TableauModel, model: dict, cert, rows: Optional[list] = None) -> dict:
+    """Solution + infeasibilityCertificate / unboundedRay (both empty unless the status matches); rows: the model's
+    constraint_rows unless given."""
     status = {"infeasible": 1, "unbounded": 2}.get(sol["status"], 0)
-    rows = _rows(model) if status == 1 else []
+    rows = (rows if rows is not None else _rows(model)) if status == 1 else []
     farkas, ray = model_certificate(tabmod.variables, rows, cert, tabmod.tableau.width, status)
     return {**sol, "infeasibilityCertificate": farkas, "unboundedRay": ray}
 
@@ -144,13 +146,14 @@ def _rows(model: dict) -> list:
     return constraint_rows(list(entries(model["constraints"])))
 
 
-def _with_sensitivity(sol: dict, tabmod: TableauModel, model: dict, reduced, ranges: Optional[tuple] = None) -> dict:
+def _with_sensitivity(sol: dict, tabmod: TableauModel, model: dict, reduced, ranges: Optional[tuple] = None,
+                      rows: Optional[list] = None) -> dict:
     """Solution + reducedCosts / shadowPrices, and costRanges / rhsRanges when `ranges` = (range_lo, range_hi) is
-    given (all empty unless optimal)."""
+    given (all empty unless optimal); rows: the model's constraint_rows unless given."""
     if sol["status"] != "optimal":
         out = {**sol, "reducedCosts": [], "shadowPrices": []}
         return out if ranges is None else {**out, "costRanges": [], "rhsRanges": []}
-    rows = _rows(model)
+    rows = rows if rows is not None else _rows(model)
     rc, sp = model_sensitivity(tabmod.variables, rows, reduced, tabmod.tableau.width, tabmod.sign)
     out = {**sol, "reducedCosts": rc, "shadowPrices": sp}
     if ranges is None:
@@ -222,11 +225,15 @@ def solve_variants(model: dict, variants: Sequence[dict], options: Optional[dict
     (Engine.solve_warm; yalps_b200.warm states the start tableau).  A variant is {"constraints": {key: {"min" | "max" |
     "equal": value}}, "objective": {variable: coefficient}}, both parts optional: a key's `max` sets its upper row's
     right-hand side, `min` its lower row's (to -min), `equal` both; a coefficient replaces the variable's objective
-    coefficient.  Returns one Solution per variant in order, the shape solve() returns; the options `sensitivity`,
-    `ranging` and `certificate` add their fields as in solve_many.  The results equal the reference's loop run from the
+    coefficient.  A variant may also add constraints and variables ("addConstraints", "addVariables";
+    yalps_b200.warm.variant_additions has their form): each is solved at its batch's largest added shape, padded with
+    zero rows and columns that no pivot chooses or changes, and mapped back with its own names.  Returns one Solution
+    per variant in order, the shape solve() returns; the options `sensitivity`, `ranging` and `certificate` add their
+    fields as in solve_many, added variables and keys included.  The results equal the reference's loop run from the
     warm tableau: statuses agree with a cold solve of the changed model and optimal results agree within the precision,
     but with alternative optima the reported vertex can differ.  ValueError for MILP models, the `iis` option, unknown
-    keys or variables, and a bound the base model does not have (an infinite bound has no tableau row)."""
+    keys or variables, a bound the base model does not have (an infinite bound has no tableau row), and the refusals of
+    variant_additions."""
     opt = {**_DEFAULTS, **(options or {})}
     if opt.get("iis"):
         raise ValueError("solve_variants does not take the iis option (a search per variant)")
@@ -236,24 +243,32 @@ def solve_variants(model: dict, variants: Sequence[dict], options: Optional[dict
         raise ValueError("solve_variants is defined for LP models only (this model has integer or binary variables)")
     t = tabmod.tableau
     rhs, obj = variant_vectors(model, list(variants), t)
+    add = variant_additions(model, list(variants), t)
     if not variants:
         return []
     duals, rng, cert = _wants(opt)
-    pairs = row_pairs(_rows(model), t.height) if rng else None
+    pairs = (row_pairs(_rows(model), t.height) if add is None else add.pairs) if rng else None
     eng = engine or get_engine()
     want = dict(options=_c_options(opt), want_duals=duals, want_ranges=rng, pairs=pairs, want_certificates=cert)
+    if add is not None:  # only then: an engine without the extend entries still serves every other variant batch
+        want.update(add_rows=add.rows, add_cols=add.cols)
     if t.matrix is None:
         r = eng.solve_warm_sparse(t.cells, t.values, t.height, t.width, rhs, obj, **want)
     else:
         r = eng.solve_warm(t.matrix, t.height, t.width, rhs, obj, **want)
     out = []
     for i in range(len(variants)):
-        sol = _solution(tabmod, STATUS_NAMES[int(r["status"][i])], float(r["value"][i]), r["rhs"][i], r["pos"][i],
+        tm, keys = tabmod, None
+        if add is not None:  # the variant's own names over the padded shape
+            H, W = t.height + add.rows.shape[1], t.width + add.cols.shape[1]
+            tm = TableauModel(Tableau(None, W, H, None, None), tabmod.sign, add.variables[i], [])
+            keys = add.keys[i]
+        sol = _solution(tm, STATUS_NAMES[int(r["status"][i])], float(r["value"][i]), r["rhs"][i], r["pos"][i],
                         r["var"][i], opt)
         if duals:
-            sol = _with_sensitivity(sol, tabmod, model, r["reduced"][i],
-                                    (r["range_lo"][i], r["range_hi"][i]) if rng else None)
-        out.append(_with_certificate(sol, tabmod, model, r["certificate"][i]) if cert else sol)
+            sol = _with_sensitivity(sol, tm, model, r["reduced"][i],
+                                    (r["range_lo"][i], r["range_hi"][i]) if rng else None, rows=keys)
+        out.append(_with_certificate(sol, tm, model, r["certificate"][i], rows=keys) if cert else sol)
     return out
 
 
